@@ -13,7 +13,9 @@ stream); `e2e` is the public call with HOST buffers: planning, H2D of the
 schedule, all layers, proband gather and D2H into pinned host memory.
 Both arms print the sha256 of the proband matrix they produced
 (`output_sha256`) next to the committed golden one (tests/golden/, made by the
-oracle alone).  Prints ONE JSON line (rank 0).
+oracle alone).  Prints ONE JSON line (rank 0).  `--dump-outputs DIR` (one GPU,
+or a full pass of the reference arm) also writes that matrix, or a seeded
+sample of its rows, to DIR as .npy for output-by-output comparison of builds.
 """
 from __future__ import annotations
 
@@ -124,6 +126,24 @@ def golden_record(args):
         return None
 
 
+DUMP_BYTES = 60 << 20                # the whole dump, .npy header included, stays below 64 MB
+
+
+def dump_outputs(out_dir: str, phi: np.ndarray):
+    """Write the proband kinship matrix of the last timed step to `out_dir`, so that two builds can be
+    compared output for output: phi.npy when it fits DUMP_BYTES, else phi_row_sample.npy, the rows
+    sorted(default_rng(0).choice(n, k, replace=False)) with k as large as fits (the same rows for the
+    same command line)."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = phi.shape[0]
+    k = DUMP_BYTES // max(1, n * phi.itemsize)
+    if k >= n:
+        np.save(os.path.join(out_dir, "phi.npy"), phi)
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        np.save(os.path.join(out_dir, "phi_row_sample.npy"), phi[rows])
+
+
 def rows_digest(rows: np.ndarray) -> bytes:
     """Concatenated sha256 digests of the rows (32 bytes each): ranks hash their own rows, the
     digest of the concatenation in proband order is independent of how the rows were sharded."""
@@ -188,6 +208,8 @@ def run_reference(args, rank, world):
     father, mother, ranks, _ = ob.workload(args.workload, args.scale)
     cores = ob.num_threads()
     full = args.ref_mode == "full" or (args.ref_mode == "auto" and not (args.workload == "C4" and args.scale > 0.25))
+    if args.dump_outputs and not full:
+        raise SystemExit("bench.py: --dump-outputs with --impl reference needs a full pass (--ref-mode full)")
     for _ in range(min(args.warmup, 1)):
         cpu_sample(father, mother, ranks, 2.0)                      # pages the pedigree in, spins the cores up
     if full:
@@ -202,6 +224,8 @@ def run_reference(args, rank, world):
                            "C restatement of the reference algorithm (Julia is not installable here)"),
                 "seconds": wall}
         par = parity_fields(args, ob.matrix_sha256(phi), hashlib.sha256(rows_digest(phi)).hexdigest())
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, phi)
     else:
         per = max(1.0, args.cpu_seconds / max(1, args.steps))
         vals, base = [], None
@@ -307,10 +331,16 @@ def main():
                     help="reference arm: one full pass (sha256, unsampled) or bounded samples")
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--layers-json", default="", help="write per-layer timings here")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the proband matrix of the last timed step to DIR as .npy (a seeded sample of its rows above 60 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        ap.error("--dump-outputs runs on one GPU only")
     if args.impl == "reference":
         return run_reference(args, rank, world)
     if world > 1:
@@ -353,6 +383,8 @@ def main():
     if args.layers_json:
         with open(args.layers_json, "w") as fh:
             json.dump([{**i, "ms_layer": float(layer_ms[:, t].mean())} for t, i in enumerate(infos)], fh, indent=1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng.fetch(dtype=np.float32 if esize == 4 else np.float64))
     eng.close()
 
     # ---- end to end: the public call with host buffers, pinned output ----
