@@ -53,6 +53,19 @@ class Stats(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
 
 
+class GcStats(C.Structure):
+    _fields_ = [("n_pro", C.c_int32), ("n_anc", C.c_int32), ("n_layers", C.c_int32), ("direction", C.c_int32),
+                ("rows", C.c_int64), ("inputs", C.c_int64), ("width", C.c_int64), ("capacity", C.c_int64),
+                ("device_bytes", C.c_int64), ("alg_bytes", C.c_double), ("ms_plan", C.c_double),
+                ("ms_kernels", C.c_double), ("ms_fetch", C.c_double), ("d2h_bytes", C.c_int64),
+                ("kernel_launches", C.c_int32), ("n_dev", C.c_int32)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+GC_DIRECTIONS = {0: "descend", 1: "ascend"}
+
 # every symbol include/genlib_cuda.h declares: (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -111,6 +124,13 @@ SYMBOLS = {
     "genlib_engine_row_sums": (C.c_int, [_P, _P]),
     "genlib_engine_set_layer_limit": (C.c_int, [_P, C.c_int32]),
     "genlib_engine_read_block": (C.c_int, [_P, C.c_int32, _P, _P]),
+    "genlib_gc": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int, C.c_int, C.c_int32, _P,
+                            C.POINTER(GcStats)]),
+    "genlib_gc_plan_create": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, C.POINTER(_P)]),
+    "genlib_gc_plan_destroy": (None, [_P]),
+    "genlib_gc_plan_info": (C.c_int, [_P, C.POINTER(GcStats)]),
+    "genlib_gc_plan_layer": (C.c_int, [_P, C.c_int32, _P, _P]),
+    "genlib_gc_plan_layer_arrays": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None

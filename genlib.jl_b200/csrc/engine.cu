@@ -18,6 +18,8 @@
 #include <vector>
 
 #include "../../include/genlib_cuda.h"
+#include "gc_kernel.cuh"
+#include "gc_plan.hpp"
 #include "kernels.cuh"
 #include "layer_kernel.cuh"
 #include "plan.hpp"
@@ -1662,6 +1664,310 @@ int genlib_plan_stream_selftest(int32_t n, const int32_t *father, const int32_t 
     for (int g = 0; g < world; g++)
         if (kept_bound ? P.rows_cap[(size_t)g] < ref.rows_cap[(size_t)g] : P.rows_cap[(size_t)g] != ref.rows_cap[(size_t)g])
             return fail(GENLIB_EINVAL, "stream selftest: rows of rank " + std::to_string(g));
+    return GENLIB_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------ gen.gc (DESIGN.md 2b)
+struct genlib_gc_plan {
+    GcPlan p;
+    double ms_plan = 0;
+};
+
+namespace {
+
+// One device's share: column positions [j0, j1) of the column-side list and the unique columns [lo, hi) they
+// name (contiguous when the list has no duplicates; a duplicate may widen the range, never the result).
+struct GcShare {
+    int device = -1;
+    int32_t j0 = 0, j1 = 0, lo = 0, hi = 0;
+    int64_t ws() const { return ((int64_t)(hi - lo) + 1) / 2 * 2; }      // row stride in doubles (16-byte rows)
+    size_t stage = 0, need = 0;
+    double ms_kernels = 0, ms_fetch = 0;
+    int32_t launches = 0;
+    int64_t d2h = 0;
+};
+
+// Output layout of a share: the stage's major dimension is the column position (cmaj) or the target position.
+struct GcLayout {
+    bool cmaj;
+    int64_t ld, nmaj, nmin, maj_off, min_off;
+};
+
+GcLayout gc_layout(const GcPlan &P, const GcShare &d, int col_major) {
+    GcLayout L;
+    L.cmaj = (P.direction == kGcDescend) == (col_major != 0);
+    L.ld = col_major ? P.n_pro : P.n_anc;
+    const int64_t T = (int64_t)P.target_uid().size(), C = d.j1 - d.j0;
+    L.nmaj = L.cmaj ? C : T; L.nmin = L.cmaj ? T : C;
+    L.maj_off = L.cmaj ? d.j0 : 0; L.min_off = L.cmaj ? 0 : d.j0;
+    return L;
+}
+
+size_t gc_device_bytes(const GcPlan &P, GcShare &d, int col_major, size_t esize) {
+    const size_t ws = (size_t)d.ws(), R = (size_t)P.rows();
+    d.stage = pad256(std::max<size_t>(kFetchStageBytes, (size_t)gc_layout(P, d, col_major).nmin * esize));
+    return pad256((size_t)P.capacity * ws * 8) + pad256((size_t)P.n_targets() * ws * 8) +
+           3 * DevBuf<int32_t>::padded(R) + DevBuf<int64_t>::padded(R + 1) + DevBuf<int32_t>::padded((size_t)P.inputs()) +
+           DevBuf<int32_t>::padded(P.target_uid().size()) + DevBuf<int32_t>::padded((size_t)(d.j1 - d.j0)) +
+           DevBuf<int32_t>::padded(1) + 2 * d.stage;
+}
+
+template <typename O>
+int gc_fetch(const GcPlan &P, GcShare &d, const double *Oblk, const int32_t *tgt_row, const int32_t *col, O *out,
+             int col_major, unsigned char *stage_base, cudaStream_t st, cudaStream_t cst) {
+    const GcLayout L = gc_layout(P, d, col_major);
+    if (L.nmaj == 0 || L.nmin == 0) return GENLIB_OK;
+    const int64_t per = std::max<int64_t>(1, std::min<int64_t>(L.nmaj, (int64_t)(d.stage / (L.nmin * sizeof(O)))));
+    O *stage[2] = {reinterpret_cast<O *>(stage_base), reinterpret_cast<O *>(stage_base + d.stage)};
+    cudaEvent_t done[2] = {nullptr, nullptr}, copied[2] = {nullptr, nullptr};
+    cudaError_t ce = cudaSuccess;
+    for (int b = 0; b < 2 && ce == cudaSuccess; b++) {
+        ce = cudaEventCreateWithFlags(&done[b], cudaEventDisableTiming);
+        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&copied[b], cudaEventDisableTiming);
+    }
+    int blk = 0;
+    for (int64_t m0 = 0; m0 < L.nmaj && ce == cudaSuccess; m0 += per, blk++) {      // gather of block b+1 overlaps the D2H of block b
+        const int b = blk & 1;
+        const int64_t nb = std::min(per, L.nmaj - m0);
+        if (blk >= 2 && (ce = cudaStreamWaitEvent(st, copied[b], 0)) != cudaSuccess) break;
+        GcGatherArgs a;
+        a.O = Oblk; a.ws = d.ws(); a.tgt_row = tgt_row; a.col = col;
+        if (L.cmaj) { a.t0 = 0; a.n_t = (int32_t)L.nmin; a.c0 = (int32_t)m0; a.n_c = (int32_t)nb; }
+        else        { a.t0 = (int32_t)m0; a.n_t = (int32_t)nb; a.c0 = 0; a.n_c = (int32_t)L.nmin; }
+        dim3 grid((unsigned)((a.n_c + 31) / 32), (unsigned)std::min<int64_t>((a.n_t + 31) / 32, 65535)), block(32, 8);
+        if (L.cmaj) gc_gather_kernel<true, O><<<grid, block, 0, st>>>(a, stage[b]);
+        else        gc_gather_kernel<false, O><<<grid, block, 0, st>>>(a, stage[b]);
+        if ((ce = cudaGetLastError()) != cudaSuccess) break;
+        cudaEventRecord(done[b], st);
+        cudaStreamWaitEvent(cst, done[b], 0);
+        ce = cudaMemcpy2DAsync(out + (L.maj_off + m0) * L.ld + L.min_off, (size_t)L.ld * sizeof(O), stage[b],
+                               (size_t)L.nmin * sizeof(O), (size_t)L.nmin * sizeof(O), (size_t)nb, cudaMemcpyDeviceToHost, cst);
+        cudaEventRecord(copied[b], cst);
+    }
+    const cudaError_t e1 = cudaStreamSynchronize(st), e2 = cudaStreamSynchronize(cst);
+    for (int b = 0; b < 2; b++) { if (done[b]) cudaEventDestroy(done[b]); if (copied[b]) cudaEventDestroy(copied[b]); }
+    if (ce != cudaSuccess || e1 != cudaSuccess || e2 != cudaSuccess)
+        return fail(GENLIB_ECUDA, std::string("gc fetch failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : e1 != cudaSuccess ? e1 : e2));
+    d.d2h += L.nmaj * L.nmin * (int64_t)sizeof(O);
+    return GENLIB_OK;
+}
+
+// Every layer of the plan over the share's columns on its device, then its block of `out`.
+int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_major) {
+    DeviceGuard guard;
+    if (int rc = guard.enter(d.device)) return rc;
+    struct Res {
+        cudaStream_t st = nullptr, cst = nullptr;
+        cudaEvent_t ev[2] = {nullptr, nullptr};
+        Arena arena;
+        ~Res() {
+            if (st) cudaStreamSynchronize(st);
+            if (cst) cudaStreamSynchronize(cst);
+            for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
+            if (st) cudaStreamDestroy(st);
+            if (cst) cudaStreamDestroy(cst);
+            g_arenas.release(arena);
+        }
+    } res;
+    CU(cudaStreamCreateWithFlags(&res.st, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&res.cst, cudaStreamNonBlocking));
+    for (cudaEvent_t &e : res.ev) CU(cudaEventCreate(&e));
+    if (g_arenas.acquire(d.device, d.need, res.arena) != cudaSuccess) {
+        res.arena = Arena();
+        cudaGetLastError();
+        size_t free_b = 0, total_b = 0;
+        cudaMemGetInfo(&free_b, &total_b);
+        char msg[256];
+        std::snprintf(msg, sizeof msg, "gen.gc needs %.2f GB on device %d, %.2f GB free (%lld frontier rows x %lld columns): "
+                      "split the columns over more devices", d.need / 1e9, d.device, free_b / 1e9,
+                      (long long)P.capacity, (long long)(d.hi - d.lo));
+        return fail(GENLIB_ENOMEM, msg);
+    }
+    const size_t ws = (size_t)d.ws(), R = (size_t)P.rows();
+    unsigned char *cur = static_cast<unsigned char *>(res.arena.base);
+    auto take = [&](size_t bytes) { unsigned char *p = cur; cur += pad256(bytes); return p; };
+    double *F = reinterpret_cast<double *>(take((size_t)P.capacity * ws * 8));
+    double *O = reinterpret_cast<double *>(take((size_t)P.n_targets() * ws * 8));
+    DevBuf<int32_t> row_slot, row_seed, row_out, in_slot, tgt_row, col, err;
+    DevBuf<int64_t> in_ptr;
+    row_slot.place(cur, R); row_seed.place(cur, R); row_out.place(cur, R); in_ptr.place(cur, R + 1);
+    in_slot.place(cur, (size_t)P.inputs()); tgt_row.place(cur, P.target_uid().size());
+    col.place(cur, (size_t)(d.j1 - d.j0)); err.place(cur, 1);
+    unsigned char *stage = cur;
+    cur += 2 * d.stage;
+    if ((size_t)(cur - static_cast<unsigned char *>(res.arena.base)) > d.need) return fail(GENLIB_EINVAL, "internal: gc arena layout overflow");
+    std::vector<int32_t> cols((size_t)(d.j1 - d.j0));
+    for (int32_t j = d.j0; j < d.j1; j++) cols[(size_t)(j - d.j0)] = P.column_uid()[(size_t)j] - d.lo;
+    CU(row_slot.upload(P.row_slot, res.st)); CU(row_seed.upload(P.row_seed, res.st)); CU(row_out.upload(P.row_out, res.st));
+    CU(in_ptr.upload(P.in_ptr, res.st)); CU(in_slot.upload(P.in_slot, res.st)); CU(tgt_row.upload(P.target_uid(), res.st));
+    CU(col.upload(cols, res.st));
+    CU(cudaMemsetAsync(err.p, 0, sizeof(int32_t), res.st));
+    if (P.n_out_rows < P.n_targets())                       // a target no path reaches: its output row is 0
+        CU(cudaMemsetAsync(O, 0, (size_t)P.n_targets() * ws * 8, res.st));
+    GcLayerArgs a;
+    a.F = reinterpret_cast<double2 *>(F); a.O = reinterpret_cast<double2 *>(O);
+    a.w2 = (int64_t)ws / 2; a.width = d.hi - d.lo; a.col_lo = d.lo;
+    a.capacity = P.capacity; a.n_targets = P.n_targets(); a.in_slot = in_slot.p; a.err = err.p;
+    const unsigned gx = (unsigned)((a.w2 + kGcChunk - 1) / kGcChunk);
+    CU(cudaEventRecord(res.ev[0], res.st));
+    for (int32_t t = 0; t < P.n_layers(); t++) {
+        const int64_t r0 = P.layer_begin[(size_t)t];
+        a.n_rows = (int32_t)(P.layer_begin[(size_t)t + 1] - r0);
+        a.row_slot = row_slot.p + r0; a.row_seed = row_seed.p + r0; a.row_out = row_out.p + r0; a.in_ptr = in_ptr.p + r0;
+        gc_layer_kernel<<<dim3(gx, (unsigned)std::min<int32_t>(a.n_rows, 65535)), kGcThreads, 0, res.st>>>(a);
+        CU(cudaGetLastError());
+        d.launches++;
+    }
+    CU(cudaEventRecord(res.ev[1], res.st));
+    CU(cudaStreamSynchronize(res.st));
+    float ms = 0;
+    CU(cudaEventElapsedTime(&ms, res.ev[0], res.ev[1]));
+    d.ms_kernels = ms;
+    int32_t errw = 0;
+    CU(cudaMemcpy(&errw, err.p, sizeof errw, cudaMemcpyDeviceToHost));
+    if (errw) return fail(GENLIB_ECUDA, "the gc layer kernel reported a bound violated at line " + std::to_string(errw - 100000));
+    const double t0 = now_ms();
+    const int rc = out_dtype == GENLIB_F64
+        ? gc_fetch<double>(P, d, O, tgt_row.p, col.p, static_cast<double *>(out), col_major, stage, res.st, res.cst)
+        : gc_fetch<float>(P, d, O, tgt_row.p, col.p, static_cast<float *>(out), col_major, stage, res.st, res.cst);
+    d.ms_fetch = now_ms() - t0;
+    return rc;
+}
+
+void gc_fill_stats(const GcPlan &P, genlib_gc_stats *s) {
+    std::memset(s, 0, sizeof *s);
+    s->n_pro = P.n_pro; s->n_anc = P.n_anc; s->n_layers = P.n_layers(); s->direction = P.direction;
+    s->rows = P.rows(); s->inputs = P.inputs(); s->width = P.width(); s->capacity = P.capacity;
+    s->alg_bytes = P.alg_bytes(P.width());
+    s->n_dev = 1;
+}
+
+}  // namespace
+
+extern "C" {
+
+int genlib_gc_plan_create(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
+                          const int32_t *proband, int32_t n_anc, const int32_t *ancestor, genlib_gc_plan **out) {
+    if (!out) return fail(GENLIB_EINVAL, "genlib_gc_plan_create: null argument");
+    *out = nullptr;
+    std::unique_ptr<genlib_gc_plan> pl(new (std::nothrow) genlib_gc_plan);
+    if (!pl) return fail(GENLIB_ENOMEM, "out of host memory");
+    const double t0 = now_ms();
+    std::string err;
+    try {
+        if (int rc = build_gc_plan(n, father, mother, n_pro, proband, n_anc, ancestor, -1, pl->p, err)) return fail(rc, err);
+    } catch (const std::bad_alloc &) {
+        return fail(GENLIB_ENOMEM, "out of host memory while planning");
+    }
+    pl->ms_plan = now_ms() - t0;
+    *out = pl.release();
+    return GENLIB_OK;
+}
+
+void genlib_gc_plan_destroy(genlib_gc_plan *plan) { delete plan; }
+
+int genlib_gc_plan_info(const genlib_gc_plan *plan, genlib_gc_stats *out) {
+    if (!plan || !out) return fail(GENLIB_EINVAL, "genlib_gc_plan_info: null argument");
+    gc_fill_stats(plan->p, out);
+    GcShare d;
+    d.j1 = (int32_t)plan->p.column_uid().size(); d.hi = plan->p.width();
+    out->device_bytes = plan->p.width() > 0 && plan->p.n_targets() > 0 ? (int64_t)gc_device_bytes(plan->p, d, 0, 8) : 0;
+    return GENLIB_OK;
+}
+
+int genlib_gc_plan_layer(const genlib_gc_plan *plan, int32_t layer, int32_t *n_rows, int64_t *n_inputs) {
+    if (!plan) return fail(GENLIB_EINVAL, "genlib_gc_plan_layer: null plan");
+    const GcPlan &P = plan->p;
+    if (layer < 0 || layer >= P.n_layers()) return fail(GENLIB_EINVAL, "layer out of range");
+    const int64_t r0 = P.layer_begin[(size_t)layer], r1 = P.layer_begin[(size_t)layer + 1];
+    if (n_rows) *n_rows = (int32_t)(r1 - r0);
+    if (n_inputs) *n_inputs = P.in_ptr[(size_t)r1] - P.in_ptr[(size_t)r0];
+    return GENLIB_OK;
+}
+
+int genlib_gc_plan_layer_arrays(const genlib_gc_plan *plan, int32_t layer, int32_t *row_ind, int32_t *row_slot,
+                                int32_t *row_seed, int32_t *row_out, int64_t *in_ptr, int32_t *in_slot) {
+    if (!plan) return fail(GENLIB_EINVAL, "genlib_gc_plan_layer_arrays: null plan");
+    const GcPlan &P = plan->p;
+    if (layer < 0 || layer >= P.n_layers()) return fail(GENLIB_EINVAL, "layer out of range");
+    const size_t r0 = (size_t)P.layer_begin[(size_t)layer], r1 = (size_t)P.layer_begin[(size_t)layer + 1];
+    auto copy = [&](const std::vector<int32_t> &v, int32_t *o) { if (o) std::copy(v.begin() + (long)r0, v.begin() + (long)r1, o); };
+    copy(P.row_ind, row_ind); copy(P.row_slot, row_slot); copy(P.row_seed, row_seed); copy(P.row_out, row_out);
+    const int64_t e0 = P.in_ptr[r0];
+    if (in_ptr) for (size_t r = r0; r <= r1; r++) in_ptr[r - r0] = P.in_ptr[r] - e0;
+    if (in_slot) std::copy(P.in_slot.begin() + e0, P.in_slot.begin() + P.in_ptr[r1], in_slot);
+    return GENLIB_OK;
+}
+
+int genlib_gc(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+              int32_t n_anc, const int32_t *ancestor, void *out, int out_dtype, int col_major, int32_t n_dev,
+              const int32_t *devices, genlib_gc_stats *stats) {
+    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
+    if (n_dev < 1 || !devices) return fail(GENLIB_EINVAL, "genlib_gc: at least one device");
+    genlib_gc_plan *plan = nullptr;
+    if (int rc = genlib_gc_plan_create(n, father, mother, n_pro, proband, n_anc, ancestor, &plan)) return rc;
+    std::unique_ptr<genlib_gc_plan> owner(plan);
+    const GcPlan &P = plan->p;
+    genlib_gc_stats st;
+    gc_fill_stats(P, &st);
+    st.ms_plan = plan->ms_plan;
+    st.n_dev = n_dev;
+    if (P.n_pro == 0 || P.n_anc == 0) {                     // an empty matrix: no device needed
+        if (stats) *stats = st;
+        return GENLIB_OK;
+    }
+    if (!out) return fail(GENLIB_EINVAL, "genlib_gc: out is null");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+        return fail(GENLIB_ECUDA, "no CUDA device: libgenlib_cuda has no CPU fallback");
+    std::vector<GcShare> share((size_t)n_dev);
+    const std::vector<int32_t> &cu = P.column_uid();
+    const int64_t m = (int64_t)cu.size();
+    const size_t esize = out_dtype == GENLIB_F64 ? 8 : 4;
+    for (int g = 0; g < n_dev; g++) {
+        GcShare &d = share[(size_t)g];
+        d.device = devices[g];
+        if (d.device < 0 && cudaGetDevice(&d.device) != cudaSuccess) return fail(GENLIB_ECUDA, "no usable CUDA device (cudaGetDevice failed)");
+        if (d.device >= ndev) return fail(GENLIB_EINVAL, "genlib_gc: no such device");
+        for (int h = 0; h < g; h++) if (share[(size_t)h].device == d.device) return fail(GENLIB_EINVAL, "genlib_gc: a device is listed twice");
+        d.j0 = (int32_t)(m * g / n_dev); d.j1 = (int32_t)(m * (g + 1) / n_dev);
+        if (d.j0 == d.j1) continue;                          // more devices than columns: nothing to do here
+        d.lo = *std::min_element(cu.begin() + d.j0, cu.begin() + d.j1);
+        d.hi = *std::max_element(cu.begin() + d.j0, cu.begin() + d.j1) + 1;
+        d.need = gc_device_bytes(P, d, col_major, esize);
+    }
+    std::vector<int> status((size_t)n_dev, GENLIB_OK);
+    std::vector<std::string> message((size_t)n_dev);
+    auto run = [&](int g) {
+        GcShare &d = share[(size_t)g];
+        if (d.j0 == d.j1) return;
+        status[(size_t)g] = gc_run_share(P, d, out, out_dtype, col_major);
+        if (status[(size_t)g] != GENLIB_OK) message[(size_t)g] = g_err;
+    };
+    if (n_dev == 1) run(0);
+    else {                                                   // one host thread per device, as genlib_phi_multi
+        std::vector<std::thread> th;
+        for (int g = 0; g < n_dev; g++) th.emplace_back(run, g);
+        for (auto &t : th) t.join();
+    }
+    for (int g = 0; g < n_dev; g++)
+        if (status[(size_t)g] != GENLIB_OK) return fail(status[(size_t)g], "device " + std::to_string(share[(size_t)g].device) + ": " + message[(size_t)g]);
+    if (stats) {
+        st.width = 0; st.alg_bytes = 0;
+        for (const GcShare &d : share) {
+            if (d.j0 == d.j1) continue;
+            st.width += d.hi - d.lo;
+            st.alg_bytes += P.alg_bytes(d.hi - d.lo);
+            st.device_bytes = std::max(st.device_bytes, (int64_t)d.need);
+            st.ms_kernels = std::max(st.ms_kernels, d.ms_kernels);
+            st.ms_fetch = std::max(st.ms_fetch, d.ms_fetch);
+            st.d2h_bytes += d.d2h;
+            st.kernel_launches += d.launches;
+        }
+        *stats = st;
+    }
     return GENLIB_OK;
 }
 

@@ -13,7 +13,8 @@ from typing import Optional
 import numpy as np
 
 from . import _lib
-from ._lib import LayerInfo, PlanBoundsExceeded, Stats, check, lib, ptr
+from . import pedigree as _pedigree
+from ._lib import GcStats, LayerInfo, PlanBoundsExceeded, Stats, check, lib, ptr
 from .pedigree import Pedigree, pro
 
 
@@ -381,6 +382,85 @@ def phi_arrays(father, mother, proband_ranks, *, numerics="reference", dtype=np.
         check(lib().genlib_phi(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), ptr(out),
                                _lib.DTYPES[np.dtype(out.dtype)], _lib.NUMERICS[numerics], device, C.byref(st)))
     return out, st.as_dict()
+
+
+class GcPlan:
+    """The schedule of gen.gc (genlib_gc_plan_*): direction, layers, frontier slots.  Needs no GPU."""
+
+    def __init__(self, father, mother, proband_ranks, ancestor_ranks):
+        self.father = np.ascontiguousarray(father, np.int32)
+        self.mother = np.ascontiguousarray(mother, np.int32)
+        self.probands = np.ascontiguousarray(proband_ranks, np.int32)
+        self.ancestors = np.ascontiguousarray(ancestor_ranks, np.int32)
+        if len(self.father) != len(self.mother):
+            raise ValueError("father and mother must have the same length")
+        h = C.c_void_p()
+        check(lib().genlib_gc_plan_create(len(self.father), ptr(self.father), ptr(self.mother), len(self.probands),
+                                          ptr(self.probands), len(self.ancestors), ptr(self.ancestors), C.byref(h)))
+        self._h = h
+
+    def __del__(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h:
+            lib().genlib_gc_plan_destroy(h)
+
+    def info(self) -> dict:
+        """genlib_gc_stats without timings; `direction` is "descend" or "ascend"."""
+        s = GcStats()
+        check(lib().genlib_gc_plan_info(self._h, C.byref(s)))
+        d = s.as_dict()
+        d["direction"] = _lib.GC_DIRECTIONS[d["direction"]]
+        return d
+
+    def layer_arrays(self, layer: int) -> dict:
+        n_rows, n_in = C.c_int32(), C.c_int64()
+        check(lib().genlib_gc_plan_layer(self._h, layer, C.byref(n_rows), C.byref(n_in)))
+        out = {k: np.zeros(n_rows.value, np.int32) for k in ("row_ind", "row_slot", "row_seed", "row_out")}
+        out["in_ptr"] = np.zeros(n_rows.value + 1, np.int64)
+        out["in_slot"] = np.zeros(n_in.value, np.int32)
+        check(lib().genlib_gc_plan_layer_arrays(self._h, layer, *(ptr(out[k]) for k in (
+            "row_ind", "row_slot", "row_seed", "row_out", "in_ptr", "in_slot"))))
+        return out
+
+    def layers(self):
+        return [self.layer_arrays(t) for t in range(self.info()["n_layers"])]
+
+
+def gc(pedigree: Pedigree, pro=None, ancestors=None, *, dtype=np.float64, device: int = -1, devices=None,
+       out: Optional[np.ndarray] = None, return_stats: bool = False):
+    """gen.gc(pedigree; pro = pro(pedigree), ancestors = founder(pedigree)) on the B200 engine
+    (src/compute.jl:518-595): the genetic contribution of every ancestor to every proband,
+    G[p, a] = sum over descent paths a -> p of (1/2)^length, a len(pro) x len(ancestors) Float64 matrix
+    in list order, duplicates kept.  KeyError on an unknown ID.  `devices=[0, 1, ...]` splits the
+    columns over several GPUs of the box (genlib_gc)."""
+    pro_ids = _pedigree.pro(pedigree) if pro is None else np.asarray(pro, np.int64)
+    anc_ids = _pedigree.founder(pedigree) if ancestors is None else np.asarray(ancestors, np.int64)
+    res, stats = gc_arrays(pedigree.father, pedigree.mother, pedigree.rank_of(pro_ids), pedigree.rank_of(anc_ids),
+                           dtype=dtype, device=device, devices=devices, out=out)
+    return (res, stats) if return_stats else res
+
+
+def gc_arrays(father, mother, proband_ranks, ancestor_ranks, *, dtype=np.float64, device: int = -1, devices=None,
+              out: Optional[np.ndarray] = None, col_major: bool = False):
+    """One-shot C-ABI call `genlib_gc` on flat rank arrays (what the Julia shim ccalls).  Returns
+    (matrix, stats); col_major=True fills a Fortran-ordered matrix (a Julia Matrix) without a transpose."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32)
+    an = np.ascontiguousarray(ancestor_ranks, np.int32)
+    shape = (len(pr), len(an))
+    if out is None:
+        out = np.empty(shape, dtype, order="F" if col_major else "C")
+    contiguous = out.flags.f_contiguous if col_major else out.flags.c_contiguous
+    if out.shape != shape or not contiguous or out.dtype not in _lib.DTYPES:
+        raise ValueError(f"out must be a {'Fortran' if col_major else 'C'}-contiguous {shape} float32/float64 array")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = GcStats()
+    check(lib().genlib_gc(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), len(an), ptr(an), ptr(out),
+                          _lib.DTYPES[np.dtype(out.dtype)], int(col_major), len(dv), ptr(dv), C.byref(st)))
+    stats = st.as_dict()
+    stats["direction"] = _lib.GC_DIRECTIONS[stats["direction"]]
+    return out, stats
 
 
 def f(pedigree: Pedigree, IDs, *, device: int = -1) -> np.ndarray:

@@ -237,4 +237,39 @@ function sparse_phi(pedigree::GenLib.Pedigree, probandIDs::Vector{Int} = GenLib.
     end
 end
 
+struct GcStats              # genlib_gc_stats
+    n_pro::Int32; n_anc::Int32; n_layers::Int32; direction::Int32
+    rows::Int64; inputs::Int64; width::Int64; capacity::Int64; device_bytes::Int64
+    alg_bytes::Float64; ms_plan::Float64; ms_kernels::Float64; ms_fetch::Float64
+    d2h_bytes::Int64; kernel_launches::Int32; n_dev::Int32
+end
+
+"""
+    gc(pedigree; pro = GenLib.pro(pedigree), ancestors = GenLib.founder(pedigree),
+       device = -1, devices = Int[]) -> Matrix{Float64}
+
+`gen.gc` (src/compute.jl:518-595) on the B200 engine: `G[p, a]` = the expected share of proband `p`'s
+genome that comes from ancestor `a`, the sum over descent paths of (1/2)^length.  Rows follow `pro`,
+columns follow `ancestors`, duplicates kept; an unknown ID throws `KeyError`.  The library writes the
+column-major matrix directly (`col_major = 1`), so there is no transpose on the host.  `devices = [0, 1, ...]`
+splits the columns over several GPUs of the box; the result is bitwise the one-GPU result.
+Like the rest of this shim it is not executed in this repository (no Julia in the build image); the same
+call is exercised through Python ctypes by tests/test_gc.py.
+"""
+function gc(pedigree::GenLib.Pedigree; pro::Vector{Int} = GenLib.pro(pedigree),
+            ancestors::Vector{Int} = GenLib.founder(pedigree), device::Integer = -1,
+            devices::Vector{<:Integer} = Int[])
+    father, mother = flatten(pedigree)
+    p = Int32[pedigree[ID].rank - 1 for ID in pro]                   # KeyError on unknown ID
+    a = Int32[pedigree[ID].rank - 1 for ID in ancestors]
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    G = Matrix{Float64}(undef, length(p), length(a))
+    stats = Ref{GcStats}()
+    GC.@preserve G check(ccall((:genlib_gc, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Cvoid}, Cint, Cint, Int32,
+         Ptr{Int32}, Ptr{GcStats}),
+        length(father), father, mother, length(p), p, length(a), a, pointer(G), 1, 1, length(devs), devs, stats))
+    G
+end
+
 end # module

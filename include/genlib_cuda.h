@@ -281,6 +281,53 @@ int genlib_engine_set_layer_limit(genlib_engine *eng, int32_t n_layers);
 /* Debug/test: copy the frontier entry block [slots x slots] (as double). */
 int genlib_engine_read_block(genlib_engine *eng, int32_t n_slots, const int32_t *slots, double *out);
 
+/* ---- gen.gc: the proband x ancestor genetic-contribution matrix (SURVEY.md 2: src/compute.jl:518-595) -----
+ *   G[p, a] = sum over descent paths a -> ... -> p of (1/2)^(path length)
+ *           = [p == a] + 1/2 G[father(p), a] + 1/2 G[mother(p), a]        (a missing parent adds 0)
+ * Rows follow `proband`, columns follow `ancestor`; duplicates are KEPT (a repeated rank gives a repeated
+ * row / column).  Every value is a sum of powers of 1/2: while no path from a listed ancestor to a listed
+ * proband is longer than 52 edges the result is exact (whatever the order of the sums), deeper pedigrees get
+ * the fixed summation order of DESIGN.md 2b.  The engine propagates the narrower side (DIRECTION below;
+ * environment GENLIB_GC_DIRECTION=descend|ascend overrides the rule) over the individuals that lie on a path
+ * from a listed ancestor to a listed proband. */
+#define GENLIB_GC_DESCEND 0 /* columns = unique ancestors, rows go down the generations              */
+#define GENLIB_GC_ASCEND 1  /* columns = unique probands, rows go up; the output is the transpose  */
+typedef struct genlib_gc_stats {
+    int32_t n_pro, n_anc;        /* output shape (duplicates kept)                                  */
+    int32_t n_layers, direction;
+    int64_t rows, inputs;        /* active rows computed, input edges read                          */
+    int64_t width, capacity;     /* columns propagated (all devices), peak live frontier rows       */
+    int64_t device_bytes;        /* largest per-device allocation                                   */
+    double alg_bytes;            /* required traffic, summed over devices: (input rows read +       */
+                                 /* frontier rows written + output rows written) x columns x 8      */
+    double ms_plan, ms_kernels, ms_fetch; /* ms_kernels: CUDA events, slowest device                */
+    int64_t d2h_bytes;
+    int32_t kernel_launches, n_dev;
+} genlib_gc_stats;
+/* out: n_pro x n_anc elements of out_dtype, row-major, or column-major when col_major != 0 (what a Julia
+ * Matrix is); host memory (pinned or pageable).  The column side's list is split into n_dev contiguous,
+ * balanced ranges, one per device (one host thread each, no peer access); every device writes its own
+ * rectangular block of `out` and the result is bitwise the one-device result.  devices[g] < 0 = the current
+ * device.  An empty list gives an empty matrix without a device.  GENLIB_ENOMEM names the bytes one device
+ * needs (more devices need less each). */
+int genlib_gc(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+              int32_t n_anc, const int32_t *ancestor, void *out, int out_dtype, int col_major, int32_t n_dev,
+              const int32_t *devices, genlib_gc_stats *stats);
+/* The schedule alone (host only; tests replay it).  Unique probands / ancestors are numbered in order of
+ * first occurrence; `columns` are the unique ancestors (descend) or probands (ascend), the output block holds
+ * one row per unique target (the other side).  Per layer: row_ind = pedigree rank, row_slot = frontier slot
+ * (-1: nobody reads the row later), row_seed = the row's own column (-1: none), row_out = output-block row
+ * (-1: not a target), in_ptr (n_rows + 1 entries, from 0) / in_slot = the frontier slots of the inputs, in
+ * the order they are added.  genlib_gc_plan_info reports no timings; device_bytes is for one device. */
+typedef struct genlib_gc_plan genlib_gc_plan;
+int genlib_gc_plan_create(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
+                          const int32_t *proband, int32_t n_anc, const int32_t *ancestor, genlib_gc_plan **out);
+void genlib_gc_plan_destroy(genlib_gc_plan *plan);
+int genlib_gc_plan_info(const genlib_gc_plan *plan, genlib_gc_stats *out);
+int genlib_gc_plan_layer(const genlib_gc_plan *plan, int32_t layer, int32_t *n_rows, int64_t *n_inputs);
+int genlib_gc_plan_layer_arrays(const genlib_gc_plan *plan, int32_t layer, int32_t *row_ind, int32_t *row_slot,
+                                int32_t *row_seed, int32_t *row_out, int64_t *in_ptr, int32_t *in_slot);
+
 #ifdef __cplusplus
 }
 #endif
