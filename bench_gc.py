@@ -1,13 +1,17 @@
 #!/usr/bin/env python
-"""bench_gc.py -- gen.gc (proband x ancestor genetic contributions) on a benchmark pedigree.
+"""bench_gc.py -- gen.gc (proband x ancestor genetic contributions), gen.occ and gen.rec on a benchmark pedigree.
 
     python bench_gc.py --config C3 --steps 5 --warmup 1 [--direction descend|ascend] [--ancestors K]
+                       [--function gc|occ|occ_total|rec]
 
 A step is one genlib_gc call: host rank arrays in, planning, upload, every layer, gather and D2H of the
-whole len(pro) x len(ancestors) Float64 matrix into pinned host memory.  `ms_kernels` (CUDA events
+whole len(pro) x len(ancestors) Float64 matrix into pinned host memory.  `--function occ` is one genlib_occ
+call that returns the len(ancestors) x len(pro) Int64 path counts the same way; `occ_total` (its row sums)
+and `rec` (descendant counts) reduce on the device and fetch len(ancestors) Int64 values.  `ms_kernels` (CUDA events
 around the layer kernels, slowest device) and `e2e_ms` (host clock around the call) are medians over
 the timed steps.  `alg_bytes` is the traffic the layers cannot avoid (input rows read, frontier and
-output rows written, binary64); `frac_of_peak` divides it by ms_kernels and the measured HBM peak.
+output rows written, 8 bytes per column -- gen.rec: per 64-column word -- plus one read of the output block
+for a reduction); `frac_of_peak` divides it by ms_kernels and the measured HBM peak.
 The C3 working set (frontier and output block, GBs) is far larger than the 126 MB L2; genea140's is
 not.  Prints one JSON line; writes nothing.
 """
@@ -55,6 +59,9 @@ def workload(gen, name: str, scale: float, n_anc: int | None, seed: int):
     return ped, ped.rank_of(pro), ped.rank_of(anc), n_anc is None
 
 
+METRIC_NAME = {"gc": "gc", "occ": "occ", "occ_total": "occ(TOTAL)", "rec": "rec"}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--config", default="C3", help="genea140, C3, C4 or C5")
@@ -65,6 +72,7 @@ def main():
     ap.add_argument("--ancestors", type=int, default=None, help="a seeded sample of this many founders")
     ap.add_argument("--seed", type=int, default=1)
     ap.add_argument("--devices", default="0", help="comma-separated device list")
+    ap.add_argument("--function", choices=["gc", "occ", "occ_total", "rec"], default="gc")
     args = ap.parse_args()
     if args.steps < 1:
         ap.error("--steps must be at least 1")
@@ -77,20 +85,29 @@ def main():
         raise SystemExit("no CUDA device: gen.gc has no CPU fallback")
     devices = [int(d) for d in args.devices.split(",")]
     ped, pro, anc, all_founders = workload(gen, args.config, args.scale, args.ancestors, args.seed)
-    shape = (len(pro), len(anc))
-    nbytes = max(1, shape[0] * shape[1] * 8)
+    shape = {"gc": (len(pro), len(anc)), "occ": (len(anc), len(pro)), "occ_total": (len(anc), 1),
+             "rec": (len(anc),)}[args.function]
+    dtype = np.float64 if args.function == "gc" else np.int64
+    nbytes = max(1, int(np.prod(shape)) * 8)
     p = C.c_void_p()
     gen._lib.check(gen.lib().genlib_pinned_alloc(nbytes, C.byref(p)))
     try:
-        out = np.frombuffer((C.c_char * nbytes).from_address(p.value), np.float64, count=shape[0] * shape[1]).reshape(shape)
+        out = np.frombuffer((C.c_char * nbytes).from_address(p.value), dtype, count=int(np.prod(shape))).reshape(shape)
+        call = {
+            "gc": lambda: gen.gc_arrays(ped.father, ped.mother, pro, anc, out=out, devices=devices),
+            "occ": lambda: gen.occ_arrays(ped.father, ped.mother, pro, anc, out=out, devices=devices),
+            "occ_total": lambda: gen.occ_arrays(ped.father, ped.mother, pro, anc, typeOcc="TOTAL", out=out,
+                                                devices=devices),
+            "rec": lambda: gen.rec_arrays(ped.father, ped.mother, pro, anc, out=out, devices=devices),
+        }[args.function]
         ms_k, e2e, stats = [], [], None
         for step in range(args.warmup + args.steps):
             t0 = time.perf_counter()
-            _, stats = gen.gc_arrays(ped.father, ped.mother, pro, anc, out=out, devices=devices)
+            _, stats = call()
             t1 = time.perf_counter()
             if step >= args.warmup:
                 ms_k.append(stats["ms_kernels"]); e2e.append((t1 - t0) * 1e3)
-        sums = out.sum(axis=1)
+        sums = out.sum(axis=1) if args.function == "gc" else None
         digest = hashlib.sha256(out.tobytes()).hexdigest()
     finally:
         gen.lib().genlib_pinned_free(p)
@@ -98,7 +115,8 @@ def main():
     ms = float(np.median(ms_k))
     name, power = gpu_card()
     res = {
-        "metric": "gen.gc required bytes / kernel time", "config": args.config, "scale": args.scale,
+        "metric": f"gen.{METRIC_NAME[args.function]} required bytes / kernel time", "config": args.config,
+        "scale": args.scale,
         "shape": list(shape), "ancestors": "founders" if all_founders else f"{len(anc)} sampled founders",
         "direction": stats["direction"], "width": stats["width"], "capacity": stats["capacity"],
         "n_layers": stats["n_layers"], "rows": stats["rows"], "inputs": stats["inputs"],
@@ -110,7 +128,7 @@ def main():
         "hbm_peak_gbs": peak_gbs, "hbm_peak_source": peak_src,
         "frac_of_peak": stats["alg_bytes"] / ms / 1e6 / peak_gbs if ms > 0 else None,
         "output_sha256": digest,
-        "rows_summing_to_one": int((sums == 1.0).sum()), "n_pro": shape[0],
+        "rows_summing_to_one": int((sums == 1.0).sum()) if args.function == "gc" else None, "n_pro": len(pro),
         "gpu": name, "power_limit": power, "steps": args.steps, "warmup": args.warmup,
     }
     print(json.dumps(res))

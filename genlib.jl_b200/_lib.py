@@ -7,13 +7,14 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import re
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GENLIB_CUDA_LIB") or os.path.join(_HERE, "libgenlib_cuda.so")
 
-OK, EINVAL, EKEY, EORDER, ECUDA, ENOMEM, ECOMM, ERESTART = range(8)
+OK, EINVAL, EKEY, EORDER, ECUDA, ENOMEM, ECOMM, ERESTART, EOVERFLOW = range(9)
 SCHEDULES = {"phi": 0, "sparse_phi": 1, "sparse_phi_symmetric": 2}
 NUMERICS = {"reference": 0, "fp64": 1, 0: 0, 1: 1}
 DTYPES = {np.dtype(np.float32): 0, np.dtype(np.float64): 1}
@@ -29,6 +30,16 @@ class PlanBoundsExceeded(GenlibError):
     """genlib_engine_run on an engine of a plan that was still being made (Plan(..., stream=True)): a size
     bound did not hold (GENLIB_ERESTART).  Close the engine, create it again -- the plan is finished by
     then -- and run."""
+
+
+class GenlibOverflowError(GenlibError, OverflowError):
+    """gen.occ: a descent-path count or a row sum does not fit an Int64 (GENLIB_EOVERFLOW).
+    `ancestor_index` / `proband_index`: the 0-based list positions of the pair the library names."""
+
+    def __init__(self, status: int, message: str):
+        super().__init__(status, message)
+        m = re.search(r"ancestor position (-?\d+).*proband position (-?\d+)", message)
+        self.ancestor_index, self.proband_index = (int(m.group(1)), int(m.group(2))) if m else (None, None)
 
 
 class LayerInfo(C.Structure):
@@ -131,6 +142,10 @@ SYMBOLS = {
     "genlib_gc_plan_info": (C.c_int, [_P, C.POINTER(GcStats)]),
     "genlib_gc_plan_layer": (C.c_int, [_P, C.c_int32, _P, _P]),
     "genlib_gc_plan_layer_arrays": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    "genlib_occ": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int, C.c_int, C.c_int32, _P,
+                             C.POINTER(GcStats)]),
+    "genlib_rec": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int32, _P,
+                             C.POINTER(GcStats)]),
 }
 
 _lib = None
@@ -166,6 +181,8 @@ def check(status: int):
             raise MemoryError(msg)
         if status == ERESTART:
             raise PlanBoundsExceeded(status, msg)
+        if status == EOVERFLOW:
+            raise GenlibOverflowError(status, msg)
         raise GenlibError(status, msg)
 
 

@@ -463,6 +463,103 @@ def gc_arrays(father, mother, proband_ranks, ancestor_ranks, *, dtype=np.float64
     return out, stats
 
 
+OCC_TYPES = {"IND": 0, "TOTAL": 1}
+
+
+def _occ_type(typeOcc) -> int:
+    if typeOcc not in OCC_TYPES:
+        raise ValueError(f"typeOcc must be \"IND\" or \"TOTAL\", not {typeOcc!r}")
+    return OCC_TYPES[typeOcc]
+
+
+def _named_overflow(pedigree: Pedigree, pro_ids, anc_ids, e):
+    """The library's overflow error with the pair it names given as IDs."""
+    i, j = e.ancestor_index, e.proband_index
+    if i is None or j is None or j < 0:
+        return e
+    err = _lib.GenlibOverflowError(e.status, f"gen.occ: the number of descent paths from ancestor {int(anc_ids[i])} "
+                                   f"to proband {int(pro_ids[j])} does not fit an Int64 ({e})")
+    err.ancestor_index, err.proband_index = i, j
+    return err
+
+
+def occ(pedigree: Pedigree, pro=None, ancestors=None, typeOcc: str = "IND", *, device: int = -1, devices=None,
+        return_stats: bool = False):
+    """gen.occ(pedigree; pro = pro(pedigree), ancestors = founder(pedigree), typeOcc = "IND") on the B200
+    engine: O[a, p] = the number of descent paths from ancestor a to proband p (1 for a == p itself), a
+    len(ancestors) x len(pro) Int64 matrix in list order, duplicates kept -- ROWS ARE ANCESTORS.
+    typeOcc = "TOTAL" returns the len(ancestors) x 1 row sums, reduced on the device.  ValueError on another
+    typeOcc, KeyError on an unknown ID, an OverflowError (also a GenlibError) naming the first
+    (ancestor, proband) pair whose count or row sum does not fit an Int64."""
+    _occ_type(typeOcc)
+    pro_ids = _pedigree.pro(pedigree) if pro is None else np.asarray(pro, np.int64)
+    anc_ids = _pedigree.founder(pedigree) if ancestors is None else np.asarray(ancestors, np.int64)
+    pr, an = pedigree.rank_of(pro_ids), pedigree.rank_of(anc_ids)
+    try:
+        res, stats = occ_arrays(pedigree.father, pedigree.mother, pr, an, typeOcc=typeOcc, device=device,
+                                devices=devices)
+    except _lib.GenlibOverflowError as e:
+        raise _named_overflow(pedigree, pro_ids, anc_ids, e) from None
+    return (res, stats) if return_stats else res
+
+
+def occ_arrays(father, mother, proband_ranks, ancestor_ranks, *, typeOcc: str = "IND", device: int = -1,
+               devices=None, out: Optional[np.ndarray] = None, col_major: bool = False):
+    """One-shot C-ABI call `genlib_occ` on flat rank arrays.  Returns (result, stats): typeOcc = "IND" gives
+    the len(ancestors) x len(pro) int64 matrix (col_major=True: Fortran order, a Julia Matrix), "TOTAL" the
+    len(ancestors) x 1 int64 row sums."""
+    kind = _occ_type(typeOcc)
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32)
+    an = np.ascontiguousarray(ancestor_ranks, np.int32)
+    ind = kind == OCC_TYPES["IND"]
+    shape = (len(an), len(pr)) if ind else (len(an), 1)
+    if out is None:
+        out = np.empty(shape, np.int64, order="F" if ind and col_major else "C")
+    contiguous = out.flags.f_contiguous if ind and col_major else out.flags.c_contiguous
+    if out.shape != shape or not contiguous or out.dtype != np.int64:
+        raise ValueError(f"out must be a {'Fortran' if ind and col_major else 'C'}-contiguous {shape} int64 array")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = GcStats()
+    check(lib().genlib_occ(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), len(an), ptr(an), ptr(out),
+                           kind, int(col_major), len(dv), ptr(dv), C.byref(st)))
+    stats = st.as_dict()
+    stats["direction"] = _lib.GC_DIRECTIONS[stats["direction"]]
+    return out, stats
+
+
+def rec(pedigree: Pedigree, pro=None, ancestors=None, *, device: int = -1, devices=None, return_stats: bool = False):
+    """gen.rec(pedigree; pro = pro(pedigree), ancestors = founder(pedigree)) on the B200 engine: for every
+    ancestor, the number of entries of `pro` that descend from it, the ancestor itself included (duplicates
+    counted) -- an Int64 vector in ancestor-list order, reduced on the device."""
+    pro_ids = _pedigree.pro(pedigree) if pro is None else np.asarray(pro, np.int64)
+    anc_ids = _pedigree.founder(pedigree) if ancestors is None else np.asarray(ancestors, np.int64)
+    res, stats = rec_arrays(pedigree.father, pedigree.mother, pedigree.rank_of(pro_ids), pedigree.rank_of(anc_ids),
+                            device=device, devices=devices)
+    return (res, stats) if return_stats else res
+
+
+def rec_arrays(father, mother, proband_ranks, ancestor_ranks, *, device: int = -1, devices=None,
+               out: Optional[np.ndarray] = None):
+    """One-shot C-ABI call `genlib_rec` on flat rank arrays.  Returns (counts, stats)."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32)
+    an = np.ascontiguousarray(ancestor_ranks, np.int32)
+    if out is None:
+        out = np.empty(len(an), np.int64)
+    if out.shape != (len(an),) or not out.flags.c_contiguous or out.dtype != np.int64:
+        raise ValueError(f"out must be a contiguous ({len(an)},) int64 array")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = GcStats()
+    check(lib().genlib_rec(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), len(an), ptr(an), ptr(out),
+                           len(dv), ptr(dv), C.byref(st)))
+    stats = st.as_dict()
+    stats["direction"] = _lib.GC_DIRECTIONS[stats["direction"]]
+    return out, stats
+
+
 def f(pedigree: Pedigree, IDs, *, device: int = -1) -> np.ndarray:
     """gen.f(pedigree, IDs): inbreeding coefficients, Float32 (src/compute.jl:500-511).
 

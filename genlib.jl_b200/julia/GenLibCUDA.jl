@@ -33,6 +33,7 @@ function check(status::Cint)
     msg = unsafe_string(ccall((:genlib_last_error, libgenlib[]), Cstring, ()))
     status == 2 && throw(KeyError(msg))            # same exception as pedigree[ID] (src/create.jl:70)
     status == 5 && throw(OutOfMemoryError())
+    status == 8 && throw(OverflowError(msg))       # genlib_occ: a count does not fit an Int64
     error("libgenlib_cuda status $status: $msg")
 end
 
@@ -270,6 +271,59 @@ function gc(pedigree::GenLib.Pedigree; pro::Vector{Int} = GenLib.pro(pedigree),
          Ptr{Int32}, Ptr{GcStats}),
         length(father), father, mother, length(p), p, length(a), a, pointer(G), 1, 1, length(devs), devs, stats))
     G
+end
+
+"""
+    occ(pedigree; pro = GenLib.pro(pedigree), ancestors = GenLib.founder(pedigree), typeOcc = "IND",
+        device = -1, devices = Int[]) -> Matrix{Int64}
+
+`gen.occ` on the B200 engine: `O[a, p]` = the number of descent paths from ancestor `a` to proband `p`
+(1 for `a == p` itself).  ROWS ARE ANCESTORS, columns follow `pro`, duplicates kept; `typeOcc = "TOTAL"`
+gives the `length(ancestors) x 1` row sums, reduced on the device.  Another `typeOcc` throws `ArgumentError`
+before the library is called; a count or row sum that does not fit an Int64 throws `OverflowError` naming
+the first offending (ancestor, proband) pair (0-based list positions and ranks).  The library writes the
+column-major matrix directly.  Exercised through Python ctypes by tests/test_occ.py, not executed here.
+"""
+function occ(pedigree::GenLib.Pedigree; pro::Vector{Int} = GenLib.pro(pedigree),
+             ancestors::Vector{Int} = GenLib.founder(pedigree), typeOcc::AbstractString = "IND",
+             device::Integer = -1, devices::Vector{<:Integer} = Int[])
+    typeOcc in ("IND", "TOTAL") || throw(ArgumentError("typeOcc must be \"IND\" or \"TOTAL\", not \"$typeOcc\""))
+    father, mother = flatten(pedigree)
+    p = Int32[pedigree[ID].rank - 1 for ID in pro]                   # KeyError on unknown ID
+    a = Int32[pedigree[ID].rank - 1 for ID in ancestors]
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    O = Matrix{Int64}(undef, length(a), typeOcc == "IND" ? length(p) : 1)
+    stats = Ref{GcStats}()
+    GC.@preserve O check(ccall((:genlib_occ, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Int64}, Cint, Cint, Int32,
+         Ptr{Int32}, Ptr{GcStats}),
+        length(father), father, mother, length(p), p, length(a), a, pointer(O), typeOcc == "IND" ? 0 : 1, 1,
+        length(devs), devs, stats))
+    O
+end
+
+"""
+    rec(pedigree; pro = GenLib.pro(pedigree), ancestors = GenLib.founder(pedigree),
+        device = -1, devices = Int[]) -> Vector{Int64}
+
+`gen.rec` on the B200 engine: for every ancestor, the number of entries of `pro` that descend from it, the
+ancestor itself included, duplicates counted.  Reduced on the device.  Exercised through Python ctypes by
+tests/test_occ.py, not executed here.
+"""
+function rec(pedigree::GenLib.Pedigree; pro::Vector{Int} = GenLib.pro(pedigree),
+             ancestors::Vector{Int} = GenLib.founder(pedigree), device::Integer = -1,
+             devices::Vector{<:Integer} = Int[])
+    father, mother = flatten(pedigree)
+    p = Int32[pedigree[ID].rank - 1 for ID in pro]
+    a = Int32[pedigree[ID].rank - 1 for ID in ancestors]
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    r = Vector{Int64}(undef, length(a))
+    stats = Ref{GcStats}()
+    GC.@preserve r check(ccall((:genlib_rec, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Int64}, Int32, Ptr{Int32},
+         Ptr{GcStats}),
+        length(father), father, mother, length(p), p, length(a), a, pointer(r), length(devs), devs, stats))
+    r
 end
 
 end # module

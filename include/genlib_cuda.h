@@ -42,6 +42,7 @@ extern "C" {
                            /* being made (genlib_plan_create_async): a size bound did    */
                            /* not hold; destroy the engine, create it again (the plan is */
                            /* finished by then) and run                                  */
+#define GENLIB_EOVERFLOW 8 /* genlib_occ: a path count or row sum does not fit an Int64   */
 
 /* numerics: how the frontier is stored between generation steps */
 #define GENLIB_NUMERICS_REFERENCE 0 /* Float32 storage, Float64 arithmetic, one RN32 per   */
@@ -300,6 +301,8 @@ typedef struct genlib_gc_stats {
     int64_t device_bytes;        /* largest per-device allocation                                   */
     double alg_bytes;            /* required traffic, summed over devices: (input rows read +       */
                                  /* frontier rows written + output rows written) x columns x 8      */
+                                 /* (genlib_rec: x 16-byte-padded 64-column words x 8; the row sums */
+                                 /* of genlib_occ and genlib_rec add one read of the output block)  */
     double ms_plan, ms_kernels, ms_fetch; /* ms_kernels: CUDA events, slowest device                */
     int64_t d2h_bytes;
     int32_t kernel_launches, n_dev;
@@ -327,6 +330,31 @@ int genlib_gc_plan_info(const genlib_gc_plan *plan, genlib_gc_stats *out);
 int genlib_gc_plan_layer(const genlib_gc_plan *plan, int32_t layer, int32_t *n_rows, int64_t *n_inputs);
 int genlib_gc_plan_layer_arrays(const genlib_gc_plan *plan, int32_t layer, int32_t *row_ind, int32_t *row_slot,
                                 int32_t *row_seed, int32_t *row_out, int64_t *in_ptr, int32_t *in_slot);
+
+/* ---- gen.occ / gen.rec: descent-path counts and proband coverage (SURVEY.md 2: src/describe.jl:133-234) --------
+ * The same plan and devices as genlib_gc (GENLIB_GC_DIRECTION applies), with the 1/2 dropped:
+ *   O[a, p] = number of descent paths a -> ... -> p (the empty path when a == p)
+ *           = [p == a] + O[a, father(p)] + O[a, mother(p)]                (a missing parent adds 0)
+ * ROWS ARE ANCESTORS (the transpose of genlib_gc's matrix); duplicates of either list are kept.
+ * Counts are added with saturation at 2^63, which is associative and commutative: every result is bitwise
+ * independent of the direction, the order of the sums and the number of devices.  A returned count or row
+ * sum that does not fit an int64 fails with GENLIB_EOVERFLOW; the message names the smallest offending
+ * (ancestor position, proband position) pair in list order (for a row sum: the ancestor and its first
+ * listed descendant), the same on every run and for every device count.
+ *   GENLIB_OCC_IND:   out = n_anc x n_pro int64, row-major, or column-major when col_major != 0
+ *   GENLIB_OCC_TOTAL: out = n_anc int64, the row sums over the proband list (duplicates counted), reduced on
+ *                     the devices: the matrix never leaves them (col_major is ignored)
+ * genlib_rec: out = n_anc int64, the number of proband list entries that descend from the ancestor, the
+ * ancestor itself included (= count(O[a, :] .> 0)); reachability rows of 64 columns per word, reduced on the
+ * devices; it cannot overflow.  Empty lists give an empty (or zero) result without a device. */
+#define GENLIB_OCC_IND 0
+#define GENLIB_OCC_TOTAL 1
+int genlib_occ(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+               int32_t n_anc, const int32_t *ancestor, int64_t *out, int type, int col_major, int32_t n_dev,
+               const int32_t *devices, genlib_gc_stats *stats);
+int genlib_rec(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+               int32_t n_anc, const int32_t *ancestor, int64_t *out, int32_t n_dev, const int32_t *devices,
+               genlib_gc_stats *stats);
 
 #ifdef __cplusplus
 }
