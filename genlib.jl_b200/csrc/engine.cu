@@ -1,121 +1,28 @@
-// engine.cu -- device runtime + C ABI of libgenlib_cuda.so (include/genlib_cuda.h).
+// engine.cu -- the phi engine and the library-wide part of the C ABI of libgenlib_cuda.so (include/genlib_cuda.h):
+// plans, engines, the one-shot genlib_phi / genlib_phi_multi, errors and caches.  gen.gc, gen.occ and gen.rec are
+// in gc_engine.cu; the host helpers both share are in runtime.hpp.
 //
 // The ABI stands where the reference's Julia method stands:
 //   phi(pedigree, probandIDs; verbose, compute)            src/compute.jl:233-304
 // There is no CPU fallback: without a usable CUDA device every compute entry
 // point returns GENLIB_ECUDA.
-#include <cuda_runtime.h>
-
-#include <algorithm>
-#include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <memory>
-#include <mutex>
-#include <string>
-#include <thread>
-#include <vector>
 
-#include "../../include/genlib_cuda.h"
-#include "gc_kernel.cuh"
-#include "gc_plan.hpp"
 #include "kernels.cuh"
 #include "layer_kernel.cuh"
 #include "plan.hpp"
+#include "runtime.hpp"
 
 using namespace genlib;
 
-namespace {
-
-thread_local std::string g_err;
-
-int fail(int code, const std::string &msg) { g_err = msg; return code; }
-}  // namespace
+thread_local std::string genlib::g_err;
+ArenaCache genlib::g_arenas;
 int genlib::set_error(int code, const std::string &msg) { return fail(code, msg); }
+
 namespace {
-
-#define CU(call)                                                                              \
-    do {                                                                                      \
-        cudaError_t e_ = (call);                                                              \
-        if (e_ != cudaSuccess)                                                                \
-            return fail(e_ == cudaErrorMemoryAllocation ? GENLIB_ENOMEM : GENLIB_ECUDA,       \
-                        std::string(#call) + ": " + cudaGetErrorString(e_));                  \
-    } while (0)
-
-double now_ms() {
-    using namespace std::chrono;
-    return duration<double, std::milli>(steady_clock::now().time_since_epoch()).count();
-}
-
-struct DeviceGuard {
-    int prev = -1;
-    bool active = false;
-    int enter(int dev) {
-        if (cudaGetDevice(&prev) != cudaSuccess) return fail(GENLIB_ECUDA, "no usable CUDA device (cudaGetDevice failed)");
-        if (dev >= 0 && dev != prev) {
-            if (cudaSetDevice(dev) != cudaSuccess) return fail(GENLIB_ECUDA, "cudaSetDevice failed");
-            active = true;
-        }
-        return GENLIB_OK;
-    }
-    ~DeviceGuard() { if (active) cudaSetDevice(prev); }
-};
-
-// ---- device arena: ONE allocation per engine, cached across calls -------------------------
-// cudaMalloc / cudaFree of tens of GB cost hundreds of milliseconds; a repeated gen.phi call
-// (and the one-shot genlib_phi) reuses the previous arena when it is large enough.
-struct Arena {
-    void *base = nullptr;
-    size_t size = 0;
-    int device = -1;
-    bool exported = false;      // a CUDA-IPC handle of it was handed out: peer processes may keep it mapped
-};
-
-class ArenaCache {
-    std::mutex mu_;
-    std::vector<Arena> free_;
-public:
-    cudaError_t acquire(int device, size_t bytes, Arena &out) {
-        {
-            std::lock_guard<std::mutex> g(mu_);
-            int best = -1;
-            for (int i = 0; i < (int)free_.size(); i++)
-                if (free_[i].device == device && free_[i].size >= bytes && (best < 0 || free_[i].size < free_[best].size)) best = i;
-            if (best >= 0) { out = free_[best]; free_.erase(free_.begin() + best); return cudaSuccess; }
-        }
-        // Nothing cached fits.  The smaller cached arenas of this device are given back first (a long-lived
-        // process would otherwise pin one arena per size it ever needed) -- except those a peer process may
-        // still have mapped (CUDA IPC: freeing exported memory under an open mapping is undefined); these go
-        // only when the device is out of memory.
-        release_device(device, /*also_exported=*/false);
-        out = Arena{nullptr, bytes, device, false};
-        cudaError_t ce = cudaMalloc(&out.base, bytes);
-        if (ce == cudaErrorMemoryAllocation) {
-            cudaGetLastError();
-            release_device(device, true);
-            ce = cudaMalloc(&out.base, bytes);
-        }
-        return ce;
-    }
-    void release(Arena a) {
-        if (!a.base) return;
-        std::lock_guard<std::mutex> g(mu_);
-        free_.push_back(a);
-    }
-    void release_device(int device, bool also_exported = true) {
-        std::lock_guard<std::mutex> g(mu_);
-        for (size_t i = 0; i < free_.size();) {
-            if ((device < 0 || free_[i].device == device) && (also_exported || !free_[i].exported)) {
-                int prev = -1; cudaGetDevice(&prev);
-                cudaSetDevice(free_[i].device); cudaFree(free_[i].base);
-                if (prev >= 0) cudaSetDevice(prev);
-                free_.erase(free_.begin() + (long)i);
-            } else i++;
-        }
-    }
-};
-ArenaCache g_arenas;
 
 // cudaIpcOpenMemHandle / CloseMemHandle of multi-GB arenas cost tens of milliseconds per peer.
 // Arenas are cached, so the same handles come back call after call: keep the mappings open.
@@ -148,19 +55,11 @@ public:
 };
 PeerMapCache g_peer_maps;
 
-// non-owning typed view into the arena
-template <typename T> struct DevBuf {
-    T *p = nullptr;
-    size_t n = 0;
-    static size_t padded(size_t count) { return (std::max<size_t>(count, 1) * sizeof(T) + 255) / 256 * 256; }
-    void place(unsigned char *&cursor, size_t count) { p = reinterpret_cast<T *>(cursor); n = count; cursor += padded(count); }
-    cudaError_t upload(const std::vector<T> &h, cudaStream_t s) {
-        if (h.empty()) return cudaSuccess;
-        return cudaMemcpyAsync(p, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, s);
-    }
+// Frees a call's transient device buffer (the caller's pointer, null until allocated) on every way out of the call.
+template <typename T> struct FreeOnExit {
+    T *&p;
+    ~FreeOnExit() { if (p) cudaFree(p); }
 };
-
-constexpr size_t kFetchStageBytes = (size_t)64 << 20;
 
 }  // namespace
 
@@ -174,6 +73,19 @@ struct genlib_plan {
     std::mutex settle_mu;
     int worker_rc = GENLIB_OK;
     std::string worker_err;
+    // build_plan into `p` (published through `ps` when given), with its status, message and time from t0.  Out of
+    // host memory fails the plan like any planner error and closes a streamed one, so that its readers stop waiting.
+    void build(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
+               const int32_t *proband, int32_t world, int schedule, PlanStream *ps, int planners, double t0) {
+        try {
+            adopt_retired_storage(p);        // the arrays of the last destroyed plan, already paged in
+            worker_rc = build_plan(n, father, mother, ids, n_pro, proband, world, schedule, p, worker_err, ps, planners);
+        } catch (const std::bad_alloc &) {
+            worker_rc = GENLIB_ENOMEM; worker_err = "out of host memory while planning";
+            if (ps) { ps->status.store(GENLIB_ENOMEM); ps->stage.store(2); ps->wake(); }
+        }
+        ms_plan = now_ms() - t0;
+    }
     void settle() {
         std::lock_guard<std::mutex> lk(settle_mu);
         if (worker.joinable()) worker.join();
@@ -184,6 +96,20 @@ struct genlib_plan {
     ~genlib_plan() { if (worker.joinable()) worker.join(); }
 };
 inline void settle(const genlib_plan *plan) { if (plan) const_cast<genlib_plan *>(plan)->settle(); }
+
+namespace {
+// A reader of a plan that is still being made (PlanStream::consumers): the planner waits for its readers to stop
+// before it reallocates anything.
+struct StreamConsumer {
+    PlanStream *ps = nullptr;
+    StreamConsumer() = default;
+    explicit StreamConsumer(PlanStream &s) : ps(&s) { ps->consumers.fetch_add(1); }
+    StreamConsumer(const StreamConsumer &) = delete;
+    StreamConsumer &operator=(StreamConsumer &&o) { reset(); ps = o.ps; o.ps = nullptr; return *this; }
+    ~StreamConsumer() { reset(); }
+    void reset() { if (ps) { ps->consumers.fetch_sub(1); ps->wake(); ps = nullptr; } }
+};
+}  // namespace
 
 // launch shape of one layer's persistent kernel (layer_kernel.cuh)
 struct LayerLaunch {
@@ -230,8 +156,7 @@ struct genlib_engine : IndexBufs {
     unsigned epoch = 0;
     long long barrier_timeout = (long long)20e9;   // cycles an inter-GPU barrier may wait (GENLIB_BARRIER_TIMEOUT_S)
     bool streamed = false;                 // built on a plan that was still being made: sized by its bounds, uploaded layer by layer
-    PlanStream *consuming = nullptr;       // registered as a reader of that plan's arrays (until the streamed run ends)
-    void stop_consuming() { if (consuming) { consuming->consumers.fetch_sub(1); consuming->wake(); consuming = nullptr; } }
+    StreamConsumer consuming;              // registered as a reader of that plan's arrays (until the streamed run ends)
     std::vector<int32_t> own_pro;          // proband indices (output rows) this rank owns, ascending
     std::vector<genlib_layer_info> info;
     std::vector<cudaEvent_t> events;
@@ -239,7 +164,7 @@ struct genlib_engine : IndexBufs {
     bool ran = false;
     int32_t layer_limit = -1;
     ~genlib_engine() {
-        stop_consuming();
+        consuming.reset();
         for (auto e : events) cudaEventDestroy(e);
         if (stream) cudaStreamSynchronize(stream);
         if (copy_stream) cudaStreamSynchronize(copy_stream);
@@ -257,8 +182,6 @@ void fill_info(const Layer &L, genlib_layer_info *o) {
     o->ref_founders = L.ref_founders; o->ref_probands = L.ref_probands; o->ref_both = L.ref_both;
     o->alg_elems = L.alg_elems;
 }
-
-size_t pad256(size_t b) { return (std::max<size_t>(b, 1) + 255) / 256 * 256; }
 
 size_t plan_index_bytes(const Plan &P) {
     return (P.mem_ind.size() * 4 + P.mem_rank.size() + P.fam_pf.size() * 6 + P.fam_start.size() + P.mtile_desc.size() +
@@ -610,38 +533,22 @@ int fetch_rows(genlib_engine &E, O *out) {
     const Plan &P = E.plan->p;
     const int32_t n = P.n_unique, nown = (int32_t)E.own_pro.size();
     if (n == 0 || nown == 0) return GENLIB_OK;
-    // stream row blocks through two staging buffers so the gather of block b+1
-    // overlaps the D2H copy of block b
     const size_t row_bytes = (size_t)n * sizeof(O);
     int32_t rows_per = (int32_t)std::max<size_t>(1, std::min<size_t>((size_t)nown, kFetchStageBytes / row_bytes));
     if ((size_t)rows_per * row_bytes > kFetchStageBytes) return fail(GENLIB_EINVAL, "proband row does not fit the staging buffer");
     rows_per = std::min(rows_per, 65535);
-    O *stage[2] = {reinterpret_cast<O *>(E.fetch_stage[0]), reinterpret_cast<O *>(E.fetch_stage[1])};
-    cudaEvent_t done[2] = {nullptr, nullptr}, copied[2] = {nullptr, nullptr};
-    cudaError_t ce = cudaSuccess;
-    for (int b = 0; b < 2 && ce == cudaSuccess; b++) {
-        ce = cudaEventCreateWithFlags(&done[b], cudaEventDisableTiming);
-        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&copied[b], cudaEventDisableTiming);
-    }
-    int blk = 0;
-    for (int32_t r0 = 0; r0 < nown && ce == cudaSuccess; r0 += rows_per, blk++) {
-        const int b = blk & 1;
-        const int32_t nr = std::min(rows_per, nown - r0);
-        if (blk >= 2 && (ce = cudaStreamWaitEvent(E.stream, copied[b], 0)) != cudaSuccess) break;
-        dim3 grid((unsigned)std::min<int32_t>((n + 255) / 256, 64), (unsigned)nr);
-        gather_kernel<T, O><<<grid, 256, 0, E.stream>>>(static_cast<const T *>(E.A), P.capacity, E.own_pro_row.p, E.pro_slot.p,
-                                                       n, r0, nr, stage[b]);
-        cudaEventRecord(done[b], E.stream);
-        cudaStreamWaitEvent(E.copy_stream, done[b], 0);
-        ce = cudaMemcpyAsync(out + (size_t)r0 * n, stage[b], (size_t)nr * row_bytes, cudaMemcpyDeviceToHost, E.copy_stream);
-        cudaEventRecord(copied[b], E.copy_stream);
-    }
-    const cudaError_t e1 = cudaStreamSynchronize(E.stream), e2 = cudaStreamSynchronize(E.copy_stream);
-    for (int b = 0; b < 2; b++) { if (done[b]) cudaEventDestroy(done[b]); if (copied[b]) cudaEventDestroy(copied[b]); }
-    if (ce != cudaSuccess || e1 != cudaSuccess || e2 != cudaSuccess)
-        return fail(GENLIB_ECUDA, std::string("proband fetch failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : e1 != cudaSuccess ? e1 : e2));
-    E.stats.d2h_bytes += (int64_t)nown * (int64_t)row_bytes;
-    return GENLIB_OK;
+    int rc = staged_d2h(E.stream, E.copy_stream, reinterpret_cast<O *>(E.fetch_stage[0]), reinterpret_cast<O *>(E.fetch_stage[1]),
+                        nown, rows_per, "proband fetch",
+        [&](O *stage, int64_t r0, int64_t nr) {
+            dim3 grid((unsigned)std::min<int32_t>((n + 255) / 256, 64), (unsigned)nr);
+            gather_kernel<T, O><<<grid, 256, 0, E.stream>>>(static_cast<const T *>(E.A), P.capacity, E.own_pro_row.p, E.pro_slot.p,
+                                                           n, (int32_t)r0, (int32_t)nr, stage);
+        },
+        [&](const O *stage, int64_t r0, int64_t nr) {
+            return cudaMemcpyAsync(out + (size_t)r0 * n, stage, (size_t)nr * row_bytes, cudaMemcpyDeviceToHost, E.copy_stream);
+        });
+    if (rc == GENLIB_OK) E.stats.d2h_bytes += (int64_t)nown * (int64_t)row_bytes;
+    return rc;
 }
 
 // Output rows [u0, u1) of the proband matrix, whoever owns them (peer reads), to host memory at their
@@ -655,31 +562,18 @@ int fetch_block(genlib_engine &E, int32_t u0, int32_t u1, O *out) {
     int32_t rows_per = (int32_t)std::max<size_t>(1, std::min<size_t>((size_t)(u1 - u0), kFetchStageBytes / row_bytes));
     if ((size_t)rows_per * row_bytes > kFetchStageBytes) return fail(GENLIB_EINVAL, "proband row does not fit the staging buffer");
     rows_per = std::min(rows_per, 65535);
-    O *stage[2] = {reinterpret_cast<O *>(E.fetch_stage[0]), reinterpret_cast<O *>(E.fetch_stage[1])};
-    cudaEvent_t done[2] = {nullptr, nullptr}, copied[2] = {nullptr, nullptr};
-    cudaError_t ce = cudaSuccess;
-    for (int b = 0; b < 2 && ce == cudaSuccess; b++) {
-        ce = cudaEventCreateWithFlags(&done[b], cudaEventDisableTiming);
-        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&copied[b], cudaEventDisableTiming);
-    }
-    int blk = 0;
-    for (int32_t r0 = u0; r0 < u1 && ce == cudaSuccess; r0 += rows_per, blk++) {
-        const int b = blk & 1;
-        const int32_t nr = std::min(rows_per, u1 - r0);
-        if (blk >= 2 && (ce = cudaStreamWaitEvent(E.stream, copied[b], 0)) != cudaSuccess) break;
-        dim3 grid((unsigned)std::min<int32_t>((n + 255) / 256, 64), (unsigned)nr);
-        gather_peer_kernel<T, O><<<grid, 256, 0, E.stream>>>(E.peers, P.capacity, E.pro_owner.p, E.pro_lrow.p, E.pro_slot.p, n, r0, nr, stage[b]);
-        cudaEventRecord(done[b], E.stream);
-        cudaStreamWaitEvent(E.copy_stream, done[b], 0);
-        ce = cudaMemcpyAsync(out + (size_t)r0 * n, stage[b], (size_t)nr * row_bytes, cudaMemcpyDeviceToHost, E.copy_stream);
-        cudaEventRecord(copied[b], E.copy_stream);
-    }
-    const cudaError_t e1 = cudaStreamSynchronize(E.stream), e2 = cudaStreamSynchronize(E.copy_stream);
-    for (int b = 0; b < 2; b++) { if (done[b]) cudaEventDestroy(done[b]); if (copied[b]) cudaEventDestroy(copied[b]); }
-    if (ce != cudaSuccess || e1 != cudaSuccess || e2 != cudaSuccess)
-        return fail(GENLIB_ECUDA, std::string("proband fetch failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : e1 != cudaSuccess ? e1 : e2));
-    E.stats.d2h_bytes += (int64_t)(u1 - u0) * (int64_t)row_bytes;
-    return GENLIB_OK;
+    int rc = staged_d2h(E.stream, E.copy_stream, reinterpret_cast<O *>(E.fetch_stage[0]), reinterpret_cast<O *>(E.fetch_stage[1]),
+                        u1 - u0, rows_per, "proband fetch",
+        [&](O *stage, int64_t i0, int64_t nr) {
+            dim3 grid((unsigned)std::min<int32_t>((n + 255) / 256, 64), (unsigned)nr);
+            gather_peer_kernel<T, O><<<grid, 256, 0, E.stream>>>(E.peers, P.capacity, E.pro_owner.p, E.pro_lrow.p, E.pro_slot.p, n,
+                                                                u0 + (int32_t)i0, (int32_t)nr, stage);
+        },
+        [&](const O *stage, int64_t i0, int64_t nr) {
+            return cudaMemcpyAsync(out + (size_t)(u0 + i0) * n, stage, (size_t)nr * row_bytes, cudaMemcpyDeviceToHost, E.copy_stream);
+        });
+    if (rc == GENLIB_OK) E.stats.d2h_bytes += (int64_t)(u1 - u0) * (int64_t)row_bytes;
+    return rc;
 }
 
 // Compulsory traffic of every layer on this rank (genlib_layer_info), from the plan.
@@ -806,17 +700,13 @@ int create_engine(const genlib_plan *plan, int numerics, int device, int rank, g
     CU(cudaStreamCreateWithFlags(&E->stream, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&E->copy_stream, cudaStreamNonBlocking));
     {
-        cudaError_t ce = g_arenas.acquire(E->device, need, E->arena);
-        if (ce != cudaSuccess) {
-            E->arena = Arena();
-            cudaGetLastError();
-            size_t free_b = 0, total_b = 0;
-            cudaMemGetInfo(&free_b, &total_b);
-            char msg[256];
-            std::snprintf(msg, sizeof msg, "rank %d needs %.2f GB on the device, %.2f GB free (capacity %lld slots, %lld rows): shard over more GPUs",
-                          rank, need / 1e9, free_b / 1e9, (long long)P.capacity, (long long)P.rows_cap[rank]);
-            return fail(GENLIB_ENOMEM, msg);
-        }
+        if (int rc = acquire_arena(E->device, need, E->arena, [&](size_t free_b) {
+                char msg[256];
+                std::snprintf(msg, sizeof msg, "rank %d needs %.2f GB on the device, %.2f GB free (capacity %lld slots, %lld rows): shard over more GPUs",
+                              rank, need / 1e9, free_b / 1e9, (long long)P.capacity, (long long)P.rows_cap[rank]);
+                return std::string(msg);
+            }))
+            return rc;
         unsigned char *base = static_cast<unsigned char *>(E->arena.base), *cur = base;
         auto take = [&](size_t bytes) { unsigned char *p = cur; cur += pad256(bytes); return p; };
         E->bar_flags = reinterpret_cast<unsigned *>(take(kFlagBytes));
@@ -923,17 +813,8 @@ int genlib_plan_create_ex(int32_t n, const int32_t *father, const int32_t *mothe
     *out = nullptr;
     std::unique_ptr<genlib_plan> pl(new (std::nothrow) genlib_plan);
     if (!pl) return fail(GENLIB_ENOMEM, "out of host memory");
-    const double t0 = now_ms();
-    std::string err;
-    int rc;
-    try {
-        adopt_retired_storage(pl->p);        // the arrays of the last destroyed plan, already paged in
-        rc = build_plan(n, father, mother, ids, n_pro, proband, world, schedule, pl->p, err);
-    } catch (const std::bad_alloc &) {
-        return fail(GENLIB_ENOMEM, "out of host memory while planning");
-    }
-    if (rc != GENLIB_OK) return fail(rc, err);
-    pl->ms_plan = now_ms() - t0;
+    pl->build(n, father, mother, ids, n_pro, proband, world, schedule, nullptr, 0, now_ms());
+    if (pl->worker_rc != GENLIB_OK) return fail(pl->worker_rc, pl->worker_err);
     *out = pl.release();
     return GENLIB_OK;
 }
@@ -950,16 +831,7 @@ int genlib_plan_create_async(int32_t n, const int32_t *father, const int32_t *mo
     genlib_plan *raw = pl.get();
     const double t0 = now_ms();
     try {
-        raw->worker = std::thread([=] {
-            try {
-                adopt_retired_storage(raw->p);
-                raw->worker_rc = build_plan(n, father, mother, ids, n_pro, proband, world, schedule, raw->p, raw->worker_err, raw->stream.get());
-            } catch (const std::bad_alloc &) {
-                raw->worker_rc = GENLIB_ENOMEM; raw->worker_err = "out of host memory while planning";
-                raw->stream->status.store(GENLIB_ENOMEM); raw->stream->stage.store(2); raw->stream->wake();
-            }
-            raw->ms_plan = now_ms() - t0;
-        });
+        raw->worker = std::thread([=] { raw->build(n, father, mother, ids, n_pro, proband, world, schedule, raw->stream.get(), 0, t0); });
     } catch (...) {                              // no thread to be had
         pl.reset();
         return genlib_plan_create_ex(n, father, mother, ids, n_pro, proband, world, schedule, out);
@@ -1129,13 +1001,12 @@ int genlib_plan_proband_slots(const genlib_plan *plan, int32_t *slots) {
 static int create_engine_public(const genlib_plan *plan, int numerics, int device, int rank, genlib_engine **out) {
     if (plan && plan->streaming()) {
         PlanStream &ps = *plan->stream;
-        ps.consumers.fetch_add(1);
+        StreamConsumer reader(ps);
         if (!ps.overflow.load() && ps.stage.load() != 2) {
             int rc = create_engine(plan, numerics, device, rank, out, true);
-            if (rc == GENLIB_OK) { (*out)->consuming = &ps; return rc; }
-            ps.consumers.fetch_sub(1); ps.wake();
+            if (rc == GENLIB_OK) { (*out)->consuming = std::move(reader); return rc; }
             if (rc != GENLIB_ENOMEM) return rc;             // (the bounds did not fit: size by the finished plan)
-        } else { ps.consumers.fetch_sub(1); ps.wake(); }
+        }
     }
     settle(plan);
     if (plan && plan->worker_rc != GENLIB_OK) return fail(plan->worker_rc, plan->worker_err);
@@ -1205,10 +1076,10 @@ int genlib_engine_run(genlib_engine *eng, int time_layers) {
     genlib_engine &E = *eng;
     if (!E.attached) return fail(GENLIB_ECOMM, "genlib_engine_run before genlib_engine_ipc_attach");
     if (E.streamed && !E.ran) {                                 // first run on a plan that is still being made
-        if (!E.consuming) return fail(GENLIB_ERESTART, "the streamed plan's bounds did not hold: create the engine again");
-        PlanStream &ps = *E.consuming;
+        if (!E.consuming.ps) return fail(GENLIB_ERESTART, "the streamed plan's bounds did not hold: create the engine again");
+        PlanStream &ps = *E.consuming.ps;
         int rc = E.numerics == GENLIB_NUMERICS_FP64 ? run_streamed<double>(E, ps) : run_streamed<float>(E, ps);
-        E.stop_consuming();
+        E.consuming.reset();
         settle(E.plan);
         if (rc == kRestart) return fail(GENLIB_ERESTART, "a size bound of the streamed plan did not hold: destroy this engine, create it again and run");
         if (rc != GENLIB_OK) return rc == E.plan->worker_rc ? fail(rc, E.plan->worker_err) : rc;
@@ -1284,8 +1155,10 @@ int genlib_engine_row_sums(genlib_engine *eng, double *out) {
     if (nown == 0) return GENLIB_OK;
     double *dsum = nullptr;
     int32_t *didx = nullptr;
+    FreeOnExit<double> free_sum{dsum};
+    FreeOnExit<int32_t> free_idx{didx};
     CU(cudaMalloc(&dsum, (size_t)nown * 2 * sizeof(double)));
-    if (cudaMalloc(&didx, (size_t)nown * sizeof(int32_t)) != cudaSuccess) { cudaFree(dsum); return fail(GENLIB_ENOMEM, "out of device memory"); }
+    if (cudaMalloc(&didx, (size_t)nown * sizeof(int32_t)) != cudaSuccess) return fail(GENLIB_ENOMEM, "out of device memory");
     cudaError_t ce = cudaMemcpyAsync(didx, eng->own_pro.data(), (size_t)nown * sizeof(int32_t), cudaMemcpyHostToDevice, eng->stream);
     if (ce == cudaSuccess) {
         if (eng->numerics == GENLIB_NUMERICS_FP64)
@@ -1295,7 +1168,6 @@ int genlib_engine_row_sums(genlib_engine *eng, double *out) {
         ce = cudaMemcpyAsync(out, dsum, (size_t)nown * 2 * sizeof(double), cudaMemcpyDeviceToHost, eng->stream);
     }
     const cudaError_t e2 = cudaStreamSynchronize(eng->stream);
-    cudaFree(dsum); cudaFree(didx);
     if (ce != cudaSuccess || e2 != cudaSuccess) return fail(GENLIB_ECUDA, std::string("row sums: ") + cudaGetErrorString(ce != cudaSuccess ? ce : e2));
     return GENLIB_OK;
 }
@@ -1330,6 +1202,8 @@ int genlib_engine_read_block(genlib_engine *eng, int32_t n_slots, const int32_t 
         if (slots[i] < 0 || slots[i] >= P.capacity) return fail(GENLIB_EINVAL, "slot out of range");
     int32_t *dslots = nullptr;
     double *dout = nullptr;
+    FreeOnExit<int32_t> free_slots{dslots};
+    FreeOnExit<double> free_out{dout};
     CU(cudaMalloc(&dslots, (size_t)n_slots * sizeof(int32_t)));
     CU(cudaMalloc(&dout, (size_t)n_slots * n_slots * sizeof(double)));
     CU(cudaMemcpyAsync(dslots, slots, (size_t)n_slots * sizeof(int32_t), cudaMemcpyHostToDevice, eng->stream));
@@ -1343,89 +1217,69 @@ int genlib_engine_read_block(genlib_engine *eng, int32_t n_slots, const int32_t 
     }
     CU(cudaMemcpyAsync(out, dout, (size_t)n_slots * n_slots * sizeof(double), cudaMemcpyDeviceToHost, eng->stream));
     CU(cudaStreamSynchronize(eng->stream));
-    cudaFree(dslots); cudaFree(dout);
     return GENLIB_OK;
 }
 
-int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
-                     const int32_t *proband, void *out, int out_dtype, int numerics, int32_t n_dev,
-                     const int32_t *devices, genlib_stats *stats) {
-    if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_multi: 1 .. 16 devices");
+// genlib_phi and genlib_phi_multi: ONE plan for all devices, made on a worker thread and handed over layer by layer
+// (PlanStream), so that the devices run the first generations while the later ones are planned.  GENLIB_STREAM=0, or
+// a bound of the streamed plan that did not hold, plans first and then runs.  One device runs on the calling thread;
+// several get a host thread each, NVLink peer access, and fetch a contiguous block of output rows each.
+static int phi_oneshot(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                       void *out, int out_dtype, int numerics, int32_t n_dev, const int32_t *devices, genlib_stats *stats) {
     if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
-    if (n_dev == 1) return genlib_phi(n, father, mother, n_pro, proband, out, out_dtype, numerics, devices[0], stats);
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(GENLIB_ECUDA, "no CUDA device: libgenlib_cuda has no CPU fallback");
-    for (int g = 0; g < n_dev; g++) {
-        if (devices[g] < 0 || devices[g] >= ndev) return fail(GENLIB_EINVAL, "genlib_phi_multi: no such device");
-        for (int h = 0; h < g; h++) if (devices[h] == devices[g]) return fail(GENLIB_EINVAL, "genlib_phi_multi: a device is listed twice");
-    }
-    // ONE plan for all ranks, made on a worker thread and handed over layer by layer (see genlib_phi)
+    const bool multi = n_dev > 1;
+    const std::string who = multi ? "genlib_phi_multi" : "genlib_phi";
+    std::vector<int> dev(devices, devices + n_dev);              // (one device: a negative one is the current device)
+    if (int rc = multi ? resolve_devices(who, n_dev, devices, false, dev) : GENLIB_OK) return rc;
     std::unique_ptr<genlib_plan> plan_owner(new (std::nothrow) genlib_plan);
     if (!plan_owner) return fail(GENLIB_ENOMEM, "out of host memory");
     genlib_plan *plan = plan_owner.get();
     const bool want_stream = env_int("GENLIB_STREAM", 1) != 0 && out != nullptr;
     const double tp0 = now_ms();
     PlanStream ps;
-    int plan_rc = GENLIB_OK;
-    std::string plan_err;
     auto make_plan = [&](PlanStream *stream) {
-        try {
-            adopt_retired_storage(plan->p);
-            plan_rc = build_plan(n, father, mother, nullptr, n_pro, proband, n_dev, GENLIB_SCHEDULE_PHI, plan->p, plan_err, stream, /*planners=*/1);
-        } catch (const std::bad_alloc &) {
-            plan_rc = GENLIB_ENOMEM; plan_err = "out of host memory while planning";
-            if (stream) { stream->status.store(plan_rc); stream->stage.store(2); stream->wake(); }
-        }
-        plan->ms_plan = now_ms() - tp0;
+        plan->build(n, father, mother, nullptr, n_pro, proband, n_dev, GENLIB_SCHEDULE_PHI, stream, /*planners=*/1, tp0);
     };
-    std::thread worker;
-    if (want_stream) { try { worker = std::thread([&] { make_plan(&ps); }); } catch (...) { } }
-    const bool streaming = worker.joinable();
-    if (!streaming) make_plan(nullptr);
-    // (destruction order: consumer registration, engines, worker joined, plan storage retired)
-    struct PlanRetire { genlib_plan *p; ~PlanRetire() { try { retire_storage(p->p); } catch (...) {} } } retire{plan};
-    struct Joiner { std::thread &t; ~Joiner() { if (t.joinable()) t.join(); } } joiner{worker};   // (joins before the plan is retired)
+    if (want_stream) { try { plan->worker = std::thread([&] { make_plan(&ps); }); } catch (...) { } }
+    const bool streaming = plan->worker.joinable();
+    if (!streaming) make_plan(nullptr);                         // (no thread to be had: plan here)
+    // (destruction order: consumer registration, engines, worker joined and plan storage retired)
+    struct PlanRetire { genlib_plan *p; ~PlanRetire() { p->settle(); try { retire_storage(p->p); } catch (...) {} } } retire{plan};
     std::vector<genlib_engine *> eng((size_t)n_dev, nullptr);
     struct EngGuard { std::vector<genlib_engine *> &e; ~EngGuard() { for (auto *&x : e) { genlib_engine_destroy(x); x = nullptr; } } } eguard{eng};
-    int prev_dev = -1;
-    cudaGetDevice(&prev_dev);
-    struct DevRestore { int d; ~DevRestore() { if (d >= 0) cudaSetDevice(d); } } restore{prev_dev};
-    // every device sees every other device's memory (NVLink peer access) -- while the planner's pre-pass runs
+    struct DevRestore { int d = -1; ~DevRestore() { if (d >= 0) cudaSetDevice(d); } } restore;
     int peer_rc = GENLIB_OK;
-    for (int g = 0; g < n_dev && peer_rc == GENLIB_OK; g++) {
-        if (cudaSetDevice(devices[g]) != cudaSuccess) { peer_rc = fail(GENLIB_ECUDA, "cudaSetDevice failed"); break; }
-        for (int h = 0; h < n_dev; h++) {
-            if (h == g) continue;
-            int can = 0;
-            cudaDeviceCanAccessPeer(&can, devices[g], devices[h]);
-            if (!can) { peer_rc = fail(GENLIB_ECOMM, "devices " + std::to_string(devices[g]) + " and " + std::to_string(devices[h]) + " have no peer access"); break; }
-            const cudaError_t ce = cudaDeviceEnablePeerAccess(devices[h], 0);
-            if (ce != cudaSuccess && ce != cudaErrorPeerAccessAlreadyEnabled) { peer_rc = fail(GENLIB_ECOMM, std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(ce)); break; }
-            cudaGetLastError();
+    if (multi) {                 // every device sees every other device's memory -- while the planner's pre-pass runs
+        cudaGetDevice(&restore.d);
+        for (int g = 0; g < n_dev && peer_rc == GENLIB_OK; g++) {
+            if (cudaSetDevice(dev[g]) != cudaSuccess) { peer_rc = fail(GENLIB_ECUDA, "cudaSetDevice failed"); break; }
+            for (int h = 0; h < n_dev; h++) {
+                if (h == g) continue;
+                int can = 0;
+                cudaDeviceCanAccessPeer(&can, dev[g], dev[h]);
+                if (!can) { peer_rc = fail(GENLIB_ECOMM, "devices " + std::to_string(dev[g]) + " and " + std::to_string(dev[h]) + " have no peer access"); break; }
+                const cudaError_t ce = cudaDeviceEnablePeerAccess(dev[h], 0);
+                if (ce != cudaSuccess && ce != cudaErrorPeerAccessAlreadyEnabled) { peer_rc = fail(GENLIB_ECOMM, std::string("cudaDeviceEnablePeerAccess: ") + cudaGetErrorString(ce)); break; }
+                cudaGetLastError();
+            }
         }
     }
-    // one host thread per device
-    std::vector<int> status((size_t)n_dev, GENLIB_OK);
-    std::vector<std::string> message((size_t)n_dev);
-    auto run_all = [&](auto &&fn) {                              // statuses stay in `status`
-        std::vector<std::thread> th;
-        for (int g = 0; g < n_dev; g++)
-            th.emplace_back([&, g] { status[(size_t)g] = fn(g); if (status[(size_t)g] != GENLIB_OK) message[(size_t)g] = g_err; });
-        for (auto &t : th) t.join();
-    };
-    auto first_error = [&](bool restart_is_error) {              // GENLIB_OK, kRestart (nothing worse happened) or an error
+    // GENLIB_OK, kRestart (a bound did not hold or did not fit, and nothing worse happened) or the first error
+    auto first_error = [&](const std::vector<DeviceStatus> &r, bool restart_is_error) {
         int rc2 = GENLIB_OK;
         for (int g = 0; g < n_dev; g++) {
-            const int st = status[(size_t)g];
+            const int st = r[(size_t)g].status;
             if (st == GENLIB_OK) continue;
             if ((st == kRestart || st == GENLIB_ENOMEM) && !restart_is_error) { if (rc2 == GENLIB_OK) rc2 = kRestart; continue; }
-            return fail(st, "device " + std::to_string(devices[g]) + ": " + message[(size_t)g]);
+            return fail(st, multi ? "device " + std::to_string(dev[g]) + ": " + r[(size_t)g].message : r[(size_t)g].message);
         }
         return rc2;
     };
-    auto on_all = [&](auto &&fn) { run_all(fn); return first_error(true); };
+    auto create_all = [&](bool streamed) {
+        return on_devices(n_dev, [&](int g) { return create_engine(plan, numerics, dev[g], g, &eng[(size_t)g], streamed); });
+    };
     auto wire_peers = [&]() {                                    // plain peer pointers instead of IPC mappings
+        if (!multi) return;
         for (int g = 0; g < n_dev; g++) {
             for (int h = 0; h < n_dev; h++) { eng[(size_t)g]->peers.A[h] = eng[(size_t)h]->A; eng[(size_t)g]->bars.flags[h] = eng[(size_t)h]->bar_flags; }
             eng[(size_t)g]->attached = true;
@@ -1436,17 +1290,12 @@ int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, in
     if (streaming) {
         ps.wait([&] { return ps.stage.load() >= 1; });
         if (peer_rc == GENLIB_OK && ps.streamed.load() && plan->p.n_unique > 0) {
-            struct Consumer {                                     // one registration for all device threads
-                PlanStream &s;
-                explicit Consumer(PlanStream &st) : s(st) { s.consumers.fetch_add(1); }
-                ~Consumer() { s.consumers.fetch_sub(1); s.wake(); }
-            } consumer(ps);
+            StreamConsumer consumer(ps);                          // one registration for all devices
             if (!ps.overflow.load()) {
-                run_all([&](int g) { return create_engine(plan, numerics, devices[g], g, &eng[(size_t)g], true); });
-                rc = first_error(false);
+                rc = first_error(create_all(true), false);
                 if (rc == GENLIB_OK) {
                     wire_peers();
-                    run_all([&](int g) {
+                    rc = first_error(on_devices(n_dev, [&](int g) {
                         genlib_engine &E = *eng[(size_t)g];
                         DeviceGuard guard;
                         if (int r = guard.enter(E.device)) return r;
@@ -1454,35 +1303,33 @@ int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, in
                         if (r == GENLIB_OK) r = check_device_errors(E);
                         if (r == GENLIB_OK) E.ran = true;
                         return r;
-                    });
-                    rc = first_error(false);
+                    }), false);
                     done = rc == GENLIB_OK;
                 }
                 if (rc == kRestart) rc = GENLIB_OK;
             }
         }
-        worker.join();
+        plan->settle();
     }
-    if (plan_rc != GENLIB_OK) return fail(plan_rc, plan_err);
+    if (plan->worker_rc != GENLIB_OK) return fail(plan->worker_rc, plan->worker_err);
     if (peer_rc != GENLIB_OK) return peer_rc;
     if (rc != GENLIB_OK) return rc;
     if (plan->p.n_unique == 0) {
         if (stats) { std::memset(stats, 0, sizeof *stats); stats->ms_plan = plan->ms_plan; }
-        return GENLIB_OK;
+        return GENLIB_OK;                                         // 0 x 0 matrix, like the reference
     }
-    if (!out) return fail(GENLIB_EINVAL, "genlib_phi_multi: out is null");
+    if (!out) return fail(GENLIB_EINVAL, who + ": out is null");
     if (!done) {                                                // plan first, then run (no streaming, or its bounds did not hold)
         for (auto *&x : eng) { genlib_engine_destroy(x); x = nullptr; }
-        rc = on_all([&](int g) { return create_engine(plan, numerics, devices[g], g, &eng[(size_t)g]); });
-        if (rc != GENLIB_OK) return rc;
+        if ((rc = first_error(create_all(false), true)) != GENLIB_OK) return rc;
         wire_peers();
-        rc = on_all([&](int g) { return genlib_engine_run(eng[(size_t)g], 0); });
-        if (rc != GENLIB_OK) return rc;
+        if ((rc = first_error(on_devices(n_dev, [&](int g) { return genlib_engine_run(eng[(size_t)g], 0); }), true)) != GENLIB_OK) return rc;
     }
     for (auto *x : eng) x->stats.ms_plan = plan->ms_plan;
     const int32_t nu = plan->p.n_unique;
     const double t0 = now_ms();
-    rc = on_all([&](int g) {                                    // contiguous row blocks, one PCIe link each
+    if (!multi) rc = genlib_engine_fetch(eng[0], out, out_dtype);
+    else rc = first_error(on_devices(n_dev, [&](int g) {        // contiguous row blocks, one PCIe link each
         genlib_engine &E = *eng[(size_t)g];
         DeviceGuard guard;
         if (int r = guard.enter(E.device)) return r;
@@ -1490,11 +1337,11 @@ int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, in
         if (numerics == GENLIB_NUMERICS_FP64)
             return out_dtype == GENLIB_F64 ? fetch_block<double, double>(E, u0, u1, (double *)out) : fetch_block<double, float>(E, u0, u1, (float *)out);
         return out_dtype == GENLIB_F64 ? fetch_block<float, double>(E, u0, u1, (double *)out) : fetch_block<float, float>(E, u0, u1, (float *)out);
-    });
+    }), true);
     if (rc != GENLIB_OK) return rc;
     if (stats) {
         *stats = eng[0]->stats;
-        stats->ms_fetch = now_ms() - t0;
+        if (multi) stats->ms_fetch = now_ms() - t0;             // (one device: genlib_engine_fetch's own time)
         for (int g = 1; g < n_dev; g++) {
             stats->ms_kernels = std::max(stats->ms_kernels, eng[(size_t)g]->stats.ms_kernels);
             stats->ms_upload = std::max(stats->ms_upload, eng[(size_t)g]->stats.ms_upload);
@@ -1507,80 +1354,18 @@ int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, in
     return GENLIB_OK;
 }
 
+int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
+                     const int32_t *proband, void *out, int out_dtype, int numerics, int32_t n_dev,
+                     const int32_t *devices, genlib_stats *stats) {
+    if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_multi: 1 .. 16 devices");
+    return phi_oneshot(n, father, mother, n_pro, proband, out, out_dtype, numerics, n_dev, devices, stats);
+}
+
 int genlib_phi(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
                const int32_t *proband, void *out, int out_dtype, int numerics, int device,
                genlib_stats *stats) {
-    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
-    // The plan is made on a worker thread and handed over layer by layer (PlanStream): the device runs the first
-    // generations while the later ones are planned.  GENLIB_STREAM=0: plan first, then run.
-    std::unique_ptr<genlib_plan> pl(new (std::nothrow) genlib_plan);
-    if (!pl) return fail(GENLIB_ENOMEM, "out of host memory");
-    const bool want_stream = env_int("GENLIB_STREAM", 1) != 0 && out != nullptr;
-    const double t0 = now_ms();
-    PlanStream ps;
-    int plan_rc = GENLIB_OK;
-    std::string plan_err;
-    auto make_plan = [&](PlanStream *stream) {
-        try {
-            adopt_retired_storage(pl->p);        // the arrays of the last destroyed plan, already paged in
-            plan_rc = build_plan(n, father, mother, nullptr, n_pro, proband, 1, GENLIB_SCHEDULE_PHI, pl->p, plan_err, stream);
-        } catch (const std::bad_alloc &) {
-            plan_rc = GENLIB_ENOMEM; plan_err = "out of host memory while planning";
-            if (stream) { stream->status.store(plan_rc); stream->stage.store(2); stream->wake(); }
-        }
-        pl->ms_plan = now_ms() - t0;
-    };
-    genlib_engine *eng = nullptr;
-    struct EngGuard { genlib_engine *&e; ~EngGuard() { genlib_engine_destroy(e); e = nullptr; } } eguard{eng};
-    int rc = GENLIB_OK;
-    bool done = false;
-    if (want_stream) {
-        std::thread worker;
-        try { worker = std::thread([&] { make_plan(&ps); }); } catch (...) { }
-        if (!worker.joinable()) make_plan(nullptr);               // no thread to be had: plan here
-        else {
-            struct Joiner { std::thread &t; ~Joiner() { if (t.joinable()) t.join(); } } joiner{worker};
-            ps.wait([&] { return ps.stage.load() >= 1; });
-            if (ps.streamed.load() && pl->p.n_unique > 0) {
-                struct Consumer {                                 // the planner waits for us before it reallocates anything
-                    PlanStream &s;
-                    explicit Consumer(PlanStream &st) : s(st) { s.consumers.fetch_add(1); }
-                    ~Consumer() { s.consumers.fetch_sub(1); s.wake(); }
-                } consumer(ps);
-                if (!ps.overflow.load()) {
-                    rc = create_engine(pl.get(), numerics, device, 0, &eng, true);
-                    if (rc == GENLIB_OK) {
-                        DeviceGuard guard;
-                        rc = guard.enter(eng->device);
-                        if (rc == GENLIB_OK) rc = numerics == GENLIB_NUMERICS_FP64 ? run_streamed<double>(*eng, ps) : run_streamed<float>(*eng, ps);
-                        if (rc == GENLIB_OK) rc = check_device_errors(*eng);
-                        if (rc == GENLIB_OK) { eng->ran = true; done = true; }
-                    }
-                    if (rc == kRestart || rc == GENLIB_ENOMEM) rc = GENLIB_OK;   // the bounds did not hold (or did not fit): run on the finished plan
-                }
-            }
-        }                                                         // (consumer released, worker joined)
-    } else make_plan(nullptr);
-    if (plan_rc != GENLIB_OK) return fail(plan_rc, plan_err);
-    if (rc != GENLIB_OK) return rc;
-    if (pl->p.n_unique == 0) {
-        if (stats) { std::memset(stats, 0, sizeof *stats); stats->ms_plan = pl->ms_plan; }
-        return GENLIB_OK;                       // 0 x 0 matrix, like the reference
-    }
-    if (!out) return fail(GENLIB_EINVAL, "genlib_phi: out is null");
-    if (!done) {
-        genlib_engine_destroy(eng); eng = nullptr;
-        rc = create_engine(pl.get(), numerics, device, 0, &eng);
-        if (rc != GENLIB_OK) return rc;
-        rc = genlib_engine_run(eng, 0);
-        if (rc != GENLIB_OK) return rc;
-    }
-    eng->stats.ms_plan = pl->ms_plan;
-    rc = genlib_engine_fetch(eng, out, out_dtype);
-    if (rc == GENLIB_OK && stats) *stats = eng->stats;
-    genlib_engine_destroy(eng); eng = nullptr;                    // before the plan it refers to
-    try { retire_storage(pl->p); } catch (...) {}
-    return rc;
+    const int32_t dev = device;
+    return phi_oneshot(n, father, mother, n_pro, proband, out, out_dtype, numerics, 1, &dev, stats);
 }
 
 int genlib_plan_stream_selftest(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
@@ -1665,517 +1450,6 @@ int genlib_plan_stream_selftest(int32_t n, const int32_t *father, const int32_t 
         if (kept_bound ? P.rows_cap[(size_t)g] < ref.rows_cap[(size_t)g] : P.rows_cap[(size_t)g] != ref.rows_cap[(size_t)g])
             return fail(GENLIB_EINVAL, "stream selftest: rows of rank " + std::to_string(g));
     return GENLIB_OK;
-}
-
-}  // extern "C"
-
-// ------------------------------------------------------------------------------ gen.gc, gen.occ, gen.rec (DESIGN.md 2b, 2c)
-struct genlib_gc_plan {
-    GcPlan p;
-    double ms_plan = 0;
-};
-
-namespace {
-
-// What a run of the gc plan computes: gen.gc's matrix, gen.occ's matrix or row sums, gen.rec's counts.
-enum GcFn { kFnGc = 0, kFnOcc, kFnOccTotal, kFnRec };
-bool gc_fn_reduces(int fn) { return fn == kFnOccTotal || fn == kFnRec; }
-
-// One device's share: column positions [j0, j1) of the column-side list and the unique columns [lo, hi) they
-// name (contiguous when the list has no duplicates; a duplicate may widen the range, never the result).
-struct GcShare {
-    int device = -1;
-    int fn = kFnGc;
-    int32_t j0 = 0, j1 = 0, lo = 0, hi = 0;
-    // row stride in 8-byte elements (16-byte rows): a column each, or for gen.rec 64 columns per word
-    int64_t ws() const {
-        const int64_t w = fn == kFnRec ? ((int64_t)(hi - lo) + 63) / 64 : (int64_t)(hi - lo);
-        return (w + 1) / 2 * 2;
-    }
-    size_t stage = 0, need = 0;
-    double ms_kernels = 0, ms_fetch = 0;
-    int32_t launches = 0;
-    int64_t d2h = 0;
-    std::vector<unsigned long long> red;   // reductions: per output-block row (ascend) or local column (descend)
-    unsigned long long ovf = ~0ull;        // gen.occ matrix: the smallest saturated (ancestor, proband) key
-};
-
-// Required traffic of a share over `cols` columns: the plan's byte model over the row's 8-byte elements
-// (gen.rec: its words, 16-byte padded as the kernel moves them), plus one read of the output block for a
-// reduction.
-double gc_fn_bytes(const GcPlan &P, int fn, int32_t cols) {
-    const int64_t w = fn == kFnRec ? (((int64_t)cols + 63) / 64 + 1) / 2 * 2 : cols;
-    double b = P.alg_bytes(w);
-    if (gc_fn_reduces(fn)) b += (double)P.n_targets() * (double)w * 8.0;
-    return b;
-}
-
-// Output layout of a share: the stage's major dimension is the column position (cmaj) or the target position.
-struct GcLayout {
-    bool cmaj;
-    int64_t ld, nmaj, nmin, maj_off, min_off;
-};
-
-GcLayout gc_layout(const GcPlan &P, const GcShare &d, int col_major) {
-    // gen.occ's ancestors x probands matrix in row-major order is gen.gc's layout in column-major order
-    const bool cm = d.fn == kFnOcc ? !col_major : col_major != 0;
-    GcLayout L;
-    L.cmaj = (P.direction == kGcDescend) == cm;
-    L.ld = cm ? P.n_pro : P.n_anc;
-    const int64_t T = (int64_t)P.target_uid().size(), C = d.j1 - d.j0;
-    L.nmaj = L.cmaj ? C : T; L.nmin = L.cmaj ? T : C;
-    L.maj_off = L.cmaj ? d.j0 : 0; L.min_off = L.cmaj ? 0 : d.j0;
-    return L;
-}
-
-// Reduction buffers: weights (ascend: per column, gen.rec also two masks per word; descend: per target row)
-// and the result (ascend: per target row; descend: per local column).
-size_t gc_reduce_bytes(const GcPlan &P, const GcShare &d) {
-    const size_t ws = (size_t)d.ws(), T = (size_t)P.n_targets(), W = (size_t)(d.hi - d.lo);
-    if (P.direction == kGcAscend)
-        return DevBuf<uint32_t>::padded(d.fn == kFnRec ? ws * 64 : ws) +
-               (d.fn == kFnRec ? 2 * DevBuf<unsigned long long>::padded(ws) : 0) + DevBuf<unsigned long long>::padded(T);
-    return DevBuf<uint32_t>::padded(T) + DevBuf<unsigned long long>::padded(W);
-}
-
-size_t gc_device_bytes(const GcPlan &P, GcShare &d, int col_major, size_t esize) {
-    const size_t ws = (size_t)d.ws(), R = (size_t)P.rows();
-    d.stage = gc_fn_reduces(d.fn) ? 0 : pad256(std::max<size_t>(kFetchStageBytes, (size_t)gc_layout(P, d, col_major).nmin * esize));
-    return pad256((size_t)P.capacity * ws * 8) + pad256((size_t)P.n_targets() * ws * 8) +
-           3 * DevBuf<int32_t>::padded(R) + DevBuf<int64_t>::padded(R + 1) + DevBuf<int32_t>::padded((size_t)P.inputs()) +
-           DevBuf<int32_t>::padded(P.target_uid().size()) + DevBuf<int32_t>::padded((size_t)(d.j1 - d.j0)) +
-           DevBuf<int32_t>::padded(1) + 2 * d.stage +
-           (d.fn == kFnGc ? 0 : DevBuf<unsigned long long>::padded(1)) + (gc_fn_reduces(d.fn) ? gc_reduce_bytes(P, d) : 0);
-}
-
-template <typename E, typename O>
-int gc_fetch(const GcPlan &P, GcShare &d, const void *Oblk, const int32_t *tgt_row, const int32_t *col, O *out,
-             int col_major, unsigned char *stage_base, unsigned long long *ovf, cudaStream_t st, cudaStream_t cst) {
-    const GcLayout L = gc_layout(P, d, col_major);
-    if (L.nmaj == 0 || L.nmin == 0) return GENLIB_OK;
-    const int64_t per = std::max<int64_t>(1, std::min<int64_t>(L.nmaj, (int64_t)(d.stage / (L.nmin * sizeof(O)))));
-    O *stage[2] = {reinterpret_cast<O *>(stage_base), reinterpret_cast<O *>(stage_base + d.stage)};
-    cudaEvent_t done[2] = {nullptr, nullptr}, copied[2] = {nullptr, nullptr};
-    cudaError_t ce = cudaSuccess;
-    for (int b = 0; b < 2 && ce == cudaSuccess; b++) {
-        ce = cudaEventCreateWithFlags(&done[b], cudaEventDisableTiming);
-        if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&copied[b], cudaEventDisableTiming);
-    }
-    int blk = 0;
-    for (int64_t m0 = 0; m0 < L.nmaj && ce == cudaSuccess; m0 += per, blk++) {      // gather of block b+1 overlaps the D2H of block b
-        const int b = blk & 1;
-        const int64_t nb = std::min(per, L.nmaj - m0);
-        if (blk >= 2 && (ce = cudaStreamWaitEvent(st, copied[b], 0)) != cudaSuccess) break;
-        GcGatherArgs a;
-        a.O = Oblk; a.ws = d.ws(); a.tgt_row = tgt_row; a.col = col;
-        a.ovf = ovf; a.j0 = d.j0; a.n_pro = P.n_pro; a.tgt_is_pro = P.direction == kGcDescend;
-        if (L.cmaj) { a.t0 = 0; a.n_t = (int32_t)L.nmin; a.c0 = (int32_t)m0; a.n_c = (int32_t)nb; }
-        else        { a.t0 = (int32_t)m0; a.n_t = (int32_t)nb; a.c0 = 0; a.n_c = (int32_t)L.nmin; }
-        dim3 grid((unsigned)((a.n_c + 31) / 32), (unsigned)std::min<int64_t>((a.n_t + 31) / 32, 65535)), block(32, 8);
-        if (L.cmaj) gc_gather_kernel<true, E, O><<<grid, block, 0, st>>>(a, stage[b]);
-        else        gc_gather_kernel<false, E, O><<<grid, block, 0, st>>>(a, stage[b]);
-        if ((ce = cudaGetLastError()) != cudaSuccess) break;
-        cudaEventRecord(done[b], st);
-        cudaStreamWaitEvent(cst, done[b], 0);
-        ce = cudaMemcpy2DAsync(out + (L.maj_off + m0) * L.ld + L.min_off, (size_t)L.ld * sizeof(O), stage[b],
-                               (size_t)L.nmin * sizeof(O), (size_t)L.nmin * sizeof(O), (size_t)nb, cudaMemcpyDeviceToHost, cst);
-        cudaEventRecord(copied[b], cst);
-    }
-    const cudaError_t e1 = cudaStreamSynchronize(st), e2 = cudaStreamSynchronize(cst);
-    for (int b = 0; b < 2; b++) { if (done[b]) cudaEventDestroy(done[b]); if (copied[b]) cudaEventDestroy(copied[b]); }
-    if (ce != cudaSuccess || e1 != cudaSuccess || e2 != cudaSuccess)
-        return fail(GENLIB_ECUDA, std::string("gc fetch failed: ") + cudaGetErrorString(ce != cudaSuccess ? ce : e1 != cudaSuccess ? e1 : e2));
-    d.d2h += L.nmaj * L.nmin * (int64_t)sizeof(O);
-    return GENLIB_OK;
-}
-
-template <typename Op>
-void gc_launch_layer(const GcLayerArgs &a, unsigned gx, cudaStream_t st) {
-    const int rpc = kGcThreads >> a.tpr_log2;
-    const unsigned gy = (unsigned)std::min<int64_t>(((int64_t)a.n_rows + rpc - 1) / rpc, 65535);
-    if (a.tpr_log2 == kGcThreadsLog2) gc_layer_kernel<Op, true><<<dim3(gx, gy), kGcThreads, 0, st>>>(a);
-    else                              gc_layer_kernel<Op, false><<<dim3(gx, gy), kGcThreads, 0, st>>>(a);
-}
-
-// Every layer of the plan over the share's columns on its device, then its block of `out` (gen.gc, gen.occ's
-// matrix) or its part of the reduction (d.red).
-int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_major) {
-    DeviceGuard guard;
-    if (int rc = guard.enter(d.device)) return rc;
-    struct Res {
-        cudaStream_t st = nullptr, cst = nullptr;
-        cudaEvent_t ev[2] = {nullptr, nullptr};
-        Arena arena;
-        ~Res() {
-            if (st) cudaStreamSynchronize(st);
-            if (cst) cudaStreamSynchronize(cst);
-            for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
-            if (st) cudaStreamDestroy(st);
-            if (cst) cudaStreamDestroy(cst);
-            g_arenas.release(arena);
-        }
-    } res;
-    CU(cudaStreamCreateWithFlags(&res.st, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&res.cst, cudaStreamNonBlocking));
-    for (cudaEvent_t &e : res.ev) CU(cudaEventCreate(&e));
-    static const char *const kName[] = {"gen.gc", "gen.occ", "gen.occ", "gen.rec"};
-    if (g_arenas.acquire(d.device, d.need, res.arena) != cudaSuccess) {
-        res.arena = Arena();
-        cudaGetLastError();
-        size_t free_b = 0, total_b = 0;
-        cudaMemGetInfo(&free_b, &total_b);
-        char msg[256];
-        std::snprintf(msg, sizeof msg, "%s needs %.2f GB on device %d, %.2f GB free (%lld frontier rows x %lld columns): "
-                      "split the columns over more devices", kName[d.fn], d.need / 1e9, d.device, free_b / 1e9,
-                      (long long)P.capacity, (long long)(d.hi - d.lo));
-        return fail(GENLIB_ENOMEM, msg);
-    }
-    const size_t ws = (size_t)d.ws(), R = (size_t)P.rows(), T = (size_t)P.n_targets(), W = (size_t)(d.hi - d.lo);
-    const bool reduce = gc_fn_reduces(d.fn), asc = P.direction == kGcAscend;
-    unsigned char *cur = static_cast<unsigned char *>(res.arena.base);
-    auto take = [&](size_t bytes) { unsigned char *p = cur; cur += pad256(bytes); return p; };
-    void *F = take((size_t)P.capacity * ws * 8);
-    void *O = take(T * ws * 8);
-    DevBuf<int32_t> row_slot, row_seed, row_out, in_slot, tgt_row, col, err;
-    DevBuf<int64_t> in_ptr;
-    DevBuf<unsigned long long> ovf, m1, m2, red;
-    DevBuf<uint32_t> wt;
-    row_slot.place(cur, R); row_seed.place(cur, R); row_out.place(cur, R); in_ptr.place(cur, R + 1);
-    in_slot.place(cur, (size_t)P.inputs()); tgt_row.place(cur, P.target_uid().size());
-    col.place(cur, (size_t)(d.j1 - d.j0)); err.place(cur, 1);
-    unsigned char *stage = cur;
-    cur += 2 * d.stage;
-    if (d.fn != kFnGc) ovf.place(cur, 1);
-    // reduction weights: how often the lists name each column (ascend) or each target row (descend)
-    std::vector<uint32_t> h_wt;
-    std::vector<unsigned long long> h_m1, h_m2;
-    if (reduce) {
-        if (asc) {
-            h_wt.assign(d.fn == kFnRec ? ws * 64 : ws, 0);
-            for (int32_t j = d.j0; j < d.j1; j++) h_wt[(size_t)(P.column_uid()[(size_t)j] - d.lo)]++;
-            if (d.fn == kFnRec) {
-                h_m1.assign(ws, 0); h_m2.assign(ws, 0);
-                for (size_t c = 0; c < W; c++) {
-                    if (h_wt[c] >= 1) h_m1[c >> 6] |= 1ull << (c & 63);
-                    if (h_wt[c] >= 2) h_m2[c >> 6] |= 1ull << (c & 63);
-                }
-                m1.place(cur, ws); m2.place(cur, ws);
-            }
-            red.place(cur, T);
-        } else {
-            h_wt.assign(T, 0);
-            for (int32_t t : P.target_uid()) h_wt[(size_t)t]++;
-            red.place(cur, W);
-        }
-        wt.place(cur, h_wt.size());
-    }
-    if ((size_t)(cur - static_cast<unsigned char *>(res.arena.base)) > d.need) return fail(GENLIB_EINVAL, "internal: gc arena layout overflow");
-    std::vector<int32_t> cols((size_t)(d.j1 - d.j0));
-    for (int32_t j = d.j0; j < d.j1; j++) cols[(size_t)(j - d.j0)] = P.column_uid()[(size_t)j] - d.lo;
-    CU(row_slot.upload(P.row_slot, res.st)); CU(row_seed.upload(P.row_seed, res.st)); CU(row_out.upload(P.row_out, res.st));
-    CU(in_ptr.upload(P.in_ptr, res.st)); CU(in_slot.upload(P.in_slot, res.st)); CU(tgt_row.upload(P.target_uid(), res.st));
-    CU(col.upload(cols, res.st));
-    CU(cudaMemsetAsync(err.p, 0, sizeof(int32_t), res.st));
-    if (d.fn != kFnGc) CU(cudaMemsetAsync(ovf.p, 0xff, sizeof(unsigned long long), res.st));
-    if (reduce) {
-        CU(wt.upload(h_wt, res.st)); CU(m1.upload(h_m1, res.st)); CU(m2.upload(h_m2, res.st));
-        if (!asc) CU(cudaMemsetAsync(red.p, 0, W * sizeof(unsigned long long), res.st));
-    }
-    if (P.n_out_rows < P.n_targets())                       // a target no path reaches: its output row is 0
-        CU(cudaMemsetAsync(O, 0, T * ws * 8, res.st));
-    GcLayerArgs a;
-    a.F = F; a.O = O;
-    a.w2 = (int64_t)ws / 2; a.width = d.hi - d.lo; a.col_lo = d.lo;
-    a.tpr_log2 = gc_tpr_log2(a.w2);
-    a.capacity = P.capacity; a.n_targets = P.n_targets(); a.in_slot = in_slot.p; a.err = err.p;
-    const unsigned gx = (unsigned)((a.w2 + ((int64_t)kGcVec << a.tpr_log2) - 1) / ((int64_t)kGcVec << a.tpr_log2));
-    CU(cudaEventRecord(res.ev[0], res.st));
-    for (int32_t t = 0; t < P.n_layers(); t++) {
-        const int64_t r0 = P.layer_begin[(size_t)t];
-        a.n_rows = (int32_t)(P.layer_begin[(size_t)t + 1] - r0);
-        a.row_slot = row_slot.p + r0; a.row_seed = row_seed.p + r0; a.row_out = row_out.p + r0; a.in_ptr = in_ptr.p + r0;
-        if (d.fn == kFnGc) gc_launch_layer<GcOpHalfSum>(a, gx, res.st);
-        else if (d.fn == kFnRec) gc_launch_layer<GcOpReach>(a, gx, res.st);
-        else gc_launch_layer<GcOpCount>(a, gx, res.st);
-        CU(cudaGetLastError());
-        d.launches++;
-    }
-    if (reduce && T > 0) {
-        if (asc) {
-            GcRowReduceArgs r;
-            r.O = static_cast<const ulonglong2 *>(O); r.w2 = (int64_t)ws / 2; r.n_rows = (int32_t)T;
-            r.wt = wt.p; r.m1 = m1.p; r.m2 = m2.p; r.out = red.p;
-            const unsigned g = (unsigned)((T + 7) / 8);
-            if (d.fn == kFnRec) gc_row_reduce_kernel<true><<<g, 256, 0, res.st>>>(r);
-            else                gc_row_reduce_kernel<false><<<g, 256, 0, res.st>>>(r);
-        } else {
-            GcColReduceArgs r;
-            r.O = static_cast<const unsigned long long *>(O); r.ws = (int64_t)ws; r.n_rows = (int32_t)T;
-            r.width = (int32_t)W; r.wt = wt.p; r.out = red.p;
-            // enough CTAs for the whole device: about 8 per SM, at least 64 rows each
-            const int64_t gxr = ((int64_t)W + 255) / 256;
-            const int64_t gyr = std::max<int64_t>(1, std::min<int64_t>(((int64_t)T + 63) / 64, (148 * 8 + gxr - 1) / gxr));
-            r.rows_per_cta = (int32_t)(((int64_t)T + gyr - 1) / gyr);
-            const dim3 g((unsigned)gxr, (unsigned)(((int64_t)T + r.rows_per_cta - 1) / r.rows_per_cta));
-            if (d.fn == kFnRec) gc_col_reduce_kernel<true><<<g, 256, 0, res.st>>>(r);
-            else                gc_col_reduce_kernel<false><<<g, 256, 0, res.st>>>(r);
-        }
-        CU(cudaGetLastError());
-        d.launches++;
-    }
-    CU(cudaEventRecord(res.ev[1], res.st));
-    CU(cudaStreamSynchronize(res.st));
-    float ms = 0;
-    CU(cudaEventElapsedTime(&ms, res.ev[0], res.ev[1]));
-    d.ms_kernels = ms;
-    int32_t errw = 0;
-    CU(cudaMemcpy(&errw, err.p, sizeof errw, cudaMemcpyDeviceToHost));
-    if (errw) return fail(GENLIB_ECUDA, "the gc layer kernel reported a bound violated at line " + std::to_string(errw - 100000));
-    const double t0 = now_ms();
-    int rc = GENLIB_OK;
-    if (reduce) {
-        d.red.assign(asc ? T : W, 0);
-        if (T > 0) CU(cudaMemcpy(d.red.data(), red.p, d.red.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-        d.d2h += (int64_t)(d.red.size() * sizeof(unsigned long long));
-    } else if (d.fn == kFnOcc) {
-        rc = gc_fetch<unsigned long long, int64_t>(P, d, O, tgt_row.p, col.p, static_cast<int64_t *>(out), col_major, stage, ovf.p, res.st, res.cst);
-        if (rc == GENLIB_OK) CU(cudaMemcpy(&d.ovf, ovf.p, sizeof d.ovf, cudaMemcpyDeviceToHost));
-    } else {
-        rc = out_dtype == GENLIB_F64
-            ? gc_fetch<double, double>(P, d, O, tgt_row.p, col.p, static_cast<double *>(out), col_major, stage, nullptr, res.st, res.cst)
-            : gc_fetch<double, float>(P, d, O, tgt_row.p, col.p, static_cast<float *>(out), col_major, stage, nullptr, res.st, res.cst);
-    }
-    d.ms_fetch = now_ms() - t0;
-    return rc;
-}
-
-void gc_fill_stats(const GcPlan &P, genlib_gc_stats *s) {
-    std::memset(s, 0, sizeof *s);
-    s->n_pro = P.n_pro; s->n_anc = P.n_anc; s->n_layers = P.n_layers(); s->direction = P.direction;
-    s->rows = P.rows(); s->inputs = P.inputs(); s->width = P.width(); s->capacity = P.capacity;
-    s->alg_bytes = P.alg_bytes(P.width());
-    s->n_dev = 1;
-}
-
-}  // namespace
-
-extern "C" {
-
-int genlib_gc_plan_create(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
-                          const int32_t *proband, int32_t n_anc, const int32_t *ancestor, genlib_gc_plan **out) {
-    if (!out) return fail(GENLIB_EINVAL, "genlib_gc_plan_create: null argument");
-    *out = nullptr;
-    std::unique_ptr<genlib_gc_plan> pl(new (std::nothrow) genlib_gc_plan);
-    if (!pl) return fail(GENLIB_ENOMEM, "out of host memory");
-    const double t0 = now_ms();
-    std::string err;
-    try {
-        if (int rc = build_gc_plan(n, father, mother, n_pro, proband, n_anc, ancestor, -1, pl->p, err)) return fail(rc, err);
-    } catch (const std::bad_alloc &) {
-        return fail(GENLIB_ENOMEM, "out of host memory while planning");
-    }
-    pl->ms_plan = now_ms() - t0;
-    *out = pl.release();
-    return GENLIB_OK;
-}
-
-void genlib_gc_plan_destroy(genlib_gc_plan *plan) { delete plan; }
-
-int genlib_gc_plan_info(const genlib_gc_plan *plan, genlib_gc_stats *out) {
-    if (!plan || !out) return fail(GENLIB_EINVAL, "genlib_gc_plan_info: null argument");
-    gc_fill_stats(plan->p, out);
-    GcShare d;
-    d.j1 = (int32_t)plan->p.column_uid().size(); d.hi = plan->p.width();
-    out->device_bytes = plan->p.width() > 0 && plan->p.n_targets() > 0 ? (int64_t)gc_device_bytes(plan->p, d, 0, 8) : 0;
-    return GENLIB_OK;
-}
-
-int genlib_gc_plan_layer(const genlib_gc_plan *plan, int32_t layer, int32_t *n_rows, int64_t *n_inputs) {
-    if (!plan) return fail(GENLIB_EINVAL, "genlib_gc_plan_layer: null plan");
-    const GcPlan &P = plan->p;
-    if (layer < 0 || layer >= P.n_layers()) return fail(GENLIB_EINVAL, "layer out of range");
-    const int64_t r0 = P.layer_begin[(size_t)layer], r1 = P.layer_begin[(size_t)layer + 1];
-    if (n_rows) *n_rows = (int32_t)(r1 - r0);
-    if (n_inputs) *n_inputs = P.in_ptr[(size_t)r1] - P.in_ptr[(size_t)r0];
-    return GENLIB_OK;
-}
-
-int genlib_gc_plan_layer_arrays(const genlib_gc_plan *plan, int32_t layer, int32_t *row_ind, int32_t *row_slot,
-                                int32_t *row_seed, int32_t *row_out, int64_t *in_ptr, int32_t *in_slot) {
-    if (!plan) return fail(GENLIB_EINVAL, "genlib_gc_plan_layer_arrays: null plan");
-    const GcPlan &P = plan->p;
-    if (layer < 0 || layer >= P.n_layers()) return fail(GENLIB_EINVAL, "layer out of range");
-    const size_t r0 = (size_t)P.layer_begin[(size_t)layer], r1 = (size_t)P.layer_begin[(size_t)layer + 1];
-    auto copy = [&](const std::vector<int32_t> &v, int32_t *o) { if (o) std::copy(v.begin() + (long)r0, v.begin() + (long)r1, o); };
-    copy(P.row_ind, row_ind); copy(P.row_slot, row_slot); copy(P.row_seed, row_seed); copy(P.row_out, row_out);
-    const int64_t e0 = P.in_ptr[r0];
-    if (in_ptr) for (size_t r = r0; r <= r1; r++) in_ptr[r - r0] = P.in_ptr[r] - e0;
-    if (in_slot) std::copy(P.in_slot.begin() + e0, P.in_slot.begin() + P.in_ptr[r1], in_slot);
-    return GENLIB_OK;
-}
-
-}  // extern "C"
-
-namespace {
-
-// The first proband list position whose individual descends from (or is) `anc`: the proband an overflowing
-// row sum is reported with.  Host only, O(n), on the error path.
-int32_t gc_first_descendant(int32_t n, const int32_t *father, const int32_t *mother, int32_t anc, int32_t n_pro,
-                            const int32_t *proband) {
-    std::vector<uint8_t> down((size_t)n, 0);
-    down[(size_t)anc] = 1;
-    for (int32_t i = anc + 1; i < n; i++)
-        down[(size_t)i] = (father[i] >= 0 && down[(size_t)father[i]]) || (mother[i] >= 0 && down[(size_t)mother[i]]);
-    for (int32_t j = 0; j < n_pro; j++) if (down[(size_t)proband[j]]) return j;
-    return -1;
-}
-
-int gc_overflow(int32_t anc_pos, int32_t anc_rank, int32_t pro_pos, int32_t pro_rank, bool total) {
-    char msg[320];
-    std::snprintf(msg, sizeof msg, "gen.occ: %s exceeds 2^63 - 1 (Int64) at ancestor position %d (rank %d), "
-                  "proband position %d (rank %d)", total ? "a row sum of descent-path counts" : "a descent-path count",
-                  anc_pos, anc_rank, pro_pos, pro_rank);
-    return fail(GENLIB_EOVERFLOW, msg);
-}
-
-// genlib_gc, genlib_occ and genlib_rec: one plan, the column-side list split over the devices, every device
-// runs the plan over its columns; the matrices are written block by block into `out`, the reductions are
-// combined here.
-int gc_driver(int fn, int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
-              int32_t n_anc, const int32_t *ancestor, void *out, int out_dtype, int col_major, int32_t n_dev,
-              const int32_t *devices, genlib_gc_stats *stats) {
-    static const char *const kEntry[] = {"genlib_gc", "genlib_occ", "genlib_occ", "genlib_rec"};
-    const std::string who = kEntry[fn];
-    if (n_dev < 1 || !devices) return fail(GENLIB_EINVAL, who + ": at least one device");
-    genlib_gc_plan *plan = nullptr;
-    if (int rc = genlib_gc_plan_create(n, father, mother, n_pro, proband, n_anc, ancestor, &plan)) return rc;
-    std::unique_ptr<genlib_gc_plan> owner(plan);
-    const GcPlan &P = plan->p;
-    genlib_gc_stats st;
-    gc_fill_stats(P, &st);
-    st.alg_bytes = gc_fn_bytes(P, fn, P.width());
-    st.ms_plan = plan->ms_plan;
-    st.n_dev = n_dev;
-    const bool reduce = gc_fn_reduces(fn);
-    if (P.n_pro == 0 || P.n_anc == 0) {                     // an empty matrix (or zero counts): no device needed
-        if (reduce && P.n_anc > 0) {
-            if (!out) return fail(GENLIB_EINVAL, who + ": out is null");
-            std::memset(out, 0, (size_t)P.n_anc * sizeof(int64_t));
-        }
-        if (stats) *stats = st;
-        return GENLIB_OK;
-    }
-    if (!out) return fail(GENLIB_EINVAL, who + ": out is null");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return fail(GENLIB_ECUDA, "no CUDA device: libgenlib_cuda has no CPU fallback");
-    std::vector<GcShare> share((size_t)n_dev);
-    const std::vector<int32_t> &cu = P.column_uid();
-    const int64_t m = (int64_t)cu.size();
-    const size_t esize = fn == kFnGc ? (out_dtype == GENLIB_F64 ? 8 : 4) : 8;
-    for (int g = 0; g < n_dev; g++) {
-        GcShare &d = share[(size_t)g];
-        d.fn = fn;
-        d.device = devices[g];
-        if (d.device < 0 && cudaGetDevice(&d.device) != cudaSuccess) return fail(GENLIB_ECUDA, "no usable CUDA device (cudaGetDevice failed)");
-        if (d.device >= ndev) return fail(GENLIB_EINVAL, who + ": no such device");
-        for (int h = 0; h < g; h++) if (share[(size_t)h].device == d.device) return fail(GENLIB_EINVAL, who + ": a device is listed twice");
-        d.j0 = (int32_t)(m * g / n_dev); d.j1 = (int32_t)(m * (g + 1) / n_dev);
-        if (d.j0 == d.j1) continue;                          // more devices than columns: nothing to do here
-        d.lo = *std::min_element(cu.begin() + d.j0, cu.begin() + d.j1);
-        d.hi = *std::max_element(cu.begin() + d.j0, cu.begin() + d.j1) + 1;
-        d.need = gc_device_bytes(P, d, col_major, esize);
-    }
-    std::vector<int> status((size_t)n_dev, GENLIB_OK);
-    std::vector<std::string> message((size_t)n_dev);
-    auto run = [&](int g) {
-        GcShare &d = share[(size_t)g];
-        if (d.j0 == d.j1) return;
-        status[(size_t)g] = gc_run_share(P, d, out, out_dtype, col_major);
-        if (status[(size_t)g] != GENLIB_OK) message[(size_t)g] = g_err;
-    };
-    if (n_dev == 1) run(0);
-    else {                                                   // one host thread per device, as genlib_phi_multi
-        std::vector<std::thread> th;
-        for (int g = 0; g < n_dev; g++) th.emplace_back(run, g);
-        for (auto &t : th) t.join();
-    }
-    for (int g = 0; g < n_dev; g++)
-        if (status[(size_t)g] != GENLIB_OK) return fail(status[(size_t)g], "device " + std::to_string(share[(size_t)g].device) + ": " + message[(size_t)g]);
-    if (stats) {
-        st.width = 0; st.alg_bytes = 0;
-        for (const GcShare &d : share) {
-            if (d.j0 == d.j1) continue;
-            st.width += d.hi - d.lo;
-            st.alg_bytes += gc_fn_bytes(P, fn, d.hi - d.lo);
-            st.device_bytes = std::max(st.device_bytes, (int64_t)d.need);
-            st.ms_kernels = std::max(st.ms_kernels, d.ms_kernels);
-            st.ms_fetch = std::max(st.ms_fetch, d.ms_fetch);
-            st.d2h_bytes += d.d2h;
-            st.kernel_launches += d.launches;
-        }
-        *stats = st;
-    }
-    if (fn == kFnOcc) {                                      // the smallest saturated pair over all devices
-        unsigned long long key = ~0ull;
-        for (const GcShare &d : share) if (d.j0 != d.j1) key = std::min(key, d.ovf);
-        if (key != ~0ull) {
-            const int32_t i = (int32_t)(key / (unsigned long long)P.n_pro), j = (int32_t)(key % (unsigned long long)P.n_pro);
-            return gc_overflow(i, ancestor[i], j, proband[j], false);
-        }
-    }
-    if (reduce) {                                            // every device's part -> one value per ancestor position
-        const bool rec = fn == kFnRec;
-        std::vector<unsigned long long> v((size_t)P.n_anc, 0);
-        if (P.direction == kGcAscend) {                      // parts per ancestor (the block's rows): add them
-            std::vector<unsigned long long> tot((size_t)P.n_targets(), 0);
-            for (const GcShare &d : share) {
-                if (d.j0 == d.j1) continue;
-                for (size_t t = 0; t < tot.size(); t++) {
-                    const unsigned long long s = tot[t] + d.red[t];
-                    tot[t] = rec ? s : (s < tot[t] || s > kOccSat) ? kOccSat : s;
-                }
-            }
-            for (int32_t i = 0; i < P.n_anc; i++) v[(size_t)i] = tot[(size_t)P.anc_uid[(size_t)i]];
-        } else {                                             // parts per ancestor column: place them
-            for (const GcShare &d : share)
-                for (int32_t j = d.j0; j < d.j1; j++) v[(size_t)j] = d.red[(size_t)(P.anc_uid[(size_t)j] - d.lo)];
-        }
-        for (int32_t i = 0; i < P.n_anc; i++)
-            if (v[(size_t)i] >= kOccSat) {
-                const int32_t j = gc_first_descendant(n, father, mother, ancestor[i], n_pro, proband);
-                return gc_overflow(i, ancestor[i], j, j >= 0 ? proband[j] : -1, true);
-            }
-        int64_t *o = static_cast<int64_t *>(out);
-        for (int32_t i = 0; i < P.n_anc; i++) o[i] = (int64_t)v[(size_t)i];
-    }
-    return GENLIB_OK;
-}
-
-}  // namespace
-
-extern "C" {
-
-int genlib_gc(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
-              int32_t n_anc, const int32_t *ancestor, void *out, int out_dtype, int col_major, int32_t n_dev,
-              const int32_t *devices, genlib_gc_stats *stats) {
-    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
-    return gc_driver(kFnGc, n, father, mother, n_pro, proband, n_anc, ancestor, out, out_dtype, col_major, n_dev,
-                     devices, stats);
-}
-
-int genlib_occ(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
-               int32_t n_anc, const int32_t *ancestor, int64_t *out, int type, int col_major, int32_t n_dev,
-               const int32_t *devices, genlib_gc_stats *stats) {
-    if (type != GENLIB_OCC_IND && type != GENLIB_OCC_TOTAL) return fail(GENLIB_EINVAL, "genlib_occ: unknown type");
-    return gc_driver(type == GENLIB_OCC_IND ? kFnOcc : kFnOccTotal, n, father, mother, n_pro, proband, n_anc, ancestor,
-                     out, 0, col_major, n_dev, devices, stats);
-}
-
-int genlib_rec(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
-               int32_t n_anc, const int32_t *ancestor, int64_t *out, int32_t n_dev, const int32_t *devices,
-               genlib_gc_stats *stats) {
-    return gc_driver(kFnRec, n, father, mother, n_pro, proband, n_anc, ancestor, out, 0, 0, n_dev, devices, stats);
 }
 
 }  // extern "C"
