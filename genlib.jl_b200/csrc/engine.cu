@@ -852,30 +852,7 @@ void genlib_plan_destroy(genlib_plan *plan) {
     try { retire_storage(plan->p); } catch (...) {}
     delete plan;
 }
-uint64_t genlib_plan_digest(const genlib_plan *plan, int with_bounds) {
-    settle(plan);
-    if (!plan) return 0;
-    const Plan &P = plan->p;
-    uint64_t h = 1469598103934665603ULL;
-    auto bytes = [&h](const void *p, size_t nb) { const unsigned char *c = (const unsigned char *)p; for (size_t i = 0; i < nb; i++) { h ^= c[i]; h *= 1099511628211ULL; } };
-    auto vec = [&bytes](const auto &v) { const uint64_t s = v.size(); bytes(&s, 8); if (s) bytes(v.data(), s * sizeof(v[0])); };
-    const int64_t hdr[6] = {P.n, P.n_unique, P.world, P.schedule, with_bounds ? P.capacity : 0, P.row_updates};
-    bytes(hdr, sizeof hdr); bytes(&P.alg_elems, 8);
-    for (const Layer &L : P.layers) {
-        const int64_t f[] = {L.n_new, L.n_fam, L.live_before, L.carried, L.ref_founders, L.ref_probands, L.ref_both, L.rt_lo, L.rt_rows,
-                             L.n_live_tiles, (int64_t)L.tile_off, (int64_t)L.ltile_off, L.nf_pad, L.n_mtiles, L.max_tile_fam,
-                             (int64_t)L.mem_off, (int64_t)L.fam_off, (int64_t)L.flag_off, (int64_t)L.mtile_off, (int64_t)L.base_off,
-                             (int64_t)L.mem_end, (int64_t)L.fam_end, (int64_t)L.flag_end, (int64_t)L.tile_end, (int64_t)L.ltile_end,
-                             (int64_t)L.mtile_end};
-        bytes(f, sizeof f); bytes(&L.alg_elems, 8);
-    }
-    vec(P.pro_ind); vec(P.pro_slot); vec(P.mem_ind); vec(P.mem_slot); vec(P.mem_fam); vec(P.mem_rank); vec(P.fam_pf); vec(P.fam_pm);
-    vec(P.fam_start); vec(P.fam_q); vec(P.flags); vec(P.tile_map); vec(P.live_tiles); vec(P.mtile_desc); vec(P.fam_base); vec(P.mem_base);
-    vec(P.mem_lrow); vec(P.fam_pf_owner); vec(P.fam_pm_owner); vec(P.fam_pf_lrow); vec(P.fam_pm_lrow); vec(P.live_owner); vec(P.live_lrow);
-    vec(P.pro_owner); vec(P.pro_lrow);
-    if (with_bounds) vec(P.rows_cap);
-    return h;
-}
+uint64_t genlib_plan_digest(const genlib_plan *plan, int with_bounds) { settle(plan); return plan ? plan_digest(plan->p, with_bounds != 0) : 0; }
 int32_t genlib_plan_n_unique(const genlib_plan *plan) { return plan ? plan->p.n_unique : -1; }
 int32_t genlib_plan_schedule(const genlib_plan *plan) { return plan ? plan->p.schedule : -1; }
 int32_t genlib_plan_n_layers(const genlib_plan *plan) { settle(plan); return plan ? (int32_t)plan->p.layers.size() : -1; }

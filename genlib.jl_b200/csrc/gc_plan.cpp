@@ -8,6 +8,7 @@
 #include <queue>
 
 #include "../../include/genlib_cuda.h"
+#include "plan.hpp"
 
 namespace genlib {
 
@@ -20,11 +21,7 @@ int build_gc_plan(int32_t n, const int32_t *father, const int32_t *mother, int32
         return GENLIB_EINVAL;
     }
     P.n = n; P.n_pro = n_pro; P.n_anc = n_anc;
-    for (int32_t i = 0; i < n; i++) {                       // the pedigree's own errors first: the first offending rank
-        const int32_t f = father[i], m = mother[i];
-        if (f < -1 || f >= n || m < -1 || m >= n) { err = "KeyError: parent index out of range at rank " + std::to_string(i); return GENLIB_EKEY; }
-        if (f >= i || m >= i) { err = "parent does not precede child at rank " + std::to_string(i); return GENLIB_EORDER; }
-    }
+    if (int rc = check_pedigree(n, father, mother, err)) return rc;   // the pedigree's own errors first
     // list position -> unique index, numbered by first occurrence; rank -> unique index (-1: not listed)
     std::vector<int32_t> pro_of((size_t)n, -1), anc_of((size_t)n, -1);
     auto unique = [&](int32_t len, const int32_t *list, const char *what, std::vector<int32_t> &of,

@@ -157,4 +157,12 @@ int build_plan(int32_t n, const int32_t *father, const int32_t *mother, const in
                const int32_t *proband, int32_t world, int schedule, Plan &plan, std::string &err,
                PlanStream *stream = nullptr, int planners = 0);
 
+// Internal to the library (hidden: not exported).
+// The pedigree's own errors, the first offending rank: a parent index out of range (GENLIB_EKEY) or a parent that
+// does not precede its child (GENLIB_EORDER).  Returns 0 or that status; `err` receives the message.
+__attribute__((visibility("hidden"))) int check_pedigree(int32_t n, const int32_t *father, const int32_t *mother, std::string &err);
+// FNV-1a over the header, every Layer field and every array of the plan, in a fixed order (genlib_plan_digest);
+// `with_bounds` adds Plan::capacity and Plan::rows_cap.  A new array of Plan belongs here as well as in each_array.
+__attribute__((visibility("hidden"))) uint64_t plan_digest(const Plan &P, bool with_bounds);
+
 }  // namespace genlib

@@ -6,30 +6,10 @@
 #include <fstream>
 namespace genlib { int set_error(int code, const std::string &) { return code; } }
 using namespace genlib;
-static uint64_t H;
-static void mixb(const void *p, size_t nbytes) { const unsigned char *c = (const unsigned char *)p; for (size_t i = 0; i < nbytes; i++) { H ^= c[i]; H *= 1099511628211ULL; } }
-template <class T> static void mixv(const std::vector<T> &v) { uint64_t s = v.size(); mixb(&s, 8); if (!v.empty()) mixb(v.data(), v.size() * sizeof(T)); }
-static uint64_t digest(Plan &P, bool with_cap) {
-    H = 1469598103934665603ULL;
-    int64_t hdr[6] = {P.n, P.n_unique, P.world, P.schedule, with_cap ? P.capacity : 0, P.row_updates};
-    mixb(hdr, sizeof hdr); mixb(&P.alg_elems, 8);
-    for (const Layer &L : P.layers) {
-        int64_t f[] = {L.n_new, L.n_fam, L.live_before, L.carried, L.ref_founders, L.ref_probands, L.ref_both, L.rt_lo, L.rt_rows,
-                       L.n_live_tiles, (int64_t)L.tile_off, (int64_t)L.ltile_off, L.nf_pad, L.n_mtiles, L.max_tile_fam, (int64_t)L.mem_off,
-                       (int64_t)L.fam_off, (int64_t)L.flag_off, (int64_t)L.mtile_off, (int64_t)L.base_off, (int64_t)L.mem_end, (int64_t)L.fam_end,
-                       (int64_t)L.flag_end, (int64_t)L.tile_end, (int64_t)L.ltile_end, (int64_t)L.mtile_end};
-        mixb(f, sizeof f); mixb(&L.alg_elems, 8);
-    }
-    mixv(P.pro_ind); mixv(P.pro_slot); mixv(P.mem_ind); mixv(P.mem_slot); mixv(P.mem_fam); mixv(P.mem_rank); mixv(P.fam_pf); mixv(P.fam_pm);
-    mixv(P.fam_start); mixv(P.fam_q); mixv(P.flags); mixv(P.tile_map); mixv(P.live_tiles); mixv(P.mtile_desc); mixv(P.fam_base); mixv(P.mem_base);
-    mixv(P.mem_lrow); mixv(P.fam_pf_owner); mixv(P.fam_pm_owner); mixv(P.fam_pf_lrow); mixv(P.fam_pm_lrow); mixv(P.live_owner); mixv(P.live_lrow);
-    mixv(P.pro_owner); mixv(P.pro_lrow);
-    if (with_cap) mixv(P.rows_cap);
-    return H;
-}
 int main(int argc, char **argv) {
     // args: file world schedule reps [stream]
     const char *file = argv[1]; int world = atoi(argv[2]), sched = atoi(argv[3]), reps = atoi(argv[4]); bool stream = argc > 5 && atoi(argv[5]);
+    const char *name = strrchr(file, '/') ? strrchr(file, '/') + 1 : file;   // (a bare file name has no '/')
     std::ifstream fh(file, std::ios::binary);
     int64_t hd[2]; fh.read((char *)hd, 16);
     std::vector<int32_t> fa(hd[0]), mo(hd[0]), pro(hd[1]); std::vector<int64_t> ids(hd[0]);
@@ -48,11 +28,11 @@ int main(int argc, char **argv) {
         } else rc = build_plan((int32_t)hd[0], fa.data(), mo.data(), sched ? ids.data() : nullptr, (int32_t)hd[1], pro.data(), world, sched, P, err, nullptr);
         double ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
         best = std::min(best, ms); best_first = std::min(best_first, first);
-        dg = digest(P, !stream);
+        dg = plan_digest(P, !stream);
         retire_storage(P);
     }
-    std::printf("%s w%d s%d%s rc %d digest %016llx", strrchr(file, '/') + 1, world, sched, stream ? " stream" : "", rc, (unsigned long long)dg);
-    std::fprintf(stderr, "   %s w%d s%d: best %.1f ms, first layer after %.1f ms\n", strrchr(file, '/') + 1, world, sched, best, best_first);
+    std::printf("%s w%d s%d%s rc %d digest %016llx", name, world, sched, stream ? " stream" : "", rc, (unsigned long long)dg);
+    std::fprintf(stderr, "   %s w%d s%d: best %.1f ms, first layer after %.1f ms\n", name, world, sched, best, best_first);
     std::printf("\n");
     return 0;
 }
