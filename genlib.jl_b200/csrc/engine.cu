@@ -221,9 +221,7 @@ LayerLaunch shape_layer(const Plan &P, int t, int rank, size_t es, int sm_count)
     // whose staged tile fits shared memory: 128 parent-row segments of sw pairs <= 64 KB).  A wide strip
     // amortises the per-tile work of the consumers; more buffers give the producers more room to run ahead.
     const size_t min_buf = (size_t)std::max(2, env_int("GENLIB_MIN_NBUF", 2));
-    // consumer groups per CTA, each with its own items and shared memory (two only fit with narrower strips)
-    const int groups = std::max(1, std::min(kConsGroups, env_int("GENLIB_CONS_GROUPS", kConsGroups)));
-    const int sw_cap = (es == 4 ? kMaxStrip : kMaxStrip / 2) / groups;
+    const int sw_cap = es == 4 ? kMaxStrip : kMaxStrip / 2;
     const size_t budget = (size_t)std::max(16, env_int("GENLIB_STRIP_BUDGET_MB", (int)(kStripBudget >> 20))) << 20;
     int sw = std::min(sw_cap, std::max(8, env_int("GENLIB_MAX_SW", kMaxStrip)));
     while (sw > 8 && (size_t)q_rows * sw * pair * min_buf > budget) sw >>= 1;
@@ -237,12 +235,13 @@ LayerLaunch shape_layer(const Plan &P, int t, int rank, size_t es, int sm_count)
     // producer items: 2 ft parent rows x one live tile; consumer items: the member tiles
     s.n_pitems = live ? (sw / s.ft) * L.n_live_tiles : 0;
     s.n_citems = L.n_mtiles;
-    s.discard = env_int("GENLIB_DISCARD", 2);     // 0: off, 1: without the release fence (experiments), 2: on
-    // One CTA per SM: four producer warps and a consumer group of eight.  Every CTA of a gang takes part in the
-    // hand-over of each of the gang's strips, whether it has an item there or not, and a switch of strips costs a
-    // CTA some microseconds of dependent loads: a strip should bring every CTA several items.  Layers with short
-    // strips (few live tiles) therefore split the CTAs into G gangs that work on G strips side by side
-    // (profiles/r02/README.md: C5 245 -> ... ms, genea140 7.3 -> ... ms); C3-sized layers stay with one gang.
+    s.discard = env_int("GENLIB_DISCARD", 1) != 0;     // 0: off
+    // One CTA per SM: four producer warps and eight consumer warps (eight and four with carried columns, below).
+    // Every CTA of a gang takes part in the hand-over of each of the gang's strips, whether it has an item there or
+    // not, and a switch of strips costs a CTA some microseconds of dependent loads: a strip should bring every CTA
+    // several items.  Layers with short strips (few live tiles) therefore split the CTAs into G gangs that work on
+    // G strips side by side (profiles/r02/README.md: C5 245 -> ... ms, genea140 7.3 -> ... ms); C3-sized layers stay
+    // with one gang.
     const int max_buf = (int)std::max<size_t>(2, budget / strip_bytes);
     int G = 1;
     if (live) {
@@ -261,21 +260,19 @@ LayerLaunch shape_layer(const Plan &P, int t, int rank, size_t es, int sm_count)
     const int few = G == 1 && (sw / s.ft) * L.n_live_tiles < 3 * sm_count / 2 ? sm_count - sm_count / 8 : sm_count;
     const int ctas = std::max(1, std::min(sm_count, env_int("GENLIB_CTAS_PER_ROLE", few))) / G;   // per gang
     s.n_prod = G * std::min(ctas, s.n_pitems);
-    s.groups = groups;
-    s.n_cons = G * std::min(ctas * groups, s.n_citems);
+    s.n_cons = G * std::min(ctas, s.n_citems);
     const size_t stage = (size_t)2 * s.ft * (kPTile * es + 16);
     // eight producer warps (and four consumer warps) where the producers have the carried columns to write as well
     {
         const int forced = env_int("GENLIB_PROD_WARPS", 0);
-        out.prod_warps = forced == 4 || forced == 8 ? forced : (L.carried > 0 && live && kConsGroups == 1 ? 8 : 4);
+        out.prod_warps = forced == 4 || forced == 8 ? forced : (L.carried > 0 && live ? 8 : 4);
     }
     const size_t cons_bytes = layer_consumer_bytes(sw, es, out.prod_warps);
     const size_t smem_cap = (size_t)227 * 1024 - 2048;      // (static shared memory and the driver's share)
-    s.stages = (int)std::max<size_t>(2, std::min<size_t>((size_t)std::min(kMaxStages, env_int("GENLIB_STAGES", kMaxStages)), (smem_cap - groups * cons_bytes) / stage));
-    s.cons_bytes = (int32_t)cons_bytes;
-    s.ring_off = (int32_t)(groups * cons_bytes);
-    out.smem = groups * cons_bytes + (size_t)s.stages * stage;
-    out.grid = std::max(s.n_prod, (s.n_cons + groups - 1) / groups);
+    s.stages = (int)std::max<size_t>(2, std::min<size_t>((size_t)std::min(kMaxStages, env_int("GENLIB_STAGES", kMaxStages)), (smem_cap - cons_bytes) / stage));
+    s.ring_off = (int32_t)cons_bytes;
+    out.smem = cons_bytes + (size_t)s.stages * stage;
+    out.grid = std::max(s.n_prod, s.n_cons);
     s.timeout_cycles = (long long)4e9;                     // ~2 s: a lost dependency becomes GENLIB_ECUDA, not a hang
     return out;
 }
@@ -339,11 +336,9 @@ LayerArgs layer_args(const genlib_engine &E, int t) {
     const Layer &L = P.layers[t];
     LayerArgs a;
     std::memset(&a, 0, sizeof a);
-    a.n_new = L.n_new; a.n_fam = L.n_fam; a.rt_lo = L.rt_lo; a.rt_rows = L.live_before > 0 ? L.rt_rows : 0; a.nf_pad = L.nf_pad;
+    a.n_new = L.n_new; a.n_fam = L.n_fam; a.rt_lo = L.rt_lo;
     a.any_carried = L.carried > 0;
-    a.rank = E.rank; a.world = E.world;
     const int32_t *fb = P.fam_base.data() + L.base_off, *mb = P.mem_base.data() + L.base_off;
-    for (int g = 0; g <= E.world; g++) a.fam_base[g] = fb[g];
     a.own_f0 = fb[E.rank]; a.own_nf = fb[E.rank + 1] - fb[E.rank];
     a.own_m0 = mb[E.rank]; a.own_nm = mb[E.rank + 1] - mb[E.rank];
     a.mem_ind = E.mem_ind.p + L.mem_off; a.mem_slot = E.mem_slot.p + L.mem_off; a.mem_fam = E.mem_fam.p + L.mem_off;
@@ -355,7 +350,6 @@ LayerArgs layer_args(const genlib_engine &E, int t) {
     a.fam_start = E.fam_start.p + L.fam_off + t;
     a.flags = E.flags.p + L.flag_off;
     a.live_owner = E.live_owner.p + L.flag_off; a.live_lrow = E.live_lrow.p + L.flag_off;
-    a.tile_map = E.tile_map.p + L.tile_off;
     a.mt_desc = reinterpret_cast<const int4 *>(E.mt_desc.p) + L.mtile_off;
     a.n_mtiles = L.n_mtiles;
     return a;
@@ -719,25 +713,6 @@ int create_engine(const genlib_plan *plan, int numerics, int device, int rank, g
         if ((size_t)(cur - base) > need) return fail(GENLIB_EINVAL, "internal: arena layout overflow");
         if ((size_t)(static_cast<unsigned char *>(E->A) - base) != off_A())
             return fail(GENLIB_EINVAL, "internal: peer-visible arena offsets drifted");
-    }
-    // Optional (GENLIB_L2_PERSIST=1): a persisting access-policy window for the strip buffers on the engine's
-    // stream.  Off by default: it limits the buffers to the 79 MB that can persist and measured slower.
-    {
-        int max_persist = 0, max_window = 0;
-        cudaDeviceGetAttribute(&max_persist, cudaDevAttrMaxPersistingL2CacheSize, E->device);
-        cudaDeviceGetAttribute(&max_window, cudaDevAttrMaxAccessPolicyWindowSize, E->device);
-        const char *env = std::getenv("GENLIB_L2_PERSIST");                // "1": persisting window (measured slower, see kStripBudget)
-        if (max_persist > 0 && max_window > 0 && env && env[0] == '1') {
-            cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)max_persist);
-            cudaStreamAttrValue attr;
-            std::memset(&attr, 0, sizeof attr);
-            attr.accessPolicyWindow.base_ptr = E->Q;
-            attr.accessPolicyWindow.num_bytes = std::min<size_t>(E->q_bytes, (size_t)max_window);
-            attr.accessPolicyWindow.hitRatio = (float)std::min(1.0, (double)max_persist / (double)std::max<size_t>(E->q_bytes, 1));
-            attr.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            attr.accessPolicyWindow.missProp = cudaAccessPropertyNormal;
-            if (cudaStreamSetAttribute(E->stream, cudaStreamAttributeAccessPolicyWindow, &attr) != cudaSuccess) cudaGetLastError();
-        }
     }
     CU(cudaMemsetAsync(E->bar_flags, 0, kFlagBytes, E->stream));
     if (!streamed) {

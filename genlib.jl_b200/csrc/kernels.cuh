@@ -25,48 +25,29 @@ struct PeerTable {
 };
 
 struct LayerArgs {
-    int32_t n_new, n_fam, rt_lo, rt_rows, nf_pad, any_carried;
+    int32_t n_new, n_fam, rt_lo, any_carried;
     // row sharding: this rank owns couples [own_f0, own_f0 + own_nf) and members [own_m0, own_m0 + own_nm)
-    int32_t rank, world, own_f0, own_nf, own_m0, own_nm;
-    int32_t fam_base[kMaxWorld + 1];
+    int32_t own_f0, own_nf, own_m0, own_nm;
     const int32_t *mem_ind, *mem_slot, *mem_fam, *mem_lrow;     // members: rank (or queue position), column slot, couple, local row
     const int32_t *fam_pf, *fam_pm, *fam_start;                  // couples: parent slots (-1 none), first member
     const int2 *fam_q;                                           // couples: the parents' rows in a strip buffer (-1 none)
     const int8_t *fam_pf_owner, *fam_pm_owner, *live_owner;      // where the parents' / the live individuals' rows are
     const int32_t *fam_pf_lrow, *fam_pm_lrow, *live_lrow;
     const uint8_t *flags;                                        // per slot of the live range: kFlagLive | kFlagCarried
-    const int32_t *tile_map;                                     // per tile of the live range: index among the live tiles (-1: hole)
     const int4 *mt_desc;                                         // member tiles: first couple, couples, first member, members
     int32_t n_mtiles;
 };
 
 constexpr int kThreads = 256;
 
-// ---- 4-wide row-segment access ------------------------------------------------------
-__device__ __forceinline__ void load4(const float *p, double (&d)[4]) {
-    float4 v = __ldg(reinterpret_cast<const float4 *>(p));
-    d[0] = v.x; d[1] = v.y; d[2] = v.z; d[3] = v.w;
-}
-__device__ __forceinline__ void load4(const double *p, double (&d)[4]) {
-    double2 a = __ldg(reinterpret_cast<const double2 *>(p));
-    double2 b = __ldg(reinterpret_cast<const double2 *>(p) + 1);
-    d[0] = a.x; d[1] = a.y; d[2] = b.x; d[3] = b.y;
-}
-__device__ __forceinline__ void store4(float *p, const double (&d)[4]) {
-    // (float)double is cvt.rn.f32.f64: round-to-nearest-even, subnormals kept (no -ftz)
-    float4 v = make_float4((float)d[0], (float)d[1], (float)d[2], (float)d[3]);
-    *reinterpret_cast<float4 *>(p) = v;
-}
-__device__ __forceinline__ void store4(double *p, const double (&d)[4]) {
-    reinterpret_cast<double2 *>(p)[0] = make_double2(d[0], d[1]);
-    reinterpret_cast<double2 *>(p)[1] = make_double2(d[2], d[3]);
-}
+// ---- 4-wide row-segment stores -------------------------------------------------------
 // New frontier rows are written once and read by the NEXT step's kernel at the earliest: streaming stores
 // (st.global.cs, evict-first) keep them from pushing the strip buffers out of L2.
-__device__ __forceinline__ void store4(float *p, const double (&d)[4], int) {
+__device__ __forceinline__ void store4(float *p, const double (&d)[4]) {
+    // (float)double is cvt.rn.f32.f64: round-to-nearest-even, subnormals kept (no -ftz)
     __stcs(reinterpret_cast<float4 *>(p), make_float4((float)d[0], (float)d[1], (float)d[2], (float)d[3]));
 }
-__device__ __forceinline__ void store4(double *p, const double (&d)[4], int) {
+__device__ __forceinline__ void store4(double *p, const double (&d)[4]) {
     __stcs(reinterpret_cast<double2 *>(p), make_double2(d[0], d[1]));
     __stcs(reinterpret_cast<double2 *>(p) + 1, make_double2(d[2], d[3]));
 }
@@ -96,15 +77,9 @@ __device__ __forceinline__ double half_sum_mode(double x, double y) {
     else return half_sum(x, y);
 }
 
-constexpr int kMaxPChunk = 32;               // live-column tiles per producer unit (upper bound)
-
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
-// 16 bytes global -> shared, cached in L2 only (coherent with what other SMs wrote before they signalled)
-__device__ __forceinline__ void cp_async16_to(unsigned smem, const void *gmem) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(smem), "l"(gmem) : "memory");
-}
 
 // mbarrier + bulk-copy (TMA, SASS UBLKCP) helpers
 __device__ __forceinline__ void mbar_init(unsigned bar, int count) {
@@ -132,8 +107,11 @@ __device__ __forceinline__ void bulk_g2s_hint(unsigned dst, const void *src, uns
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar), "l"(pol) : "memory");
 }
-__device__ __forceinline__ void zero16_shared(unsigned smem) {
-    asm volatile("st.shared.v4.u32 [%0], {%1, %1, %1, %1};\n" ::"r"(smem), "r"(0) : "memory");
+// An unknown parent contributes 0 (compute.jl:111-126): its row (`bytes`, a multiple of 16) is zeroed instead of copied.
+// Bulk copies (async proxy) fill the same place at other times: the fence orders these ordinary stores against them.
+__device__ __forceinline__ void zero_row_shared(unsigned smem, unsigned bytes) {
+    for (unsigned c = 0; c < bytes; c += 16) asm volatile("st.shared.v4.u32 [%0], {%1, %1, %1, %1};\n" ::"r"(smem + c), "r"(0) : "memory");
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 __device__ __forceinline__ void lds4(const float *p, double (&d)[4]) {
     const float4 v = *reinterpret_cast<const float4 *>(p);
