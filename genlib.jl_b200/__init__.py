@@ -1,4 +1,4 @@
-"""genlib.jl_b200 -- B200-native kinship engine behind GenLib.jl's `gen.phi` (and `gen.gc`, `gen.occ`, `gen.rec`).
+"""genlib.jl_b200 -- B200-native kinship engine behind GenLib.jl's `gen.phi` (and `gen.gc`, `gen.occ`, `gen.rec`, `gen.findMRCA`).
 
 Usage mirrors the reference (`import GenLib as gen`):
     import genlib_b200 as gen
@@ -7,12 +7,14 @@ Usage mirrors the reference (`import GenLib as gen`):
     g = gen.gc(ped)                        # float64, gen.pro(ped) x gen.founder(ped)
     o = gen.occ(ped)                       # int64 path counts, gen.founder(ped) x gen.pro(ped)
     r = gen.rec(ped)                       # int64, probands descending from each founder
+    m = gen.findMRCA(ped, [1, 2])          # GenMatrix: MRCAs sorted by ID, int64 meioses
 """
 import os as _os
 
 from .pedigree import Individual, Pedigree, founder, genealogy, pro  # noqa: F401
-from .engine import (Engine, GcPlan, KinshipMatrix, PinnedMatrix, Plan, f, gc, gc_arrays, occ, occ_arrays,  # noqa: F401
-                     phi, phi_arrays, phi_distributed, phiMean, rec, rec_arrays, run_distributed, sparse_phi)
+from .engine import (Engine, GcPlan, GenMatrix, KinshipMatrix, PinnedMatrix, Plan, f, findDistance,  # noqa: F401
+                     findMRCA, gc, gc_arrays, meioses_arrays, mrca_arrays, occ, occ_arrays, phi, phi_arrays,
+                     phi_distributed, phiMean, rec, rec_arrays, run_distributed, sparse_phi)
 from . import synth  # noqa: F401
 from ._lib import GenlibError, GenlibOverflowError, LIB_PATH, PlanBoundsExceeded, lib  # noqa: F401
 

@@ -146,6 +146,9 @@ SYMBOLS = {
                              C.POINTER(GcStats)]),
     "genlib_rec": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int32, _P,
                              C.POINTER(GcStats)]),
+    "genlib_meioses": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int, C.c_int32, _P,
+                                 C.POINTER(GcStats)]),
+    "genlib_mrca": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, _P, C.c_int32, _P, C.POINTER(GcStats)]),
 }
 
 _lib = None

@@ -1,4 +1,4 @@
-// gc_engine.cu -- gen.gc, gen.occ and gen.rec on the device (DESIGN.md 2b, 2c): the C ABI entry points, the split of
+// gc_engine.cu -- gen.gc, gen.occ, gen.rec and gen.findMRCA on the device (DESIGN.md 2b-2d): the C ABI entry points, the split of
 // the column-side list over the devices and each device's run of the plan (gc_plan.hpp) with the kernels of
 // gc_kernel.cuh.
 #include <cstdio>
@@ -8,6 +8,7 @@
 #include "runtime.hpp"
 #include "gc_kernel.cuh"
 #include "gc_plan.hpp"
+#include "plan.hpp"
 
 using namespace genlib;
 
@@ -18,10 +19,18 @@ struct genlib_gc_plan {
 
 namespace {
 
-// What a run of the gc plan computes: gen.gc's matrix, gen.occ's matrix or row sums, gen.rec's counts.
-enum GcFn { kFnGc = 0, kFnOcc, kFnOccTotal, kFnRec };
-const char *const kGcFnName[] = {"gc", "occ", "occ", "rec"};     // gen.<name> in Python, genlib_<name> in C
+// What a run of the gc plan computes: gen.gc's matrix, gen.occ's matrix or row sums, gen.rec's counts, the
+// meioses matrix of gen.findMRCA / gen.findDistance.
+enum GcFn { kFnGc = 0, kFnOcc, kFnOccTotal, kFnRec, kFnMeioses };
+const char *const kGcFnName[] = {"gc", "occ", "occ", "rec", "meioses"};   // genlib_<name> in C
 bool gc_fn_reduces(int fn) { return fn == kFnOccTotal || fn == kFnRec; }
+// gen.occ's matrix is the one output whose gather reports saturated counts (an 8-byte key on the device)
+bool gc_fn_reports_overflow(int fn) { return fn == kFnOcc; }
+// 8-byte words of a 16-byte-padded row of `cols` columns
+int64_t gc_fn_words(int fn, int64_t cols) {
+    const int64_t w = fn == kFnRec ? (cols + 63) / 64 : fn == kFnMeioses ? (cols + 3) / 4 : cols;
+    return (w + 1) / 2 * 2;
+}
 
 // One device's share: column positions [j0, j1) of the column-side list and the unique columns [lo, hi) they
 // name (contiguous when the list has no duplicates; a duplicate may widen the range, never the result).
@@ -29,11 +38,9 @@ struct GcShare {
     int device = -1;
     int fn = kFnGc;
     int32_t j0 = 0, j1 = 0, lo = 0, hi = 0;
-    // row stride in 8-byte elements (16-byte rows): a column each, or for gen.rec 64 columns per word
-    int64_t ws() const {
-        const int64_t w = fn == kFnRec ? ((int64_t)(hi - lo) + 63) / 64 : (int64_t)(hi - lo);
-        return (w + 1) / 2 * 2;
-    }
+    // row stride in 8-byte elements (16-byte rows): a column each, for gen.rec 64 columns per word, for the
+    // meioses 4 uint16 columns per word
+    int64_t ws() const { return gc_fn_words(fn, hi - lo); }
     size_t stage = 0, need = 0;
     double ms_kernels = 0, ms_fetch = 0;
     int32_t launches = 0;
@@ -43,10 +50,10 @@ struct GcShare {
 };
 
 // Required traffic of a share over `cols` columns: the plan's byte model over the row's 8-byte elements
-// (gen.rec: its words, 16-byte padded as the kernel moves them), plus one read of the output block for a
-// reduction.
+// (gen.rec and the meioses: their words, 16-byte padded as the kernel moves them), plus one read of the
+// output block for a reduction.
 double gc_fn_bytes(const GcPlan &P, int fn, int32_t cols) {
-    const int64_t w = fn == kFnRec ? (((int64_t)cols + 63) / 64 + 1) / 2 * 2 : cols;
+    const int64_t w = fn == kFnRec || fn == kFnMeioses ? gc_fn_words(fn, cols) : cols;
     double b = P.alg_bytes(w);
     if (gc_fn_reduces(fn)) b += (double)P.n_targets() * (double)w * 8.0;
     return b;
@@ -87,7 +94,7 @@ size_t gc_device_bytes(const GcPlan &P, GcShare &d, int col_major, size_t esize)
            3 * DevBuf<int32_t>::padded(R) + DevBuf<int64_t>::padded(R + 1) + DevBuf<int32_t>::padded((size_t)P.inputs()) +
            DevBuf<int32_t>::padded(P.target_uid().size()) + DevBuf<int32_t>::padded((size_t)(d.j1 - d.j0)) +
            DevBuf<int32_t>::padded(1) + 2 * d.stage +
-           (d.fn == kFnGc ? 0 : DevBuf<unsigned long long>::padded(1)) + (gc_fn_reduces(d.fn) ? gc_reduce_bytes(P, d) : 0);
+           (gc_fn_reports_overflow(d.fn) ? DevBuf<unsigned long long>::padded(1) : 0) + (gc_fn_reduces(d.fn) ? gc_reduce_bytes(P, d) : 0);
 }
 
 template <typename E, typename O>
@@ -99,7 +106,7 @@ int gc_fetch(const GcPlan &P, GcShare &d, const void *Oblk, const int32_t *tgt_r
     int rc = staged_d2h(st, cst, reinterpret_cast<O *>(stage_base), reinterpret_cast<O *>(stage_base + d.stage), L.nmaj, per, "gc fetch",
         [&](O *stage, int64_t m0, int64_t nb) {
             GcGatherArgs a;
-            a.O = Oblk; a.ws = d.ws(); a.tgt_row = tgt_row; a.col = col;
+            a.O = Oblk; a.ws = d.ws() * (int64_t)(8 / sizeof(E)); a.tgt_row = tgt_row; a.col = col;
             a.ovf = ovf; a.j0 = d.j0; a.n_pro = P.n_pro; a.tgt_is_pro = P.direction == kGcDescend;
             if (L.cmaj) { a.t0 = 0; a.n_t = (int32_t)L.nmin; a.c0 = (int32_t)m0; a.n_c = (int32_t)nb; }
             else        { a.t0 = (int32_t)m0; a.n_t = (int32_t)nb; a.c0 = 0; a.n_c = (int32_t)L.nmin; }
@@ -167,7 +174,7 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
     col.place(cur, (size_t)(d.j1 - d.j0)); err.place(cur, 1);
     unsigned char *stage = cur;
     cur += 2 * d.stage;
-    if (d.fn != kFnGc) ovf.place(cur, 1);
+    if (gc_fn_reports_overflow(d.fn)) ovf.place(cur, 1);
     // reduction weights: how often the lists name each column (ascend) or each target row (descend)
     std::vector<uint32_t> h_wt;
     std::vector<unsigned long long> h_m1, h_m2;
@@ -198,13 +205,13 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
     CU(in_ptr.upload(P.in_ptr, res.st)); CU(in_slot.upload(P.in_slot, res.st)); CU(tgt_row.upload(P.target_uid(), res.st));
     CU(col.upload(cols, res.st));
     CU(cudaMemsetAsync(err.p, 0, sizeof(int32_t), res.st));
-    if (d.fn != kFnGc) CU(cudaMemsetAsync(ovf.p, 0xff, sizeof(unsigned long long), res.st));
+    if (gc_fn_reports_overflow(d.fn)) CU(cudaMemsetAsync(ovf.p, 0xff, sizeof(unsigned long long), res.st));
     if (reduce) {
         CU(wt.upload(h_wt, res.st)); CU(m1.upload(h_m1, res.st)); CU(m2.upload(h_m2, res.st));
         if (!asc) CU(cudaMemsetAsync(red.p, 0, W * sizeof(unsigned long long), res.st));
     }
     if (P.n_out_rows < P.n_targets())                       // a target no path reaches: its output row is 0
-        CU(cudaMemsetAsync(O, 0, T * ws * 8, res.st));
+        CU(cudaMemsetAsync(O, d.fn == kFnMeioses ? 0xFF : 0, T * ws * 8, res.st));   // (meioses: unreachable)
     GcLayerArgs a;
     a.F = F; a.O = O;
     a.w2 = (int64_t)ws / 2; a.width = d.hi - d.lo; a.col_lo = d.lo;
@@ -218,6 +225,7 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
         a.row_slot = row_slot.p + r0; a.row_seed = row_seed.p + r0; a.row_out = row_out.p + r0; a.in_ptr = in_ptr.p + r0;
         if (d.fn == kFnGc) gc_launch_layer<GcOpHalfSum>(a, gx, res.st);
         else if (d.fn == kFnRec) gc_launch_layer<GcOpReach>(a, gx, res.st);
+        else if (d.fn == kFnMeioses) gc_launch_layer<GcOpMinPlus>(a, gx, res.st);
         else gc_launch_layer<GcOpCount>(a, gx, res.st);
         CU(cudaGetLastError());
         d.launches++;
@@ -262,6 +270,8 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
     } else if (d.fn == kFnOcc) {
         rc = gc_fetch<unsigned long long, int64_t>(P, d, O, tgt_row.p, col.p, static_cast<int64_t *>(out), col_major, stage, ovf.p, res.st, res.cst);
         if (rc == GENLIB_OK) CU(cudaMemcpy(&d.ovf, ovf.p, sizeof d.ovf, cudaMemcpyDeviceToHost));
+    } else if (d.fn == kFnMeioses) {
+        rc = gc_fetch<uint16_t, int64_t>(P, d, O, tgt_row.p, col.p, static_cast<int64_t *>(out), col_major, stage, nullptr, res.st, res.cst);
     } else {
         rc = out_dtype == GENLIB_F64
             ? gc_fetch<double, double>(P, d, O, tgt_row.p, col.p, static_cast<double *>(out), col_major, stage, nullptr, res.st, res.cst)
@@ -372,6 +382,9 @@ int gc_driver(int fn, int32_t n, const int32_t *father, const int32_t *mother, i
     if (int rc = genlib_gc_plan_create(n, father, mother, n_pro, proband, n_anc, ancestor, &plan)) return rc;
     std::unique_ptr<genlib_gc_plan> owner(plan);
     const GcPlan &P = plan->p;
+    if (fn == kFnMeioses && P.n_layers() >= (int32_t)kMeiosesNone)   // d <= n_layers - 1 must stay below the sentinel
+        return fail(GENLIB_EOVERFLOW, who + ": " + std::to_string(P.n_layers()) + " layers: a distance could reach "
+                    "the uint16 sentinel 0xFFFF");
     genlib_gc_stats st;
     gc_fill_stats(P, &st);
     st.alg_bytes = gc_fn_bytes(P, fn, P.width());
@@ -483,6 +496,64 @@ int genlib_rec(int32_t n, const int32_t *father, const int32_t *mother, int32_t 
                int32_t n_anc, const int32_t *ancestor, int64_t *out, int32_t n_dev, const int32_t *devices,
                genlib_gc_stats *stats) {
     return gc_driver(kFnRec, n, father, mother, n_pro, proband, n_anc, ancestor, out, 0, 0, n_dev, devices, stats);
+}
+
+int genlib_meioses(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                   int32_t n_anc, const int32_t *ancestor, int64_t *out, int col_major, int32_t n_dev,
+                   const int32_t *devices, genlib_gc_stats *stats) {
+    return gc_driver(kFnMeioses, n, father, mother, n_pro, proband, n_anc, ancestor, out, 0, col_major, n_dev,
+                     devices, stats);
+}
+
+int genlib_mrca(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_ids, const int32_t *ids,
+                int32_t *mrca, int32_t *n_mrca, int32_t n_dev, const int32_t *devices, genlib_gc_stats *stats) {
+    if (n < 0 || n_ids < 0 || (n > 0 && (!father || !mother)) || (n_ids > 0 && !ids) || !n_mrca || (n > 0 && !mrca))
+        return fail(GENLIB_EINVAL, "genlib_mrca: null pointer or negative size");
+    try {
+        *n_mrca = 0;
+        std::string err;
+        if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);
+        std::vector<uint8_t> listed((size_t)n, 0);
+        std::vector<int32_t> uniq;                               // the distinct IDs, first occurrence order
+        for (int32_t k = 0; k < n_ids; k++) {
+            const int32_t x = ids[k];
+            if (x < 0 || x >= n) return fail(GENLIB_EKEY, "KeyError: ID index " + std::to_string(x) + " not in pedigree");
+            if (!listed[(size_t)x]) { listed[(size_t)x] = 1; uniq.push_back(x); }
+        }
+        if (uniq.empty()) {
+            if (stats) std::memset(stats, 0, sizeof *stats);
+            return GENLIB_OK;
+        }
+        // S = the ancestors-or-self of the IDs (a reverse sweep: children have larger ranks), in ascending rank
+        std::vector<uint8_t> in_s(listed);
+        for (int32_t i = n - 1; i >= 0; i--) {
+            if (!in_s[(size_t)i]) continue;
+            if (father[i] >= 0) in_s[(size_t)father[i]] = 1;
+            if (mother[i] >= 0) in_s[(size_t)mother[i]] = 1;
+        }
+        std::vector<int32_t> S;
+        for (int32_t i = 0; i < n; i++) if (in_s[(size_t)i]) S.push_back(i);
+        // on the devices: how many distinct IDs descend from (or are) each member of S
+        std::vector<int64_t> cnt(S.size());
+        if (int rc = gc_driver(kFnRec, n, father, mother, (int32_t)uniq.size(), uniq.data(), (int32_t)S.size(), S.data(),
+                               cnt.data(), 0, 0, n_dev, devices, stats))
+            return rc;
+        // common: a proper ancestor of every ID; an MRCA: a common ancestor none of whose children is common
+        std::vector<uint8_t> common((size_t)n, 0), parent_of_common((size_t)n, 0);
+        for (size_t k = 0; k < S.size(); k++) {
+            const int32_t a = S[k];
+            if (cnt[k] != (int64_t)uniq.size() || listed[(size_t)a]) continue;
+            common[(size_t)a] = 1;
+            if (father[a] >= 0) parent_of_common[(size_t)father[a]] = 1;
+            if (mother[a] >= 0) parent_of_common[(size_t)mother[a]] = 1;
+        }
+        int32_t m = 0;
+        for (int32_t a : S) if (common[(size_t)a] && !parent_of_common[(size_t)a]) mrca[m++] = a;
+        *n_mrca = m;
+        return GENLIB_OK;
+    } catch (const std::bad_alloc &) {
+        return fail(GENLIB_ENOMEM, "genlib_mrca: out of host memory");
+    }
 }
 
 }  // extern "C"

@@ -1,17 +1,19 @@
-// gc_kernel.cuh -- the sm_100a kernels of gen.gc, gen.occ and gen.rec (DESIGN.md 2b, 2c).
+// gc_kernel.cuh -- the sm_100a kernels of gen.gc, gen.occ, gen.rec and gen.findMRCA (DESIGN.md 2b, 2c, 2d).
 //
 // gc_layer_kernel<Op>: one launch per layer.  A CTA takes a chunk of columns (threads per row x kGcVec
 // 16-byte vectors) for a group of the layer's rows -- several rows per CTA when rows are narrow; per row it
 // combines the input rows in CSR order, finishes the row with the seed in the row's own column and writes
 // it to its frontier slot and/or (streaming store: never read again by a layer) its output-block row.  For
 // gen.gc the order of the additions is part of the result's contract: ((0 + in_1) + in_2) + ..., then
-// 1/2 * sum + seed.  gen.occ adds counts with saturation, gen.rec ORs bit rows: both are order-free.
+// 1/2 * sum + seed.  gen.occ adds counts with saturation, gen.rec ORs bit rows, the meioses of gen.findMRCA
+// take the minimum of saturating uint16 sums: all three are order-free.
 //
 // gc_row_reduce_kernel / gc_col_reduce_kernel: the row sums of gen.occ(typeOcc = "TOTAL") and the counts of
 // gen.rec, one pass over the output block, so the matrix never leaves the device.
 //
 // gc_gather_kernel: a 32 x 32 tile of the output block, with duplicates of either list expanded, to a
-// staging buffer in the layout of the caller's matrix (row- or column-major; float64, float32 or int64),
+// staging buffer in the layout of the caller's matrix (row- or column-major; float64, float32 or int64; uint16
+// distances widen to int64),
 // transposed through shared memory where the output block's rows are the matrix's columns.
 #pragma once
 #include <cstdint>
@@ -73,6 +75,35 @@ struct GcOpReach {              // gen.rec: reachability, 64 columns per uint64 
         if (seed >= 0 && (seed >> 7) == c) {
             const unsigned long long bit = 1ull << (seed & 63);
             if (seed & 64) a.y |= bit; else a.x |= bit;
+        }
+        return a;
+    }
+};
+
+// gen.findMRCA / gen.findDistance: the shortest descent path in the (min, +1) semiring, eight uint16 distances
+// per vector, 0xFFFF = unreachable.  +1 saturates at 0xFFFF, so an unreachable input stays unreachable; the
+// host refuses plans of 0xFFFF layers or more, so a reachable distance (< layers) never meets the sentinel.
+// Descending the inputs are the parents and the columns ancestors, ascending the children and the columns
+// probands: the same rules give d(ancestor, proband) both ways.
+constexpr uint16_t kMeiosesNone = 0xFFFF;
+struct GcOpMinPlus {
+    using V = uint4;
+    static constexpr int kColsPerVec = 8;
+    __device__ static V zero() { return make_uint4(~0u, ~0u, ~0u, ~0u); }
+    __device__ static void add(V &a, V x) {
+        constexpr unsigned one = 0x00010001u;
+        a.x = __vminu2(a.x, __vaddus2(x.x, one)); a.y = __vminu2(a.y, __vaddus2(x.y, one));
+        a.z = __vminu2(a.z, __vaddus2(x.z, one)); a.w = __vminu2(a.w, __vaddus2(x.w, one));
+    }
+    __device__ static V finish(V a, int64_t c, int32_t seed) {
+        if (seed >= 0 && (seed >> 3) == c) {
+            const unsigned keep = (seed & 1) ? 0x0000FFFFu : 0xFFFF0000u;   // d(p, p) = 0
+            switch ((seed >> 1) & 3) {
+                case 0: a.x &= keep; break;
+                case 1: a.y &= keep; break;
+                case 2: a.z &= keep; break;
+                default: a.w &= keep; break;
+            }
         }
         return a;
     }
@@ -234,7 +265,7 @@ __global__ void __launch_bounds__(256) gc_col_reduce_kernel(GcColReduceArgs a) {
 }
 
 struct GcGatherArgs {
-    const void *O;              // output block, rows of ws 8-byte elements
+    const void *O;              // output block, rows of ws elements of E
     int64_t ws;
     const int32_t *tgt_row;     // target list position -> output-block row
     const int32_t *col;         // column list position (the device's range) -> local column
@@ -246,6 +277,13 @@ struct GcGatherArgs {
     int32_t j0, n_pro;          // list position of the device's first column; proband list length
     int32_t tgt_is_pro;         // the targets are the probands (descend)
 };
+
+// An output-block element as the caller's type: a uint16 distance widens, the unreachable sentinel to -1.
+template <typename Out, typename E>
+__device__ __forceinline__ Out gc_widen(E v) {
+    if constexpr (std::is_same<E, uint16_t>::value) return v == kMeiosesNone ? (Out)-1 : (Out)v;
+    else return (Out)v;
+}
 
 // stage (major x minor, minor contiguous): C_MAJOR = false: major = target, minor = column position;
 // C_MAJOR = true: major = column position, minor = target.  Tiles of 32 x 32, 32 x 8 threads.
@@ -275,7 +313,7 @@ __global__ void __launch_bounds__(256) gc_gather_kernel(GcGatherArgs a, Out *sta
         if (!C_MAJOR) {
             for (int k = ty; k < 32; k += 8) {
                 const int32_t t = tb + k;
-                if (t < a.n_t && c < a.n_c) stage[(int64_t)t * a.n_c + c] = (Out)tile[k][tx];
+                if (t < a.n_t && c < a.n_c) stage[(int64_t)t * a.n_c + c] = gc_widen<Out>(tile[k][tx]);
             }
             continue;
         }
@@ -283,7 +321,7 @@ __global__ void __launch_bounds__(256) gc_gather_kernel(GcGatherArgs a, Out *sta
         // write: lanes along the targets
         for (int k = ty; k < 32; k += 8) {
             const int32_t cc = cb + k, t = tb + tx;
-            if (t < a.n_t && cc < a.n_c) stage[(int64_t)cc * a.n_t + t] = (Out)tile[tx][k];
+            if (t < a.n_t && cc < a.n_c) stage[(int64_t)cc * a.n_t + t] = gc_widen<Out>(tile[tx][k]);
         }
         __syncthreads();
     }

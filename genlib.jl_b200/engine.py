@@ -560,6 +560,102 @@ def rec_arrays(father, mother, proband_ranks, ancestor_ranks, *, device: int = -
     return out, stats
 
 
+class GenMatrix:
+    """gen.GenMatrix (src/identify.jl:129-133), what `findMRCA` returns: `individuals` (the IDs as given),
+    `ancestors` (the MRCAs, sorted by ID) and `meioses[i, j]`, the number of meioses on the shortest descent
+    path from ancestors[j] down to individuals[i] (Int64)."""
+
+    def __init__(self, individuals, ancestors, meioses):
+        self.individuals = np.asarray(individuals, np.int64)
+        self.ancestors = np.asarray(ancestors, np.int64)
+        self.meioses = np.asarray(meioses, np.int64)
+        if self.meioses.shape != (len(self.individuals), len(self.ancestors)):
+            raise ValueError("meioses must be len(individuals) x len(ancestors)")
+
+    def __repr__(self) -> str:
+        return (f"GenMatrix({len(self.individuals)} individuals x {len(self.ancestors)} ancestors: "
+                f"{self.ancestors.tolist()})")
+
+
+def meioses_arrays(father, mother, proband_ranks, ancestor_ranks, *, device: int = -1, devices=None,
+                   out: Optional[np.ndarray] = None, col_major: bool = False):
+    """One-shot C-ABI call `genlib_meioses` on flat rank arrays.  Returns (matrix, stats): the
+    len(pro) x len(ancestors) int64 minimum meioses from each ancestor down to each proband, -1 where the
+    proband does not descend from the ancestor (0 on the diagonal a == p); col_major=True: Fortran order."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32)
+    an = np.ascontiguousarray(ancestor_ranks, np.int32)
+    shape = (len(pr), len(an))
+    if out is None:
+        out = np.empty(shape, np.int64, order="F" if col_major else "C")
+    contiguous = out.flags.f_contiguous if col_major else out.flags.c_contiguous
+    if out.shape != shape or not contiguous or out.dtype != np.int64:
+        raise ValueError(f"out must be a {'Fortran' if col_major else 'C'}-contiguous {shape} int64 array")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = GcStats()
+    check(lib().genlib_meioses(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), len(an), ptr(an), ptr(out),
+                               int(col_major), len(dv), ptr(dv), C.byref(st)))
+    stats = st.as_dict()
+    stats["direction"] = _lib.GC_DIRECTIONS[stats["direction"]]
+    return out, stats
+
+
+def mrca_arrays(father, mother, ranks, *, device: int = -1, devices=None):
+    """One-shot C-ABI call `genlib_mrca` on flat rank arrays.  Returns (MRCA ranks ascending, stats of the
+    device pass that decides who is a common ancestor)."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    r = np.ascontiguousarray(ranks, np.int32)
+    out = np.empty(max(len(father), 1), np.int32)
+    m = C.c_int32(0)
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = GcStats()
+    check(lib().genlib_mrca(len(father), ptr(father), ptr(mother), len(r), ptr(r), ptr(out), C.byref(m), len(dv),
+                            ptr(dv), C.byref(st)))
+    stats = st.as_dict()
+    stats["direction"] = _lib.GC_DIRECTIONS[stats["direction"]]
+    return out[:m.value].copy(), stats
+
+
+def findMRCA(pedigree: Pedigree, IDs, *, device: int = -1, devices=None, return_stats: bool = False):
+    """gen.findMRCA(pedigree, IDs) (src/identify.jl:153-161) on the B200 engine: the most recent common
+    ancestors of IDs and the minimum meioses from each of them to each ID, as a `GenMatrix`.  A common ancestor
+    is a proper ancestor of every ID (an individual is not its own ancestor); an MRCA is a common ancestor
+    none of whose descendants is common.  `ancestors` are sorted by ID; no common ancestor gives a
+    len(IDs) x 0 matrix.  KeyError on an unknown ID.  return_stats: also {"mrca": the common-ancestor pass,
+    "meioses": the distance pass}."""
+    ids = np.asarray(IDs, np.int64).reshape(-1)
+    ranks = pedigree.rank_of(ids)                       # KeyError, like pedigree[ID]
+    stats = {}
+    if len(ids) == 0:
+        res = GenMatrix(ids, np.zeros(0, np.int64), np.zeros((0, 0), np.int64))
+        return (res, stats) if return_stats else res
+    anc, stats["mrca"] = mrca_arrays(pedigree.father, pedigree.mother, ranks, device=device, devices=devices)
+    anc_ids = np.sort(pedigree.ids[anc])
+    d, stats["meioses"] = meioses_arrays(pedigree.father, pedigree.mother, ranks, pedigree.rank_of(anc_ids),
+                                         device=device, devices=devices)
+    res = GenMatrix(ids, anc_ids, d)
+    return (res, stats) if return_stats else res
+
+
+def findDistance(pedigree: Pedigree, IDs, ancestorID, *, device: int = -1) -> int:
+    """gen.findDistance(pedigree, IDs, ancestorID) (src/describe.jl:296-300) on the B200 engine: the sum over
+    IDs of the minimum meioses from ancestorID down to each of them (for two individuals, the meioses that
+    separate them through that ancestor).  An ID equal to ancestorID adds 0.  ValueError naming the first ID
+    that does not descend from ancestorID; KeyError on an unknown ID."""
+    ids = np.asarray(IDs, np.int64).reshape(-1)
+    ranks = pedigree.rank_of(ids)
+    anc = pedigree.rank_of([ancestorID])
+    if len(ids) == 0:
+        return 0
+    d, _ = meioses_arrays(pedigree.father, pedigree.mother, ranks, anc, device=device)
+    bad = np.flatnonzero(d[:, 0] < 0)
+    if len(bad):
+        raise ValueError(f"gen.findDistance: {int(ids[bad[0]])} does not descend from {int(ancestorID)}")
+    return int(d[:, 0].sum())
+
+
 def f(pedigree: Pedigree, IDs, *, device: int = -1) -> np.ndarray:
     """gen.f(pedigree, IDs): inbreeding coefficients, Float32 (src/compute.jl:500-511).
 

@@ -326,4 +326,63 @@ function rec(pedigree::GenLib.Pedigree; pro::Vector{Int} = GenLib.pro(pedigree),
     r
 end
 
+# d(ancestor, proband) for every pair, length(p) x length(a), -1 where there is no descent path
+function meioses(father, mother, p::Vector{Int32}, a::Vector{Int32}, devs::Vector{Int32})
+    M = Matrix{Int64}(undef, length(p), length(a))
+    stats = Ref{GcStats}()
+    GC.@preserve M check(ccall((:genlib_meioses, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Int64}, Cint, Int32, Ptr{Int32},
+         Ptr{GcStats}),
+        length(father), father, mother, length(p), p, length(a), a, pointer(M), 1, length(devs), devs, stats))
+    M
+end
+
+"""
+    findMRCA(pedigree, IDs; device = -1, devices = Int[]) -> GenLib.GenMatrix
+
+`gen.findMRCA` (src/identify.jl:153-161) on the B200 engine: the most recent common ancestors of `IDs` --
+proper ancestors of every ID (an individual is not its own ancestor) none of whose descendants is one -- and
+the minimum meioses from each of them down to each ID.  `genlib_mrca` finds the MRCAs (ranks), they are
+sorted by ID, and `genlib_meioses` writes the `length(IDs) x length(ancestors)` Int64 matrix column-major.
+Builds `GenLib.GenMatrix(individuals, ancestors, meioses)`: this argument order (IDs, MRCA IDs, matrix with
+rows = IDs) is assumed from the field list SURVEY.md gives for `GenMatrix` (src/identify.jl:129-133).
+Exercised through Python ctypes by tests/test_mrca.py, not executed here.
+"""
+function findMRCA(pedigree::GenLib.Pedigree, IDs::Vector{Int}; device::Integer = -1,
+                  devices::Vector{<:Integer} = Int[])
+    father, mother = flatten(pedigree)
+    p = Int32[pedigree[ID].rank - 1 for ID in IDs]                   # KeyError on unknown ID
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    isempty(p) && return GenLib.GenMatrix(IDs, Int[], Matrix{Int64}(undef, 0, 0))
+    ranks = Vector{Int32}(undef, length(father))
+    n_mrca = Ref{Int32}(0)
+    stats = Ref{GcStats}()
+    check(ccall((:genlib_mrca, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{GcStats}),
+        length(father), father, mother, length(p), p, ranks, n_mrca, length(devs), devs, stats))
+    by_rank = Dict(individual.rank - 1 => individual.ID for individual in values(pedigree))
+    ancestors = sort([by_rank[r] for r in ranks[1:n_mrca[]]])
+    a = Int32[pedigree[ID].rank - 1 for ID in ancestors]
+    GenLib.GenMatrix(IDs, ancestors, meioses(father, mother, p, a, devs))
+end
+
+"""
+    findDistance(pedigree, IDs, ancestorID; device = -1) -> Int
+
+`gen.findDistance` (src/describe.jl:296-300) on the B200 engine: the sum over `IDs` of the minimum meioses
+from `ancestorID` down to each ID (0 for `ancestorID` itself).  An ID that does not descend from
+`ancestorID` throws `ArgumentError` naming it.  Exercised through Python ctypes by tests/test_mrca.py, not
+executed here.
+"""
+function findDistance(pedigree::GenLib.Pedigree, IDs::Vector{Int}, ancestorID::Int; device::Integer = -1)
+    father, mother = flatten(pedigree)
+    p = Int32[pedigree[ID].rank - 1 for ID in IDs]
+    a = Int32[pedigree[ancestorID].rank - 1]
+    isempty(p) && return 0
+    d = meioses(father, mother, p, a, Int32[device])
+    k = findfirst(<(0), d[:, 1])
+    k === nothing || throw(ArgumentError("$(IDs[k]) does not descend from $ancestorID"))
+    sum(d[:, 1])
+end
+
 end # module

@@ -356,6 +356,32 @@ int genlib_rec(int32_t n, const int32_t *father, const int32_t *mother, int32_t 
                int32_t n_anc, const int32_t *ancestor, int64_t *out, int32_t n_dev, const int32_t *devices,
                genlib_gc_stats *stats);
 
+/* ---- gen.findMRCA / gen.findDistance: most recent common ancestors and minimum meioses ------------------------
+ * (SURVEY.md 2: src/identify.jl _findMRCA :101-107, _findMinDistanceMRCA :114-118, GenMatrix :129-133,
+ * findMRCA :153-161; src/describe.jl _get_paths :241-258, findDistance :296-300)
+ * The reference enumerates every descent path and keeps the shortest; here the same plan and devices as
+ * genlib_gc (GENLIB_GC_DIRECTION applies) propagate shortest distances in the (min, +1) semiring:
+ *   d(a, p) = number of parent -> child edges on the shortest descent path a -> ... -> p, d(p, p) = 0
+ *           = min(d(a, father(p)), d(a, mother(p))) + 1                     (a missing parent: no path)
+ * Distances are uint16 on the device; a plan of 0xFFFF layers or more fails with GENLIB_EOVERFLOW before any
+ * launch (a distance is below the plan's layer count), so a distance is never confused with "no path".
+ * The minimum is order-free: the result is bitwise independent of the direction and the number of devices.
+ * genlib_meioses: out = n_pro x n_anc int64, out[i, j] = d(ancestor[j], proband[i]), -1 where proband[i] does
+ * not descend from (and is not) ancestor[j]; row-major, or column-major when col_major != 0; duplicates of
+ * either list are kept.  Stats and alg_bytes as genlib_gc with 2 bytes per (16-byte padded) column. */
+int genlib_meioses(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                   int32_t n_anc, const int32_t *ancestor, int64_t *out, int col_major, int32_t n_dev,
+                   const int32_t *devices, genlib_gc_stats *stats);
+/* genlib_mrca: the most recent common ancestors of the ranks `ids` (duplicates allowed).  A common ancestor is
+ * a PROPER ancestor of every distinct ID (an individual is not its own ancestor: for [parent, child] the
+ * MRCAs are the parent's parents); an MRCA is a common ancestor none of whose children is common (equivalent
+ * to "none of whose descendants is common", DESIGN.md 2d).  `mrca` has room for n ranks; it receives *n_mrca
+ * ranks in ascending order.  One genlib_rec pass on the devices (pro = the distinct IDs, anc = their
+ * ancestors-or-self) decides who is common; everything else is O(n) on the host.  `stats` are the rec pass's.
+ * No ID gives no MRCA without a device. */
+int genlib_mrca(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_ids, const int32_t *ids,
+                int32_t *mrca, int32_t *n_mrca, int32_t n_dev, const int32_t *devices, genlib_gc_stats *stats);
+
 #ifdef __cplusplus
 }
 #endif
