@@ -1,5 +1,5 @@
 // engine.cu -- the phi engine and the library-wide part of the C ABI of libgenlib_cuda.so (include/genlib_cuda.h):
-// plans, engines, the one-shot genlib_phi / genlib_phi_multi, errors and caches.  gen.gc, gen.occ and gen.rec are
+// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_f, errors and caches.  gen.gc, gen.occ and gen.rec are
 // in gc_engine.cu; the host helpers both share are in runtime.hpp.
 //
 // The ABI stands where the reference's Julia method stands:
@@ -9,6 +9,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <memory>
 
 #include "kernels.cuh"
@@ -129,6 +130,7 @@ struct IndexBufs {
     DevBuf<int32_t> mem_rank;
     DevBuf<uint8_t> flags;
     DevBuf<double> acc;
+    DevBuf<double> fam_kin;                // kScheduleF: Psi[father, mother] per couple (couples whose father row is own)
 };
 
 struct genlib_engine : IndexBufs {
@@ -186,6 +188,15 @@ void fill_info(const Layer &L, genlib_layer_info *o) {
 size_t plan_index_bytes(const Plan &P) {
     return (P.mem_ind.size() * 4 + P.mem_rank.size() + P.fam_pf.size() * 6 + P.fam_start.size() + P.mtile_desc.size() +
             P.pro_slot.size() * 2 + P.live_lrow.size() + P.tile_map.size() + P.live_tiles.size()) * sizeof(int32_t) + P.fam_pf.size() * 2 + P.live_owner.size() + P.flags.size();
+}
+
+// The traffic the layers cannot avoid: s (4 n L + 3 n^2) per layer, and for kScheduleF 8 bytes per couple with
+// both parents (its Psi[father, mother], read once and written once).
+double plan_alg_bytes(const Plan &P, size_t es) {
+    double b = P.alg_elems * (double)es;
+    if (P.schedule == kScheduleF)
+        for (size_t k = 0; k < P.fam_pf.size(); k++) b += (P.fam_pf[k] >= 0 && P.fam_pm[k] >= 0) ? 8.0 : 0.0;
+    return b;
 }
 
 // Arena layout of rank g.  The first two regions are what peers address (barrier flags, frontier rows).
@@ -298,6 +309,7 @@ unsigned char *place_arrays(IndexBufs &B, const Plan &P, bool streamed, unsigned
     B.live_owner.place(cur, cnt(P.live_owner));
     B.flags.place(cur, cnt(P.flags)); B.acc.place(cur, 4);
     B.pro_owner.place(cur, npro); B.pro_lrow.place(cur, npro);
+    if (P.schedule == kScheduleF) B.fam_kin.place(cur, cnt(P.fam_pf));
     return cur;
 }
 
@@ -391,6 +403,12 @@ int launch_layer(genlib_engine &E, int t, bool timed, size_t &ev, int &launches)
     LayerArgs a = layer_args(E, t);
     LayerLaunch &ll = E.launch[t];
     auto layer_fn = layer_function<T>(P, ll.prod_warps);
+    if (P.schedule == kScheduleF && L.n_fam > 0) {              // the parents' kinships, while both rows are live
+        couple_kinship_kernel<T><<<(unsigned)((L.n_fam + kThreads - 1) / kThreads), kThreads, 0, E.stream>>>(
+            A, ld, E.fam_pf_owner.p + L.fam_off, E.fam_pf_lrow.p + L.fam_off, E.fam_pm.p + L.fam_off, L.n_fam, E.rank,
+            E.fam_kin.p + L.fam_off);
+        launches++;
+    }
     if (timed) CU(cudaEventRecord(E.events[ev++], E.stream));
     if (ll.grid > 0) {
         ll.s.Q = E.Q;
@@ -516,7 +534,7 @@ int run_streamed(genlib_engine &E, PlanStream &ps) {
     float ms = 0;
     CU(cudaEventElapsedTime(&ms, E.events[nev - 2], E.events[nev - 1]));
     E.stats.ms_kernels = ms;                                    // first launch to last: includes waiting for the planner
-    E.stats.row_updates = P.row_updates; E.stats.alg_bytes = P.alg_elems * (double)E.esize;
+    E.stats.row_updates = P.row_updates; E.stats.alg_bytes = plan_alg_bytes(P, E.esize);
     E.stats.h2d_bytes = (int64_t)plan_index_bytes(P);
     return GENLIB_OK;
 }
@@ -614,7 +632,7 @@ int upload_probands(genlib_engine &E) {
     const Plan &P = E.plan->p;
     std::vector<int32_t> own_rows;
     E.own_pro.clear();
-    for (size_t u = 0; u < P.pro_ind.size(); u++)
+    for (size_t u = 0; u < P.pro_owner.size(); u++)            // (empty for kScheduleF: no proband matrix)
         if (P.pro_owner[u] == E.rank) { E.own_pro.push_back((int32_t)u); own_rows.push_back(P.pro_lrow[u]); }
     CU(E.pro_slot.upload(P.pro_slot, E.stream));
     CU(E.own_pro_row.upload(own_rows, E.stream));
@@ -655,6 +673,8 @@ int create_engine(const genlib_plan *plan, int numerics, int device, int rank, g
     const Plan &P = plan->p;
     if (sparse_schedule(P.schedule) && numerics != GENLIB_NUMERICS_REFERENCE)
         return fail(GENLIB_EINVAL, "the sparse_phi schedule stores Float32 (numerics must be GENLIB_NUMERICS_REFERENCE)");
+    if (P.schedule == kScheduleF && numerics != GENLIB_NUMERICS_FP64)
+        return fail(GENLIB_EINVAL, "the gen.f schedule stores Float64 (numerics must be GENLIB_NUMERICS_FP64)");
     if (rank < 0 || rank >= P.world) return fail(GENLIB_EINVAL, "rank outside the plan's world");
     if (P.world > kMaxWorld) return fail(GENLIB_EINVAL, "the engine supports at most 16 ranks");
     if (P.n_unique == 0) return fail(GENLIB_EINVAL, "empty proband list: nothing to run");
@@ -732,7 +752,8 @@ int create_engine(const genlib_plan *plan, int numerics, int device, int rank, g
     for (auto &e : E->events) CU(cudaEventCreate(&e));
     genlib_stats &s = E->stats;
     s.n_unique = P.n_unique; s.n_layers = (int32_t)P.layers.size(); s.row_updates = P.row_updates;
-    s.capacity = P.capacity; s.device_bytes = (int64_t)need; s.alg_bytes = P.alg_elems * (double)E->esize;
+    s.capacity = P.capacity; s.device_bytes = (int64_t)need;
+    s.alg_bytes = streamed ? P.alg_elems * (double)E->esize : plan_alg_bytes(P, E->esize);   // (streamed: final in run_streamed)
     s.ms_plan = plan->ms_plan; s.ms_upload = now_ms() - t0;
     s.h2d_bytes = (int64_t)plan_index_bytes(P);
     *out = E.release();
@@ -928,7 +949,7 @@ int32_t genlib_plan_world(const genlib_plan *plan) { return plan ? plan->p.world
 int genlib_plan_proband_rows(const genlib_plan *plan, int32_t *owner, int32_t *lrow) {
     settle(plan);
     if (!plan || !owner || !lrow) return fail(GENLIB_EINVAL, "null argument");
-    for (size_t u = 0; u < plan->p.pro_ind.size(); u++) { owner[u] = plan->p.pro_owner[u]; lrow[u] = plan->p.pro_lrow[u]; }
+    for (size_t u = 0; u < plan->p.pro_owner.size(); u++) { owner[u] = plan->p.pro_owner[u]; lrow[u] = plan->p.pro_lrow[u]; }
     return GENLIB_OK;
 }
 
@@ -951,6 +972,9 @@ int genlib_plan_proband_slots(const genlib_plan *plan, int32_t *slots) {
 
 // An engine on a plan that is still being made registers as a reader of its arrays before it looks at them.
 static int create_engine_public(const genlib_plan *plan, int numerics, int device, int rank, genlib_engine **out) {
+    if (out) *out = nullptr;
+    if (plan && plan->p.schedule == kScheduleF)                  // (set before genlib_plan_create* returns)
+        return fail(GENLIB_EINVAL, "a GENLIB_SCHEDULE_F plan has no matrix to fetch: call genlib_f");
     if (plan && plan->streaming()) {
         PlanStream &ps = *plan->stream;
         StreamConsumer reader(ps);
@@ -1172,25 +1196,31 @@ int genlib_engine_read_block(genlib_engine *eng, int32_t n_slots, const int32_t 
     return GENLIB_OK;
 }
 
-// genlib_phi and genlib_phi_multi: ONE plan for all devices, made on a worker thread and handed over layer by layer
-// (PlanStream), so that the devices run the first generations while the later ones are planned.  GENLIB_STREAM=0, or
-// a bound of the streamed plan that did not hold, plans first and then runs.  One device runs on the calling thread;
-// several get a host thread each, NVLink peer access, and fetch a contiguous block of output rows each.
-static int phi_oneshot(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
-                       void *out, int out_dtype, int numerics, int32_t n_dev, const int32_t *devices, genlib_stats *stats) {
-    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
+// What a one-shot call takes out of the engines once every device has run: `prepare` (may be empty) reads the
+// finished plan on the calling thread, then `device(E, g)` runs on device g's host thread.
+struct OneshotFetch {
+    std::function<void(const Plan &)> prepare;
+    std::function<int(genlib_engine &, int)> device;
+};
+
+// genlib_phi, genlib_phi_multi and genlib_f: ONE plan for all devices, made on a worker thread and handed over layer
+// by layer (PlanStream), so that the devices run the first generations while the later ones are planned.
+// GENLIB_STREAM=0, or a bound of the streamed plan that did not hold, plans first and then runs.  One device runs on
+// the calling thread; several get a host thread each and NVLink peer access.  `has_out`: the caller wants a result.
+static int oneshot(const std::string &who, int schedule, int32_t n, const int32_t *father, const int32_t *mother,
+                   int32_t n_pro, const int32_t *proband, bool has_out, int numerics, int32_t n_dev, const int32_t *devices,
+                   genlib_stats *stats, const OneshotFetch &fetch) {
     const bool multi = n_dev > 1;
-    const std::string who = multi ? "genlib_phi_multi" : "genlib_phi";
     std::vector<int> dev(devices, devices + n_dev);              // (one device: a negative one is the current device)
     if (int rc = multi ? resolve_devices(who, n_dev, devices, false, dev) : GENLIB_OK) return rc;
     std::unique_ptr<genlib_plan> plan_owner(new (std::nothrow) genlib_plan);
     if (!plan_owner) return fail(GENLIB_ENOMEM, "out of host memory");
     genlib_plan *plan = plan_owner.get();
-    const bool want_stream = env_int("GENLIB_STREAM", 1) != 0 && out != nullptr;
+    const bool want_stream = env_int("GENLIB_STREAM", 1) != 0 && has_out;
     const double tp0 = now_ms();
     PlanStream ps;
     auto make_plan = [&](PlanStream *stream) {
-        plan->build(n, father, mother, nullptr, n_pro, proband, n_dev, GENLIB_SCHEDULE_PHI, stream, /*planners=*/1, tp0);
+        plan->build(n, father, mother, nullptr, n_pro, proband, n_dev, schedule, stream, /*planners=*/1, tp0);
     };
     if (want_stream) { try { plan->worker = std::thread([&] { make_plan(&ps); }); } catch (...) { } }
     const bool streaming = plan->worker.joinable();
@@ -1270,7 +1300,7 @@ static int phi_oneshot(int32_t n, const int32_t *father, const int32_t *mother, 
         if (stats) { std::memset(stats, 0, sizeof *stats); stats->ms_plan = plan->ms_plan; }
         return GENLIB_OK;                                         // 0 x 0 matrix, like the reference
     }
-    if (!out) return fail(GENLIB_EINVAL, who + ": out is null");
+    if (!has_out) return fail(GENLIB_EINVAL, who + ": out is null");
     if (!done) {                                                // plan first, then run (no streaming, or its bounds did not hold)
         for (auto *&x : eng) { genlib_engine_destroy(x); x = nullptr; }
         if ((rc = first_error(create_all(false), true)) != GENLIB_OK) return rc;
@@ -1278,18 +1308,9 @@ static int phi_oneshot(int32_t n, const int32_t *father, const int32_t *mother, 
         if ((rc = first_error(on_devices(n_dev, [&](int g) { return genlib_engine_run(eng[(size_t)g], 0); }), true)) != GENLIB_OK) return rc;
     }
     for (auto *x : eng) x->stats.ms_plan = plan->ms_plan;
-    const int32_t nu = plan->p.n_unique;
     const double t0 = now_ms();
-    if (!multi) rc = genlib_engine_fetch(eng[0], out, out_dtype);
-    else rc = first_error(on_devices(n_dev, [&](int g) {        // contiguous row blocks, one PCIe link each
-        genlib_engine &E = *eng[(size_t)g];
-        DeviceGuard guard;
-        if (int r = guard.enter(E.device)) return r;
-        const int32_t u0 = (int32_t)((int64_t)nu * g / n_dev), u1 = (int32_t)((int64_t)nu * (g + 1) / n_dev);
-        if (numerics == GENLIB_NUMERICS_FP64)
-            return out_dtype == GENLIB_F64 ? fetch_block<double, double>(E, u0, u1, (double *)out) : fetch_block<double, float>(E, u0, u1, (float *)out);
-        return out_dtype == GENLIB_F64 ? fetch_block<float, double>(E, u0, u1, (double *)out) : fetch_block<float, float>(E, u0, u1, (float *)out);
-    }), true);
+    if (fetch.prepare) fetch.prepare(plan->p);
+    rc = first_error(on_devices(n_dev, [&](int g) { return fetch.device(*eng[(size_t)g], g); }), true);
     if (rc != GENLIB_OK) return rc;
     if (stats) {
         *stats = eng[0]->stats;
@@ -1306,11 +1327,93 @@ static int phi_oneshot(int32_t n, const int32_t *father, const int32_t *mother, 
     return GENLIB_OK;
 }
 
+// genlib_phi / genlib_phi_multi: one device fetches the whole matrix (genlib_engine_fetch); several fetch a
+// contiguous block of output rows each, over their own PCIe links.
+static int phi_oneshot(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                       void *out, int out_dtype, int numerics, int32_t n_dev, const int32_t *devices, genlib_stats *stats) {
+    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
+    const bool multi = n_dev > 1;
+    int32_t nu = 0;
+    OneshotFetch fetch;
+    fetch.prepare = [&](const Plan &P) { nu = P.n_unique; };
+    fetch.device = [&](genlib_engine &E, int g) {
+        if (!multi) return genlib_engine_fetch(&E, out, out_dtype);
+        DeviceGuard guard;
+        if (int r = guard.enter(E.device)) return r;
+        const int32_t u0 = (int32_t)((int64_t)nu * g / n_dev), u1 = (int32_t)((int64_t)nu * (g + 1) / n_dev);
+        if (numerics == GENLIB_NUMERICS_FP64)
+            return out_dtype == GENLIB_F64 ? fetch_block<double, double>(E, u0, u1, (double *)out) : fetch_block<double, float>(E, u0, u1, (float *)out);
+        return out_dtype == GENLIB_F64 ? fetch_block<float, double>(E, u0, u1, (double *)out) : fetch_block<float, float>(E, u0, u1, (float *)out);
+    };
+    return oneshot(multi ? "genlib_phi_multi" : "genlib_phi", GENLIB_SCHEDULE_PHI, n, father, mother, n_pro, proband,
+                   out != nullptr, numerics, n_dev, devices, stats, fetch);
+}
+
 int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
                      const int32_t *proband, void *out, int out_dtype, int numerics, int32_t n_dev,
                      const int32_t *devices, genlib_stats *stats) {
     if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_multi: 1 .. 16 devices");
     return phi_oneshot(n, father, mother, n_pro, proband, out, out_dtype, numerics, n_dev, devices, stats);
+}
+
+// genlib_f: a GENLIB_SCHEDULE_F plan of the listed individuals with both parents; every device copies its per-couple
+// kinships to the host once, and each list position takes the value of its couple from the device that holds the
+// couple's father row.
+int genlib_f(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_ids, const int32_t *ids,
+             void *out, int out_dtype, int32_t n_dev, const int32_t *devices, genlib_stats *stats) {
+    if (n < 0 || n_ids < 0 || (n > 0 && (!father || !mother)) || (n_ids > 0 && (!ids || !out)))
+        return fail(GENLIB_EINVAL, "genlib_f: null pointer or negative size");
+    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
+    if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_f: 1 .. 16 devices");
+    bool any = false;                                            // a listed individual with both parents
+    for (int32_t i = 0; i < n_ids; i++) {
+        const int32_t x = ids[i];
+        if (x < 0 || x >= n) {
+            std::string err;
+            if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);   // (a broken pedigree is reported first)
+            return fail(GENLIB_EKEY, "KeyError: index " + std::to_string(x) + " not in pedigree");
+        }
+        any = any || (father[x] >= 0 && mother[x] >= 0);
+    }
+    auto put = [&](int32_t i, double v) {
+        if (out_dtype == GENLIB_F64) static_cast<double *>(out)[i] = v;
+        else static_cast<float *>(out)[i] = (float)v;
+    };
+    for (int32_t i = 0; i < n_ids; i++) put(i, 0.0);             // a missing parent: F = 0
+    if (!any) {                                                  // no plan, no device
+        std::string err;
+        if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);
+        if (stats) std::memset(stats, 0, sizeof *stats);
+        return GENLIB_OK;
+    }
+    std::vector<int64_t> couple;                                 // per list position: its couple (-1: F = 0)
+    OneshotFetch fetch;
+    fetch.prepare = [&](const Plan &P) {
+        std::vector<int64_t> of((size_t)n, -1);
+        for (const Layer &L : P.layers)
+            for (int32_t q = 0; q < L.n_new; q++) of[(size_t)P.mem_ind[L.mem_off + q]] = (int64_t)L.fam_off + P.mem_fam[L.mem_off + q];
+        couple.assign((size_t)n_ids, -1);
+        for (int32_t i = 0; i < n_ids; i++)
+            if (father[ids[i]] >= 0 && mother[ids[i]] >= 0) couple[(size_t)i] = of[(size_t)ids[i]];
+    };
+    fetch.device = [&](genlib_engine &E, int g) {
+        DeviceGuard guard;
+        if (int r = guard.enter(E.device)) return r;
+        const double t0 = now_ms();
+        const Plan &P = E.plan->p;
+        std::vector<double> kin(P.fam_pf.size());
+        CU(cudaMemcpyAsync(kin.data(), E.fam_kin.p, kin.size() * sizeof(double), cudaMemcpyDeviceToHost, E.stream));
+        CU(cudaStreamSynchronize(E.stream));
+        for (int32_t i = 0; i < n_ids; i++) {
+            const int64_t c = couple[(size_t)i];
+            if (c >= 0 && P.fam_pf_owner[(size_t)c] == g) put(i, kin[(size_t)c]);
+        }
+        E.stats.d2h_bytes += (int64_t)(kin.size() * sizeof(double));
+        E.stats.ms_fetch = now_ms() - t0;
+        return GENLIB_OK;
+    };
+    return oneshot("genlib_f", kScheduleF, n, father, mother, n_ids, ids, true, GENLIB_NUMERICS_FP64, n_dev, devices,
+                   stats, fetch);
 }
 
 int genlib_phi(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,

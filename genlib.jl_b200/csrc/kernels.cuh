@@ -1,6 +1,6 @@
 // kernels.cuh -- device-side vocabulary shared by the sm_100a kernels of the kinship sweep, and the
 // small kernels around the layer kernel (layer_kernel.cuh): proband gather, phiMean reduction, the
-// inter-GPU barrier and sparse_phi's misfiled pairs.
+// inter-GPU barrier, sparse_phi's misfiled pairs and gen.f's parents' kinships.
 //
 // Arithmetic is binary64 in the reference's grouping; storage type T is float
 // (GENLIB_NUMERICS_REFERENCE: one RN32 per step, like src/compute.jl:296) or double.
@@ -145,6 +145,21 @@ misfile_kernel(T *__restrict__ A, int64_t ld, const int32_t *__restrict__ mem_ra
     T *row = A + (int64_t)L.mem_lrow[i] * ld;
     for (int j = blockIdx.y * kThreads + threadIdx.x; j < L.n_new; j += gridDim.y * kThreads)
         if (j != i && ((seq_i > L.mem_ind[j]) != (rank_i > mem_rank[j]))) row[L.mem_slot[j]] = (T)0;
+}
+
+// =====================================================================================
+// couple_kinship_kernel (GENLIB_SCHEDULE_F), launched just BEFORE the layer kernel of the couples' layer: the
+// inbreeding coefficient of a child is the kinship of its parents, Psi[father, mother], the entry at the mother's
+// slot of the father's row.  During the layer both parents are live and nobody writes that entry; after it the
+// mother's slot may be recycled, by a peer rank too.  Every rank reads the couples whose father row it holds.
+// =====================================================================================
+template <typename T>
+__global__ void couple_kinship_kernel(const T *__restrict__ A, int64_t ld, const int8_t *__restrict__ pf_owner,
+                                      const int32_t *__restrict__ pf_lrow, const int32_t *__restrict__ pm, int32_t n_fam,
+                                      int rank, double *__restrict__ out) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= n_fam || pf_owner[f] != rank || pm[f] < 0) return;
+    out[f] = (double)A[(int64_t)pf_lrow[f] * ld + pm[f]];
 }
 
 // =====================================================================================

@@ -135,6 +135,8 @@ struct Scratch {
     std::vector<int64_t> d_cut, d_both;
     std::vector<LiveRec> live, next_live;
     std::vector<int32_t> last_of;
+    std::vector<int32_t> dead_slots;                            // kScheduleF: slots / rows (per owner) of the members that no
+    std::vector<std::vector<int32_t>> dead_rows;                // later layer reads, freed at the end of their own layer
     std::vector<int32_t> fam_of, fam_count, fam_first, fam_key, fam_n;   // couples of every layer (grouped ahead by helper threads)
     std::vector<int32_t> order, newid, nf_of, load, freed, evicted[2], cnt, cnt_order, ipos;   // order / newid: by member / couple of every layer
     std::vector<FamilyTable> tables;          // one per planning thread
@@ -190,6 +192,9 @@ int verify_plan(const Plan &P, std::string &err) {
                 const int32_t q0 = P.fam_q[2 * (L.fam_off + (size_t)f) + s2], q = q0 >= 0 ? (q0 & ~kSoleReader) : q0;
                 const int32_t slot = s2 ? P.fam_pm[L.fam_off + f] : P.fam_pf[L.fam_off + f];
                 if (q < -1 || q >= qrows || (q < 0) != (slot < 0)) { err = "verify: fam_q out of range in layer " + std::to_string(t) + " couple " + std::to_string(f) + " q " + std::to_string(q) + " qrows " + std::to_string(qrows) + " slot " + std::to_string(slot) + " rt_lo " + std::to_string(L.rt_lo); return GENLIB_EINVAL; }
+                // a parent's row is live in its child's layer (for kScheduleF: the engine reads Psi[father, mother] there)
+                if (slot >= 0 && (slot < L.rt_lo || slot >= L.rt_lo + L.rt_rows || !(P.flags[L.flag_off + (size_t)(slot - L.rt_lo)] & kFlagLive)))
+                    { err = "verify: a parent of couple " + std::to_string(f) + " is not live in layer " + std::to_string(t); return GENLIB_EINVAL; }
             }
         for (int32_t j = 0; j < L.n_mtiles; j++) {
             const int32_t *d = &P.mtile_desc[4 * (L.mtile_off + (size_t)j)];
@@ -229,6 +234,8 @@ struct Planner {
     Scratch &W; Plan &P; std::string &err; PlanStream *ps;
     const int32_t n, *father, *mother; const int64_t *ids; const int32_t n_pro, *proband, world; const int schedule, planners;
     const bool by_seq = sparse_schedule(schedule);              // members of a layer in processing order
+    const bool by_depth = by_seq || schedule == kScheduleF;     // layers by depth below the founders
+    const bool short_rows = schedule == kScheduleF;             // rows that no later layer reads (childless members)
     PhaseTimer clock{};
     std::vector<uint8_t> &is_pro = W.is_pro;
     std::vector<Pre> &pre = W.pre;
@@ -248,7 +255,7 @@ struct Planner {
 
     int run() {
         P.reset();
-        if (schedule != kSchedulePhi && !sparse_schedule(schedule)) { err = "unknown schedule"; return GENLIB_EINVAL; }
+        if (schedule != kSchedulePhi && !sparse_schedule(schedule) && schedule != kScheduleF) { err = "unknown schedule"; return GENLIB_EINVAL; }
         P.schedule = schedule;
         if (n < 0 || n_pro < 0 || world < 1 || (n > 0 && (!father || !mother)) || (n_pro > 0 && !proband))
             { err = "genlib_plan_create: null pointer or negative size"; return GENLIB_EINVAL; }
@@ -258,6 +265,7 @@ struct Planner {
         clock.phase("probands");
         if (int rc = sweep()) return rc;
         if (int rc = by_seq ? queue_order() : GENLIB_OK) return rc;
+        if (schedule == kScheduleF) depth_layers();
         clock.phase("heights");
         buckets();
         clock.phase("buckets");
@@ -268,7 +276,8 @@ struct Planner {
         return finish();
     }
 
-    // probands: first occurrence wins (intersect/union keep first-argument order, compute.jl:247,251)
+    // probands: first occurrence wins (intersect/union keep first-argument order, compute.jl:247,251); kScheduleF
+    // leaves out the listed individuals with a missing parent (their F is 0 without a plan)
     int probands() {
         is_pro.assign((size_t)n + 1, 0);
         for (int32_t t = 0; t < n_pro; t++) {
@@ -278,6 +287,7 @@ struct Planner {
                 err = "KeyError: proband index " + std::to_string(x) + " not in pedigree";
                 return GENLIB_EKEY;
             }
+            if (schedule == kScheduleF && (father[x] < 0 || mother[x] < 0)) continue;
             if (!is_pro[x]) { is_pro[x] = 1; P.pro_ind.push_back(x); }
         }
         P.n_unique = (int32_t)P.pro_ind.size();
@@ -299,7 +309,7 @@ struct Planner {
         bool bad_pedigree = false;
         // Threads of the bucket pass (buckets()): it works on equal ranges of ranks, and this sweep counts the heights
         // per range for it (hist[h * kC + c]).
-        const int kC = this->kC = by_seq ? 1 : plan_threads(n, 400000, planners, world);
+        const int kC = this->kC = by_depth ? 1 : plan_threads(n, 400000, planners, world);
         const int32_t chunk = this->chunk = n / kC + 1;
         std::vector<int32_t> &hist = this->hist; hist.clear();
         int32_t c_of_x = kC - 1, c_lo = (kC - 1) * chunk;
@@ -331,26 +341,54 @@ struct Planner {
         return bad_pedigree ? check_pedigree(n, father, mother, err) : GENLIB_OK;
     }
 
-    // Schedule of sparse_phi (compute.jl:335-439): individuals are processed in the order of a queue
-    // that starts with the founders and receives a child when its last parent has been processed --
-    // i.e. by depth below the founders, ties in queue order -- and of a pair, the one processed LATER
-    // is climbed.  The layer is then the depth, `seq` (the position in that queue) replaces the rank
-    // wherever the kernels decide who is climbed, and eviction is sparse_phi's own rule (:400-430).
-    // The sweep marked the ancestors of the probands (branching, :323); re-label them.
-    int queue_order() {
+    // Layers by depth below the founders (sparse_phi's schedule and kScheduleF): the sweep marked the ancestors of
+    // the probands; re-label them so that layer = S-1-h = depth, and the last child is the deepest one.
+    void depth_layers() {
         const int32_t n = this->n, *father = this->father, *mother = this->mother;
-        std::vector<int32_t> &cstart = W.cstart, &clist = W.clist, &depth = W.depth;
-        seq_order.clear();
-        cstart.assign((size_t)n + 2, 0);
+        std::vector<int32_t> &depth = W.depth;
         depth.assign((size_t)n, 0);
         int32_t dmax = 0;
         for (int32_t x = 0; x < n; x++) {                       // parents precede children
             if (pre[x].h < 0) continue;
             const int32_t f = father[x], m = mother[x];
             int32_t d = 0;
-            if (f >= 0) { d = std::max(d, depth[f] + 1); cstart[(size_t)f + 2]++; }
-            if (m >= 0 && m != f) { d = std::max(d, depth[m] + 1); cstart[(size_t)m + 2]++; }
+            if (f >= 0) d = std::max(d, depth[f] + 1);
+            if (m >= 0) d = std::max(d, depth[m] + 1);
             depth[x] = d; dmax = std::max(dmax, d);
+        }
+        std::fill(hist.begin(), hist.end(), 0);
+        hist.resize((size_t)dmax + 1, 0);
+        hmax = dmax;
+        for (int32_t x = 0; x < n; x++) {
+            if (pre[x].h < 0) continue;
+            pre[x].h = dmax - depth[x];                          // layer = S-1-h = depth
+            pre[x].minch = INT_MAX;
+            pre[x].rl = pre[x].h;                                // the reference's cut counts do not apply
+            hist[(size_t)pre[x].h]++;
+        }
+        for (int32_t x = 0; x < n; x++) {                       // last child: the deepest one
+            if (pre[x].h < 0) continue;
+            const int32_t par[2] = {father[x], mother[x]};
+            for (int32_t p : par) if (p >= 0 && pre[p].minch > pre[x].h) pre[p].minch = pre[x].h;
+        }
+    }
+
+    // Schedule of sparse_phi (compute.jl:335-439): individuals are processed in the order of a queue
+    // that starts with the founders and receives a child when its last parent has been processed --
+    // i.e. by depth below the founders, ties in queue order -- and of a pair, the one processed LATER
+    // is climbed.  The layer is then the depth, `seq` (the position in that queue) replaces the rank
+    // wherever the kernels decide who is climbed, and eviction is sparse_phi's own rule (:400-430).
+    int queue_order() {
+        const int32_t n = this->n, *father = this->father, *mother = this->mother;
+        std::vector<int32_t> &cstart = W.cstart, &clist = W.clist, &depth = W.depth;
+        depth_layers();
+        seq_order.clear();
+        cstart.assign((size_t)n + 2, 0);
+        for (int32_t x = 0; x < n; x++) {
+            if (pre[x].h < 0) continue;
+            const int32_t f = father[x], m = mother[x];
+            if (f >= 0) cstart[(size_t)f + 2]++;
+            if (m >= 0 && m != f) cstart[(size_t)m + 2]++;
         }
         for (int32_t x = 0; x < n; x++) cstart[(size_t)x + 2] += cstart[(size_t)x + 1];
         clist.resize((size_t)cstart[(size_t)n + 1]);
@@ -361,7 +399,7 @@ struct Planner {
             if (m >= 0 && m != f) clist[(size_t)cstart[(size_t)m + 1]++] = x;
         }                                                       // now children of p = clist[cstart[p] .. cstart[p+1])
         orient.assign((size_t)n, -1);
-        seq_order.reserve(hist.empty() ? 0 : (size_t)n);
+        seq_order.reserve((size_t)n);
         for (int32_t x = 0; x < n; x++)                         // founder(isolated_pedigree) (:335-339) ...
             if (pre[x].h >= 0 && father[x] < 0 && mother[x] < 0) seq_order.push_back(x);
         if (ids)                                                // ... is sorted by ID (identify.jl:15-19)
@@ -381,21 +419,6 @@ struct Planner {
         for (int32_t i : seq_order) {                           // the queue order is sorted by depth (asserted, not assumed)
             if (depth[i] < last_depth) { err = "sparse_phi schedule: queue order is not sorted by depth"; return GENLIB_EINVAL; }
             last_depth = depth[i];
-        }
-        std::fill(hist.begin(), hist.end(), 0);
-        hist.resize((size_t)dmax + 1, 0);
-        hmax = dmax;
-        for (int32_t x = 0; x < n; x++) {
-            if (pre[x].h < 0) continue;
-            pre[x].h = dmax - depth[x];                          // layer = S-1-h = depth
-            pre[x].minch = INT_MAX;
-            pre[x].rl = pre[x].h;                                // the reference's cut counts do not apply
-            hist[(size_t)pre[x].h]++;
-        }
-        for (int32_t x = 0; x < n; x++) {                       // last child: the deepest one
-            if (pre[x].h < 0) continue;
-            const int32_t par[2] = {father[x], mother[x]};
-            for (int32_t p : par) if (p >= 0 && pre[p].minch > pre[x].h) pre[p].minch = pre[x].h;
         }
         return GENLIB_OK;
     }
@@ -424,7 +447,8 @@ struct Planner {
                 if (px.h < 0) continue;
                 const int32_t lx = S - 1 - px.h, ref_last = S - 1 - px.rl;
                 by_layer[pos[lx]++] = x;
-                const int32_t last = is_pro[x] ? INT_MAX : S - 1 - px.minch;     // probands stay to the end
+                // probands stay to the end (kScheduleF: nobody does); a row without children leaves after its own layer
+                const int32_t last = is_pro[x] && schedule != kScheduleF ? INT_MAX : px.minch == INT_MAX ? lx : S - 1 - px.minch;
                 last_of[x] = last;
                 occ[(size_t)std::min<int64_t>(std::max(last, lx), S - 1) + 1]--;   // born in or before, read in or after
                 cut[ref_last + 1]--;                                   // in cut[k] for layer <= k <= ref_last
@@ -527,8 +551,12 @@ struct Planner {
         int32_t *fam_of = W.fam_of.data() + lstart[t], *fam_count = W.fam_count.data() + lstart[t];
         int32_t *fam_first = W.fam_first.data() + lstart[t], *fam_key = W.fam_key.data() + lstart[t];
         table.next_layer((size_t)nn);
+        // kScheduleF: the siblings that nobody reads after this layer form couples of their own, so that their lines
+        // of slots come back whole at its end (mixed with the carried siblings they would leave holes in the frontier)
+        const bool split_dead = short_rows;
         auto couple_key = [&](int32_t x) {
-            return ((uint64_t)(uint32_t)(father[x] + 1) << 32) | (uint32_t)(mother[x] + 1);
+            const uint64_t dead = split_dead && last_of[x] == t ? 1ULL << 63 : 0;     // (father + 1 < 2^31)
+            return dead | ((uint64_t)(uint32_t)(father[x] + 1) << 32) | (uint32_t)(mother[x] + 1);
         };
         constexpr int32_t kAhead = 16;
         int32_t nfr = 0;
@@ -537,7 +565,7 @@ struct Planner {
             if (q + kAhead < nn) table.prefetch(couple_key(X[q + kAhead]));
             bool found;
             FamilyTable::Bucket &bk = table.find(couple_key(X[q]), &found);
-            const int32_t key = std::min(last_of[X[q]] - t, kKeys - 1);   // >= 1: somebody is born later, or proband
+            const int32_t key = std::min(last_of[X[q]] - t, kKeys - 1);   // >= 1: somebody is born later, or proband; 0: nobody (kScheduleF)
             if (found && fam_count[bk.val] < kMaxFamily) {
                 fam_of[q] = bk.val;
                 fam_key[bk.val] = std::max(fam_key[bk.val], key);
@@ -578,6 +606,7 @@ struct Planner {
             const int32_t np = count[t - 1];
             for (int32_t q = 0; q < np; q++) {             // (ranks ascend: nearly sequential reads)
                 const int32_t x = Xp[q];
+                if (short_rows && last_of[x] < t) continue;    // nobody reads the row after its own layer
                 const Home hx = home[x];
                 live.push_back(LiveRec{hx.slot, hx.lrow, last_of[x], hx.owner});
                 live_lo = std::min(live_lo, hx.slot); live_hi = std::max(live_hi, hx.slot);
@@ -740,6 +769,10 @@ struct Planner {
             if (streaming && (s >= bound_slots || lr >= bound_rows)) give_up_streaming();
             Home &hx = home[x];
             hx.slot = s; hx.lrow = lr; hx.owner = (int8_t)g;
+            if (short_rows && last_of[x] == t) {          // read by nobody after this layer: never joins the live list
+                W.dead_slots.push_back(s);
+                if (world > 1) W.dead_rows[(size_t)g].push_back(lr);
+            }
             mi[q] = by_seq ? orient[x] : x; ms[q] = s; mf[q] = newid[f]; ml[q] = lr;
             if (by_seq) P.mem_rank[L.mem_off + (size_t)q] = x;
         }
@@ -820,12 +853,22 @@ struct Planner {
         if (streaming) { ps->layers_done.store(t + 1, std::memory_order_release); ps->wake(); }
     }
 
-    // lane A: after the step, evicted slots / rows become reusable from the next layer on
+    // lane A: after the step, evicted slots / rows become reusable from the next layer on (and those of the layer's
+    // members that no later layer reads)
     void end_layer(int32_t t) {
         freed.clear();
         for (int32_t s : W.evicted[t & 1]) slots.release(s, freed);
+        if (!W.dead_slots.empty()) {
+            const size_t mid = freed.size();
+            for (int32_t s : W.dead_slots) slots.release(s, freed);      // (slots of one layer ascend)
+            std::inplace_merge(freed.begin(), freed.begin() + (ptrdiff_t)mid, freed.end());
+            W.dead_slots.clear();
+        }
         slots.end_layer(freed);
-        for (int32_t g = 0; g < world && world > 1; g++) rows[g].end_layer(W.freed_rows[t & 1][(size_t)g]);
+        for (int32_t g = 0; g < world && world > 1; g++) {
+            rows[g].end_layer(W.freed_rows[t & 1][(size_t)g]);
+            rows[g].end_layer(W.dead_rows[(size_t)g]);
+        }
     }
 
     // ---- the layers, as a pipeline.  What is sequential in planning is the slot assignment: the members of layer t
@@ -849,6 +892,8 @@ struct Planner {
         for (Alloc &a : rows) a.reset();
         // (two sets: lane B fills those of layer t+1 while lane A still returns those of layer t)
         for (auto &fr : W.freed_rows) { fr.resize((size_t)world); for (auto &v : fr) v.clear(); }
+        W.dead_slots.clear(); W.dead_rows.resize((size_t)world);
+        for (auto &v : W.dead_rows) v.clear();
         if (!streaming) P.rows_cap.assign((size_t)world, 0);
         load.assign((size_t)world, 0);
         // the owners once more, one byte per individual: the owner rule reads two parents per couple, and a generation of
@@ -1003,7 +1048,7 @@ struct Planner {
             for (int32_t g = 0; g < world; g++) P.rows_cap[g] = world > 1 ? std::max(rows[g].next_fresh, 1) : P.capacity;
         }
         if (int rc = std::getenv("GENLIB_PLAN_VERIFY") ? verify_plan(P, err) : GENLIB_OK) return rc;
-        const size_t np = P.pro_ind.size();
+        const size_t np = schedule == kScheduleF ? 0 : P.pro_ind.size();    // (kScheduleF: no proband matrix)
         P.pro_slot.resize(np); P.pro_owner.resize(np); P.pro_lrow.resize(np);
         for (size_t u = 0; u < np; u++) {
             const Home &hu = home[P.pro_ind[u]];

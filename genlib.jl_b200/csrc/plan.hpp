@@ -37,7 +37,15 @@ constexpr int kMaxTileFam = 64;  // couples per member tile (bounds the couple t
 //                                    the reference files phi[earlier][later] and reads phi[lower rank][higher
 //                                    rank] (compute.jl:393 vs :367-389), losing the pairs whose queue order
 //                                    inverts their rank order; kScheduleSparsePhi reproduces that loss
-constexpr int kSchedulePhi = 0, kScheduleSparsePhi = 1, kScheduleSparsePhiSymmetric = 2;
+//   f                                gen.f for many individuals: the members are the ancestors-or-self of the listed
+//                                    individuals that have both parents, layered by depth below the founders (a
+//                                    childless member of generation 3 is born in layer 3, not with the last one),
+//                                    with phi's arithmetic (the higher RANK is climbed, mem_ind is the rank).  No
+//                                    row is kept to the end: a row leaves after the layer of its last child, a row
+//                                    without children after its own layer (the layer still writes it).  The engine
+//                                    reads Psi[father, mother] of every couple just before its layer; there is no
+//                                    proband matrix (pro_slot / pro_owner / pro_lrow are empty).
+constexpr int kSchedulePhi = 0, kScheduleSparsePhi = 1, kScheduleSparsePhiSymmetric = 2, kScheduleF = 3;
 inline bool sparse_schedule(int s) { return s == kScheduleSparsePhi || s == kScheduleSparsePhiSymmetric; }
 
 constexpr int32_t kTileCarried = 1 << 30;   // live_tiles entry: the tile has a carried column
@@ -73,7 +81,7 @@ struct Plan {
     int64_t row_updates = 0;
     double alg_elems = 0;
     std::vector<Layer> layers;
-    std::vector<int32_t> pro_ind, pro_slot;
+    std::vector<int32_t> pro_ind, pro_slot;          // kScheduleF: pro_ind = the distinct listed individuals with both parents
     // concatenated per-layer arrays
     std::vector<int32_t> mem_ind, mem_slot, mem_fam;   // family-major order inside a layer
     std::vector<int32_t> mem_rank;                     // sparse_phi schedules: the members' pedigree ranks (mem_ind = queue position)

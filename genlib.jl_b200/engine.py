@@ -656,25 +656,40 @@ def findDistance(pedigree: Pedigree, IDs, ancestorID, *, device: int = -1) -> in
     return int(d[:, 0].sum())
 
 
-def f(pedigree: Pedigree, IDs, *, device: int = -1) -> np.ndarray:
-    """gen.f(pedigree, IDs): inbreeding coefficients, Float32 (src/compute.jl:500-511).
+def f(pedigree: Pedigree, IDs, *, device: int = -1, devices=None, return_stats: bool = False):
+    """gen.f(pedigree, IDs): inbreeding coefficients, Float32 in list order (src/compute.jl:500-511).
 
-    The reference evaluates phi(father, mother) by the exponential pairwise recursion in Float64
-    and rounds once; here the parents of all requested individuals go through ONE sweep of the
-    engine with Float64 storage (exact while kinships fit 53 bits, i.e. up to ~26 generations)
-    and the result is rounded to Float32.  SURVEY.md 8(f) N3."""
-    IDs = np.asarray(IDs, np.int64)
-    ranks = pedigree.rank_of(IDs)
-    fa, mo = pedigree.father[ranks], pedigree.mother[ranks]
-    both = (fa >= 0) & (mo >= 0)
-    out = np.zeros(len(IDs), np.float32)
-    if both.any():
-        parents = np.unique(np.concatenate([fa[both], mo[both]]))
-        k = phi(pedigree, pedigree.ids[parents], numerics="fp64", dtype=np.float64, device=device)
-        pos = {int(r): i for i, r in enumerate(parents)}
-        idx = np.nonzero(both)[0]
-        out[idx] = [np.float32(k[pos[int(fa[i])], pos[int(mo[i])]]) for i in idx]
-    return out
+    F of an individual is the kinship of its parents, 0 when a parent is missing.  The reference runs the
+    exponential pairwise recursion in Float64 per ID and rounds once; here ONE sweep of the engine with Float64
+    storage over the IDs' ancestors-or-self, layered by depth below the founders, reads Psi[father, mother] of
+    every couple on the device just before the couple's layer (genlib_f), so the cost grows with the pedigree,
+    not with the square of the number of IDs: the inbreeding of a whole population is one call.  Exact while
+    kinships fit 53 bits (about 26 generations, e.g. genea140); in deeper pedigrees the last Float64 bits follow
+    this schedule's order of the sums and may differ from the reference's before the rounding to Float32.
+    Duplicates are kept; KeyError on an unknown ID.  `devices=[0, 1, ...]` shards the frontier over several
+    GPUs of the box, with the same result.  SURVEY.md 8(f) N3."""
+    IDs = np.asarray(IDs, np.int64).reshape(-1)
+    ranks = pedigree.rank_of(IDs)                       # KeyError, like pedigree[ID]
+    res, stats = f_arrays(pedigree.father, pedigree.mother, ranks, device=device, devices=devices)
+    return (res, stats) if return_stats else res
+
+
+def f_arrays(father, mother, ranks, *, dtype=np.float32, device: int = -1, devices=None,
+             out: Optional[np.ndarray] = None):
+    """One-shot C-ABI call `genlib_f` on flat rank arrays (what the Julia shim ccalls).  Returns
+    (coefficients in list order as float32 or float64, stats)."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    r = np.ascontiguousarray(ranks, np.int32)
+    if out is None:
+        out = np.empty(len(r), dtype)
+    if out.shape != (len(r),) or not out.flags.c_contiguous or out.dtype not in _lib.DTYPES:
+        raise ValueError(f"out must be a contiguous ({len(r)},) float32/float64 array")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = Stats()
+    check(lib().genlib_f(len(father), ptr(father), ptr(mother), len(r), ptr(r), ptr(out),
+                         _lib.DTYPES[np.dtype(out.dtype)], len(dv), ptr(dv), C.byref(st)))
+    return out, st.as_dict()
 
 
 class KinshipMatrix:

@@ -169,24 +169,23 @@ function phiMean(pedigree::GenLib.Pedigree, probandIDs::Vector{Int} = GenLib.pro
 end
 
 """
-    f(pedigree, IDs) -> Vector{Float32}
+    f(pedigree, IDs; device = -1, devices = Int[]) -> Vector{Float32}
 
-`gen.f` (src/compute.jl:500-511): inbreeding = kinship of the parents.  The reference runs the
-exponential pairwise recursion once per ID; here the parents of all IDs go through ONE sweep of the
-engine with Float64 storage (exact while kinships fit 53 bits, i.e. pedigrees up to ~26 generations deep;
-beyond that the last bits can differ from the reference's Float64 recursion) and are rounded to Float32.
+`gen.f` (src/compute.jl:500-511): inbreeding = kinship of the parents, 0 when a parent is missing.  The reference
+runs the exponential pairwise recursion once per ID; here ONE sweep of the engine with Float64 storage over the
+IDs' ancestors-or-self, layered by depth below the founders, reads each couple's kinship on the device just before
+the couple's layer (`genlib_f`): the inbreeding of a whole population is one call.  Exact while kinships fit 53 bits
+(about 26 generations); beyond that the last Float64 bits follow this schedule's order of the sums and can differ
+from the reference's recursion.  Duplicates are kept; KeyError on an unknown ID.
 """
-function f(pedigree::GenLib.Pedigree, IDs::Vector{Int}; device::Integer = -1)
-    coefficients = zeros(Float32, length(IDs))
-    pairs = [(pedigree[ID].father, pedigree[ID].mother) for ID in IDs]          # KeyError on unknown ID
-    parents = sort(unique(Int[p.ID for pr in pairs for p in pr if !isnothing(pr[1]) && !isnothing(pr[2])]))
-    isempty(parents) && return coefficients
-    k = phi(pedigree, parents; numerics = :fp64, device = device)   # Float32 view of the Float64-storage sweep
-    pos = Dict(ID => i for (i, ID) in enumerate(parents))
-    for (i, (fa, mo)) in enumerate(pairs)
-        (isnothing(fa) || isnothing(mo)) && continue
-        coefficients[i] = k[pos[fa.ID], pos[mo.ID]]
-    end
+function f(pedigree::GenLib.Pedigree, IDs::Vector{Int}; device::Integer = -1, devices::Vector{<:Integer} = Int[])
+    father, mother = flatten(pedigree)
+    ranks = Int32[pedigree[ID].rank - 1 for ID in IDs]                 # KeyError on unknown ID
+    coefficients = Vector{Float32}(undef, length(ranks))
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    GC.@preserve coefficients check(ccall((:genlib_f, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Cvoid}, Cint, Int32, Ptr{Int32}, Ptr{Cvoid}),
+        length(father), father, mother, length(ranks), ranks, coefficients, 0, length(devs), devs, C_NULL))
     coefficients
 end
 

@@ -151,10 +151,16 @@ int genlib_plan_create(int32_t n, const int32_t *father, const int32_t *mother, 
  *       phi[lower rank][higher rank] (:36-40, :367-389); when the queue order of two individuals of the
  *       same depth inverts their rank order the value is never found again and the reference carries on
  *       as if they were unrelated.  GENLIB_SCHEDULE_SPARSE_PHI reproduces that (bit-identical to the
- *       reference's KinshipMatrix look-ups); this variant keeps those kinships. */
+ *       reference's KinshipMatrix look-ups); this variant keeps those kinships.
+ *   GENLIB_SCHEDULE_F  the schedule of genlib_f: the members are the ancestors-or-self of the listed individuals
+ *       that have both parents (the others never reach the plan), layered by depth below the founders, with
+ *       phi's arithmetic; no row is kept to the end (a row leaves after the layer of its last child, or after
+ *       its own layer when it has none).  Such a plan has no proband matrix: it can be inspected with the
+ *       genlib_plan_* calls, genlib_engine_create* refuses it (GENLIB_EINVAL). */
 #define GENLIB_SCHEDULE_PHI 0
 #define GENLIB_SCHEDULE_SPARSE_PHI 1
 #define GENLIB_SCHEDULE_SPARSE_PHI_SYMMETRIC 2
+#define GENLIB_SCHEDULE_F 3
 int genlib_plan_create_scheduled(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
                                  const int32_t *proband, int32_t world, int schedule, genlib_plan **out);
 /* The same with the individuals' IDs (by rank; may be NULL).  sparse_phi seeds its queue with
@@ -242,6 +248,20 @@ int genlib_plan_stream_selftest(int32_t n, const int32_t *father, const int32_t 
 int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
                      const int32_t *proband, void *out, int out_dtype, int numerics, int32_t n_dev,
                      const int32_t *devices, genlib_stats *stats);
+
+/* ---- gen.f: inbreeding coefficients (src/compute.jl:500-511) ---------------------------------------------------
+ * F[i] = Psi[father(ids[i]), mother(ids[i])], 0 when a parent is missing.  One sweep of the engine over the IDs'
+ * ancestors-or-self (GENLIB_SCHEDULE_F, Float64 storage) reads each couple's Psi[father, mother] on the device just
+ * before the couple's layer; nothing quadratic in the number of IDs is formed or leaves the device (8 bytes per
+ * couple are copied back).  The value is read directly, not as 2 Psi[i, i] - 1.  While kinships fit 53 bits (about
+ * 26 generations) every value is exact and equals the reference's Float64 recursion; deeper pedigrees are summed in
+ * the depth-layered order of this schedule, so their last Float64 bits may differ.
+ * out: n_ids elements of out_dtype in list order (duplicates kept).  An index out of range gives GENLIB_EKEY.  A list
+ * without an individual that has both parents gives zeros without a device.  devices[0] < 0 = the current device
+ * (one device); several devices shard the frontier rows as genlib_phi_multi does, with the same result bitwise.
+ * GENLIB_ENOMEM names the bytes one device needs.  stats->n_unique counts the distinct IDs with both parents. */
+int genlib_f(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_ids, const int32_t *ids,
+             void *out, int out_dtype, int32_t n_dev, const int32_t *devices, genlib_stats *stats);
 
 /* ---- handle API: keep the schedule on the device, run, fetch ---------------
  * (what the benchmark and a multi-call Julia session use) */
