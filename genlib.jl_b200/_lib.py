@@ -15,7 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("GENLIB_CUDA_LIB") or os.path.join(_HERE, "libgenlib_cuda.so")
 
 OK, EINVAL, EKEY, EORDER, ECUDA, ENOMEM, ECOMM, ERESTART, EOVERFLOW = range(9)
-SCHEDULES = {"phi": 0, "sparse_phi": 1, "sparse_phi_symmetric": 2, "f": 3}
+SCHEDULES = {"phi": 0, "sparse_phi": 1, "sparse_phi_symmetric": 2, "f": 3, "pairs": 4}
 NUMERICS = {"reference": 0, "fp64": 1, 0: 0, 1: 1}
 DTYPES = {np.dtype(np.float32): 0, np.dtype(np.float64): 1}
 
@@ -120,6 +120,9 @@ SYMBOLS = {
     "genlib_phi_multi": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_int, C.c_int, C.c_int32, _P,
                                    C.POINTER(Stats)]),
     "genlib_f": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_int, C.c_int32, _P, C.POINTER(Stats)]),
+    "genlib_phi_pairs": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, _P, C.c_int, C.c_int32, _P, C.POINTER(Stats)]),
+    "genlib_plan_create_pairs": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, C.c_int32, C.c_int, C.POINTER(_P)]),
+    "genlib_plan_pair_reads": (C.c_int64, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "genlib_plan_create_async": (C.c_int, [C.c_int32, _P, _P, _P, C.c_int32, _P, C.c_int32, C.c_int, C.POINTER(_P)]),
     "genlib_plan_stream_selftest": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, C.c_double, _P, _P]),
     "genlib_engine_create": (C.c_int, [_P, C.c_int, C.c_int, C.POINTER(_P)]),

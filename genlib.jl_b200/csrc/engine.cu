@@ -1,5 +1,5 @@
 // engine.cu -- the phi engine and the library-wide part of the C ABI of libgenlib_cuda.so (include/genlib_cuda.h):
-// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_f, errors and caches.  gen.gc, gen.occ and gen.rec are
+// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_f / genlib_phi_pairs, errors and caches.  gen.gc, gen.occ and gen.rec are
 // in gc_engine.cu; the host helpers both share are in runtime.hpp.
 //
 // The ABI stands where the reference's Julia method stands:
@@ -77,10 +77,11 @@ struct genlib_plan {
     // build_plan into `p` (published through `ps` when given), with its status, message and time from t0.  Out of
     // host memory fails the plan like any planner error and closes a streamed one, so that its readers stop waiting.
     void build(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
-               const int32_t *proband, int32_t world, int schedule, PlanStream *ps, int planners, double t0) {
+               const int32_t *proband, int32_t world, int schedule, PlanStream *ps, int planners, double t0,
+               const PairList &pairs = PairList{}) {
         try {
             adopt_retired_storage(p);        // the arrays of the last destroyed plan, already paged in
-            worker_rc = build_plan(n, father, mother, ids, n_pro, proband, world, schedule, p, worker_err, ps, planners);
+            worker_rc = build_plan(n, father, mother, ids, n_pro, proband, world, schedule, p, worker_err, ps, planners, pairs);
         } catch (const std::bad_alloc &) {
             worker_rc = GENLIB_ENOMEM; worker_err = "out of host memory while planning";
             if (ps) { ps->status.store(GENLIB_ENOMEM); ps->stage.store(2); ps->wake(); }
@@ -131,6 +132,9 @@ struct IndexBufs {
     DevBuf<uint8_t> flags;
     DevBuf<double> acc;
     DevBuf<double> fam_kin;                // kScheduleF: Psi[father, mother] per couple (couples whose father row is own)
+    DevBuf<int8_t> pair_owner;             // kSchedulePairs: per read, the row's owner, local row and column slot,
+    DevBuf<int32_t> pair_lrow, pair_col;
+    DevBuf<double> pair_kin;               // and Psi[a, b] (reads whose row is own)
 };
 
 struct genlib_engine : IndexBufs {
@@ -187,16 +191,17 @@ void fill_info(const Layer &L, genlib_layer_info *o) {
 
 size_t plan_index_bytes(const Plan &P) {
     return (P.mem_ind.size() * 4 + P.mem_rank.size() + P.fam_pf.size() * 6 + P.fam_start.size() + P.mtile_desc.size() +
-            P.pro_slot.size() * 2 + P.live_lrow.size() + P.tile_map.size() + P.live_tiles.size()) * sizeof(int32_t) + P.fam_pf.size() * 2 + P.live_owner.size() + P.flags.size();
+            P.pro_slot.size() * 2 + P.live_lrow.size() + P.tile_map.size() + P.live_tiles.size() + P.pair_lrow.size() * 2) * sizeof(int32_t) +
+           P.fam_pf.size() * 2 + P.live_owner.size() + P.flags.size() + P.pair_owner.size();
 }
 
-// The traffic the layers cannot avoid: s (4 n L + 3 n^2) per layer, and for kScheduleF 8 bytes per couple with
-// both parents (its Psi[father, mother], read once and written once).
+// The traffic the layers cannot avoid: s (4 n L + 3 n^2) per layer, for kScheduleF 8 bytes per couple with
+// both parents (its Psi[father, mother], read once and written once), for kSchedulePairs 8 bytes per read.
 double plan_alg_bytes(const Plan &P, size_t es) {
     double b = P.alg_elems * (double)es;
     if (P.schedule == kScheduleF)
         for (size_t k = 0; k < P.fam_pf.size(); k++) b += (P.fam_pf[k] >= 0 && P.fam_pm[k] >= 0) ? 8.0 : 0.0;
-    return b;
+    return b + 8.0 * (double)P.pair_pos.size();
 }
 
 // Arena layout of rank g.  The first two regions are what peers address (barrier flags, frontier rows).
@@ -310,6 +315,10 @@ unsigned char *place_arrays(IndexBufs &B, const Plan &P, bool streamed, unsigned
     B.flags.place(cur, cnt(P.flags)); B.acc.place(cur, 4);
     B.pro_owner.place(cur, npro); B.pro_lrow.place(cur, npro);
     if (P.schedule == kScheduleF) B.fam_kin.place(cur, cnt(P.fam_pf));
+    if (P.schedule == kSchedulePairs) {
+        const size_t K = P.pair_pos.size();                    // (sized at the list's length before any layer is published)
+        B.pair_owner.place(cur, K); B.pair_lrow.place(cur, K); B.pair_col.place(cur, K); B.pair_kin.place(cur, K);
+    }
     return cur;
 }
 
@@ -392,11 +401,25 @@ int prepare_launches(genlib_engine &E, size_t smem_max) {
     return GENLIB_OK;
 }
 
+// kSchedulePairs: the reads of layer t (t == S: after the last layer and its barrier), while their rows hold them
+// (such a plan's engine stores Float64: create_engine refuses any other numerics)
+void launch_pair_reads(genlib_engine &E, int t, int &launches) {
+    const Plan &P = E.plan->p;
+    if (P.schedule != kSchedulePairs) return;
+    const int64_t i0 = P.pair_start[(size_t)t], nr = P.pair_start[(size_t)t + 1] - i0;
+    if (nr == 0) return;
+    pair_kinship_kernel<<<(unsigned)((nr + kThreads - 1) / kThreads), kThreads, 0, E.stream>>>(
+        static_cast<const double *>(E.A), P.capacity, E.pair_owner.p + i0, E.pair_lrow.p + i0, E.pair_col.p + i0, nr, E.rank,
+        E.pair_kin.p + i0);
+    launches++;
+}
+
 // one generation step: the layer kernel (and sparse_phi's misfiled pairs), then the inter-GPU barrier
 template <typename T>
 int launch_layer(genlib_engine &E, int t, bool timed, size_t &ev, int &launches) {
     const Plan &P = E.plan->p;
     const Layer &L = P.layers[t];
+    launch_pair_reads(E, t, launches);                          // the pairs read before this layer
     if (L.n_new == 0) return GENLIB_OK;
     T *A = static_cast<T *>(E.A);
     const int64_t ld = P.capacity;
@@ -442,10 +465,12 @@ int launch_layers(genlib_engine &E, bool timed) {
     if (int rc = prepare_launches<T>(E, smem_max)) return rc;
     int launches = 0;
     size_t ev = 0;
-    for (int t = 0; t < (int)P.layers.size(); t++) {
+    const int S = (int)P.layers.size();
+    for (int t = 0; t < S; t++) {
         if (E.layer_limit >= 0 && t >= E.layer_limit) break;
         if (int rc = launch_layer<T>(E, t, timed, ev, launches)) return rc;
     }
+    if (E.layer_limit < 0 || E.layer_limit >= S) launch_pair_reads(E, S, launches);   // the pairs read after the last layer
     CU(cudaGetLastError());
     E.stats.kernel_launches = launches;
 #ifdef GENLIB_PROFILE
@@ -468,6 +493,7 @@ int launch_layers(genlib_engine &E, bool timed) {
 
 int upload_layers(genlib_engine &E, int t0, int t1);
 int upload_probands(genlib_engine &E);
+int upload_pair_reads(genlib_engine &E, int64_t i0, int64_t i1);
 
 // what the kernels of a run left in their error words
 int check_device_errors(genlib_engine &E) {
@@ -523,12 +549,13 @@ int run_streamed(genlib_engine &E, PlanStream &ps) {
         done = avail;
         if (overflow || too_small) { cudaStreamSynchronize(E.stream); return kRestart; }
     }
-    CU(cudaGetLastError());
-    E.stats.kernel_launches = launches;
     ps.wait([&] { return ps.stage.load() == 2; });              // the probands' homes close the plan
     if (ps.status.load() != GENLIB_OK) return ps.status.load();
     if (ps.overflow.load()) { cudaStreamSynchronize(E.stream); return kRestart; }
     if (int rc = upload_probands(E)) return rc;
+    launch_pair_reads(E, S, launches);                          // the pairs read after the last layer
+    CU(cudaGetLastError());
+    E.stats.kernel_launches = launches;
     CU(cudaEventRecord(E.events[nev - 1], E.stream));
     CU(cudaStreamSynchronize(E.stream));
     float ms = 0;
@@ -627,9 +654,14 @@ void account_layers(genlib_engine &E) {
     E.info_ready = true;
 }
 
-// this rank's probands in output order, and where their rows and columns are (needs the finished plan)
+// this rank's probands in output order, and where their rows and columns are, and the pair reads after the last
+// layer (needs the finished plan)
 int upload_probands(genlib_engine &E) {
     const Plan &P = E.plan->p;
+    if (P.schedule == kSchedulePairs) {
+        const size_t S = P.layers.size();
+        if (int rc = upload_pair_reads(E, P.pair_start[S], P.pair_start[S + 1])) return rc;
+    }
     std::vector<int32_t> own_rows;
     E.own_pro.clear();
     for (size_t u = 0; u < P.pro_owner.size(); u++)            // (empty for kScheduleF: no proband matrix)
@@ -639,6 +671,17 @@ int upload_probands(genlib_engine &E) {
     CU(E.pro_owner.upload(P.pro_owner, E.stream));
     CU(E.pro_lrow.upload(P.pro_lrow, E.stream));
     CU(cudaStreamSynchronize(E.stream));                       // (own_rows is a local)
+    return GENLIB_OK;
+}
+
+// reads [i0, i1) of a kSchedulePairs plan -> device
+int upload_pair_reads(genlib_engine &E, int64_t i0, int64_t i1) {
+    const Plan &P = E.plan->p;
+    if (i1 <= i0) return GENLIB_OK;
+    const size_t a = (size_t)i0, k = (size_t)(i1 - i0);
+    CU(cudaMemcpyAsync(E.pair_owner.p + a, P.pair_owner.data() + a, k * sizeof(int8_t), cudaMemcpyHostToDevice, E.stream));
+    CU(cudaMemcpyAsync(E.pair_lrow.p + a, P.pair_lrow.data() + a, k * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    CU(cudaMemcpyAsync(E.pair_col.p + a, P.pair_col_slot.data() + a, k * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
     return GENLIB_OK;
 }
 
@@ -663,6 +706,8 @@ int upload_layers(genlib_engine &E, int t0, int t1) {
     CU(up(E.flags, P.flags, A.flag_off, Z.flag_end));
     CU(up(E.live_owner, P.live_owner, A.flag_off, Z.flag_end)); CU(up(E.live_lrow, P.live_lrow, A.flag_off, Z.flag_end));
     CU(up(E.tile_map, P.tile_map, A.tile_off, Z.tile_end)); CU(up(E.live_tiles, P.live_tiles, A.ltile_off, Z.ltile_end));
+    if (P.schedule == kSchedulePairs)
+        if (int rc = upload_pair_reads(E, P.pair_start[(size_t)t0], P.pair_start[(size_t)t1])) return rc;
     return GENLIB_OK;
 }
 
@@ -673,8 +718,8 @@ int create_engine(const genlib_plan *plan, int numerics, int device, int rank, g
     const Plan &P = plan->p;
     if (sparse_schedule(P.schedule) && numerics != GENLIB_NUMERICS_REFERENCE)
         return fail(GENLIB_EINVAL, "the sparse_phi schedule stores Float32 (numerics must be GENLIB_NUMERICS_REFERENCE)");
-    if (P.schedule == kScheduleF && numerics != GENLIB_NUMERICS_FP64)
-        return fail(GENLIB_EINVAL, "the gen.f schedule stores Float64 (numerics must be GENLIB_NUMERICS_FP64)");
+    if ((P.schedule == kScheduleF || P.schedule == kSchedulePairs) && numerics != GENLIB_NUMERICS_FP64)
+        return fail(GENLIB_EINVAL, "the gen.f and gen.phi_pairs schedules store Float64 (numerics must be GENLIB_NUMERICS_FP64)");
     if (rank < 0 || rank >= P.world) return fail(GENLIB_EINVAL, "rank outside the plan's world");
     if (P.world > kMaxWorld) return fail(GENLIB_EINVAL, "the engine supports at most 16 ranks");
     if (P.n_unique == 0) return fail(GENLIB_EINVAL, "empty proband list: nothing to run");
@@ -803,23 +848,29 @@ int genlib_plan_create_scheduled(int32_t n, const int32_t *father, const int32_t
     return genlib_plan_create_ex(n, father, mother, nullptr, n_pro, proband, world, schedule, out);
 }
 
-int genlib_plan_create_ex(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
-                          const int32_t *proband, int32_t world, int schedule, genlib_plan **out) {
+static int plan_create(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
+                       const int32_t *proband, int32_t world, int schedule, const PairList &pairs, genlib_plan **out) {
     if (!out) return fail(GENLIB_EINVAL, "genlib_plan_create: out is null");
     *out = nullptr;
     std::unique_ptr<genlib_plan> pl(new (std::nothrow) genlib_plan);
     if (!pl) return fail(GENLIB_ENOMEM, "out of host memory");
-    pl->build(n, father, mother, ids, n_pro, proband, world, schedule, nullptr, 0, now_ms());
+    pl->build(n, father, mother, ids, n_pro, proband, world, schedule, nullptr, 0, now_ms(), pairs);
     if (pl->worker_rc != GENLIB_OK) return fail(pl->worker_rc, pl->worker_err);
     *out = pl.release();
     return GENLIB_OK;
 }
 
-int genlib_plan_create_async(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
-                             const int32_t *proband, int32_t world, int schedule, genlib_plan **out) {
+int genlib_plan_create_ex(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
+                          const int32_t *proband, int32_t world, int schedule, genlib_plan **out) {
+    return plan_create(n, father, mother, ids, n_pro, proband, world, schedule, PairList{}, out);
+}
+
+// a plan made on a worker thread and published layer by layer (the caller's arrays stay alive until it is settled)
+static int plan_create_async(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
+                             const int32_t *proband, int32_t world, int schedule, const PairList &pairs, genlib_plan **out) {
     if (!out) return fail(GENLIB_EINVAL, "genlib_plan_create: out is null");
     *out = nullptr;
-    if (env_int("GENLIB_STREAM", 1) == 0) return genlib_plan_create_ex(n, father, mother, ids, n_pro, proband, world, schedule, out);
+    if (env_int("GENLIB_STREAM", 1) == 0) return plan_create(n, father, mother, ids, n_pro, proband, world, schedule, pairs, out);
     std::unique_ptr<genlib_plan> pl(new (std::nothrow) genlib_plan);
     if (!pl) return fail(GENLIB_ENOMEM, "out of host memory");
     pl->stream.reset(new (std::nothrow) PlanStream);
@@ -827,10 +878,10 @@ int genlib_plan_create_async(int32_t n, const int32_t *father, const int32_t *mo
     genlib_plan *raw = pl.get();
     const double t0 = now_ms();
     try {
-        raw->worker = std::thread([=] { raw->build(n, father, mother, ids, n_pro, proband, world, schedule, raw->stream.get(), 0, t0); });
+        raw->worker = std::thread([=] { raw->build(n, father, mother, ids, n_pro, proband, world, schedule, raw->stream.get(), 0, t0, pairs); });
     } catch (...) {                              // no thread to be had
         pl.reset();
-        return genlib_plan_create_ex(n, father, mother, ids, n_pro, proband, world, schedule, out);
+        return plan_create(n, father, mother, ids, n_pro, proband, world, schedule, pairs, out);
     }
     PlanStream &ps = *raw->stream;
     ps.wait([&] { return ps.stage.load() >= 1; });
@@ -840,6 +891,36 @@ int genlib_plan_create_async(int32_t n, const int32_t *father, const int32_t *mo
     }
     *out = pl.release();
     return GENLIB_OK;
+}
+
+int genlib_plan_create_async(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
+                             const int32_t *proband, int32_t world, int schedule, genlib_plan **out) {
+    return plan_create_async(n, father, mother, ids, n_pro, proband, world, schedule, PairList{}, out);
+}
+
+int genlib_plan_create_pairs(int32_t n, const int32_t *father, const int32_t *mother, int64_t n_pairs, const int32_t *a,
+                             const int32_t *b, int32_t world, int stream, genlib_plan **out) {
+    const PairList pairs{n_pairs, a, b};
+    return stream ? plan_create_async(n, father, mother, nullptr, 0, nullptr, world, GENLIB_SCHEDULE_PAIRS, pairs, out)
+                  : plan_create(n, father, mother, nullptr, 0, nullptr, world, GENLIB_SCHEDULE_PAIRS, pairs, out);
+}
+
+int64_t genlib_plan_pair_reads(const genlib_plan *plan, int32_t layer, int64_t *pos, int32_t *row_slot, int32_t *col_slot,
+                               int32_t *owner, int32_t *lrow) {
+    settle(plan);
+    if (!plan || plan->p.schedule != kSchedulePairs || plan->p.pair_start.empty() || layer < 0 || layer > (int32_t)plan->p.layers.size())
+        { fail(GENLIB_EINVAL, "genlib_plan_pair_reads: not a GENLIB_SCHEDULE_PAIRS plan, or no such layer"); return -1; }
+    const Plan &P = plan->p;
+    const int64_t i0 = P.pair_start[(size_t)layer], i1 = P.pair_start[(size_t)layer + 1];
+    for (int64_t i = i0; i < i1; i++) {
+        const size_t k = (size_t)(i - i0), j = (size_t)i;
+        if (pos) pos[k] = P.pair_pos[j];
+        if (row_slot) row_slot[k] = P.pair_row_slot[j];
+        if (col_slot) col_slot[k] = P.pair_col_slot[j];
+        if (owner) owner[k] = P.pair_owner[j];
+        if (lrow) lrow[k] = P.pair_lrow[j];
+    }
+    return i1 - i0;
 }
 
 void genlib_plan_destroy(genlib_plan *plan) {
@@ -975,6 +1056,8 @@ static int create_engine_public(const genlib_plan *plan, int numerics, int devic
     if (out) *out = nullptr;
     if (plan && plan->p.schedule == kScheduleF)                  // (set before genlib_plan_create* returns)
         return fail(GENLIB_EINVAL, "a GENLIB_SCHEDULE_F plan has no matrix to fetch: call genlib_f");
+    if (plan && plan->p.schedule == kSchedulePairs)
+        return fail(GENLIB_EINVAL, "a GENLIB_SCHEDULE_PAIRS plan has no matrix to fetch: call genlib_phi_pairs");
     if (plan && plan->streaming()) {
         PlanStream &ps = *plan->stream;
         StreamConsumer reader(ps);
@@ -1203,13 +1286,13 @@ struct OneshotFetch {
     std::function<int(genlib_engine &, int)> device;
 };
 
-// genlib_phi, genlib_phi_multi and genlib_f: ONE plan for all devices, made on a worker thread and handed over layer
+// genlib_phi, genlib_phi_multi, genlib_f and genlib_phi_pairs: ONE plan for all devices, made on a worker thread and handed over layer
 // by layer (PlanStream), so that the devices run the first generations while the later ones are planned.
 // GENLIB_STREAM=0, or a bound of the streamed plan that did not hold, plans first and then runs.  One device runs on
 // the calling thread; several get a host thread each and NVLink peer access.  `has_out`: the caller wants a result.
 static int oneshot(const std::string &who, int schedule, int32_t n, const int32_t *father, const int32_t *mother,
                    int32_t n_pro, const int32_t *proband, bool has_out, int numerics, int32_t n_dev, const int32_t *devices,
-                   genlib_stats *stats, const OneshotFetch &fetch) {
+                   genlib_stats *stats, const OneshotFetch &fetch, const PairList &pairs = PairList{}) {
     const bool multi = n_dev > 1;
     std::vector<int> dev(devices, devices + n_dev);              // (one device: a negative one is the current device)
     if (int rc = multi ? resolve_devices(who, n_dev, devices, false, dev) : GENLIB_OK) return rc;
@@ -1220,7 +1303,7 @@ static int oneshot(const std::string &who, int schedule, int32_t n, const int32_
     const double tp0 = now_ms();
     PlanStream ps;
     auto make_plan = [&](PlanStream *stream) {
-        plan->build(n, father, mother, nullptr, n_pro, proband, n_dev, schedule, stream, /*planners=*/1, tp0);
+        plan->build(n, father, mother, nullptr, n_pro, proband, n_dev, schedule, stream, /*planners=*/1, tp0, pairs);
     };
     if (want_stream) { try { plan->worker = std::thread([&] { make_plan(&ps); }); } catch (...) { } }
     const bool streaming = plan->worker.joinable();
@@ -1414,6 +1497,51 @@ int genlib_f(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_
     };
     return oneshot("genlib_f", kScheduleF, n, father, mother, n_ids, ids, true, GENLIB_NUMERICS_FP64, n_dev, devices,
                    stats, fetch);
+}
+
+// genlib_phi_pairs: a GENLIB_SCHEDULE_PAIRS plan of everybody named; every device copies its per-read kinships to the
+// host once (all K entries: a device leaves the reads it does not own unwritten, and they are not used), and each
+// list position takes the value of its read from the device that holds the read's row.
+int genlib_phi_pairs(int32_t n, const int32_t *father, const int32_t *mother, int64_t n_pairs, const int32_t *a,
+                     const int32_t *b, void *out, int out_dtype, int32_t n_dev, const int32_t *devices, genlib_stats *stats) {
+    if (n < 0 || n_pairs < 0 || (n > 0 && (!father || !mother)) || (n_pairs > 0 && (!a || !b || !out)))
+        return fail(GENLIB_EINVAL, "genlib_phi_pairs: null pointer or negative size");
+    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
+    if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_pairs: 1 .. 16 devices");
+    for (int64_t k = 0; k < n_pairs; k++)
+        for (const int32_t x : {a[k], b[k]})
+            if (x < 0 || x >= n) {
+                std::string err;
+                if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);   // (a broken pedigree is reported first)
+                return fail(GENLIB_EKEY, "KeyError: index " + std::to_string(x) + " not in pedigree");
+            }
+    if (n_pairs == 0) {                                          // no plan, no device
+        std::string err;
+        if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);
+        if (stats) std::memset(stats, 0, sizeof *stats);
+        return GENLIB_OK;
+    }
+    auto put = [&](int64_t i, double v) {
+        if (out_dtype == GENLIB_F64) static_cast<double *>(out)[i] = v;
+        else static_cast<float *>(out)[i] = (float)v;
+    };
+    OneshotFetch fetch;
+    fetch.device = [&](genlib_engine &E, int g) {
+        DeviceGuard guard;
+        if (int r = guard.enter(E.device)) return r;
+        const double t0 = now_ms();
+        const Plan &P = E.plan->p;
+        std::vector<double> kin(P.pair_pos.size());
+        CU(cudaMemcpyAsync(kin.data(), E.pair_kin.p, kin.size() * sizeof(double), cudaMemcpyDeviceToHost, E.stream));
+        CU(cudaStreamSynchronize(E.stream));
+        for (size_t i = 0; i < kin.size(); i++)
+            if (P.pair_owner[i] == g) put(P.pair_pos[i], kin[i]);
+        E.stats.d2h_bytes += (int64_t)(kin.size() * sizeof(double));
+        E.stats.ms_fetch = now_ms() - t0;
+        return GENLIB_OK;
+    };
+    return oneshot("genlib_phi_pairs", kSchedulePairs, n, father, mother, 0, nullptr, true, GENLIB_NUMERICS_FP64, n_dev,
+                   devices, stats, fetch, PairList{n_pairs, a, b});
 }
 
 int genlib_phi(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,

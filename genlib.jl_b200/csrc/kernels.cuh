@@ -1,6 +1,6 @@
 // kernels.cuh -- device-side vocabulary shared by the sm_100a kernels of the kinship sweep, and the
 // small kernels around the layer kernel (layer_kernel.cuh): proband gather, phiMean reduction, the
-// inter-GPU barrier, sparse_phi's misfiled pairs and gen.f's parents' kinships.
+// inter-GPU barrier, sparse_phi's misfiled pairs, gen.f's parents' kinships and gen.phi_pairs' reads.
 //
 // Arithmetic is binary64 in the reference's grouping; storage type T is float
 // (GENLIB_NUMERICS_REFERENCE: one RN32 per step, like src/compute.jl:296) or double.
@@ -160,6 +160,20 @@ __global__ void couple_kinship_kernel(const T *__restrict__ A, int64_t ld, const
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= n_fam || pf_owner[f] != rank || pm[f] < 0) return;
     out[f] = (double)A[(int64_t)pf_lrow[f] * ld + pm[f]];
+}
+
+// =====================================================================================
+// pair_kinship_kernel (GENLIB_SCHEDULE_PAIRS), launched just BEFORE the layer kernel of the reads' layer (or once after
+// the last layer): Psi[a, b] of a pair is the entry at the other member's slot of the higher-ranked member's row.  Both
+// rows are live then and nobody writes that entry; one thread per read of the layer, every rank reads the rows it holds.
+// Such a plan always stores Float64.
+// =====================================================================================
+__global__ void pair_kinship_kernel(const double *__restrict__ A, int64_t ld, const int8_t *__restrict__ owner,
+                                    const int32_t *__restrict__ lrow, const int32_t *__restrict__ col, int64_t n_reads,
+                                    int rank, double *__restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_reads || owner[i] != rank) return;
+    out[i] = A[(int64_t)lrow[i] * ld + col[i]];
 }
 
 // =====================================================================================

@@ -137,6 +137,7 @@ struct Scratch {
     std::vector<int32_t> last_of;
     std::vector<int32_t> dead_slots;                            // kScheduleF: slots / rows (per owner) of the members that no
     std::vector<std::vector<int32_t>> dead_rows;                // later layer reads, freed at the end of their own layer
+    std::vector<int32_t> read_last;                             // kSchedulePairs: per individual, its last read layer (-1: none)
     std::vector<int32_t> fam_of, fam_count, fam_first, fam_key, fam_n;   // couples of every layer (grouped ahead by helper threads)
     std::vector<int32_t> order, newid, nf_of, load, freed, evicted[2], cnt, cnt_order, ipos;   // order / newid: by member / couple of every layer
     std::vector<FamilyTable> tables;          // one per planning thread
@@ -181,6 +182,49 @@ struct PhaseTimer {
     void add(int k) { if (on) sum[k] += lap(); }
     void phase(const char *name) { if (on) std::fprintf(stderr, "[plan] %-12s %.2f ms\n", name, lap()); }
 };
+
+// kSchedulePairs: both slots of every read hold the pair's members when it is read.  Before layer t (t < S) they are
+// live there, and the row side is where the live list says; after the last layer (t == S) the slots' last members are
+// the pair's own (no one born later took them), and an earlier-born member's row was carried through the last layer
+// (only carried rows receive the columns of the last layer's members).
+int verify_pair_reads(const Plan &P, const PairList &pairs, std::string &err) {
+    const int32_t S = (int32_t)P.layers.size();
+    if ((int64_t)P.pair_pos.size() != pairs.n || (int32_t)P.pair_start.size() != S + 2 || P.pair_start[(size_t)S + 1] != pairs.n)
+        { err = "verify: the pair reads do not cover the list"; return GENLIB_EINVAL; }
+    std::vector<int32_t> last_in((size_t)P.capacity, -1);            // slot -> its last member (mem_ind is the rank)
+    std::vector<uint8_t> born_last((size_t)P.capacity, 0);           // slot of a member of the last layer
+    for (int32_t t = 0; t < S; t++) {
+        const Layer &L = P.layers[(size_t)t];
+        for (int32_t q = 0; q < L.n_new; q++) {
+            last_in[(size_t)P.mem_slot[L.mem_off + q]] = P.mem_ind[L.mem_off + q];
+            if (t == S - 1) born_last[(size_t)P.mem_slot[L.mem_off + q]] = 1;
+        }
+    }
+    for (int32_t t = 0; t <= S; t++)
+        for (int64_t i = P.pair_start[(size_t)t]; i < P.pair_start[(size_t)t + 1]; i++) {
+            const int64_t p = P.pair_pos[(size_t)i];
+            const int32_t x = pairs.a[p], y = pairs.b[p], slots[2] = {P.pair_row_slot[(size_t)i], P.pair_col_slot[(size_t)i]};
+            const std::string at = " of list position " + std::to_string(p) + " read in layer " + std::to_string(t);
+            if (t < S) {
+                const Layer &L = P.layers[(size_t)t];
+                for (int32_t s : slots)
+                    if (s < L.rt_lo || s >= L.rt_lo + L.rt_rows || !(P.flags[L.flag_off + (size_t)(s - L.rt_lo)] & kFlagLive))
+                        { err = "verify: a slot" + at + " is not live"; return GENLIB_EINVAL; }
+                const size_t r = L.flag_off + (size_t)(slots[0] - L.rt_lo);
+                if (P.live_owner[r] != P.pair_owner[(size_t)i] || P.live_lrow[r] != P.pair_lrow[(size_t)i])
+                    { err = "verify: the row" + at + " is not where the live list has it"; return GENLIB_EINVAL; }
+            } else {
+                if (last_in[(size_t)slots[0]] != std::max(x, y) || last_in[(size_t)slots[1]] != std::min(x, y))
+                    { err = "verify: a slot" + at + " was handed to someone born later"; return GENLIB_EINVAL; }
+                const Layer &L = P.layers[(size_t)S - 1];
+                for (int32_t s : slots) {
+                    const bool carried = s >= L.rt_lo && s < L.rt_lo + L.rt_rows && (P.flags[L.flag_off + (size_t)(s - L.rt_lo)] & kFlagCarried);
+                    if (!born_last[(size_t)s] && !carried) { err = "verify: a row" + at + " was not carried through the last layer"; return GENLIB_EINVAL; }
+                }
+            }
+        }
+    return GENLIB_OK;
+}
 
 // GENLIB_PLAN_VERIFY (a debugging aid): the index ranges the layer kernel relies on.
 int verify_plan(const Plan &P, std::string &err) {
@@ -233,9 +277,11 @@ int verify_plan(const Plan &P, std::string &err) {
 struct Planner {
     Scratch &W; Plan &P; std::string &err; PlanStream *ps;
     const int32_t n, *father, *mother; const int64_t *ids; const int32_t n_pro, *proband, world; const int schedule, planners;
+    const PairList &pairs;                                      // kSchedulePairs
     const bool by_seq = sparse_schedule(schedule);              // members of a layer in processing order
-    const bool by_depth = by_seq || schedule == kScheduleF;     // layers by depth below the founders
-    const bool short_rows = schedule == kScheduleF;             // rows that no later layer reads (childless members)
+    const bool reads = schedule == kSchedulePairs;              // rows read by pairs (pair_* arrays)
+    const bool by_depth = by_seq || schedule == kScheduleF || reads;     // layers by depth below the founders
+    const bool short_rows = schedule == kScheduleF || reads;    // rows that no later layer reads (childless members)
     PhaseTimer clock{};
     std::vector<uint8_t> &is_pro = W.is_pro;
     std::vector<Pre> &pre = W.pre;
@@ -255,17 +301,21 @@ struct Planner {
 
     int run() {
         P.reset();
-        if (schedule != kSchedulePhi && !sparse_schedule(schedule) && schedule != kScheduleF) { err = "unknown schedule"; return GENLIB_EINVAL; }
+        if (schedule != kSchedulePhi && !sparse_schedule(schedule) && schedule != kScheduleF && !reads) { err = "unknown schedule"; return GENLIB_EINVAL; }
         P.schedule = schedule;
-        if (n < 0 || n_pro < 0 || world < 1 || (n > 0 && (!father || !mother)) || (n_pro > 0 && !proband))
+        if (n < 0 || n_pro < 0 || world < 1 || (n > 0 && (!father || !mother)) || (n_pro > 0 && !proband) ||
+            pairs.n < 0 || (pairs.n > 0 && (!pairs.a || !pairs.b)))
             { err = "genlib_plan_create: null pointer or negative size"; return GENLIB_EINVAL; }
+        if (reads ? n_pro > 0 : pairs.n > 0)
+            { err = "genlib_plan_create: a GENLIB_SCHEDULE_PAIRS plan takes pairs and no probands, the other schedules no pairs"; return GENLIB_EINVAL; }
         P.n = n; P.world = world;
         if (int rc = probands()) return rc;
         if (P.n_unique == 0) return check_pedigree(n, father, mother, err);     // nothing to plan
         clock.phase("probands");
         if (int rc = sweep()) return rc;
         if (int rc = by_seq ? queue_order() : GENLIB_OK) return rc;
-        if (schedule == kScheduleF) depth_layers();
+        if (by_depth && !by_seq) depth_layers();
+        if (reads) read_layers();
         clock.phase("heights");
         buckets();
         clock.phase("buckets");
@@ -278,17 +328,24 @@ struct Planner {
 
     // probands: first occurrence wins (intersect/union keep first-argument order, compute.jl:247,251); kScheduleF
     // leaves out the listed individuals with a missing parent (their F is 0 without a plan)
+    // (kSchedulePairs: everybody named in a pair, in list order, a before b)
     int probands() {
         is_pro.assign((size_t)n + 1, 0);
-        for (int32_t t = 0; t < n_pro; t++) {
-            int32_t x = proband[t];
+        auto add = [&](int32_t x) {
             if (x < 0 || x >= n) {
                 if (int rc = check_pedigree(n, father, mother, err)) return rc;   // (a broken pedigree is reported first)
                 err = "KeyError: proband index " + std::to_string(x) + " not in pedigree";
-                return GENLIB_EKEY;
+                return (int)GENLIB_EKEY;
             }
-            if (schedule == kScheduleF && (father[x] < 0 || mother[x] < 0)) continue;
+            if (schedule == kScheduleF && (father[x] < 0 || mother[x] < 0)) return (int)GENLIB_OK;
             if (!is_pro[x]) { is_pro[x] = 1; P.pro_ind.push_back(x); }
+            return (int)GENLIB_OK;
+        };
+        for (int32_t t = 0; t < n_pro; t++)
+            if (int rc = add(proband[t])) return rc;
+        for (int64_t k = 0; k < pairs.n; k++) {
+            if (int rc = add(pairs.a[k])) return rc;
+            if (int rc = add(pairs.b[k])) return rc;
         }
         P.n_unique = (int32_t)P.pro_ind.size();
         return GENLIB_OK;
@@ -373,6 +430,46 @@ struct Planner {
         }
     }
 
+    // kSchedulePairs: the read layer of every pair, r = max(depth a, depth b) + 1 in [1, S] -- just before layer r
+    // both rows hold the pair's kinship (the later-born member's row got the other one's column, the other row the
+    // mirror of it) and nobody has written over it.  The reads are bucketed by r with a counting sort, list order
+    // kept, and each named individual learns its last read layer.  A pair read after the last layer (r == S) keeps
+    // its rows through that layer as CARRIED rows: only carried rows receive the columns of a layer's members.
+    void read_layers() {
+        const int32_t S = hmax + 1, *a = pairs.a, *b = pairs.b;
+        const int64_t K = pairs.n;
+        const std::vector<int32_t> &depth = W.depth;
+        std::vector<int32_t> &read_last = W.read_last;
+        read_last.assign((size_t)n, -1);
+        std::vector<int64_t> &start = P.pair_start;
+        start.assign((size_t)S + 2, 0);
+        for (int64_t k = 0; k < K; k++) {
+            const int32_t r = std::max(depth[a[k]], depth[b[k]]) + 1;
+            start[(size_t)r + 1]++;
+            read_last[a[k]] = std::max(read_last[a[k]], r);
+            read_last[b[k]] = std::max(read_last[b[k]], r);
+        }
+        for (int32_t t = 0; t <= S; t++) start[(size_t)t + 1] += start[(size_t)t];
+        P.pair_pos.resize((size_t)K);
+        std::vector<int64_t> at(start.begin(), start.end() - 1);
+        for (int64_t k = 0; k < K; k++) P.pair_pos[(size_t)at[(size_t)std::max(depth[a[k]], depth[b[k]]) + 1]++] = k;
+        // (exactly K entries each, sized before the first layer is published: a streamed plan never outgrows them)
+        P.pair_row_slot.resize((size_t)K); P.pair_col_slot.resize((size_t)K);
+        P.pair_owner.resize((size_t)K); P.pair_lrow.resize((size_t)K);
+    }
+
+    // kSchedulePairs, lane A: where the reads of layer t (t == S: after the last layer) find their two slots -- every
+    // member was born before t, and a home does not move while its row is live
+    void pair_reads(int32_t t) {
+        for (int64_t i = P.pair_start[(size_t)t]; i < P.pair_start[(size_t)t + 1]; i++) {
+            const int64_t k = P.pair_pos[(size_t)i];
+            const int32_t hi = std::max(pairs.a[k], pairs.b[k]), lo = std::min(pairs.a[k], pairs.b[k]);
+            const Home hr = home[hi];
+            P.pair_row_slot[(size_t)i] = hr.slot; P.pair_col_slot[(size_t)i] = home[lo].slot;
+            P.pair_owner[(size_t)i] = hr.owner; P.pair_lrow[(size_t)i] = hr.lrow;
+        }
+    }
+
     // Schedule of sparse_phi (compute.jl:335-439): individuals are processed in the order of a queue
     // that starts with the founders and receives a child when its last parent has been processed --
     // i.e. by depth below the founders, ties in queue order -- and of a pair, the one processed LATER
@@ -440,15 +537,17 @@ struct Planner {
         last_of.resize((size_t)n);                                    // last layer that reads the row (a sequential write here)
         // One range of visits: its members go to their layers from `pos` on, its share of the difference arrays to d[0..2].
         auto bucket_range = [&](int32_t v0, int32_t v1, size_t *pos, int64_t *occ, int64_t *cut, int64_t *both) {
-            const int32_t S = this->S; const bool by_seq = this->by_seq;   // (copies: not reloaded after every store below)
+            const int32_t S = this->S; const bool by_seq = this->by_seq, short_rows = this->short_rows, reads = this->reads;   // (copies: not reloaded after every store below)
             for (int32_t v = v0; v < v1; v++) {
                 const int32_t x = by_seq ? seq_order[(size_t)v] : v;
                 const Pre px = pre[x];
                 if (px.h < 0) continue;
                 const int32_t lx = S - 1 - px.h, ref_last = S - 1 - px.rl;
                 by_layer[pos[lx]++] = x;
-                // probands stay to the end (kScheduleF: nobody does); a row without children leaves after its own layer
-                const int32_t last = is_pro[x] && schedule != kScheduleF ? INT_MAX : px.minch == INT_MAX ? lx : S - 1 - px.minch;
+                // probands stay to the end (kScheduleF, kSchedulePairs: nobody does); a row without children leaves after
+                // its own layer; kSchedulePairs: not before its last read (S: carried through the last layer)
+                int32_t last = is_pro[x] && !short_rows ? INT_MAX : px.minch == INT_MAX ? lx : S - 1 - px.minch;
+                if (reads) last = std::max(last, W.read_last[x]);
                 last_of[x] = last;
                 occ[(size_t)std::min<int64_t>(std::max(last, lx), S - 1) + 1]--;   // born in or before, read in or after
                 cut[ref_last + 1]--;                                   // in cut[k] for layer <= k <= ref_last
@@ -848,6 +947,7 @@ struct Planner {
         L.alg_elems = 4.0 * nn * (double)L.live_before + 3.0 * (double)nn * nn;
         P.alg_elems += L.alg_elems;
         P.row_updates += nn;
+        if (reads) pair_reads(t);                  // (published with the layer)
 
         L.mem_end = P.mem_ind.size(); L.mtile_end = P.mtile_desc.size() / 4;     // (lane B has set the ends of its arrays)
         if (streaming) { ps->layers_done.store(t + 1, std::memory_order_release); ps->wake(); }
@@ -1047,8 +1147,10 @@ struct Planner {
             P.rows_cap.resize((size_t)world);
             for (int32_t g = 0; g < world; g++) P.rows_cap[g] = world > 1 ? std::max(rows[g].next_fresh, 1) : P.capacity;
         }
+        if (reads) pair_reads(S);                  // after the last layer (published with the finished plan)
         if (int rc = std::getenv("GENLIB_PLAN_VERIFY") ? verify_plan(P, err) : GENLIB_OK) return rc;
-        const size_t np = schedule == kScheduleF ? 0 : P.pro_ind.size();    // (kScheduleF: no proband matrix)
+        if (int rc = reads && std::getenv("GENLIB_PLAN_VERIFY") ? verify_pair_reads(P, pairs, err) : GENLIB_OK) return rc;
+        const size_t np = short_rows ? 0 : P.pro_ind.size();    // (kScheduleF, kSchedulePairs: no proband matrix)
         P.pro_slot.resize(np); P.pro_owner.resize(np); P.pro_lrow.resize(np);
         for (size_t u = 0; u < np; u++) {
             const Home &hu = home[P.pro_ind[u]];
@@ -1100,15 +1202,19 @@ uint64_t plan_digest(const Plan &P, bool with_bounds) {
     vec(P.mem_lrow); vec(P.fam_pf_owner); vec(P.fam_pm_owner); vec(P.fam_pf_lrow); vec(P.fam_pm_lrow); vec(P.live_owner); vec(P.live_lrow);
     vec(P.pro_owner); vec(P.pro_lrow);
     if (with_bounds) vec(P.rows_cap);
+    if (P.schedule == kSchedulePairs) {        // (the other schedules' digests stay what they were)
+        vec(P.pair_start); vec(P.pair_pos); vec(P.pair_row_slot); vec(P.pair_col_slot); vec(P.pair_owner); vec(P.pair_lrow);
+    }
     return h;
 }
 
 int build_plan(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
-               const int32_t *proband, int32_t world, int schedule, Plan &P, std::string &err, PlanStream *ps, int planners) {
+               const int32_t *proband, int32_t world, int schedule, Plan &P, std::string &err, PlanStream *ps, int planners,
+               const PairList &pairs) {
     int rc;
     try {
         std::unique_ptr<Scratch> W = take_scratch();
-        rc = Planner{*W, P, err, ps, n, father, mother, ids, n_pro, proband, world, schedule, planners}.run();
+        rc = Planner{*W, P, err, ps, n, father, mother, ids, n_pro, proband, world, schedule, planners, pairs}.run();
         give_scratch(std::move(W));
     } catch (const std::bad_alloc &) {
         if (!ps) throw;

@@ -45,7 +45,13 @@ constexpr int kMaxTileFam = 64;  // couples per member tile (bounds the couple t
 //                                    without children after its own layer (the layer still writes it).  The engine
 //                                    reads Psi[father, mother] of every couple just before its layer; there is no
 //                                    proband matrix (pro_slot / pro_owner / pro_lrow are empty).
-constexpr int kSchedulePhi = 0, kScheduleSparsePhi = 1, kScheduleSparsePhiSymmetric = 2, kScheduleF = 3;
+//   pairs                            gen.phi_pairs: f's layers, arithmetic and short rows, over the ancestors-or-self
+//                                    of everybody named in a pair (a, b).  The pair is read in layer
+//                                    r = max(depth a, depth b) + 1, just before that layer's kernel (r == S: once after
+//                                    the last layer), from the row of the higher-ranked member; both rows live until
+//                                    then (a row's last layer is the later of its last child and its last read).
+//                                    pro_ind = the distinct named individuals; no proband matrix either.
+constexpr int kSchedulePhi = 0, kScheduleSparsePhi = 1, kScheduleSparsePhiSymmetric = 2, kScheduleF = 3, kSchedulePairs = 4;
 inline bool sparse_schedule(int s) { return s == kScheduleSparsePhi || s == kScheduleSparsePhiSymmetric; }
 
 constexpr int32_t kTileCarried = 1 << 30;   // live_tiles entry: the tile has a carried column
@@ -104,6 +110,13 @@ struct Plan {
     std::vector<int8_t> pro_owner;
     std::vector<int32_t> pro_lrow;
     std::vector<int64_t> rows_cap;                     // per rank: rows of the frontier it holds
+    // ---- kSchedulePairs: one read per list position, bucketed by read layer (list order inside a bucket).  The
+    //      reads of layer t are [pair_start[t], pair_start[t + 1]) for t in [0, S]; t == S: after the last layer.
+    //      Sized at the list's length before the first layer is published, filled layer by layer. ----
+    std::vector<int64_t> pair_start, pair_pos;         // pair_pos: the read's list position
+    std::vector<int32_t> pair_row_slot, pair_col_slot; // the higher-ranked member's slot (its row), the other one's (the column)
+    std::vector<int8_t> pair_owner;                    // the rank that holds the row, and its local row there
+    std::vector<int32_t> pair_lrow;
 
     // Every array above, for reset(): the storage of a destroyed plan is handed to the next
     // genlib_plan_create, because first-touch page faults on a few hundred MB of fresh vectors
@@ -115,6 +128,7 @@ struct Plan {
         f(mtile_desc); f(fam_base); f(mem_base); f(mem_lrow);
         f(fam_pf_owner); f(fam_pm_owner); f(fam_pf_lrow); f(fam_pm_lrow); f(live_owner); f(live_lrow);
         f(pro_owner); f(pro_lrow); f(rows_cap);
+        f(pair_start); f(pair_pos); f(pair_row_slot); f(pair_col_slot); f(pair_owner); f(pair_lrow);
     }
     void reset() {                     // empty plan, capacities kept
         each_array([](auto &v) { v.clear(); });
@@ -161,9 +175,15 @@ int set_error(int code, const std::string &msg);
 // `planners`: how many planners share this host's cores while this one runs -- `world` when every rank is a process
 // of its own that plans for itself (0: assume that), 1 when one process plans for all its devices; the planner
 // takes up to three threads out of cores / planners (GENLIB_PLAN_THREADS overrides).
+// The pairs of a kSchedulePairs plan: ranks a[k], b[k] for k in [0, n), in list order.
+struct PairList {
+    int64_t n = 0;
+    const int32_t *a = nullptr, *b = nullptr;
+};
+
 int build_plan(int32_t n, const int32_t *father, const int32_t *mother, const int64_t *ids, int32_t n_pro,
                const int32_t *proband, int32_t world, int schedule, Plan &plan, std::string &err,
-               PlanStream *stream = nullptr, int planners = 0);
+               PlanStream *stream = nullptr, int planners = 0, const PairList &pairs = PairList{});
 
 // Internal to the library (hidden: not exported).
 // The pedigree's own errors, the first offending rank: a parent index out of range (GENLIB_EKEY) or a parent that

@@ -15,7 +15,7 @@ import numpy as np
 from . import _lib
 from . import pedigree as _pedigree
 from ._lib import GcStats, LayerInfo, PlanBoundsExceeded, Stats, check, lib, ptr
-from .pedigree import Pedigree, pro
+from .pedigree import Individual, Pedigree, pro
 
 
 class Plan:
@@ -41,6 +41,34 @@ class Plan:
         self._h = h
         self.world = world
         self.schedule = schedule
+
+    @classmethod
+    def pairs(cls, father, mother, a, b, world: int = 1, stream: bool = False) -> "Plan":
+        """The plan of gen.phi_pairs (genlib_plan_create_pairs): the pairs (a[k], b[k]) of ranks, read by the layers
+        (`pair_reads`); stream=True makes it on a worker thread like Plan(..., stream=True)."""
+        self = cls.__new__(cls)
+        self.father = np.ascontiguousarray(father, np.int32)
+        self.mother = np.ascontiguousarray(mother, np.int32)
+        self.a, self.b = np.ascontiguousarray(a, np.int32), np.ascontiguousarray(b, np.int32)
+        if len(self.father) != len(self.mother) or len(self.a) != len(self.b):
+            raise ValueError("father and mother, and the two sides of the pairs, must have the same length")
+        self.probands, self.ids = np.zeros(0, np.int32), None
+        h = C.c_void_p()
+        check(lib().genlib_plan_create_pairs(len(self.father), ptr(self.father), ptr(self.mother), len(self.a),
+                                             ptr(self.a), ptr(self.b), world, int(stream), C.byref(h)))
+        self._h, self.world, self.schedule = h, world, "pairs"
+        return self
+
+    def pair_reads(self, layer: int) -> dict:
+        """The reads of a pairs plan just before `layer` (layer == n_layers: after the last one), in list order:
+        list position, row slot (the higher-ranked member), column slot, the row's owner and local row."""
+        n = lib().genlib_plan_pair_reads(self._h, layer, None, None, None, None, None)
+        if n < 0:
+            check(_lib.EINVAL)
+        out = {"pos": np.zeros(n, np.int64)}
+        out.update({k: np.zeros(n, np.int32) for k in ("row_slot", "col_slot", "owner", "lrow")})
+        lib().genlib_plan_pair_reads(self._h, layer, *(ptr(out[k]) for k in ("pos", "row_slot", "col_slot", "owner", "lrow")))
+        return out
 
     def __del__(self):
         h, self._h = getattr(self, "_h", None), None
@@ -243,7 +271,17 @@ def phi(pedigree: Pedigree, probandIDs=None, *, verbose: bool = False, compute: 
         numerics="reference", dtype=np.float32, device: int = -1, out: Optional[np.ndarray] = None,
         return_stats: bool = False, devices=None):
     """gen.phi(pedigree, probandIDs; verbose, compute) on the B200 engine.  `devices=[0, 1, ...]` shards
-    the frontier over several GPUs of the box from this one process (genlib_phi_multi)."""
+    the frontier over several GPUs of the box from this one process (genlib_phi_multi).
+
+    gen.phi(ind1, ind2) with two Individuals of one pedigree is the reference's scalar method
+    (src/compute.jl:66-95): their kinship as a Python float, through `phi_pairs` with one pair."""
+    if isinstance(pedigree, Individual):
+        ind1, ind2 = pedigree, probandIDs
+        if not isinstance(ind2, Individual) or ind2._ped is not ind1._ped:
+            raise ValueError("gen.phi(ind1, ind2): two Individuals of one pedigree")
+        ped = ind1._ped
+        res, _ = phi_pairs_arrays(ped.father, ped.mother, [ind1._r], [ind2._r], device=device, devices=devices)
+        return float(res[0])
     IDs = pro(pedigree) if probandIDs is None else np.asarray(probandIDs, np.int64)
     ranks = pedigree.rank_of(IDs)                       # KeyError, like pedigree[ID]
     plan = Plan(pedigree.father, pedigree.mother, ranks, stream=compute and not verbose and devices is None)
@@ -689,6 +727,47 @@ def f_arrays(father, mother, ranks, *, dtype=np.float32, device: int = -1, devic
     st = Stats()
     check(lib().genlib_f(len(father), ptr(father), ptr(mother), len(r), ptr(r), ptr(out),
                          _lib.DTYPES[np.dtype(out.dtype)], len(dv), ptr(dv), C.byref(st)))
+    return out, st.as_dict()
+
+
+def phi_pairs(pedigree: Pedigree, IDs1, IDs2, *, dtype=np.float64, device: int = -1, devices=None,
+              return_stats: bool = False):
+    """The kinship of each pair (IDs1[k], IDs2[k]), in list order (duplicates and reversed pairs kept): what the
+    reference's scalar phi(ind1, ind2) (src/compute.jl:66-95) gives one pair at a time, for a whole list.
+
+    ONE sweep of the engine with Float64 storage over the ancestors-or-self of everybody named, layered by depth
+    below the founders, reads each pair on the device in the layer after its later-born member's (genlib_phi_pairs);
+    no matrix is formed.  phi(a, b) == phi(b, a) bitwise, phi(a, a) = 1/2 + 1/2 F_a, unrelated pairs give 0.  Exact
+    while kinships fit 53 bits; deeper pedigrees follow this schedule's order of the sums, like gen.f.  Both rows of
+    a pair stay on the device until it is read: pairs of members born many generations apart widen the frontier
+    (MemoryError when it does not fit).  ValueError on lists of unequal length, KeyError on an unknown ID.
+    `devices=[0, 1, ...]` shards the frontier over several GPUs of the box, with the same result."""
+    a = np.asarray(IDs1, np.int64).reshape(-1)
+    b = np.asarray(IDs2, np.int64).reshape(-1)
+    if len(a) != len(b):
+        raise ValueError(f"gen.phi_pairs: {len(a)} IDs against {len(b)}")
+    ra, rb = pedigree.rank_of(a), pedigree.rank_of(b)   # KeyError, like pedigree[ID]
+    res, stats = phi_pairs_arrays(pedigree.father, pedigree.mother, ra, rb, dtype=dtype, device=device, devices=devices)
+    return (res, stats) if return_stats else res
+
+
+def phi_pairs_arrays(father, mother, a, b, *, dtype=np.float64, device: int = -1, devices=None,
+                     out: Optional[np.ndarray] = None):
+    """One-shot C-ABI call `genlib_phi_pairs` on flat rank arrays (what the Julia shim ccalls).  Returns
+    (kinships in list order as float64 or float32, stats)."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    a, b = np.ascontiguousarray(a, np.int32).reshape(-1), np.ascontiguousarray(b, np.int32).reshape(-1)
+    if len(a) != len(b):
+        raise ValueError(f"phi_pairs_arrays: {len(a)} ranks against {len(b)}")
+    if out is None:
+        out = np.empty(len(a), dtype)
+    if out.shape != (len(a),) or not out.flags.c_contiguous or out.dtype not in _lib.DTYPES:
+        raise ValueError(f"out must be a contiguous ({len(a)},) float32/float64 array")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = Stats()
+    check(lib().genlib_phi_pairs(len(father), ptr(father), ptr(mother), len(a), ptr(a), ptr(b), ptr(out),
+                                 _lib.DTYPES[np.dtype(out.dtype)], len(dv), ptr(dv), C.byref(st)))
     return out, st.as_dict()
 
 

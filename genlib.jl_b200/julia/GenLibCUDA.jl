@@ -190,6 +190,30 @@ function f(pedigree::GenLib.Pedigree, IDs::Vector{Int}; device::Integer = -1, de
 end
 
 """
+    phi_pairs(pedigree, IDs1, IDs2; device = -1, devices = Int[]) -> Vector{Float64}
+
+The reference's scalar `phi(ind₁, ind₂)` (src/compute.jl:66-95) for every pair `(IDs1[k], IDs2[k])`, in list order
+(duplicates and reversed pairs kept).  ONE sweep of the engine with Float64 storage over the ancestors-or-self of
+everybody named, layered by depth below the founders, reads each pair on the device in the layer after its
+later-born member's (`genlib_phi_pairs`); no matrix is formed.  Exact while kinships fit 53 bits; beyond that the
+last bits follow this schedule's order of the sums, as in `f`.  ArgumentError on lists of unequal length, KeyError
+on an unknown ID.
+"""
+function phi_pairs(pedigree::GenLib.Pedigree, IDs1::Vector{Int}, IDs2::Vector{Int};
+                   device::Integer = -1, devices::Vector{<:Integer} = Int[])
+    length(IDs1) == length(IDs2) || throw(ArgumentError("phi_pairs: $(length(IDs1)) IDs against $(length(IDs2))"))
+    father, mother = flatten(pedigree)
+    a = Int32[pedigree[ID].rank - 1 for ID in IDs1]                     # KeyError on unknown ID
+    b = Int32[pedigree[ID].rank - 1 for ID in IDs2]
+    kinships = Vector{Float64}(undef, length(a))
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    GC.@preserve kinships check(ccall((:genlib_phi_pairs, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int64, Ptr{Int32}, Ptr{Int32}, Ptr{Cvoid}, Cint, Int32, Ptr{Int32}, Ptr{Cvoid}),
+        length(father), father, mother, length(a), a, b, kinships, 1, length(devs), devs, C_NULL))
+    kinships
+end
+
+"""
     sparse_phi(pedigree, probandIDs = pro(pedigree)) -> GenLib.KinshipMatrix
 
 `gen.sparse_phi` (src/compute.jl:321-447) on the GPU: the same engine, planned for sparse_phi's own

@@ -156,11 +156,17 @@ int genlib_plan_create(int32_t n, const int32_t *father, const int32_t *mother, 
  *       that have both parents (the others never reach the plan), layered by depth below the founders, with
  *       phi's arithmetic; no row is kept to the end (a row leaves after the layer of its last child, or after
  *       its own layer when it has none).  Such a plan has no proband matrix: it can be inspected with the
- *       genlib_plan_* calls, genlib_engine_create* refuses it (GENLIB_EINVAL). */
+ *       genlib_plan_* calls, genlib_engine_create* refuses it (GENLIB_EINVAL). *
+ *   GENLIB_SCHEDULE_PAIRS  the schedule of genlib_phi_pairs (made by genlib_plan_create_pairs, which takes pairs
+ *       instead of probands): GENLIB_SCHEDULE_F's layers and arithmetic over the ancestors-or-self of everybody
+ *       named in a pair.  The pair (a, b) is read in layer r = max(depth a, depth b) + 1, just before that layer
+ *       (r == the number of layers: once after the last one), from the row of the higher-ranked member; a row
+ *       leaves after the later of its last child and its last read.  No proband matrix either. */
 #define GENLIB_SCHEDULE_PHI 0
 #define GENLIB_SCHEDULE_SPARSE_PHI 1
 #define GENLIB_SCHEDULE_SPARSE_PHI_SYMMETRIC 2
 #define GENLIB_SCHEDULE_F 3
+#define GENLIB_SCHEDULE_PAIRS 4
 int genlib_plan_create_scheduled(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
                                  const int32_t *proband, int32_t world, int schedule, genlib_plan **out);
 /* The same with the individuals' IDs (by rank; may be NULL).  sparse_phi seeds its queue with
@@ -219,6 +225,16 @@ int genlib_plan_proband_slots(const genlib_plan *plan, int32_t *slots);
  * GENLIB_PLAN_THREADS) and the streamed hand-over must not change it.  with_bounds = 0 leaves out the frontier
  * width and the rows per rank (a streamed plan keeps the upper bounds its engine was sized with).  CPU only. */
 uint64_t genlib_plan_digest(const genlib_plan *plan, int with_bounds);
+/* A GENLIB_SCHEDULE_PAIRS plan of the pairs (a[k], b[k]), k < n_pairs (ranks; duplicates and a == b allowed), for
+ * `world` ranks.  stream != 0: made on a worker thread and published layer by layer, like genlib_plan_create_async
+ * (a, b, father and mother stay valid until the plan is finished).  An index out of range gives GENLIB_EKEY. */
+int genlib_plan_create_pairs(int32_t n, const int32_t *father, const int32_t *mother, int64_t n_pairs, const int32_t *a,
+                             const int32_t *b, int32_t world, int stream, genlib_plan **out);
+/* The reads of a GENLIB_SCHEDULE_PAIRS plan in layer `layer` (just before it), or after the last layer
+ * (layer == n_layers), in list order: the list position, the row's slot (the higher-ranked member), the column's slot,
+ * the rank that holds the row and its local row there.  Returns their number (any pointer may be NULL), -1 on error. */
+int64_t genlib_plan_pair_reads(const genlib_plan *plan, int32_t layer, int64_t *pos, int32_t *row_slot,
+                               int32_t *col_slot, int32_t *owner, int32_t *lrow);
 
 /* ---- one-shot: the `gen.phi(ped, probandIDs)` call -------------------------
  * out: n_unique^2 elements of out_dtype (row-major == column-major: symmetric),
@@ -262,6 +278,21 @@ int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, in
  * GENLIB_ENOMEM names the bytes one device needs.  stats->n_unique counts the distinct IDs with both parents. */
 int genlib_f(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_ids, const int32_t *ids,
              void *out, int out_dtype, int32_t n_dev, const int32_t *devices, genlib_stats *stats);
+
+/* ---- gen.phi_pairs: the kinship of each pair of a list (src/compute.jl:66-95, one value per pair) --------------
+ * out[k] = Psi[a[k], b[k]] for k < n_pairs, in list order (duplicates and reversed pairs kept; Psi[a, a] = 1/2 + 1/2 F_a).
+ * One sweep of the engine over the ancestors-or-self of everybody named (GENLIB_SCHEDULE_PAIRS, Float64 storage)
+ * reads each pair on the device in the layer after its later-born member's; no matrix is formed.  Every device
+ * copies its per-read array back once, 8 bytes per pair, and the host takes each entry from the device that holds the
+ * pair's row (stats->d2h_bytes = 8 * n_pairs * n_dev; entries of reads a device does not own are not used).  Both rows of a pair stay in the frontier until it is read, so pairs whose members are born
+ * generations apart widen it (GENLIB_ENOMEM, naming the bytes one device needs, when it does not fit).  While
+ * kinships fit 53 bits every value is exact; deeper pedigrees follow the depth-layered order of the sums, like
+ * genlib_f (genlib_phi_pairs of a couple equals genlib_f of its child bitwise).  An index out of range gives
+ * GENLIB_EKEY (a broken pedigree is reported first); n_pairs == 0 returns without a device.  devices as in genlib_f.
+ * stats->n_unique counts the distinct individuals named. */
+int genlib_phi_pairs(int32_t n, const int32_t *father, const int32_t *mother, int64_t n_pairs, const int32_t *a,
+                     const int32_t *b, void *out, int out_dtype, int32_t n_dev, const int32_t *devices,
+                     genlib_stats *stats);
 
 /* ---- handle API: keep the schedule on the device, run, fetch ---------------
  * (what the benchmark and a multi-call Julia session use) */
