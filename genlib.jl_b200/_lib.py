@@ -53,6 +53,15 @@ class LayerInfo(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
 
 
+class LaunchShape(C.Structure):
+    _fields_ = [(k, C.c_int32) for k in ("sw", "ft", "prod_warps", "gangs", "nbuf", "stages", "n_strips", "n_pitems",
+                                          "n_citems", "n_prod", "n_cons", "grid", "fast_transpose", "reserved")] + \
+               [("smem", C.c_int64)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+
+
 class Stats(C.Structure):
     _fields_ = [("n_unique", C.c_int32), ("n_layers", C.c_int32), ("row_updates", C.c_int64),
                 ("capacity", C.c_int64), ("device_bytes", C.c_int64), ("alg_bytes", C.c_double),
@@ -106,6 +115,7 @@ SYMBOLS = {
     "genlib_plan_row_updates": (C.c_int64, [_P]),
     "genlib_plan_layer_info": (C.c_int, [_P, C.c_int32, C.POINTER(LayerInfo)]),
     "genlib_plan_device_bytes": (C.c_int64, [_P, C.c_int, C.c_int32]),
+    "genlib_plan_launch_shape": (C.c_int, [_P, C.c_int32, C.c_int, C.c_int32, C.c_int32, C.POINTER(LaunchShape)]),
     "genlib_plan_layer_arrays": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),
     "genlib_plan_layer_shard": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, _P]),
     "genlib_plan_layer_live_rows": (C.c_int, [_P, C.c_int32, _P, _P]),

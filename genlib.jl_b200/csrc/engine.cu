@@ -239,13 +239,25 @@ LayerLaunch shape_layer(const Plan &P, int t, int rank, size_t es, int sm_count)
     const size_t min_buf = (size_t)std::max(2, env_int("GENLIB_MIN_NBUF", 2));
     const int sw_cap = es == 4 ? kMaxStrip : kMaxStrip / 2;
     const size_t budget = (size_t)std::max(16, env_int("GENLIB_STRIP_BUDGET_MB", (int)(kStripBudget >> 20))) << 20;
-    int sw = std::min(sw_cap, std::max(8, env_int("GENLIB_MAX_SW", kMaxStrip)));
+    // (a power of two: the consumers index the strip by shifts, the producers split it into whole items)
+    int sw = 8;
+    while (2 * sw <= std::min(sw_cap, env_int("GENLIB_MAX_SW", kMaxStrip))) sw *= 2;
     while (sw > 8 && (size_t)q_rows * sw * pair * min_buf > budget) sw >>= 1;
     const size_t strip_bytes = std::max<size_t>((size_t)q_rows * sw * pair, 256);
     s.sw = sw;
-    // couples per producer item: 32 rows of 512 B (float) / 16 rows of 1 KB (double); at most two items per live tile
-    s.ft = std::max(sw / 2, std::min(sw, std::max(8, env_int("GENLIB_FT", es == 4 ? 32 : 16))));
+    // eight producer warps (and four consumer warps) where the producers have the carried columns to write as well
+    {
+        const int forced = env_int("GENLIB_PROD_WARPS", 0);
+        out.prod_warps = forced == 4 || forced == 8 ? forced : (L.carried > 0 && live ? 8 : 4);
+    }
+    const size_t cons_bytes = layer_consumer_bytes(sw, es, out.prod_warps);
+    const size_t smem_cap = (size_t)227 * 1024 - 2048;      // (static shared memory and the driver's share)
+    auto stage_bytes = [&](int ft) { return (size_t)2 * ft * (kPTile * es + 16); };
+    // couples per producer item: 32 rows of 512 B (float) / 16 rows of 1 KB (double); one or two items per live
+    // tile (ft = sw or sw / 2, at most 32), and the ring must hold two stages of items next to the consumers' part
+    s.ft = env_int("GENLIB_FT", es == 4 ? 32 : 16) >= sw || sw == 8 ? sw : sw / 2;
     if (s.ft > 32) s.ft = 32;
+    if (s.ft == sw && sw > 8 && cons_bytes + 2 * stage_bytes(s.ft) > smem_cap) s.ft = sw / 2;
     s.n_strips = (int)((own_nf + sw - 1) / sw);
     s.qstride = (int64_t)(strip_bytes / pair);
     // producer items: 2 ft parent rows x one live tile; consumer items: the member tiles
@@ -267,24 +279,19 @@ LayerLaunch shape_layer(const Plan &P, int t, int rank, size_t es, int sm_count)
         else while (G < kMaxGangs && (int64_t)s.n_pitems * G < (int64_t)want_items * sm_count) G *= 2;
         while (G > 1 && (2 * G > max_buf || s.n_strips < 2 * G || G > sm_count / 4)) G /= 2;
     }
-    s.gangs = G;
-    // (at most eight buffers per gang: the producer warps of a CTA count themselves off in eight slots by strip)
-    s.nbuf = std::min(8 * G, std::max(2 * G, std::min(std::max(2 * G, env_int("GENLIB_MAX_NBUF", 8)), max_buf)) / G * G);
     // (one gang) layers with few items per strip run faster on 7/8 of the SMs (C5: 148 CTAs 246 ms, 128 to 136 CTAs
     // 148 ms; genea140: 8.9 -> 6.4 ms); layers with several items per CTA and strip want every SM (C3: 70.8 ms on
     // 148, 74.3 ms on 132).
     const int few = G == 1 && (sw / s.ft) * L.n_live_tiles < 3 * sm_count / 2 ? sm_count - sm_count / 8 : sm_count;
-    const int ctas = std::max(1, std::min(sm_count, env_int("GENLIB_CTAS_PER_ROLE", few))) / G;   // per gang
+    const int role_ctas = std::max(1, std::min(sm_count, env_int("GENLIB_CTAS_PER_ROLE", few)));
+    while (G > 1 && G > role_ctas) G /= 2;                  // every gang has a CTA of each role
+    s.gangs = G;
+    // (at most eight buffers per gang: the producer warps of a CTA count themselves off in eight slots by strip)
+    s.nbuf = std::min(8 * G, std::max(2 * G, std::min(std::max(2 * G, env_int("GENLIB_MAX_NBUF", 8)), max_buf)) / G * G);
+    const int ctas = role_ctas / G;                         // per gang
     s.n_prod = G * std::min(ctas, s.n_pitems);
     s.n_cons = G * std::min(ctas, s.n_citems);
-    const size_t stage = (size_t)2 * s.ft * (kPTile * es + 16);
-    // eight producer warps (and four consumer warps) where the producers have the carried columns to write as well
-    {
-        const int forced = env_int("GENLIB_PROD_WARPS", 0);
-        out.prod_warps = forced == 4 || forced == 8 ? forced : (L.carried > 0 && live ? 8 : 4);
-    }
-    const size_t cons_bytes = layer_consumer_bytes(sw, es, out.prod_warps);
-    const size_t smem_cap = (size_t)227 * 1024 - 2048;      // (static shared memory and the driver's share)
+    const size_t stage = stage_bytes(s.ft);                 // (two of them fit: ft above)
     s.stages = (int)std::max<size_t>(2, std::min<size_t>((size_t)std::min(kMaxStages, env_int("GENLIB_STAGES", kMaxStages)), (smem_cap - cons_bytes) / stage));
     s.ring_off = (int32_t)cons_bytes;
     out.smem = cons_bytes + (size_t)s.stages * stage;
@@ -947,6 +954,25 @@ int64_t genlib_plan_device_bytes(const genlib_plan *plan, int numerics, int32_t 
     settle(plan);
     if (!plan || rank < 0 || rank >= plan->p.world || plan->p.n_unique == 0) return plan ? 0 : -1;
     return (int64_t)engine_bytes(plan->p, numerics, rank);      // strip buffers sized for 148 SMs
+}
+
+int genlib_plan_launch_shape(const genlib_plan *plan, int32_t layer, int numerics, int32_t rank, int32_t sm_count,
+                             genlib_launch_shape *out) {
+    settle(plan);
+    if (!plan || !out || layer < 0 || layer >= (int32_t)plan->p.layers.size()) return fail(GENLIB_EINVAL, "bad layer");
+    if (numerics != GENLIB_NUMERICS_REFERENCE && numerics != GENLIB_NUMERICS_FP64) return fail(GENLIB_EINVAL, "unknown numerics mode");
+    if (rank < 0 || rank >= plan->p.world || sm_count < 1) return fail(GENLIB_EINVAL, "genlib_plan_launch_shape: bad rank or SM count");
+    const size_t es = numerics == GENLIB_NUMERICS_FP64 ? 8 : 4;
+    const LayerLaunch ll = shape_layer(plan->p, layer, rank, es, sm_count);
+    const StripArgs &s = ll.s;
+    std::memset(out, 0, sizeof *out);
+    if (s.sw == 0) return GENLIB_OK;                             // (no couple of the rank in this layer)
+    out->sw = s.sw; out->ft = s.ft; out->prod_warps = ll.prod_warps; out->gangs = s.gangs; out->nbuf = s.nbuf;
+    out->stages = s.stages; out->n_strips = s.n_strips; out->n_pitems = s.n_pitems; out->n_citems = s.n_citems;
+    out->n_prod = s.n_prod; out->n_cons = s.n_cons; out->grid = ll.grid;
+    out->fast_transpose = s.n_pitems > 0 && fast_transpose_shape((int)es, s.sw, s.ft);
+    out->smem = (int64_t)ll.smem;
+    return GENLIB_OK;
 }
 
 int genlib_plan_layer_arrays(const genlib_plan *plan, int32_t layer, int32_t *member_ind,

@@ -69,6 +69,9 @@ constexpr int kMaxStrip = 64;                   // couples per strip (upper boun
 constexpr int kVPitch = kMaxTileFam + 1;        // row pitch of the staged couple tile (65: conflict-free)
 constexpr int kMaxStages = 4;
 constexpr int kSyncStride = 16;                 // ints per strip in StripArgs::sync: every counter has its own 32-byte sector
+// The shapes whose producers take the Float32 transpose with immediate offsets (Producer::transpose); every other
+// shape takes the generic one.
+__host__ __device__ constexpr bool fast_transpose_shape(int esize, int sw, int ft) { return esize == 4 && ft == 32 && (sw == 64 || sw == 32); }
 
 struct StripArgs {
     int32_t sw;          // strip width: couples per strip (8, 16, 32 or 64)
@@ -398,7 +401,7 @@ struct Producer {
     __device__ __forceinline__ void transpose(const unsigned char *st, P2 *const Q, int pt, int lt) {
         bool done = false;
         if constexpr (sizeof(T) == 4) {
-            if (ft == 32) {                                        // the common shape: lane = couple, offsets are immediates
+            if (fast_transpose_shape(4, sw, ft)) {                 // the common shape: lane = couple, offsets are immediates
                 auto fast = [&](auto SWC) {
                     constexpr int SW = decltype(SWC)::value;
                     const unsigned char *xr = st + lane * RB + pw * (kProdCols * 4), *yr = xr + 32 * RB;

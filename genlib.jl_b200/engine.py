@@ -14,7 +14,7 @@ import numpy as np
 
 from . import _lib
 from . import pedigree as _pedigree
-from ._lib import GcStats, LayerInfo, PlanBoundsExceeded, Stats, check, lib, ptr
+from ._lib import GcStats, LaunchShape, LayerInfo, PlanBoundsExceeded, Stats, check, lib, ptr
 from .pedigree import Individual, Pedigree, pro
 
 
@@ -93,6 +93,14 @@ class Plan:
         info = LayerInfo()
         check(lib().genlib_plan_layer_info(self._h, layer, C.byref(info)))
         return info.as_dict()
+
+    def launch_shape(self, layer: int, numerics="reference", rank: int = 0, sm_count: int = 148) -> dict:
+        """How an engine of `rank` would launch the layer kernel of `layer` on a device with `sm_count` SMs
+        (genlib_plan_launch_shape: the GENLIB_* tuning variables of the environment apply); all zero when the
+        rank has no couple in the layer."""
+        shape = LaunchShape()
+        check(lib().genlib_plan_launch_shape(self._h, layer, _lib.NUMERICS[numerics], rank, sm_count, C.byref(shape)))
+        return shape.as_dict()
 
     def layers(self):
         return [self.layer_info(t) for t in range(self.n_layers)]

@@ -194,6 +194,28 @@ int64_t genlib_plan_row_updates(const genlib_plan *plan);
 int genlib_plan_layer_info(const genlib_plan *plan, int32_t layer, genlib_layer_info *out);
 /* Device bytes rank `rank` needs for the given numerics. */
 int64_t genlib_plan_device_bytes(const genlib_plan *plan, int numerics, int32_t rank);
+/* The launch shape of one layer's kernel, as an engine of `rank` with the given numerics would launch it on a
+ * device with `sm_count` SMs (host only: no device is needed).  It follows the GENLIB_* tuning variables of the
+ * environment like the engine does.  All zero for a layer in which the rank has no couple. */
+typedef struct genlib_launch_shape {
+    int32_t sw;             /* couples per strip: 8, 16, 32 or 64 (at most 32 with Float64 storage)  */
+    int32_t ft;             /* couples per producer item: sw or sw / 2, and 8, 16 or 32             */
+    int32_t prod_warps;     /* producer warps per CTA, 4 or 8 (the other warps of 12 consume)      */
+    int32_t gangs;          /* independent gangs of CTAs, each on its own strips                    */
+    int32_t nbuf;           /* strip buffers in rotation (a multiple of gangs)                      */
+    int32_t stages;         /* stages of the producers' shared-memory ring                          */
+    int32_t n_strips;       /* strips of the rank's couples                                         */
+    int32_t n_pitems;       /* producer items per strip: (sw / ft) x live tiles                     */
+    int32_t n_citems;       /* consumer items per strip: the layer's member tiles                   */
+    int32_t n_prod;         /* CTAs with producer items                                             */
+    int32_t n_cons;         /* CTAs with consumer items                                             */
+    int32_t grid;           /* CTAs launched: max(n_prod, n_cons); 0: the layer kernel is skipped   */
+    int32_t fast_transpose; /* 1: the producers take the Float32 transpose with immediate offsets   */
+    int32_t reserved;
+    int64_t smem;           /* dynamic shared memory per CTA, bytes                                 */
+} genlib_launch_shape;
+int genlib_plan_launch_shape(const genlib_plan *plan, int32_t layer, int numerics, int32_t rank, int32_t sm_count,
+                             genlib_launch_shape *out);
 /* Schedule export (tests replay it on the CPU to check the planner).  Arrays
  * may be NULL; sizes come from genlib_plan_layer_info.  member_*: n_new
  * entries in family-major order; fam_*: n_fam entries; slots are columns of
