@@ -10,13 +10,14 @@ Usage mirrors the reference (`import GenLib as gen`):
     m = gen.findMRCA(ped, [1, 2])          # GenMatrix: MRCAs sorted by ID, int64 meioses
     F = gen.f(ped, ped.ids)                # float32 inbreeding of everyone, one device sweep
     k = gen.phi_pairs(ped, [1, 2], [29, 2])  # float64 kinship of each pair, list order, no matrix formed
+    o = gen.phiOver(ped, 1 / 64)           # proband pairs at or above 1/64, selected on the device
 """
 import os as _os
 
 from .pedigree import Individual, Pedigree, founder, genealogy, pro  # noqa: F401
 from .engine import (Engine, GcPlan, GenMatrix, KinshipMatrix, PinnedMatrix, Plan, f, f_arrays,  # noqa: F401
                      findDistance, findMRCA, gc, gc_arrays, meioses_arrays, mrca_arrays, occ, occ_arrays, phi, phi_arrays,
-                     phi_distributed, phi_pairs, phi_pairs_arrays, phiMean, rec, rec_arrays, run_distributed,
+                     phi_distributed, phi_over_arrays, phi_pairs, phi_pairs_arrays, phiMean, phiOver, PhiOver, rec, rec_arrays, run_distributed,
                      sparse_phi)
 from . import synth  # noqa: F401
 from ._lib import GenlibError, GenlibOverflowError, LIB_PATH, PlanBoundsExceeded, lib  # noqa: F401

@@ -34,12 +34,15 @@ class PlanBoundsExceeded(GenlibError):
 
 class GenlibOverflowError(GenlibError, OverflowError):
     """gen.occ: a descent-path count or a row sum does not fit an Int64 (GENLIB_EOVERFLOW).
-    `ancestor_index` / `proband_index`: the 0-based list positions of the pair the library names."""
+    `ancestor_index` / `proband_index`: the 0-based list positions of the pair the library names.
+    gen.phiOver: more pairs reach the threshold than `max_pairs`; `count` is their number."""
 
     def __init__(self, status: int, message: str):
         super().__init__(status, message)
         m = re.search(r"ancestor position (-?\d+).*proband position (-?\d+)", message)
         self.ancestor_index, self.proband_index = (int(m.group(1)), int(m.group(2))) if m else (None, None)
+        m = re.search(r"(\d+) pairs reach the threshold", message)
+        self.count = int(m.group(1)) if m else None
 
 
 class LayerInfo(C.Structure):
@@ -71,6 +74,12 @@ class Stats(C.Structure):
 
     def as_dict(self):
         return {k: getattr(self, k) for k, _ in self._fields_ if k != "reserved"}
+
+
+class KinshipPairs(C.Structure):
+    """genlib_kinship_pairs: what genlib_phi_over allocates (release with genlib_kinship_pairs_free)."""
+    _fields_ = [("n", C.c_int64), ("row", C.c_void_p), ("col", C.c_void_p), ("value", C.c_void_p),
+                ("value_dtype", C.c_int)]
 
 
 class GcStats(C.Structure):
@@ -131,6 +140,9 @@ SYMBOLS = {
                                    C.POINTER(Stats)]),
     "genlib_f": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_int, C.c_int32, _P, C.POINTER(Stats)]),
     "genlib_phi_pairs": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, _P, C.c_int, C.c_int32, _P, C.POINTER(Stats)]),
+    "genlib_phi_over": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_double, C.c_int64, C.c_int, C.c_int, C.c_int32,
+                                  _P, C.POINTER(KinshipPairs), C.POINTER(Stats)]),
+    "genlib_kinship_pairs_free": (C.c_int, [C.POINTER(KinshipPairs)]),
     "genlib_plan_create_pairs": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, C.c_int32, C.c_int, C.POINTER(_P)]),
     "genlib_plan_pair_reads": (C.c_int64, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "genlib_plan_create_async": (C.c_int, [C.c_int32, _P, _P, _P, C.c_int32, _P, C.c_int32, C.c_int, C.POINTER(_P)]),

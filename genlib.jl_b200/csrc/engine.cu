@@ -1,11 +1,12 @@
 // engine.cu -- the phi engine and the library-wide part of the C ABI of libgenlib_cuda.so (include/genlib_cuda.h):
-// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_f / genlib_phi_pairs, errors and caches.  gen.gc, gen.occ and gen.rec are
+// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_phi_over / genlib_f / genlib_phi_pairs, errors and caches.  gen.gc, gen.occ and gen.rec are
 // in gc_engine.cu; the host helpers both share are in runtime.hpp.
 //
 // The ABI stands where the reference's Julia method stands:
 //   phi(pedigree, probandIDs; verbose, compute)            src/compute.jl:233-304
 // There is no CPU fallback: without a usable CUDA device every compute entry
 // point returns GENLIB_ECUDA.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -619,6 +620,88 @@ int fetch_block(genlib_engine &E, int32_t u0, int32_t u1, O *out) {
             return cudaMemcpyAsync(out + (size_t)(u0 + i0) * n, stage, (size_t)nr * row_bytes, cudaMemcpyDeviceToHost, E.copy_stream);
         });
     if (rc == GENLIB_OK) E.stats.d2h_bytes += (int64_t)(u1 - u0) * (int64_t)row_bytes;
+    return rc;
+}
+
+// ---- gen.phiOver (genlib_phi_over) ----------------------------------------------------------------------
+// One device's share of the selection: its own proband rows (own_pro order), their per-row counts and then offsets,
+// and on the device the same offsets, the rows' positions in the proband list and the rows that have pairs.
+struct OverRows {
+    int device = -1;
+    const std::vector<int32_t> *own = nullptr;   // the engine's own_pro
+    std::vector<int64_t> off;                    // nown + 1: the counts after the first pass, exclusive offsets after
+    int64_t base = 0;                            // (several devices) where this device's pairs start in the scratch
+    int64_t *d_off = nullptr;                    // one allocation: d_off (nown + 1), d_index (nown), d_sel (nown)
+    int32_t *d_index = nullptr, *d_sel = nullptr;
+    OverRows() = default;
+    OverRows(const OverRows &) = delete;
+    ~OverRows() {
+        if (!d_off) return;
+        DeviceGuard guard;
+        guard.enter(device);
+        cudaFree(d_off);
+    }
+};
+
+// First pass: each own row's count of columns j > i with M[i, j] >= threshold, to R.off.
+template <typename T, typename O>
+int phi_over_count(genlib_engine &E, OverRows &R, double threshold) {
+    const Plan &P = E.plan->p;
+    const int32_t nown = (int32_t)E.own_pro.size();
+    R.device = E.device;
+    R.own = &E.own_pro;
+    R.off.assign((size_t)nown + 1, 0);
+    if (nown == 0) return GENLIB_OK;
+    CU(cudaMalloc(&R.d_off, (size_t)(nown + 1) * sizeof(int64_t) + 2 * (size_t)nown * sizeof(int32_t)));
+    R.d_index = reinterpret_cast<int32_t *>(R.d_off + nown + 1);
+    R.d_sel = R.d_index + nown;
+    CU(cudaMemcpyAsync(R.d_index, E.own_pro.data(), (size_t)nown * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    phi_over_count_kernel<T, O><<<(unsigned)nown, kThreads, 0, E.stream>>>(static_cast<const T *>(E.A), P.capacity, E.own_pro_row.p,
+                                                                           R.d_index, E.pro_slot.p, P.n_unique, threshold, R.d_off);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(R.off.data(), R.d_off, (size_t)nown * sizeof(int64_t), cudaMemcpyDeviceToHost, E.stream));
+    CU(cudaStreamSynchronize(E.stream));
+    E.stats.d2h_bytes += (int64_t)nown * (int64_t)sizeof(int64_t);
+    return GENLIB_OK;
+}
+
+// Second pass (R.off holds the offsets by now): the device's pairs in its own row order to col / val in host memory,
+// through the staging buffers, in blocks of rows whose pairs fit one buffer (columns first, then the values).
+template <typename T, typename O>
+int phi_over_select(genlib_engine &E, OverRows &R, double threshold, int32_t *col, O *val) {
+    const Plan &P = E.plan->p;
+    const int32_t nown = (int32_t)E.own_pro.size();
+    std::vector<int32_t> sel;                                    // own rows with at least one pair
+    for (int32_t r = 0; r < nown; r++)
+        if (R.off[(size_t)r + 1] > R.off[(size_t)r]) sel.push_back(r);
+    if (sel.empty()) return GENLIB_OK;
+    const int64_t cap = (int64_t)(kFetchStageBytes / (sizeof(int32_t) + sizeof(O))) / 2 * 2;   // (values 8-byte aligned)
+    auto first = [&](size_t k) { return R.off[(size_t)sel[k]]; };
+    auto last = [&](size_t k) { return R.off[(size_t)sel[k] + 1]; };
+    std::vector<size_t> blk{0};                                  // blocks of sel: [blk[b], blk[b + 1])
+    for (size_t k = 0; k < sel.size(); k++) {
+        if (last(k) - first(k) > cap) return fail(GENLIB_EINVAL, "the pairs of one proband row do not fit the staging buffer");
+        if (last(k) - first(blk.back()) > cap) blk.push_back(k);
+    }
+    blk.push_back(sel.size());
+    CU(cudaMemcpyAsync(R.d_off, R.off.data(), ((size_t)nown + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, E.stream));
+    CU(cudaMemcpyAsync(R.d_sel, sel.data(), sel.size() * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    auto cols_of = [](unsigned char *s) { return reinterpret_cast<int32_t *>(s); };
+    auto vals_of = [&](unsigned char *s) { return reinterpret_cast<O *>(s + (size_t)cap * sizeof(int32_t)); };
+    int rc = staged_d2h(E.stream, E.copy_stream, E.fetch_stage[0], E.fetch_stage[1], (int64_t)blk.size() - 1, 1, "phiOver fetch",
+        [&](unsigned char *stage, int64_t b, int64_t) {
+            const size_t k0 = blk[(size_t)b], k1 = blk[(size_t)b + 1];
+            phi_over_select_kernel<T, O><<<(unsigned)(k1 - k0), kThreads, 0, E.stream>>>(
+                static_cast<const T *>(E.A), P.capacity, E.own_pro_row.p, R.d_index, E.pro_slot.p, P.n_unique, threshold,
+                R.d_sel + k0, R.d_off, first(k0), cols_of(stage), vals_of(stage));
+        },
+        [&](unsigned char *stage, int64_t b, int64_t) {
+            const int64_t a = first(blk[(size_t)b]), m = last(blk[(size_t)b + 1] - 1) - a;
+            cudaError_t ce = cudaMemcpyAsync(col + a, cols_of(stage), (size_t)m * sizeof(int32_t), cudaMemcpyDeviceToHost, E.copy_stream);
+            if (ce == cudaSuccess) ce = cudaMemcpyAsync(val + a, vals_of(stage), (size_t)m * sizeof(O), cudaMemcpyDeviceToHost, E.copy_stream);
+            return ce;
+        });
+    if (rc == GENLIB_OK) E.stats.d2h_bytes += R.off[(size_t)nown] * (int64_t)(sizeof(int32_t) + sizeof(O));
     return rc;
 }
 
@@ -1306,13 +1389,17 @@ int genlib_engine_read_block(genlib_engine *eng, int32_t n_slots, const int32_t 
 }
 
 // What a one-shot call takes out of the engines once every device has run: `prepare` (may be empty) reads the
-// finished plan on the calling thread, then `device(E, g)` runs on device g's host thread.
+// finished plan on the calling thread, then `device(E, g)` runs on device g's host thread.  A fetch that needs what
+// every device found first (gen.phiOver's global offsets) adds `combine`, on the calling thread once every `device`
+// has returned, and `finish(E, g)`, again on the devices' threads.
 struct OneshotFetch {
     std::function<void(const Plan &)> prepare;
     std::function<int(genlib_engine &, int)> device;
+    std::function<int()> combine;
+    std::function<int(genlib_engine &, int)> finish;
 };
 
-// genlib_phi, genlib_phi_multi, genlib_f and genlib_phi_pairs: ONE plan for all devices, made on a worker thread and handed over layer
+// genlib_phi, genlib_phi_multi, genlib_phi_over, genlib_f and genlib_phi_pairs: ONE plan for all devices, made on a worker thread and handed over layer
 // by layer (PlanStream), so that the devices run the first generations while the later ones are planned.
 // GENLIB_STREAM=0, or a bound of the streamed plan that did not hold, plans first and then runs.  One device runs on
 // the calling thread; several get a host thread each and NVLink peer access.  `has_out`: the caller wants a result.
@@ -1420,6 +1507,8 @@ static int oneshot(const std::string &who, int schedule, int32_t n, const int32_
     const double t0 = now_ms();
     if (fetch.prepare) fetch.prepare(plan->p);
     rc = first_error(on_devices(n_dev, [&](int g) { return fetch.device(*eng[(size_t)g], g); }), true);
+    if (rc == GENLIB_OK && fetch.combine) rc = fetch.combine();
+    if (rc == GENLIB_OK && fetch.finish) rc = first_error(on_devices(n_dev, [&](int g) { return fetch.finish(*eng[(size_t)g], g); }), true);
     if (rc != GENLIB_OK) return rc;
     if (stats) {
         *stats = eng[0]->stats;
@@ -1463,6 +1552,133 @@ int genlib_phi_multi(int32_t n, const int32_t *father, const int32_t *mother, in
                      const int32_t *devices, genlib_stats *stats) {
     if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_multi: 1 .. 16 devices");
     return phi_oneshot(n, father, mother, n_pro, proband, out, out_dtype, numerics, n_dev, devices, stats);
+}
+
+// genlib_phi_over: the genlib_phi run, then on every device a count of each own row's pairs; the host turns the counts
+// into offsets in (row, col) order over all devices and allocates the result; every device then writes its pairs in
+// its own row order and the host puts each run of consecutive rows in place (one device: they are in place already).
+int genlib_phi_over(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                    double threshold, int64_t max_pairs, int out_dtype, int numerics, int32_t n_dev, const int32_t *devices,
+                    genlib_kinship_pairs *out, genlib_stats *stats) {
+    if (!out) return fail(GENLIB_EINVAL, "genlib_phi_over: out is null");
+    *out = genlib_kinship_pairs{0, nullptr, nullptr, nullptr, out_dtype};
+    if (n < 0 || n_pro < 0 || (n > 0 && (!father || !mother)) || (n_pro > 0 && !proband))
+        return fail(GENLIB_EINVAL, "genlib_phi_over: null pointer or negative size");
+    if (std::isnan(threshold)) return fail(GENLIB_EINVAL, "genlib_phi_over: the threshold is NaN");
+    if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
+    if (numerics != GENLIB_NUMERICS_REFERENCE && numerics != GENLIB_NUMERICS_FP64) return fail(GENLIB_EINVAL, "unknown numerics mode");
+    if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_over: 1 .. 16 devices");
+    std::vector<char> seen((size_t)n, 0);
+    int32_t distinct = 0;
+    for (int32_t k = 0; k < n_pro; k++) {
+        const int32_t x = proband[k];
+        if (x < 0 || x >= n) {
+            std::string err;
+            if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);   // (a broken pedigree is reported first)
+            return fail(GENLIB_EKEY, "KeyError: index " + std::to_string(x) + " not in pedigree");
+        }
+        if (!seen[(size_t)x]) { seen[(size_t)x] = 1; distinct++; }
+    }
+    if (distinct < 2) {                                          // no pair: no plan, no device
+        std::string err;
+        if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);
+        if (stats) { std::memset(stats, 0, sizeof *stats); stats->n_unique = distinct; }
+        return GENLIB_OK;
+    }
+    const bool multi = n_dev > 1, f64 = out_dtype == GENLIB_F64;
+    const size_t es = f64 ? sizeof(double) : sizeof(float);
+    std::vector<OverRows> rows((size_t)n_dev);
+    std::vector<int64_t> goff;                                   // per proband: where its pairs start in the result
+    unsigned char *scratch = nullptr;                            // several devices: their pairs in their own row order
+    struct FreeHost { unsigned char *&p; ~FreeHost() { if (p) cudaFreeHost(p); } } free_scratch{scratch};
+    double t0 = 0;
+    int32_t nu = 0;
+    OneshotFetch fetch;
+    fetch.prepare = [&](const Plan &P) { t0 = now_ms(); nu = P.n_unique; };
+    fetch.device = [&](genlib_engine &E, int g) {
+        DeviceGuard guard;
+        if (int r = guard.enter(E.device)) return r;
+        OverRows &R = rows[(size_t)g];
+        if (numerics == GENLIB_NUMERICS_FP64)
+            return f64 ? phi_over_count<double, double>(E, R, threshold) : phi_over_count<double, float>(E, R, threshold);
+        return f64 ? phi_over_count<float, double>(E, R, threshold) : phi_over_count<float, float>(E, R, threshold);
+    };
+    fetch.combine = [&]() {
+        goff.assign((size_t)nu + 1, 0);
+        for (const OverRows &R : rows)
+            for (size_t r = 0; r < R.own->size(); r++) goff[(size_t)(*R.own)[r] + 1] = R.off[r];
+        for (int32_t u = 0; u < nu; u++) goff[(size_t)u + 1] += goff[(size_t)u];
+        const int64_t total = goff[(size_t)nu];
+        if (max_pairs >= 0 && total > max_pairs) {
+            out->n = total;
+            char msg[160];
+            std::snprintf(msg, sizeof msg, "genlib_phi_over: %lld pairs reach the threshold %.17g, more than max_pairs = %lld",
+                          (long long)total, threshold, (long long)max_pairs);
+            return fail(GENLIB_EOVERFLOW, msg);
+        }
+        int64_t base = 0;
+        for (OverRows &R : rows) {                               // counts -> offsets in the device's own row order
+            R.base = base;
+            for (int64_t &o : R.off) { const int64_t c = o; o = base - R.base; base += c; }
+        }
+        if (total == 0) return (int)GENLIB_OK;
+        void *block = nullptr;
+        CU(cudaHostAlloc(&block, (size_t)total * (2 * sizeof(int32_t) + es), cudaHostAllocPortable));
+        out->row = static_cast<int32_t *>(block);
+        out->col = out->row + total;
+        out->value = out->col + total;                           // (8 total bytes in: aligned)
+        out->n = total;
+        for (int32_t u = 0; u < nu; u++) std::fill(out->row + goff[(size_t)u], out->row + goff[(size_t)u + 1], u);
+        if (multi) CU(cudaHostAlloc(reinterpret_cast<void **>(&scratch), (size_t)total * (sizeof(int32_t) + es), cudaHostAllocPortable));
+        return (int)GENLIB_OK;
+    };
+    fetch.finish = [&](genlib_engine &E, int g) {
+        DeviceGuard guard;
+        if (int r = guard.enter(E.device)) return r;
+        OverRows &R = rows[(size_t)g];
+        const int64_t total = out->n;
+        if (total > 0) {
+            // scratch: every device's values, then every device's columns
+            unsigned char *val = multi ? scratch + (size_t)R.base * es : static_cast<unsigned char *>(out->value);
+            int32_t *col = multi ? reinterpret_cast<int32_t *>(scratch + (size_t)total * es) + R.base : out->col;
+            int r;
+            if (numerics == GENLIB_NUMERICS_FP64)
+                r = f64 ? phi_over_select<double, double>(E, R, threshold, col, (double *)val) : phi_over_select<double, float>(E, R, threshold, col, (float *)val);
+            else
+                r = f64 ? phi_over_select<float, double>(E, R, threshold, col, (double *)val) : phi_over_select<float, float>(E, R, threshold, col, (float *)val);
+            if (r != GENLIB_OK) return r;
+            const std::vector<int32_t> &own = *R.own;
+            for (size_t a = 0; multi && a < own.size();) {       // runs of consecutive proband rows
+                size_t b = a + 1;
+                while (b < own.size() && own[b] == own[b - 1] + 1) b++;
+                const int64_t from = R.off[a], m = R.off[b] - from, to = goff[(size_t)own[a]];
+                if (m > 0) {
+                    std::memcpy(out->col + to, col + from, (size_t)m * sizeof(int32_t));
+                    std::memcpy(static_cast<unsigned char *>(out->value) + (size_t)to * es, val + (size_t)from * es, (size_t)m * es);
+                }
+                a = b;
+            }
+        }
+        E.stats.ms_fetch = now_ms() - t0;
+        return (int)GENLIB_OK;
+    };
+    const int rc = oneshot("genlib_phi_over", GENLIB_SCHEDULE_PHI, n, father, mother, n_pro, proband, true, numerics, n_dev,
+                           devices, stats, fetch);
+    if (rc != GENLIB_OK && rc != GENLIB_EOVERFLOW) {             // (over max_pairs: out->n is the count)
+        const std::string msg = g_err;
+        genlib_kinship_pairs_free(out);
+        g_err = msg;
+    }
+    return rc;
+}
+
+int genlib_kinship_pairs_free(genlib_kinship_pairs *pairs) {
+    if (!pairs) return GENLIB_OK;
+    if (pairs->row) CU(cudaFreeHost(pairs->row));
+    pairs->n = 0;
+    pairs->row = pairs->col = nullptr;
+    pairs->value = nullptr;
+    return GENLIB_OK;
 }
 
 // genlib_f: a GENLIB_SCHEDULE_F plan of the listed individuals with both parents; every device copies its per-couple

@@ -1,6 +1,6 @@
 // kernels.cuh -- device-side vocabulary shared by the sm_100a kernels of the kinship sweep, and the
-// small kernels around the layer kernel (layer_kernel.cuh): proband gather, phiMean reduction, the
-// inter-GPU barrier, sparse_phi's misfiled pairs, gen.f's parents' kinships and gen.phi_pairs' reads.
+// small kernels around the layer kernel (layer_kernel.cuh): proband gather, gen.phiOver's selection, phiMean
+// reduction, the inter-GPU barrier, sparse_phi's misfiled pairs, gen.f's parents' kinships and gen.phi_pairs' reads.
 //
 // Arithmetic is binary64 in the reference's grouping; storage type T is float
 // (GENLIB_NUMERICS_REFERENCE: one RN32 per step, like src/compute.jl:296) or double.
@@ -204,6 +204,68 @@ __global__ void gather_peer_kernel(PeerTable PT, int64_t ld, const int8_t *__res
     O *dst = out + (size_t)blockIdx.y * P;
     for (int v = blockIdx.x * blockDim.x + threadIdx.x; v < P; v += gridDim.x * blockDim.x)
         dst[v] = (O)row[cols[v]];
+}
+
+// =====================================================================================
+// gen.phiOver: the proband pairs (i, j), i < j, whose kinship reaches a threshold, selected from this rank's own
+// proband rows (rows[] local rows, index[] their positions i in the proband list, ascending; columns read as
+// gather_kernel reads them, so no peer reads).  M[i, j] is the entry gen.phi returns in the output type O, compared as
+// a binary64 number.  Two passes over the same columns j > i, one CTA per row: the first counts them, the second writes
+// (j, M[i, j]) of each row, ascending in j, from the row's offset on.
+// =====================================================================================
+template <typename T, typename O>
+__global__ void __launch_bounds__(kThreads)
+phi_over_count_kernel(const T *__restrict__ A, int64_t ld, const int32_t *__restrict__ rows, const int32_t *__restrict__ index,
+                      const int32_t *__restrict__ cols, int32_t P, double threshold, int64_t *__restrict__ count) {
+    __shared__ int part[kThreads / 32];
+    const int r = blockIdx.x;
+    const T *row = A + (int64_t)rows[r] * ld;
+    int c = 0;
+    for (int j = index[r] + 1 + threadIdx.x; j < P; j += kThreads) c += (double)(O)row[cols[j]] >= threshold;
+    c = __reduce_add_sync(0xffffffffu, c);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int64_t s = 0;
+        for (int w = 0; w < kThreads / 32; w++) s += part[w];
+        count[r] = s;
+    }
+}
+
+// The rows sel[0, gridDim.x) of one block (own rows with at least one pair), row r's pairs written from
+// offset[r] - base on: per chunk of kThreads columns a warp ballot orders the hits inside a warp and a scan of the
+// warps' counts in shared memory orders the warps.
+template <typename T, typename O>
+__global__ void __launch_bounds__(kThreads)
+phi_over_select_kernel(const T *__restrict__ A, int64_t ld, const int32_t *__restrict__ rows, const int32_t *__restrict__ index,
+                       const int32_t *__restrict__ cols, int32_t P, double threshold, const int32_t *__restrict__ sel,
+                       const int64_t *__restrict__ offset, int64_t base, int32_t *__restrict__ col_out, O *__restrict__ val_out) {
+    __shared__ int warp_hits[kThreads / 32];
+    const int r = sel[blockIdx.x];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const T *row = A + (int64_t)rows[r] * ld;
+    int64_t at = offset[r] - base;
+    for (int j0 = index[r] + 1; j0 < P; j0 += kThreads) {       // (the same trip count for every thread of the CTA)
+        const int j = j0 + threadIdx.x;
+        const O v = j < P ? (O)row[cols[j]] : (O)0;
+        const bool hit = j < P && (double)v >= threshold;
+        const unsigned ballot = __ballot_sync(0xffffffffu, hit);
+        if (lane == 0) warp_hits[w] = __popc(ballot);
+        __syncthreads();
+        int before = 0, total = 0;
+        for (int k = 0; k < kThreads / 32; k++) {
+            const int h = warp_hits[k];
+            before += k < w ? h : 0;
+            total += h;
+        }
+        if (hit) {
+            const int64_t p = at + before + __popc(ballot & ((1u << lane) - 1u));
+            col_out[p] = j;
+            val_out[p] = v;
+        }
+        at += total;
+        __syncthreads();                                          // (warp_hits is written again by the next chunk)
+    }
 }
 
 // Row sums of the proband block for phiMean (src/compute.jl:454-459), deterministic: one CTA per own

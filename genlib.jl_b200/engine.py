@@ -430,6 +430,115 @@ def phi_arrays(father, mother, proband_ranks, *, numerics="reference", dtype=np.
     return out, st.as_dict()
 
 
+class PhiOver:
+    """What gen.phiOver returns, GENLIB's data frame `line, column, pro1, pro2, kinship`: one entry per proband pair whose
+    kinship reaches the threshold, ordered by line, then column.  `line` < `column` are 0-based positions in the
+    deduplicated proband list (the rows and columns of gen.phi's matrix), `pro1` / `pro2` the IDs at those positions,
+    `kinship` the matrix entry, bit for bit (float32, or float64)."""
+
+    def __init__(self, line, column, pro1, pro2, kinship, threshold: float):
+        self.line, self.column = np.asarray(line, np.int64), np.asarray(column, np.int64)
+        self.pro1, self.pro2 = np.asarray(pro1, np.int64), np.asarray(pro2, np.int64)
+        self.kinship = np.asarray(kinship)
+        self.threshold = threshold
+
+    def __len__(self) -> int:
+        return len(self.line)
+
+    def __repr__(self) -> str:
+        return f"PhiOver({len(self)} pairs with kinship >= {self.threshold!r}, {self.kinship.dtype})"
+
+
+def _first_occurrences(ids) -> np.ndarray:
+    """The IDs with duplicates collapsed onto their first occurrence (the rows of gen.phi's matrix)."""
+    _, first = np.unique(ids, return_index=True)
+    return ids[np.sort(first)]
+
+
+def _phi_over_host(phi_matrix, threshold: float, probandIDs) -> PhiOver:
+    """GENLIB's phiOver(phiMatrix, threshold) on a matrix in host memory: the pairs (i, j), i < j, with
+    M[i, j] >= threshold, M[i, j] compared as a float64."""
+    m = np.asarray(phi_matrix)
+    if m.ndim != 2 or m.shape[0] != m.shape[1]:
+        raise ValueError(f"gen.phiOver: a Pedigree or a square kinship matrix, not an array of shape {m.shape}")
+    n = m.shape[0]
+    ids = np.arange(n, dtype=np.int64) if probandIDs is None else \
+        _first_occurrences(np.asarray(probandIDs, np.int64).reshape(-1))
+    if len(ids) != n:
+        raise ValueError(f"gen.phiOver: {len(ids)} distinct proband IDs for a {n} x {n} matrix")
+    lines, cols = [np.zeros(0, np.int64)], [np.zeros(0, np.int64)]
+    step = max(1, (1 << 24) // max(n, 1))                  # rows per block: the float64 copy stays at 128 MB
+    for r0 in range(0, n, step):
+        i, j = np.nonzero(m[r0:r0 + step].astype(np.float64) >= threshold)
+        i += r0
+        keep = j > i
+        lines.append(i[keep])
+        cols.append(j[keep])
+    line, column = np.concatenate(lines), np.concatenate(cols)
+    return PhiOver(line, column, ids[line], ids[column], m[line, column], threshold)
+
+
+def phiOver(pedigree, threshold, probandIDs=None, *, numerics="reference", dtype=np.float32, max_pairs=None,
+            device: int = -1, devices=None, return_stats: bool = False):
+    """GENLIB's phiOver: the proband pairs whose kinship is at least `threshold`, as a `PhiOver` record.
+
+    gen.phiOver(pedigree, threshold, probandIDs = pro(pedigree)) runs gen.phi's plan and layers on the device and
+    selects there, from the proband rows each device holds (genlib_phi_over): only the pairs (and 8 bytes per row)
+    leave the device, never the matrix.  The result is `np.nonzero(np.triu(M >= threshold, 1))` of the matrix M that
+    gen.phi(pedigree, probandIDs, numerics=numerics, dtype=dtype) returns, with M at those positions, the same bits
+    for any number of devices: the diagonal is never selected, M[i, j] is compared as a float64 (a float32 entry is
+    widened exactly), threshold <= 0 selects every pair, +inf none.  More than `max_pairs` pairs raise
+    GenlibOverflowError (an OverflowError) naming their number and the threshold; fewer than two distinct probands
+    give an empty result without a device.  ValueError on a NaN threshold, KeyError on an unknown ID.
+
+    gen.phiOver(phi_matrix, threshold, probandIDs=None), with a square array first, is the same selection on a matrix
+    already in host memory; `probandIDs` (duplicates collapse, as in gen.phi) names its rows, else pro1 / pro2 are the
+    positions."""
+    threshold = float(threshold)
+    if np.isnan(threshold):
+        raise ValueError("gen.phiOver: the threshold is NaN")
+    if not isinstance(pedigree, Pedigree):
+        res, stats = _phi_over_host(pedigree, threshold, probandIDs), {}
+        return (res, stats) if return_stats else res
+    IDs = pro(pedigree) if probandIDs is None else np.asarray(probandIDs, np.int64).reshape(-1)
+    ranks = pedigree.rank_of(IDs)                       # KeyError, like pedigree[ID]
+    ids = _first_occurrences(IDs)
+    line, column, kinship, stats = phi_over_arrays(pedigree.father, pedigree.mother, ranks, threshold, numerics=numerics,
+                                                   dtype=dtype, max_pairs=max_pairs, device=device, devices=devices)
+    res = PhiOver(line, column, ids[line], ids[column], kinship, threshold)
+    return (res, stats) if return_stats else res
+
+
+def phi_over_arrays(father, mother, proband_ranks, threshold, *, numerics="reference", dtype=np.float32,
+                    max_pairs=None, device: int = -1, devices=None):
+    """One-shot C-ABI call `genlib_phi_over` on flat rank arrays (what the Julia shim ccalls).  Returns
+    (line, column, kinship, stats): 0-based positions in the deduplicated proband list, line < column, in (line,
+    column) order, and the matrix entries as float32 or float64.  The library's arrays are copied and freed."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32)
+    dt = np.dtype(dtype)
+    if dt not in _lib.DTYPES:
+        raise ValueError("dtype must be float32 or float64")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    res, st = _lib.KinshipPairs(), Stats()
+    rc = lib().genlib_phi_over(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), float(threshold),
+                               -1 if max_pairs is None else int(max_pairs), _lib.DTYPES[dt], _lib.NUMERICS[numerics],
+                               len(dv), ptr(dv), C.byref(res), C.byref(st))
+    try:
+        check(rc)
+        n = res.n
+
+        def take(p, t):
+            t = np.dtype(t)
+            return np.frombuffer((C.c_char * (n * t.itemsize)).from_address(p), t, n).copy() if n else np.zeros(0, t)
+
+        line, column, kinship = take(res.row, np.int32), take(res.col, np.int32), take(res.value, dt)
+    finally:
+        lib().genlib_kinship_pairs_free(C.byref(res))
+    return line.astype(np.int64), column.astype(np.int64), kinship, st.as_dict()
+
+
 class GcPlan:
     """The schedule of gen.gc (genlib_gc_plan_*): direction, layers, frontier slots.  Needs no GPU."""
 

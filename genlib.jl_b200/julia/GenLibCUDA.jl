@@ -33,7 +33,7 @@ function check(status::Cint)
     msg = unsafe_string(ccall((:genlib_last_error, libgenlib[]), Cstring, ()))
     status == 2 && throw(KeyError(msg))            # same exception as pedigree[ID] (src/create.jl:70)
     status == 5 && throw(OutOfMemoryError())
-    status == 8 && throw(OverflowError(msg))       # genlib_occ: a count does not fit an Int64
+    status == 8 && throw(OverflowError(msg))       # genlib_occ: a count does not fit an Int64; phiOver: max_pairs
     error("libgenlib_cuda status $status: $msg")
 end
 
@@ -211,6 +211,47 @@ function phi_pairs(pedigree::GenLib.Pedigree, IDs1::Vector{Int}, IDs2::Vector{In
         (Int32, Ptr{Int32}, Ptr{Int32}, Int64, Ptr{Int32}, Ptr{Int32}, Ptr{Cvoid}, Cint, Int32, Ptr{Int32}, Ptr{Cvoid}),
         length(father), father, mother, length(a), a, b, kinships, 1, length(devs), devs, C_NULL))
     kinships
+end
+
+struct KinshipPairs         # genlib_kinship_pairs: allocated by the library, released by genlib_kinship_pairs_free
+    n::Int64; row::Ptr{Int32}; col::Ptr{Int32}; value::Ptr{Cvoid}; value_dtype::Cint
+end
+
+"""
+    phiOver(pedigree, threshold, probandIDs = pro(pedigree); numerics = :reference, max_pairs = -1,
+            device = -1, devices = Int[]) -> NamedTuple (line, column, pro1, pro2, kinship)
+
+GENLIB's `phiOver(phi(pedigree, probandIDs), threshold)` without the matrix leaving the device
+(`genlib_phi_over`): `phi`'s plan and layers run, then every device selects the pairs `line < column` with
+`ϕ[line, column] >= threshold` from the proband rows it holds and copies back only those.  `line` / `column` are
+1-based positions in the deduplicated proband list (as in GENLIB), `pro1` / `pro2` the IDs there, `kinship` the
+`Float32` entries of `phi`'s matrix bit for bit, ordered by line, then column; the same for any number of devices.
+More than `max_pairs` (>= 0) pairs throw `OverflowError` naming their number; a NaN threshold is an error,
+an unknown ID a KeyError.
+"""
+function phiOver(pedigree::GenLib.Pedigree, threshold::Real, probandIDs::Vector{Int} = GenLib.pro(pedigree);
+                 numerics::Symbol = :reference, max_pairs::Integer = -1, device::Integer = -1,
+                 devices::Vector{<:Integer} = Int[])
+    father, mother = flatten(pedigree)
+    probands = Int32[pedigree[ID].rank - 1 for ID in probandIDs]      # KeyError on unknown ID
+    ids = unique(probandIDs)                                           # the matrix's rows (src/compute.jl:251)
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    pairs = Ref{KinshipPairs}(KinshipPairs(0, C_NULL, C_NULL, C_NULL, 0))
+    status = ccall((:genlib_phi_over, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Cdouble, Int64, Cint, Cint, Int32, Ptr{Int32},
+         Ref{KinshipPairs}, Ptr{Cvoid}),
+        length(father), father, mother, length(probands), probands, Float64(threshold), max_pairs, 0,
+        numerics === :fp64 ? 1 : 0, length(devs), devs, pairs, C_NULL)
+    try
+        check(status)
+        n = Int(pairs[].n)
+        line = n == 0 ? Int[] : Int.(unsafe_wrap(Array, pairs[].row, n)) .+ 1
+        column = n == 0 ? Int[] : Int.(unsafe_wrap(Array, pairs[].col, n)) .+ 1
+        kinship = n == 0 ? Float32[] : copy(unsafe_wrap(Array, Ptr{Float32}(pairs[].value), n))
+        return (line = line, column = column, pro1 = ids[line], pro2 = ids[column], kinship = kinship)
+    finally
+        ccall((:genlib_kinship_pairs_free, libgenlib[]), Cint, (Ref{KinshipPairs},), pairs)
+    end
 end
 
 """

@@ -7,8 +7,10 @@
  *         verbose::Bool = false, compute::Bool = true)      src/compute.jl:233-304
  * so these entry points are what a `ccall` shim (genlib.jl_b200/julia/GenLibCUDA.jl,
  * INTEGRATION.md) binds in its place.  Everything is plain pointers and sizes;
- * the caller owns every buffer; no call throws, exits or keeps a pointer after
- * it returns (handles excepted).
+ * the caller owns every buffer (except the result of genlib_phi_over, whose
+ * size only the device knows: the library allocates it, genlib_kinship_pairs_free
+ * releases it); no call throws, exits or keeps a pointer after it returns
+ * (handles excepted).
  *
  * Pedigree encoding (what `values(pedigree)` yields, src/create.jl:234-254):
  *   individuals are numbered by 0-based rank (Individual.rank - 1); father[i] /
@@ -42,7 +44,8 @@ extern "C" {
                            /* being made (genlib_plan_create_async): a size bound did    */
                            /* not hold; destroy the engine, create it again (the plan is */
                            /* finished by then) and run                                  */
-#define GENLIB_EOVERFLOW 8 /* genlib_occ: a path count or row sum does not fit an Int64   */
+#define GENLIB_EOVERFLOW 8 /* genlib_occ: a path count or row sum does not fit an Int64;  */
+                           /* genlib_phi_over: more pairs than max_pairs (out->n = count) */
 
 /* numerics: how the frontier is stored between generation steps */
 #define GENLIB_NUMERICS_REFERENCE 0 /* Float32 storage, Float64 arithmetic, one RN32 per   */
@@ -315,6 +318,32 @@ int genlib_f(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_
 int genlib_phi_pairs(int32_t n, const int32_t *father, const int32_t *mother, int64_t n_pairs, const int32_t *a,
                      const int32_t *b, void *out, int out_dtype, int32_t n_dev, const int32_t *devices,
                      genlib_stats *stats);
+
+/* ---- gen.phiOver: the proband pairs whose kinship reaches a threshold (GENLIB's phiOver(phiMatrix, threshold)) ---
+ * M is the matrix genlib_phi returns for the same arguments (numerics, out_dtype); rows and columns are positions in
+ * the deduplicated proband list.  (i, j) is selected when i < j and M[i, j] >= threshold, M[i, j] compared as a binary64
+ * number (a Float32 entry is widened exactly): the diagonal never, threshold <= 0 every pair, +inf none.  The pairs come
+ * in (row, col) order with the stored M[i, j] bit for bit, the same for every number of devices.  The genlib_phi plan
+ * runs unchanged (streamed, several devices as genlib_phi_multi); then every device selects from the proband rows it
+ * holds, counts per row first, and copies back only its per-row counts and its pairs: no matrix leaves the device.
+ *   THE LIBRARY ALLOCATES the result (host memory, exactly n entries of each array, page-locked); release it with
+ *   genlib_kinship_pairs_free and nothing else.  n == 0 leaves the pointers NULL.
+ *   max_pairs >= 0 and more pairs than that: GENLIB_EOVERFLOW with out->n = the count and nothing allocated or copied.
+ *   A NaN threshold gives GENLIB_EINVAL, an index out of range GENLIB_EKEY (a broken pedigree is reported first);
+ *   fewer than two distinct probands give n = 0 without a device.  devices[0] < 0 = the current device (one device).
+ *   stats as genlib_phi's, but ms_fetch = the selection and the copy back, d2h_bytes = the bytes copied (8 per own
+ *   row and device, 4 + element size per pair). */
+typedef struct genlib_kinship_pairs {
+    int64_t n;            /* pairs selected (or, with GENLIB_EOVERFLOW, pairs that would have been)       */
+    int32_t *row, *col;   /* positions in the deduplicated proband list, row < col, (row, col) ascending   */
+    void *value;          /* n elements of value_dtype (GENLIB_F32 / GENLIB_F64): M[row, col]              */
+    int value_dtype;
+} genlib_kinship_pairs;
+int genlib_phi_over(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                    double threshold, int64_t max_pairs /* < 0: no limit */, int out_dtype, int numerics,
+                    int32_t n_dev, const int32_t *devices, genlib_kinship_pairs *out, genlib_stats *stats);
+/* Frees what genlib_phi_over allocated and zeroes the struct (NULL or an empty result: nothing to do). */
+int genlib_kinship_pairs_free(genlib_kinship_pairs *pairs);
 
 /* ---- handle API: keep the schedule on the device, run, fetch ---------------
  * (what the benchmark and a multi-call Julia session use) */
