@@ -11,13 +11,15 @@ Usage mirrors the reference (`import GenLib as gen`):
     F = gen.f(ped, ped.ids)                # float32 inbreeding of everyone, one device sweep
     k = gen.phi_pairs(ped, [1, 2], [29, 2])  # float64 kinship of each pair, list order, no matrix formed
     o = gen.phiOver(ped, 1 / 64)           # proband pairs at or above 1/64, selected on the device
+    g = gen.phiMeanGroups(ped, {1: "a", 2: "a", 29: "b"})  # mean kinship within / between groups, and per proband
 """
 import os as _os
 
 from .pedigree import Individual, Pedigree, founder, genealogy, pro  # noqa: F401
-from .engine import (Engine, GcPlan, GenMatrix, KinshipMatrix, PinnedMatrix, Plan, f, f_arrays,  # noqa: F401
+from .engine import (Engine, GcPlan, GenMatrix, GroupKinship, KinshipMatrix, PinnedMatrix, Plan, f, f_arrays,  # noqa: F401
                      findDistance, findMRCA, gc, gc_arrays, meioses_arrays, mrca_arrays, occ, occ_arrays, phi, phi_arrays,
-                     phi_distributed, phi_over_arrays, phi_pairs, phi_pairs_arrays, phiMean, phiOver, PhiOver, rec, rec_arrays, run_distributed,
+                     phi_distributed, phi_groups_arrays, phi_over_arrays, phi_pairs, phi_pairs_arrays, phiMean,
+                     phiMeanGroups, phiOver, PhiOver, rec, rec_arrays, run_distributed,
                      sparse_phi)
 from . import synth  # noqa: F401
 from ._lib import GenlibError, GenlibOverflowError, LIB_PATH, PlanBoundsExceeded, lib  # noqa: F401

@@ -143,6 +143,8 @@ SYMBOLS = {
     "genlib_phi_over": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_double, C.c_int64, C.c_int, C.c_int, C.c_int32,
                                   _P, C.POINTER(KinshipPairs), C.POINTER(Stats)]),
     "genlib_kinship_pairs_free": (C.c_int, [C.POINTER(KinshipPairs)]),
+    "genlib_phi_groups": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_int32, C.c_int, C.c_int32, _P, _P, _P,
+                                    C.POINTER(Stats)]),
     "genlib_plan_create_pairs": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, C.c_int32, C.c_int, C.POINTER(_P)]),
     "genlib_plan_pair_reads": (C.c_int64, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "genlib_plan_create_async": (C.c_int, [C.c_int32, _P, _P, _P, C.c_int32, _P, C.c_int32, C.c_int, C.POINTER(_P)]),

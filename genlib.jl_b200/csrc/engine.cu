@@ -1,5 +1,5 @@
 // engine.cu -- the phi engine and the library-wide part of the C ABI of libgenlib_cuda.so (include/genlib_cuda.h):
-// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_phi_over / genlib_f / genlib_phi_pairs, errors and caches.  gen.gc, gen.occ and gen.rec are
+// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_phi_over / genlib_phi_groups / genlib_f / genlib_phi_pairs, errors and caches.  gen.gc, gen.occ and gen.rec are
 // in gc_engine.cu; the host helpers both share are in runtime.hpp.
 //
 // The ABI stands where the reference's Julia method stands:
@@ -702,6 +702,44 @@ int phi_over_select(genlib_engine &E, OverRows &R, double threshold, int32_t *co
             return ce;
         });
     if (rc == GENLIB_OK) E.stats.d2h_bytes += R.off[(size_t)nown] * (int64_t)(sizeof(int32_t) + sizeof(O));
+    return rc;
+}
+
+// ---- gen.phiMeanGroups (genlib_phi_groups) --------------------------------------------------------------------
+// The grouped column list (phi_groups_kernel): the probands' frontier slots in group-major order (list order within a
+// group), where each group starts, and where each list position went.
+struct GroupColumns {
+    std::vector<int32_t> gcol, gptr, gat;
+};
+
+// This device's S rows (own_pro order) to host rows dst[0, nown) of G doubles each, in blocks of rows that fit one
+// staging buffer.
+template <typename T>
+int phi_groups_rows(genlib_engine &E, const GroupColumns &C, double *dst) {
+    const Plan &P = E.plan->p;
+    const int32_t np = P.n_unique, nown = (int32_t)E.own_pro.size(), G = (int32_t)C.gptr.size() - 1;
+    if (nown == 0) return GENLIB_OK;
+    const size_t row_bytes = (size_t)G * sizeof(double);
+    if (row_bytes > kFetchStageBytes) return fail(GENLIB_EINVAL, "the group means of one proband do not fit the staging buffer");
+    const int64_t rows_per = (int64_t)std::min<size_t>((size_t)nown, kFetchStageBytes / row_bytes);
+    int32_t *d = nullptr;                                        // d_index (nown), gcol (np), gat (np), gptr (G + 1)
+    FreeOnExit<int32_t> free_d{d};
+    CU(cudaMalloc(&d, ((size_t)nown + 2 * (size_t)np + (size_t)G + 1) * sizeof(int32_t)));
+    int32_t *d_index = d, *d_gcol = d + nown, *d_gat = d_gcol + np, *d_gptr = d_gat + np;
+    CU(cudaMemcpyAsync(d_index, E.own_pro.data(), (size_t)nown * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    CU(cudaMemcpyAsync(d_gcol, C.gcol.data(), (size_t)np * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    CU(cudaMemcpyAsync(d_gat, C.gat.data(), (size_t)np * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    CU(cudaMemcpyAsync(d_gptr, C.gptr.data(), ((size_t)G + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    const int rc = staged_d2h(E.stream, E.copy_stream, reinterpret_cast<double *>(E.fetch_stage[0]),
+                              reinterpret_cast<double *>(E.fetch_stage[1]), nown, rows_per, "phiMeanGroups fetch",
+        [&](double *stage, int64_t r0, int64_t nr) {
+            phi_groups_kernel<T><<<(unsigned)nr, kThreads, 0, E.stream>>>(static_cast<const T *>(E.A), P.capacity, E.own_pro_row.p,
+                                                                          d_index, d_gcol, d_gat, d_gptr, G, np, (int32_t)r0, stage);
+        },
+        [&](const double *stage, int64_t r0, int64_t nr) {
+            return cudaMemcpyAsync(dst + (size_t)r0 * G, stage, (size_t)nr * row_bytes, cudaMemcpyDeviceToHost, E.copy_stream);
+        });
+    if (rc == GENLIB_OK) E.stats.d2h_bytes += (int64_t)nown * (int64_t)row_bytes;
     return rc;
 }
 
@@ -1679,6 +1717,112 @@ int genlib_kinship_pairs_free(genlib_kinship_pairs *pairs) {
     pairs->row = pairs->col = nullptr;
     pairs->value = nullptr;
     return GENLIB_OK;
+}
+
+// genlib_phi_groups: the genlib_phi run, then every device reduces its own proband rows to S (phi_groups_kernel) and
+// copies them into proband_mean, device after device in own_pro order (one device: row i lands at row i); the host
+// moves the rows to list order, adds T in list order and divides both outputs in place.
+int genlib_phi_groups(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                      const int32_t *group, int32_t n_groups, int numerics, int32_t n_dev, const int32_t *devices,
+                      double *proband_mean, double *group_mean, genlib_stats *stats) {
+    if (n < 0 || n_pro < 0 || n_groups < 0 || (n > 0 && (!father || !mother)) ||
+        (n_pro > 0 && (!proband || !group || !proband_mean || !group_mean)))
+        return fail(GENLIB_EINVAL, "genlib_phi_groups: null pointer or negative size");
+    if (numerics != GENLIB_NUMERICS_REFERENCE && numerics != GENLIB_NUMERICS_FP64) return fail(GENLIB_EINVAL, "unknown numerics mode");
+    if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_groups: 1 .. 16 devices");
+    if (n_pro > 0 && n_groups < 1) return fail(GENLIB_EINVAL, "genlib_phi_groups: probands without groups");
+    const int32_t G = n_groups;
+    std::vector<int64_t> members((size_t)G, 0);    // n_g
+    for (int32_t k = 0; k < n_pro; k++) {
+        if (group[k] < 0 || group[k] >= G)
+            return fail(GENLIB_EINVAL, "genlib_phi_groups: group index " + std::to_string(group[k]) + " of proband position " +
+                                       std::to_string(k) + " is not in [0, " + std::to_string(G) + ")");
+        members[(size_t)group[k]]++;
+    }
+    for (int32_t g = 0; g < G; g++)
+        if (members[(size_t)g] == 0) return fail(GENLIB_EINVAL, "genlib_phi_groups: group " + std::to_string(g) + " has no proband");
+    std::vector<char> seen((size_t)n, 0);
+    for (int32_t k = 0; k < n_pro; k++) {
+        const int32_t x = proband[k];
+        if (x < 0 || x >= n) {
+            std::string err;
+            if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);   // (a broken pedigree is reported first)
+            return fail(GENLIB_EKEY, "KeyError: index " + std::to_string(x) + " not in pedigree");
+        }
+        if (seen[(size_t)x]) return fail(GENLIB_EINVAL, "genlib_phi_groups: duplicate proband rank " + std::to_string(x));
+        seen[(size_t)x] = 1;
+    }
+    if (n_pro < 2) {                                             // no pair: no plan, no device
+        std::string err;
+        if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);
+        if (stats) { std::memset(stats, 0, sizeof *stats); stats->n_unique = n_pro; }
+        if (n_pro == 1) proband_mean[0] = group_mean[0] = std::nan("");
+        return GENLIB_OK;
+    }
+    GroupColumns cols;
+    std::vector<int64_t> base((size_t)n_dev + 1, 0);             // where each device's rows land in proband_mean
+    std::vector<int32_t> at;                                     // at[p]: the list position of the row landed at p
+    double t0 = 0;
+    OneshotFetch fetch;
+    fetch.prepare = [&](const Plan &P) {
+        t0 = now_ms();
+        cols.gptr.assign((size_t)G + 1, 0);                      // (the plan's proband u is list position u: no duplicates)
+        for (int32_t g = 0; g < G; g++) cols.gptr[(size_t)g + 1] = cols.gptr[(size_t)g] + (int32_t)members[(size_t)g];
+        cols.gcol.resize((size_t)n_pro);
+        cols.gat.resize((size_t)n_pro);
+        std::vector<int32_t> next(cols.gptr.begin(), cols.gptr.end() - 1);
+        for (int32_t u = 0; u < n_pro; u++) {
+            const int32_t k = next[(size_t)group[u]]++;
+            cols.gcol[(size_t)k] = P.pro_slot[(size_t)u];
+            cols.gat[(size_t)u] = k;
+        }
+        for (int32_t u = 0; u < n_pro; u++) base[(size_t)P.pro_owner[(size_t)u] + 1]++;
+        for (int32_t g = 0; g < n_dev; g++) base[(size_t)g + 1] += base[(size_t)g];
+        at.resize((size_t)n_pro);
+        std::vector<int64_t> fill(base.begin(), base.end() - 1);
+        for (int32_t u = 0; u < n_pro; u++) at[(size_t)fill[(size_t)P.pro_owner[(size_t)u]]++] = u;   // own_pro: ascending
+    };
+    fetch.device = [&](genlib_engine &E, int g) {
+        DeviceGuard guard;
+        if (int r = guard.enter(E.device)) return r;
+        double *dst = proband_mean + (size_t)base[(size_t)g] * G;
+        return numerics == GENLIB_NUMERICS_FP64 ? phi_groups_rows<double>(E, cols, dst) : phi_groups_rows<float>(E, cols, dst);
+    };
+    fetch.combine = [&]() {
+        const size_t Gs = (size_t)G;
+        for (int32_t p = 0; p < n_pro; p++)                      // rows to list order (one device: in place already)
+            while (at[(size_t)p] != p) {
+                const int32_t q = at[(size_t)p];
+                std::swap_ranges(proband_mean + (size_t)p * Gs, proband_mean + (size_t)(p + 1) * Gs, proband_mean + (size_t)q * Gs);
+                std::swap(at[(size_t)p], at[(size_t)q]);
+            }
+        std::fill(group_mean, group_mean + Gs * Gs, 0.0);         // T, in list order
+        for (int32_t i = 0; i < n_pro; i++) {
+            double *t = group_mean + (size_t)group[i] * Gs;
+            const double *s = proband_mean + (size_t)i * Gs;
+            for (size_t g = 0; g < Gs; g++) t[g] += s[g];
+        }
+        const double nan = std::nan("");                       // (no pair to average over)
+        for (size_t a = 0; a < Gs; a++)                          // T[a][b], a <= b, to both means
+            for (size_t b = a; b < Gs; b++) {
+                const int64_t pairs = members[a] * members[b] - (a == b ? members[a] : 0);
+                group_mean[a * Gs + b] = group_mean[b * Gs + a] = pairs ? group_mean[a * Gs + b] / (double)pairs : nan;
+            }
+        for (int32_t i = 0; i < n_pro; i++) {
+            double *s = proband_mean + (size_t)i * Gs;
+            for (size_t g = 0; g < Gs; g++) {
+                const int64_t others = members[g] - ((size_t)group[i] == g ? 1 : 0);
+                s[g] = others ? s[g] / (double)others : nan;
+            }
+        }
+        return (int)GENLIB_OK;
+    };
+    fetch.finish = [&](genlib_engine &E, int) {                  // (one device: stats come from its engine)
+        E.stats.ms_fetch = now_ms() - t0;
+        return (int)GENLIB_OK;
+    };
+    return oneshot("genlib_phi_groups", GENLIB_SCHEDULE_PHI, n, father, mother, n_pro, proband, true, numerics, n_dev,
+                   devices, stats, fetch);
 }
 
 // genlib_f: a GENLIB_SCHEDULE_F plan of the listed individuals with both parents; every device copies its per-couple

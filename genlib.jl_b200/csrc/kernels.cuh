@@ -1,6 +1,6 @@
 // kernels.cuh -- device-side vocabulary shared by the sm_100a kernels of the kinship sweep, and the
-// small kernels around the layer kernel (layer_kernel.cuh): proband gather, gen.phiOver's selection, phiMean
-// reduction, the inter-GPU barrier, sparse_phi's misfiled pairs, gen.f's parents' kinships and gen.phi_pairs' reads.
+// small kernels around the layer kernel (layer_kernel.cuh): proband gather, gen.phiOver's selection, gen.phiMeanGroups'
+// and phiMean's reductions, the inter-GPU barrier, sparse_phi's misfiled pairs, gen.f's parents' kinships and gen.phi_pairs' reads.
 //
 // Arithmetic is binary64 in the reference's grouping; storage type T is float
 // (GENLIB_NUMERICS_REFERENCE: one RN32 per step, like src/compute.jl:296) or double.
@@ -265,6 +265,82 @@ phi_over_select_kernel(const T *__restrict__ A, int64_t ld, const int32_t *__res
         }
         at += total;
         __syncthreads();                                          // (warp_hits is written again by the next chunk)
+    }
+}
+
+// =====================================================================================
+// gen.phiMeanGroups: S[i][g] = sum of M[i, j] over the probands j != i of group g, for this rank's own proband rows
+// row0 + blockIdx.x (rows[] local rows, index[] their list positions i; no peer reads).  The columns come in group-major
+// order: column k is the proband at frontier slot gcol[k], group g holds columns [gptr[g], gptr[g + 1]), never empty,
+// and list position i is column gat[i] (the diagonal, skipped).  out[r * G + g] = S[row0 + r][g].  Every entry of the
+// row is read once, all sums are binary64, and their order depends only on P, the groups and kThreads:
+//   - thread t adds the columns [P t / kThreads, P (t + 1) / kThreads) in ascending order, one running sum per group;
+//   - a group whose columns all lie in one chunk is written by that thread;
+//   - the open group at the end of each chunk enters a segmented scan over the threads (Kogge-Stone shuffles inside a
+//     warp, then the warps' totals in warp order); the thread that holds a group's last column adds its own partial to
+//     the scan's value before it, and writes the group.
+// Work per row is P / kThreads columns and a binary search in gptr per thread, whatever G is.
+// =====================================================================================
+template <typename T>
+__global__ void __launch_bounds__(kThreads)
+phi_groups_kernel(const T *__restrict__ A, int64_t ld, const int32_t *__restrict__ rows, const int32_t *__restrict__ index,
+                  const int32_t *__restrict__ gcol, const int32_t *__restrict__ gat, const int32_t *__restrict__ gptr,
+                  int32_t G, int32_t P, int32_t row0, double *__restrict__ out) {
+    __shared__ double warp_v[kThreads / 32];
+    __shared__ int warp_f[kThreads / 32];
+    const int r = row0 + blockIdx.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const T *row = A + (int64_t)rows[r] * ld;
+    const int diag = gat[index[r]];
+    double *dst = out + (size_t)blockIdx.x * G;
+    const int c0 = (int)((int64_t)P * threadIdx.x / kThreads), c1 = (int)((int64_t)P * (threadIdx.x + 1) / kThreads);
+    double s = 0.0, head = 0.0;        // the open group's partial; the first group's, when it began before c0 and ends here
+    int g = 0, g_head = -1;
+    bool began_here = false;           // the open group began in this chunk (an empty chunk is the scan's identity)
+    if (c0 < c1) {
+        int lo = 0, hi = G - 1;        // the group of column c0: the last g with gptr[g] <= c0
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (gptr[mid] <= c0) lo = mid; else hi = mid - 1;
+        }
+        g = lo;
+        began_here = gptr[g] == c0;
+        int end = gptr[g + 1];
+        for (int k = c0; k < c1; k++) {
+            if (k == end) {            // group g ended at column k - 1
+                if (began_here) dst[g] = s; else { head = s; g_head = g; }
+                end = gptr[++g + 1];
+                s = 0.0;
+                began_here = true;
+            }
+            if (k != diag) s += (double)row[gcol[k]];
+        }
+        if (end == c1) {               // the last group ends with the chunk
+            if (began_here) dst[g] = s; else { head = s; g_head = g; }
+        }
+    }
+    // segmented inclusive scan of (began_here, s): a later element that began its group discards what came before
+    double v = s;
+    int f = began_here;
+    for (int o = 1; o < 32; o <<= 1) {
+        const double pv = __shfl_up_sync(0xffffffffu, v, o);
+        const int pf = __shfl_up_sync(0xffffffffu, f, o);
+        if (lane >= o) {
+            if (!f) v = pv + v;
+            f |= pf;
+        }
+    }
+    if (lane == 31) { warp_v[w] = v; warp_f[w] = f; }
+    double ev = __shfl_up_sync(0xffffffffu, v, 1);      // exclusive: the threads before this one
+    int ef = __shfl_up_sync(0xffffffffu, f, 1);
+    if (lane == 0) { ev = 0.0; ef = 0; }
+    __syncthreads();
+    if (g_head >= 0) {
+        if (!ef) {
+            double pv = 0.0;                              // the warps before this one, in warp order
+            for (int k = 0; k < w; k++) pv = warp_f[k] ? warp_v[k] : pv + warp_v[k];
+            ev = pv + ev;
+        }
+        dst[g_head] = ev + head;
     }
 }
 

@@ -539,6 +539,68 @@ def phi_over_arrays(father, mother, proband_ranks, threshold, *, numerics="refer
     return line.astype(np.int64), column.astype(np.int64), kinship, st.as_dict()
 
 
+class GroupKinship:
+    """What gen.phiMeanGroups returns.  `ids`: the probands, sorted; `groups`: the group labels, sorted; `size`: the
+    probands per group (int64); `mean[h, g]`: the mean kinship between groups h and g, pairs of distinct probands
+    (G x G, symmetric, float64); `proband[i, g]`: the mean kinship of proband ids[i] with the other members of group g
+    (P x G, float64).  A proband alone in its group has NaN in its own column; a one-member group NaN on the diagonal."""
+
+    def __init__(self, ids, groups, size, mean, proband):
+        self.ids, self.groups, self.size = ids, groups, size
+        self.mean, self.proband = mean, proband
+
+    def __repr__(self) -> str:
+        return f"GroupKinship({len(self.ids)} probands in {len(self.groups)} groups)"
+
+
+def phiMeanGroups(pedigree: Pedigree, groups, *, numerics="reference", device: int = -1, devices=None,
+                  return_stats: bool = False) -> GroupKinship:
+    """Mean kinship within and between groups of probands, and of each proband with each group, as a `GroupKinship`.
+
+    `groups` maps proband IDs to labels (`{ID: population}`, what GenLib's `_pop` reads from pop140.csv).  The probands
+    are its IDs sorted ascending, the groups its distinct labels sorted (TypeError when labels do not compare, e.g. str
+    and int).  M is the matrix gen.phi(pedigree, ids, numerics=numerics) returns, widened exactly to float64; the means
+    are over pairs of distinct probands (the diagonal is skipped).  gen.phi's plan and layers run on the device and
+    every device reduces the proband rows it holds (genlib_phi_groups): only P x G doubles leave the device, never the
+    matrix.  The order of every sum is fixed by the list and the groups, so the result is the same bits on any number
+    of devices; where every partial sum is a float64 number each mean is the exact rational rounded once.  An empty
+    mapping gives an empty record without a device; KeyError on an unknown ID."""
+    ids = np.array(sorted(int(i) for i in groups), np.int64)
+    labels = np.empty(len(ids), object)
+    labels[:] = [groups[int(i)] for i in ids]
+    levels, index = np.unique(labels, return_inverse=True)          # (TypeError on labels that do not compare)
+    levels = np.array(levels.tolist())
+    size = np.bincount(index, minlength=len(levels)).astype(np.int64)
+    ranks = pedigree.rank_of(ids)                                   # KeyError, like pedigree[ID]
+    if len(ids) == 0:
+        res, stats = GroupKinship(ids, levels, size, np.zeros((0, 0)), np.zeros((0, 0))), {}
+    else:
+        pm, gm, stats = phi_groups_arrays(pedigree.father, pedigree.mother, ranks, index, len(levels), numerics=numerics,
+                                          device=device, devices=devices)
+        res = GroupKinship(ids, levels, size, gm, pm)
+    return (res, stats) if return_stats else res
+
+
+def phi_groups_arrays(father, mother, proband_ranks, group_index, n_groups, *, numerics="reference", device: int = -1,
+                      devices=None):
+    """One-shot C-ABI call `genlib_phi_groups` on flat rank arrays (what the Julia shim ccalls): distinct proband ranks
+    in list order, each one's group in [0, n_groups).  Returns (proband_mean (P x G), group_mean (G x G), stats)."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32).reshape(-1)
+    gi = np.ascontiguousarray(group_index, np.int32).reshape(-1)
+    if len(gi) != len(pr):
+        raise ValueError(f"phi_groups_arrays: {len(gi)} group indices for {len(pr)} probands")
+    n_groups = int(n_groups)
+    pm = np.empty((len(pr), max(n_groups, 0)), np.float64)
+    gm = np.empty((max(n_groups, 0), max(n_groups, 0)), np.float64)
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = Stats()
+    check(lib().genlib_phi_groups(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), ptr(gi), n_groups,
+                                  _lib.NUMERICS[numerics], len(dv), ptr(dv), ptr(pm), ptr(gm), C.byref(st)))
+    return pm, gm, st.as_dict()
+
+
 class GcPlan:
     """The schedule of gen.gc (genlib_gc_plan_*): direction, layers, frontier slots.  Needs no GPU."""
 

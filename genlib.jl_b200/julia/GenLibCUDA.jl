@@ -255,6 +255,43 @@ function phiOver(pedigree::GenLib.Pedigree, threshold::Real, probandIDs::Vector{
 end
 
 """
+    phiMeanGroups(pedigree, groups; numerics = :reference, device = -1, devices = Int[])
+        -> NamedTuple (ids, groups, size, mean, proband)
+
+Mean kinship within and between groups of probands, and of each proband with each group, without the matrix leaving
+the device (`genlib_phi_groups`).  `groups` maps proband IDs to labels, e.g. `GenLib._pop(...)` on pop140.csv for
+genea140.  `ids` are its IDs sorted, `groups` its labels sorted, `size` the probands per group; `mean[h, g]` is the
+mean of `ϕ[i, j]` over `i` in group `h`, `j` in group `g`, `i ≠ j` (symmetric, `Float64`), `proband[i, g]` the mean
+of `ϕ[i, j]` over the other members `j` of group `g`, where `ϕ = phi(pedigree, ids; numerics)` widened exactly to
+`Float64`.  NaN where there is no pair (a one-member group's diagonal, a proband alone in its group).  The order of
+every sum is fixed by the list and the groups: the same bits on any number of devices.  KeyError on an unknown ID.
+"""
+function phiMeanGroups(pedigree::GenLib.Pedigree, groups::AbstractDict{Int}; numerics::Symbol = :reference,
+                       device::Integer = -1, devices::Vector{<:Integer} = Int[])
+    ids = sort!(collect(keys(groups)))
+    labels = sort!(unique(collect(values(groups))))
+    level = Dict(l => Int32(k - 1) for (k, l) in enumerate(labels))
+    P, G = length(ids), length(labels)
+    index = Int32[level[groups[ID]] for ID in ids]
+    counts = zeros(Int, G)
+    for k in index
+        counts[k + 1] += 1
+    end
+    P == 0 && return (ids = ids, groups = labels, size = counts, mean = zeros(0, 0), proband = zeros(0, 0))
+    father, mother = flatten(pedigree)
+    probands = Int32[pedigree[ID].rank - 1 for ID in ids]               # KeyError on unknown ID
+    rows = Matrix{Float64}(undef, G, P)                                 # C's row-major P x G
+    mean = Matrix{Float64}(undef, G, G)                                 # symmetric: layout-free
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    GC.@preserve rows mean check(ccall((:genlib_phi_groups, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Int32}, Int32, Cint, Int32, Ptr{Int32},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Cvoid}),
+        length(father), father, mother, P, probands, index, G, numerics === :fp64 ? 1 : 0, length(devs), devs,
+        rows, mean, C_NULL))
+    (ids = ids, groups = labels, size = counts, mean = mean, proband = permutedims(rows))
+end
+
+"""
     sparse_phi(pedigree, probandIDs = pro(pedigree)) -> GenLib.KinshipMatrix
 
 `gen.sparse_phi` (src/compute.jl:321-447) on the GPU: the same engine, planned for sparse_phi's own

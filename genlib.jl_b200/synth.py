@@ -57,6 +57,7 @@ class SyntheticPedigree:
     probands: np.ndarray    # IDs, sorted
     generation: np.ndarray
     params: dict
+    deme: np.ndarray        # per individual, in [0, demes): a natural grouping for gen.phiMeanGroups
 
     def to_csv(self, path: str):
         with open(path, "w") as fh:
@@ -134,7 +135,7 @@ def generate(n_individuals: int, generations: int, n_probands: int, alpha: float
     probands = np.sort(ind[last[rng.permutation(len(last))[:P]]])
     params = dict(n_individuals=N, generations=G, n_probands=P, alpha=alpha, demes=demes,
                   migration=migration, overlap=overlap, seed=seed)
-    return SyntheticPedigree(ind, father, mother, sex, probands, gen, params)
+    return SyntheticPedigree(ind, father, mother, sex, probands, gen, params, deme)
 
 
 # The shapes BASELINE.json's configs name (SURVEY.md 8d table).

@@ -345,6 +345,28 @@ int genlib_phi_over(int32_t n, const int32_t *father, const int32_t *mother, int
 /* Frees what genlib_phi_over allocated and zeroes the struct (NULL or an empty result: nothing to do). */
 int genlib_kinship_pairs_free(genlib_kinship_pairs *pairs);
 
+/* ---- gen.phiMeanGroups: mean kinship within and between groups of probands ---------------------------------------
+ * proband[0 .. n_pro) are distinct ranks in list order, group[k] in [0, n_groups) the group of proband[k]; every group
+ * has at least one member (n_g of them).  M is the matrix genlib_phi returns for the same list and numerics (Float32
+ * or Float64 storage), each entry widened exactly to binary64:
+ *   S[i][g]            = sum of M[i, j] over j in group g, j != i (the diagonal is skipped, not subtracted)
+ *   proband_mean[i][g] = S[i][g] / (n_g - [group[i] == g])                       (n_pro x n_groups, row-major)
+ *   T[h][g]            = sum of S[i][g] over i in group h, added in list order on the host
+ *   group_mean[h][g]   = group_mean[g][h] = T[a][b] / (n_a n_b - [a == b] n_a), a = min(h, g), b = max(h, g)
+ * A proband alone in its group gives NaN in its own column, a one-member group NaN on the diagonal.  The order of every
+ * sum depends only on the list and the groups, so the result is the same bits on any number of devices; where every
+ * partial sum is a binary64 number, each mean is the exact rational rounded once.  The genlib_phi plan runs unchanged
+ * (streamed, several devices as genlib_phi_multi); then every device reduces the proband rows it holds and copies back
+ * n_groups doubles per row: no matrix leaves the device.  The caller owns both outputs.
+ *   GENLIB_EINVAL: a null pointer or negative size, unknown numerics, not 1 .. 16 devices, n_groups < 1 with probands,
+ *   a group index out of range, a group without a proband, a rank listed twice.  A rank out of range gives GENLIB_EKEY
+ *   (a broken pedigree is reported first).  n_pro == 0 writes nothing, n_pro == 1 writes NaN to both outputs, neither
+ *   with a device.  devices[0] < 0 = the current device (one device).
+ *   stats as genlib_phi's, but ms_fetch = the reduction, the copy back and the host's part, d2h_bytes = 8 n_pro n_groups. */
+int genlib_phi_groups(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                      const int32_t *group, int32_t n_groups, int numerics, int32_t n_dev, const int32_t *devices,
+                      double *proband_mean, double *group_mean, genlib_stats *stats);
+
 /* ---- handle API: keep the schedule on the device, run, fetch ---------------
  * (what the benchmark and a multi-call Julia session use) */
 int genlib_engine_create(const genlib_plan *plan, int numerics, int device, genlib_engine **out);
