@@ -12,12 +12,13 @@ Usage mirrors the reference (`import GenLib as gen`):
     k = gen.phi_pairs(ped, [1, 2], [29, 2])  # float64 kinship of each pair, list order, no matrix formed
     o = gen.phiOver(ped, 1 / 64)           # proband pairs at or above 1/64, selected on the device
     g = gen.phiMeanGroups(ped, {1: "a", 2: "a", 29: "b"})  # mean kinship within / between groups, and per proband
+    c = gen.gcGroups(ped, {1: "a", 2: "a", 29: "b"})       # gen.gc summed over proband groups, no matrix formed
 """
 import os as _os
 
 from .pedigree import Individual, Pedigree, founder, genealogy, pro  # noqa: F401
 from .engine import (Engine, GcPlan, GenMatrix, GroupKinship, KinshipMatrix, PinnedMatrix, Plan, f, f_arrays,  # noqa: F401
-                     findDistance, findMRCA, gc, gc_arrays, meioses_arrays, mrca_arrays, occ, occ_arrays, phi, phi_arrays,
+                     findDistance, findMRCA, gc, gc_arrays, gc_groups_arrays, gcGroups, GroupContribution, meioses_arrays, mrca_arrays, occ, occ_arrays, phi, phi_arrays,
                      phi_distributed, phi_groups_arrays, phi_over_arrays, phi_pairs, phi_pairs_arrays, phiMean,
                      phiMeanGroups, phiOver, PhiOver, rec, rec_arrays, run_distributed,
                      sparse_phi)

@@ -170,6 +170,10 @@ SYMBOLS = {
     "genlib_gc_plan_info": (C.c_int, [_P, C.POINTER(GcStats)]),
     "genlib_gc_plan_layer": (C.c_int, [_P, C.c_int32, _P, _P]),
     "genlib_gc_plan_layer_arrays": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P]),
+    "genlib_gc_groups": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, C.c_int32, _P,
+                                   C.c_int, C.c_int32, _P, C.POINTER(GcStats)]),
+    "genlib_gc_groups_plan_create": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P,
+                                               C.c_int32, C.POINTER(_P)]),
     "genlib_occ": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int, C.c_int, C.c_int32, _P,
                              C.POINTER(GcStats)]),
     "genlib_rec": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int32, _P,

@@ -1,4 +1,4 @@
-// gc_engine.cu -- gen.gc, gen.occ, gen.rec and gen.findMRCA on the device (DESIGN.md 2b-2d): the C ABI entry points, the split of
+// gc_engine.cu -- gen.gc, gen.gcGroups, gen.occ, gen.rec and gen.findMRCA on the device (DESIGN.md 2b-2d, 2i): the C ABI entry points, the split of
 // the column-side list over the devices and each device's run of the plan (gc_plan.hpp) with the kernels of
 // gc_kernel.cuh.
 #include <cstdio>
@@ -51,11 +51,11 @@ struct GcShare {
 
 // Required traffic of a share over `cols` columns: the plan's byte model over the row's 8-byte elements
 // (gen.rec and the meioses: their words, 16-byte padded as the kernel moves them), plus one read of the
-// output block for a reduction.
+// output block for a reduction (gen.occ's and gen.rec's, or gen.gcGroups' sums over target groups).
 double gc_fn_bytes(const GcPlan &P, int fn, int32_t cols) {
     const int64_t w = fn == kFnRec || fn == kFnMeioses ? gc_fn_words(fn, cols) : cols;
     double b = P.alg_bytes(w);
-    if (gc_fn_reduces(fn)) b += (double)P.n_targets() * (double)w * 8.0;
+    if (gc_fn_reduces(fn) || P.target_grouped()) b += (double)P.n_targets() * (double)w * 8.0;
     return b;
 }
 
@@ -94,7 +94,9 @@ size_t gc_device_bytes(const GcPlan &P, GcShare &d, int col_major, size_t esize)
            3 * DevBuf<int32_t>::padded(R) + DevBuf<int64_t>::padded(R + 1) + DevBuf<int32_t>::padded((size_t)P.inputs()) +
            DevBuf<int32_t>::padded(P.target_uid().size()) + DevBuf<int32_t>::padded((size_t)(d.j1 - d.j0)) +
            DevBuf<int32_t>::padded(1) + 2 * d.stage +
-           (gc_fn_reports_overflow(d.fn) ? DevBuf<unsigned long long>::padded(1) : 0) + (gc_fn_reduces(d.fn) ? gc_reduce_bytes(P, d) : 0);
+           (gc_fn_reports_overflow(d.fn) ? DevBuf<unsigned long long>::padded(1) : 0) + (gc_fn_reduces(d.fn) ? gc_reduce_bytes(P, d) : 0) +
+           (P.target_grouped() ? pad256((size_t)P.n_target_groups() * ws * 8) + DevBuf<int64_t>::padded(P.grp_ptr.size()) +
+                                 DevBuf<int32_t>::padded(P.grp_row.size()) : 0);
 }
 
 template <typename E, typename O>
@@ -131,7 +133,8 @@ void gc_launch_layer(const GcLayerArgs &a, unsigned gx, cudaStream_t st) {
 }
 
 // Every layer of the plan over the share's columns on its device, then its block of `out` (gen.gc, gen.occ's
-// matrix) or its part of the reduction (d.red).
+// matrix; gen.gcGroups with the target side grouped: after summing the rows of every target group) or its
+// part of the reduction (d.red).
 int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_major) {
     DeviceGuard guard;
     if (int rc = guard.enter(d.device)) return rc;
@@ -165,8 +168,10 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
     auto take = [&](size_t bytes) { unsigned char *p = cur; cur += pad256(bytes); return p; };
     void *F = take((size_t)P.capacity * ws * 8);
     void *O = take(T * ws * 8);
-    DevBuf<int32_t> row_slot, row_seed, row_out, in_slot, tgt_row, col, err;
-    DevBuf<int64_t> in_ptr;
+    const bool grouped = P.target_grouped();
+    void *Og = grouped ? take((size_t)P.n_target_groups() * ws * 8) : nullptr;   // one row per target group
+    DevBuf<int32_t> row_slot, row_seed, row_out, in_slot, tgt_row, col, err, grp_row;
+    DevBuf<int64_t> in_ptr, grp_ptr;
     DevBuf<unsigned long long> ovf, m1, m2, red;
     DevBuf<uint32_t> wt;
     row_slot.place(cur, R); row_seed.place(cur, R); row_out.place(cur, R); in_ptr.place(cur, R + 1);
@@ -175,6 +180,7 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
     unsigned char *stage = cur;
     cur += 2 * d.stage;
     if (gc_fn_reports_overflow(d.fn)) ovf.place(cur, 1);
+    if (grouped) { grp_ptr.place(cur, P.grp_ptr.size()); grp_row.place(cur, P.grp_row.size()); }
     // reduction weights: how often the lists name each column (ascend) or each target row (descend)
     std::vector<uint32_t> h_wt;
     std::vector<unsigned long long> h_m1, h_m2;
@@ -204,6 +210,7 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
     CU(row_slot.upload(P.row_slot, res.st)); CU(row_seed.upload(P.row_seed, res.st)); CU(row_out.upload(P.row_out, res.st));
     CU(in_ptr.upload(P.in_ptr, res.st)); CU(in_slot.upload(P.in_slot, res.st)); CU(tgt_row.upload(P.target_uid(), res.st));
     CU(col.upload(cols, res.st));
+    if (grouped) { CU(grp_ptr.upload(P.grp_ptr, res.st)); CU(grp_row.upload(P.grp_row, res.st)); }
     CU(cudaMemsetAsync(err.p, 0, sizeof(int32_t), res.st));
     if (gc_fn_reports_overflow(d.fn)) CU(cudaMemsetAsync(ovf.p, 0xff, sizeof(unsigned long long), res.st));
     if (reduce) {
@@ -253,6 +260,17 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
         CU(cudaGetLastError());
         d.launches++;
     }
+    if (grouped && P.n_target_groups() > 0) {
+        GcGroupReduceArgs g;
+        g.O = static_cast<const double *>(O); g.out = static_cast<double *>(Og); g.ws = (int64_t)ws;
+        g.n_groups = P.n_target_groups(); g.grp_ptr = grp_ptr.p; g.grp_row = grp_row.p;
+        // about 8 CTAs per SM over the columns and the groups
+        const int64_t gxg = ((int64_t)ws + 255) / 256;
+        const unsigned gyg = (unsigned)std::max<int64_t>(1, std::min<int64_t>(g.n_groups, (148 * 8 + gxg - 1) / gxg));
+        gc_group_reduce_kernel<<<dim3((unsigned)gxg, gyg), 256, 0, res.st>>>(g);
+        CU(cudaGetLastError());
+        d.launches++;
+    }
     CU(cudaEventRecord(res.ev[1], res.st));
     CU(cudaStreamSynchronize(res.st));
     float ms = 0;
@@ -274,7 +292,7 @@ int gc_run_share(const GcPlan &P, GcShare &d, void *out, int out_dtype, int col_
         rc = gc_fetch<uint16_t, int64_t>(P, d, O, tgt_row.p, col.p, static_cast<int64_t *>(out), col_major, stage, nullptr, res.st, res.cst);
     } else {
         rc = out_dtype == GENLIB_F64
-            ? gc_fetch<double, double>(P, d, O, tgt_row.p, col.p, static_cast<double *>(out), col_major, stage, nullptr, res.st, res.cst)
+            ? gc_fetch<double, double>(P, d, grouped ? Og : O, tgt_row.p, col.p, static_cast<double *>(out), col_major, stage, nullptr, res.st, res.cst)
             : gc_fetch<double, float>(P, d, O, tgt_row.p, col.p, static_cast<float *>(out), col_major, stage, nullptr, res.st, res.cst);
     }
     d.ms_fetch = now_ms() - t0;
@@ -289,12 +307,9 @@ void gc_fill_stats(const GcPlan &P, genlib_gc_stats *s) {
     s->n_dev = 1;
 }
 
-}  // namespace
-
-extern "C" {
-
-int genlib_gc_plan_create(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
-                          const int32_t *proband, int32_t n_anc, const int32_t *ancestor, genlib_gc_plan **out) {
+int gc_plan_create(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                   const int32_t *pro_group, int32_t n_pro_groups, int32_t n_anc, const int32_t *ancestor,
+                   const int32_t *anc_group, int32_t n_anc_groups, genlib_gc_plan **out) {
     if (!out) return fail(GENLIB_EINVAL, "genlib_gc_plan_create: null argument");
     *out = nullptr;
     std::unique_ptr<genlib_gc_plan> pl(new (std::nothrow) genlib_gc_plan);
@@ -302,13 +317,39 @@ int genlib_gc_plan_create(int32_t n, const int32_t *father, const int32_t *mothe
     const double t0 = now_ms();
     std::string err;
     try {
-        if (int rc = build_gc_plan(n, father, mother, n_pro, proband, n_anc, ancestor, -1, pl->p, err)) return fail(rc, err);
+        if (int rc = build_gc_plan(n, father, mother, n_pro, proband, n_anc, ancestor, -1, pl->p, err, pro_group,
+                                   n_pro_groups, anc_group, n_anc_groups))
+            return fail(rc, err);
     } catch (const std::bad_alloc &) {
         return fail(GENLIB_ENOMEM, "out of host memory while planning");
     }
     pl->ms_plan = now_ms() - t0;
     *out = pl.release();
     return GENLIB_OK;
+}
+
+// gen.gcGroups with neither side grouped is gen.gc
+int gc_groups_check(const int32_t *pro_group, const int32_t *anc_group) {
+    if (!pro_group && !anc_group) return fail(GENLIB_EINVAL, "genlib_gc_groups: neither side is grouped (that is genlib_gc)");
+    return GENLIB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int genlib_gc_plan_create(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
+                          const int32_t *proband, int32_t n_anc, const int32_t *ancestor, genlib_gc_plan **out) {
+    return gc_plan_create(n, father, mother, n_pro, proband, nullptr, 0, n_anc, ancestor, nullptr, 0, out);
+}
+
+int genlib_gc_groups_plan_create(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro,
+                                 const int32_t *proband, const int32_t *pro_group, int32_t n_pro_groups, int32_t n_anc,
+                                 const int32_t *ancestor, const int32_t *anc_group, int32_t n_anc_groups,
+                                 genlib_gc_plan **out) {
+    if (int rc = gc_groups_check(pro_group, anc_group)) return rc;
+    return gc_plan_create(n, father, mother, n_pro, proband, pro_group, n_pro_groups, n_anc, ancestor, anc_group,
+                          n_anc_groups, out);
 }
 
 void genlib_gc_plan_destroy(genlib_gc_plan *plan) { delete plan; }
@@ -375,11 +416,14 @@ int gc_overflow(int32_t anc_pos, int32_t anc_rank, int32_t pro_pos, int32_t pro_
 // combined here.
 int gc_driver(int fn, int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
               int32_t n_anc, const int32_t *ancestor, void *out, int out_dtype, int col_major, int32_t n_dev,
-              const int32_t *devices, genlib_gc_stats *stats) {
+              const int32_t *devices, genlib_gc_stats *stats, const int32_t *pro_group = nullptr,
+              int32_t n_pro_groups = 0, const int32_t *anc_group = nullptr, int32_t n_anc_groups = 0) {
     const std::string who = std::string("genlib_") + kGcFnName[fn];
     if (n_dev < 1 || !devices) return fail(GENLIB_EINVAL, who + ": at least one device");
     genlib_gc_plan *plan = nullptr;
-    if (int rc = genlib_gc_plan_create(n, father, mother, n_pro, proband, n_anc, ancestor, &plan)) return rc;
+    if (int rc = gc_plan_create(n, father, mother, n_pro, proband, pro_group, n_pro_groups, n_anc, ancestor, anc_group,
+                                n_anc_groups, &plan))
+        return rc;
     std::unique_ptr<genlib_gc_plan> owner(plan);
     const GcPlan &P = plan->p;
     if (fn == kFnMeioses && P.n_layers() >= (int32_t)kMeiosesNone)   // d <= n_layers - 1 must stay below the sentinel
@@ -482,6 +526,15 @@ int genlib_gc(int32_t n, const int32_t *father, const int32_t *mother, int32_t n
     if (out_dtype != GENLIB_F32 && out_dtype != GENLIB_F64) return fail(GENLIB_EINVAL, "unknown out_dtype");
     return gc_driver(kFnGc, n, father, mother, n_pro, proband, n_anc, ancestor, out, out_dtype, col_major, n_dev,
                      devices, stats);
+}
+
+int genlib_gc_groups(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                     const int32_t *pro_group, int32_t n_pro_groups, int32_t n_anc, const int32_t *ancestor,
+                     const int32_t *anc_group, int32_t n_anc_groups, double *out, int col_major, int32_t n_dev,
+                     const int32_t *devices, genlib_gc_stats *stats) {
+    if (int rc = gc_groups_check(pro_group, anc_group)) return rc;
+    return gc_driver(kFnGc, n, father, mother, n_pro, proband, n_anc, ancestor, out, GENLIB_F64, col_major, n_dev,
+                     devices, stats, pro_group, n_pro_groups, anc_group, n_anc_groups);
 }
 
 int genlib_occ(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,

@@ -11,6 +11,9 @@
 // gc_row_reduce_kernel / gc_col_reduce_kernel: the row sums of gen.occ(typeOcc = "TOTAL") and the counts of
 // gen.rec, one pass over the output block, so the matrix never leaves the device.
 //
+// gc_group_reduce_kernel: gen.gcGroups with the target side grouped -- every group's output-block rows summed
+// into one row, so only a groups x columns block is gathered.
+//
 // gc_gather_kernel: a 32 x 32 tile of the output block, with duplicates of either list expanded, to a
 // staging buffer in the layout of the caller's matrix (row- or column-major; float64, float32 or int64; uint16
 // distances widen to int64),
@@ -324,6 +327,40 @@ __global__ void __launch_bounds__(256) gc_gather_kernel(GcGatherArgs a, Out *sta
             if (t < a.n_t && cc < a.n_c) stage[(int64_t)cc * a.n_t + t] = gc_widen<Out>(tile[tx][k]);
         }
         __syncthreads();
+    }
+}
+
+// gen.gcGroups, target side grouped: out[g][c] = the sum of O[row][c] over group g's output-block rows, in list
+// order, one binary64 running sum per (group, column).  The order is fixed and there are no atomics, and every
+// column lives on one device, so the bits do not depend on the device count.  A thread per column (coalesced
+// along the row), a y-stride over the groups; the row indices and values of kGcGroupBatch members are loaded
+// before they are added, in order.
+constexpr int kGcGroupBatch = 8;
+struct GcGroupReduceArgs {
+    const double *O;            // output block: rows of ws doubles
+    double *out;                // n_groups rows of ws doubles
+    int64_t ws;
+    int32_t n_groups;
+    const int64_t *grp_ptr;     // n_groups + 1 entries
+    const int32_t *grp_row;
+};
+
+__global__ void __launch_bounds__(256) gc_group_reduce_kernel(GcGroupReduceArgs a) {
+    const int64_t c = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (c >= a.ws) return;
+    for (int32_t g = blockIdx.y; g < a.n_groups; g += gridDim.y) {
+        const int64_t k1 = a.grp_ptr[g + 1];
+        double s = 0.0;
+        int64_t k = a.grp_ptr[g];
+        for (; k + kGcGroupBatch <= k1; k += kGcGroupBatch) {
+            double v[kGcGroupBatch];
+#pragma unroll
+            for (int u = 0; u < kGcGroupBatch; u++) v[u] = __ldcs(a.O + (int64_t)a.grp_row[k + u] * a.ws + c);
+#pragma unroll
+            for (int u = 0; u < kGcGroupBatch; u++) s += v[u];
+        }
+        for (; k < k1; k++) s += __ldcs(a.O + (int64_t)a.grp_row[k] * a.ws + c);
+        a.out[(int64_t)g * a.ws + c] = s;
     }
 }
 

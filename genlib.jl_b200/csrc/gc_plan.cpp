@@ -13,10 +13,11 @@
 namespace genlib {
 
 int build_gc_plan(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
-                  int32_t n_anc, const int32_t *ancestor, int direction, GcPlan &P, std::string &err) {
+                  int32_t n_anc, const int32_t *ancestor, int direction, GcPlan &P, std::string &err,
+                  const int32_t *pro_group, int32_t n_pro_groups, const int32_t *anc_group, int32_t n_anc_groups) {
     P = GcPlan();
-    if (n < 0 || n_pro < 0 || n_anc < 0 || (n > 0 && (!father || !mother)) || (n_pro > 0 && !proband) ||
-        (n_anc > 0 && !ancestor)) {
+    if (n < 0 || n_pro < 0 || n_anc < 0 || n_pro_groups < 0 || n_anc_groups < 0 || (n > 0 && (!father || !mother)) ||
+        (n_pro > 0 && !proband) || (n_anc > 0 && !ancestor)) {
         err = "genlib_gc: null pointer or negative size";
         return GENLIB_EINVAL;
     }
@@ -37,8 +38,29 @@ int build_gc_plan(int32_t n, const int32_t *father, const int32_t *mother, int32
     };
     if (int rc = unique(n_pro, proband, "proband", pro_of, P.pro_uid, P.n_pro_u)) return rc;
     if (int rc = unique(n_anc, ancestor, "ancestor", anc_of, P.anc_uid, P.n_anc_u)) return rc;
+    // a grouped side: distinct ranks (so its unique index is its list position), every group named
+    auto check_groups = [&](int32_t len, const int32_t *list, const int32_t *group, int32_t n_groups, const char *what,
+                            const std::vector<int32_t> &uid) {
+        std::vector<int32_t> members((size_t)n_groups, 0);
+        for (int32_t k = 0; k < len; k++) {
+            if (uid[(size_t)k] != k) { err = std::string("genlib_gc_groups: duplicate ") + what + " rank " + std::to_string(list[k]); return GENLIB_EINVAL; }
+            if (group[k] < 0 || group[k] >= n_groups) {
+                err = "genlib_gc_groups: group index " + std::to_string(group[k]) + " of " + what + " position " +
+                      std::to_string(k) + " is not in [0, " + std::to_string(n_groups) + ")";
+                return GENLIB_EINVAL;
+            }
+            members[(size_t)group[k]]++;
+        }
+        for (int32_t g = 0; g < n_groups; g++)
+            if (!members[(size_t)g]) { err = "genlib_gc_groups: " + std::string(what) + " group " + std::to_string(g) + " has no member"; return GENLIB_EINVAL; }
+        return GENLIB_OK;
+    };
+    P.pro_grouped = pro_group != nullptr; P.anc_grouped = anc_group != nullptr;
+    if (P.pro_grouped) if (int rc = check_groups(n_pro, proband, pro_group, n_pro_groups, "proband", P.pro_uid)) return rc;
+    if (P.anc_grouped) if (int rc = check_groups(n_anc, ancestor, anc_group, n_anc_groups, "ancestor", P.anc_uid)) return rc;
     if (direction < 0) {
-        direction = P.n_pro_u < P.n_anc_u ? kGcAscend : kGcDescend;
+        const int32_t w_pro = P.pro_grouped ? n_pro_groups : P.n_pro_u, w_anc = P.anc_grouped ? n_anc_groups : P.n_anc_u;
+        direction = w_pro < w_anc ? kGcAscend : kGcDescend;
         if (const char *env = std::getenv("GENLIB_GC_DIRECTION")) {      // test / benchmark knob
             if (!std::strcmp(env, "descend")) direction = kGcDescend;
             else if (!std::strcmp(env, "ascend")) direction = kGcAscend;
@@ -46,6 +68,27 @@ int build_gc_plan(int32_t n, const int32_t *father, const int32_t *mother, int32
     }
     if (direction != kGcDescend && direction != kGcAscend) { err = "genlib_gc: unknown direction"; return GENLIB_EINVAL; }
     P.direction = direction;
+    // a grouped side's output positions are its groups: as the column side every member seeds its group's
+    // column, as the target side every member keeps its own output-block row and the groups list those rows
+    auto regroup = [&](bool is_column, int32_t len, const int32_t *list, const int32_t *group, int32_t n_groups,
+                       std::vector<int32_t> &of, std::vector<int32_t> &uid, int32_t &n_u, int32_t &n_out) {
+        if (is_column) {
+            for (int32_t k = 0; k < len; k++) of[(size_t)list[k]] = group[k];
+            n_u = n_groups;
+        } else {
+            P.grp_ptr.assign((size_t)n_groups + 1, 0);
+            for (int32_t k = 0; k < len; k++) P.grp_ptr[(size_t)group[k] + 1]++;
+            for (int32_t g = 0; g < n_groups; g++) P.grp_ptr[(size_t)g + 1] += P.grp_ptr[(size_t)g];
+            P.grp_row.resize((size_t)len);
+            std::vector<int64_t> at(P.grp_ptr.begin(), P.grp_ptr.end() - 1);
+            for (int32_t k = 0; k < len; k++) P.grp_row[(size_t)at[(size_t)group[k]]++] = k;
+        }
+        uid.resize((size_t)n_groups);
+        for (int32_t g = 0; g < n_groups; g++) uid[(size_t)g] = g;
+        n_out = n_groups;
+    };
+    if (P.pro_grouped) regroup(direction == kGcAscend, n_pro, proband, pro_group, n_pro_groups, pro_of, P.pro_uid, P.n_pro_u, P.n_pro);
+    if (P.anc_grouped) regroup(direction == kGcDescend, n_anc, ancestor, anc_group, n_anc_groups, anc_of, P.anc_uid, P.n_anc_u, P.n_anc);
     P.layer_begin.assign(1, 0);
     if (P.n_pro_u == 0 || P.n_anc_u == 0) return GENLIB_OK;
 

@@ -8,6 +8,7 @@ returns a symmetric Float32 matrix in probandIDs order (duplicates collapsed),
 from __future__ import annotations
 
 import ctypes as C
+from collections.abc import Mapping
 from typing import Optional
 
 import numpy as np
@@ -553,6 +554,18 @@ class GroupKinship:
         return f"GroupKinship({len(self.ids)} probands in {len(self.groups)} groups)"
 
 
+def _group_mapping(pedigree: Pedigree, groups):
+    """A {ID: label} mapping read as (IDs sorted, labels sorted, each ID's label index, members per label (int64),
+    the IDs' ranks).  TypeError on labels that do not compare, KeyError on an unknown ID."""
+    ids = np.array(sorted(int(i) for i in groups), np.int64)
+    labels = np.empty(len(ids), object)
+    labels[:] = [groups[int(i)] for i in ids]
+    levels, index = np.unique(labels, return_inverse=True)          # (TypeError on labels that do not compare)
+    levels = np.array(levels.tolist())
+    size = np.bincount(index, minlength=len(levels)).astype(np.int64)
+    return ids, levels, index, size, pedigree.rank_of(ids)          # KeyError, like pedigree[ID]
+
+
 def phiMeanGroups(pedigree: Pedigree, groups, *, numerics="reference", device: int = -1, devices=None,
                   return_stats: bool = False) -> GroupKinship:
     """Mean kinship within and between groups of probands, and of each proband with each group, as a `GroupKinship`.
@@ -565,13 +578,7 @@ def phiMeanGroups(pedigree: Pedigree, groups, *, numerics="reference", device: i
     matrix.  The order of every sum is fixed by the list and the groups, so the result is the same bits on any number
     of devices; where every partial sum is a float64 number each mean is the exact rational rounded once.  An empty
     mapping gives an empty record without a device; KeyError on an unknown ID."""
-    ids = np.array(sorted(int(i) for i in groups), np.int64)
-    labels = np.empty(len(ids), object)
-    labels[:] = [groups[int(i)] for i in ids]
-    levels, index = np.unique(labels, return_inverse=True)          # (TypeError on labels that do not compare)
-    levels = np.array(levels.tolist())
-    size = np.bincount(index, minlength=len(levels)).astype(np.int64)
-    ranks = pedigree.rank_of(ids)                                   # KeyError, like pedigree[ID]
+    ids, levels, index, size, ranks = _group_mapping(pedigree, groups)
     if len(ids) == 0:
         res, stats = GroupKinship(ids, levels, size, np.zeros((0, 0)), np.zeros((0, 0))), {}
     else:
@@ -604,7 +611,10 @@ def phi_groups_arrays(father, mother, proband_ranks, group_index, n_groups, *, n
 class GcPlan:
     """The schedule of gen.gc (genlib_gc_plan_*): direction, layers, frontier slots.  Needs no GPU."""
 
-    def __init__(self, father, mother, proband_ranks, ancestor_ranks):
+    def __init__(self, father, mother, proband_ranks, ancestor_ranks, *, pro_group=None, n_pro_groups: int = 0,
+                 anc_group=None, n_anc_groups: int = 0):
+        """With `pro_group` and/or `anc_group` (a group index per rank), gen.gcGroups' schedule
+        (genlib_gc_groups_plan_create)."""
         self.father = np.ascontiguousarray(father, np.int32)
         self.mother = np.ascontiguousarray(mother, np.int32)
         self.probands = np.ascontiguousarray(proband_ranks, np.int32)
@@ -612,8 +622,15 @@ class GcPlan:
         if len(self.father) != len(self.mother):
             raise ValueError("father and mother must have the same length")
         h = C.c_void_p()
-        check(lib().genlib_gc_plan_create(len(self.father), ptr(self.father), ptr(self.mother), len(self.probands),
-                                          ptr(self.probands), len(self.ancestors), ptr(self.ancestors), C.byref(h)))
+        if pro_group is None and anc_group is None:
+            check(lib().genlib_gc_plan_create(len(self.father), ptr(self.father), ptr(self.mother), len(self.probands),
+                                              ptr(self.probands), len(self.ancestors), ptr(self.ancestors), C.byref(h)))
+        else:
+            pg, ag = _group_array(pro_group, self.probands), _group_array(anc_group, self.ancestors)
+            check(lib().genlib_gc_groups_plan_create(len(self.father), ptr(self.father), ptr(self.mother),
+                                                     len(self.probands), ptr(self.probands), ptr(pg), int(n_pro_groups),
+                                                     len(self.ancestors), ptr(self.ancestors), ptr(ag),
+                                                     int(n_anc_groups), C.byref(h)))
         self._h = h
 
     def __del__(self):
@@ -675,6 +692,81 @@ def gc_arrays(father, mother, proband_ranks, ancestor_ranks, *, dtype=np.float64
     st = GcStats()
     check(lib().genlib_gc(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), len(an), ptr(an), ptr(out),
                           _lib.DTYPES[np.dtype(out.dtype)], int(col_major), len(dv), ptr(dv), C.byref(st)))
+    stats = st.as_dict()
+    stats["direction"] = _lib.GC_DIRECTIONS[stats["direction"]]
+    return out, stats
+
+
+class GroupContribution:
+    """What gen.gcGroups returns.  `rows` / `cols`: the output positions of the proband / ancestor side -- a grouped
+    side's labels, sorted, or a list's IDs in list order; `row_size` / `col_size`: the individuals in each (int64, 1 for
+    a list entry); `total[r, c]`: the sum of G[p, a] over the probands p of row r and the ancestors a of column c
+    (float64); `mean = total / row_size[:, None]`: the mean contribution of column c to one proband of row r."""
+
+    def __init__(self, rows, cols, row_size, col_size, total):
+        self.rows, self.cols, self.row_size, self.col_size = rows, cols, row_size, col_size
+        self.total = total
+        self.mean = total / row_size[:, None]
+
+    def __repr__(self) -> str:
+        return f"GroupContribution({len(self.rows)} x {len(self.cols)})"
+
+
+def gcGroups(pedigree: Pedigree, pro=None, ancestors=None, *, device: int = -1, devices=None,
+             return_stats: bool = False) -> GroupContribution:
+    """gen.gc summed over groups, as a `GroupContribution`: total[r, c] = the sum of G[p, a] over p in row r and a in
+    column c, where G is what gen.gc returns for the same lists.
+
+    Each of `pro` and `ancestors` is None (gen.pro / gen.founder, as in gen.gc), a list of IDs (one row / column per
+    entry, duplicates kept) or a {ID: label} mapping (one row / column per label; IDs sorted, labels sorted, TypeError
+    when labels do not compare).  At least one side must be a mapping (ValueError otherwise: that is gen.gc).  G is
+    linear, so the engine propagates one column per group and sums the other side's rows per group on the device
+    (genlib_gc_groups): only the R x C result leaves it, never the proband x ancestor matrix.  Where every partial
+    sum is a float64 number (founders as ancestors, any realistic group size) the result is the exact sum.  KeyError
+    on an unknown ID."""
+    sides = []
+    for arg, default in ((pro, _pedigree.pro), (ancestors, _pedigree.founder)):
+        if isinstance(arg, Mapping):
+            _, levels, index, size, ranks = _group_mapping(pedigree, arg)
+            sides.append((levels, size, ranks, index, len(levels)))
+        else:
+            ids = default(pedigree) if arg is None else np.asarray(arg, np.int64)
+            sides.append((ids, np.ones(len(ids), np.int64), pedigree.rank_of(ids), None, 0))
+    (rows, row_size, pr, pg, npg), (cols, col_size, an, ag, nag) = sides
+    if pg is None and ag is None:
+        raise ValueError("gen.gcGroups needs a {ID: group} mapping for pro or ancestors; for two lists use gen.gc")
+    total, stats = gc_groups_arrays(pedigree.father, pedigree.mother, pr, an, pro_group=pg, n_pro_groups=npg,
+                                    anc_group=ag, n_anc_groups=nag, device=device, devices=devices)
+    res = GroupContribution(rows, cols, row_size, col_size, total)
+    return (res, stats) if return_stats else res
+
+
+def _group_array(group, ranks):
+    if group is None:
+        return None
+    g = np.ascontiguousarray(group, np.int32).reshape(-1)
+    if len(g) != len(ranks):
+        raise ValueError(f"{len(g)} group indices for {len(ranks)} ranks")
+    return g
+
+
+def gc_groups_arrays(father, mother, proband_ranks, ancestor_ranks, *, pro_group=None, n_pro_groups: int = 0,
+                     anc_group=None, n_anc_groups: int = 0, device: int = -1, devices=None, col_major: bool = False):
+    """One-shot C-ABI call `genlib_gc_groups` on flat rank arrays (what the Julia shim ccalls).  A side with a group
+    array (distinct ranks, each one's group in [0, n_groups)) is grouped, a side without one is a list as in
+    gc_arrays.  Returns (total, stats): R x C float64, R = n_pro_groups or len(proband_ranks), C likewise."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32).reshape(-1)
+    an = np.ascontiguousarray(ancestor_ranks, np.int32).reshape(-1)
+    pg, ag = _group_array(pro_group, pr), _group_array(anc_group, an)
+    shape = (len(pr) if pg is None else max(int(n_pro_groups), 0), len(an) if ag is None else max(int(n_anc_groups), 0))
+    out = np.empty(shape, np.float64, order="F" if col_major else "C")
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = GcStats()
+    check(lib().genlib_gc_groups(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), ptr(pg), int(n_pro_groups),
+                                 len(an), ptr(an), ptr(ag), int(n_anc_groups), ptr(out), int(col_major), len(dv),
+                                 ptr(dv), C.byref(st)))
     stats = st.as_dict()
     stats["direction"] = _lib.GC_DIRECTIONS[stats["direction"]]
     return out, stats

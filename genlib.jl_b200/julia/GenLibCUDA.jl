@@ -375,6 +375,48 @@ function gc(pedigree::GenLib.Pedigree; pro::Vector{Int} = GenLib.pro(pedigree),
 end
 
 """
+    gcGroups(pedigree; pro = GenLib.pro(pedigree), ancestors = GenLib.founder(pedigree),
+             device = -1, devices = Int[]) -> NamedTuple (rows, cols, row_size, col_size, total, mean)
+
+`gc` summed over groups without the proband × ancestor matrix leaving the device (`genlib_gc_groups`).  Each of
+`pro` and `ancestors` is a `Vector{Int}` of IDs (one row / column per entry, duplicates kept) or an
+`AbstractDict{Int}` mapping IDs to group labels (one row / column per label; IDs sorted, labels sorted); at least
+one must be a mapping (an `ArgumentError` otherwise: that is `gc`).  `total[r, c]` is the sum of `G[p, a]` over the
+probands `p` of row `r` and the ancestors `a` of column `c`, `mean = total ./ row_size`.  An unknown ID throws
+`KeyError`.  Not executed in this repository (no Julia in the build image); the same call is exercised through
+Python ctypes by tests/test_gc_groups.py.
+"""
+function gcGroups(pedigree::GenLib.Pedigree; pro::Union{Vector{Int}, AbstractDict{Int}} = GenLib.pro(pedigree),
+                  ancestors::Union{Vector{Int}, AbstractDict{Int}} = GenLib.founder(pedigree), device::Integer = -1,
+                  devices::Vector{<:Integer} = Int[])
+    side(list::Vector{Int}) = (list, ones(Int, length(list)), Int32[pedigree[ID].rank - 1 for ID in list], nothing)
+    function side(groups::AbstractDict{Int})
+        ids = sort!(collect(keys(groups)))
+        labels = sort!(unique(collect(values(groups))))
+        level = Dict(l => Int32(k - 1) for (k, l) in enumerate(labels))
+        index = Int32[level[groups[ID]] for ID in ids]
+        counts = zeros(Int, length(labels))
+        for k in index
+            counts[k + 1] += 1
+        end
+        (labels, counts, Int32[pedigree[ID].rank - 1 for ID in ids], index)       # KeyError on unknown ID
+    end
+    rows, row_size, p, pg = side(pro)
+    cols, col_size, a, ag = side(ancestors)
+    pg === nothing && ag === nothing && throw(ArgumentError("gcGroups needs a mapping for pro or ancestors; use gc"))
+    father, mother = flatten(pedigree)
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    total = Matrix{Float64}(undef, length(rows), length(cols))
+    stats = Ref{GcStats}()
+    GC.@preserve total check(ccall((:genlib_gc_groups, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Ptr{Int32}, Int32, Int32, Ptr{Int32}, Ptr{Int32}, Int32,
+         Ptr{Float64}, Cint, Int32, Ptr{Int32}, Ptr{GcStats}),
+        length(father), father, mother, length(p), p, pg === nothing ? C_NULL : pg, length(rows),
+        length(a), a, ag === nothing ? C_NULL : ag, length(cols), total, 1, length(devs), devs, stats))
+    (rows = rows, cols = cols, row_size = row_size, col_size = col_size, total = total, mean = total ./ row_size)
+end
+
+"""
     occ(pedigree; pro = GenLib.pro(pedigree), ancestors = GenLib.founder(pedigree), typeOcc = "IND",
         device = -1, devices = Int[]) -> Matrix{Int64}
 

@@ -455,6 +455,37 @@ int genlib_gc_plan_layer(const genlib_gc_plan *plan, int32_t layer, int32_t *n_r
 int genlib_gc_plan_layer_arrays(const genlib_gc_plan *plan, int32_t layer, int32_t *row_ind, int32_t *row_slot,
                                 int32_t *row_seed, int32_t *row_out, int64_t *in_ptr, int32_t *in_slot);
 
+/* ---- gen.gcGroups: genetic contributions summed over groups of probands and/or ancestors (DESIGN.md 2i) -------
+ * Each side is a list of ranks as in genlib_gc (group pointer null: list order, duplicates kept, one row / column
+ * per entry) or GROUPED: distinct ranks, rank k in group pro_group[k] (anc_group[k]) in [0, n_groups), every group
+ * non-empty.  With G = genlib_gc's matrix for the same lists,
+ *   out[r, c] = sum over p in row r, a in column c of G[p, a]                  (R x C float64)
+ * R = n_pro_groups if the probands are grouped, else n_pro; C likewise.  Row-major, or column-major when
+ * col_major != 0.  G is linear, so the engine propagates one column per group of the column side (the narrower
+ * side, counting a grouped side's groups and an ungrouped side's unique entries; descend on ties;
+ * GENLIB_GC_DIRECTION overrides) and, when the other side is grouped, sums its output rows per group on the device
+ * (members in list order, no atomics); only R x C doubles leave the devices.  Every G[p, a] is a multiple of 2^-L
+ * (L = the longest listed path) and every sum adds non-negative values: while every partial sum is a multiple of
+ * 2^-L below 2^(53 - L) the result is the exact sum, in either direction and on any device count; otherwise the
+ * order is fixed (the same bits on a repeat and on any device count; the two directions may differ in the last
+ * bits).  Devices as genlib_gc.
+ *   GENLIB_EINVAL: a null pointer or negative size, neither side grouped (that is genlib_gc), a group index out of
+ *   range, an empty group, a rank listed twice on a grouped side, no device.  A rank out of range gives GENLIB_EKEY
+ *   (a broken pedigree is reported first).  R == 0 or C == 0 writes nothing, without a device.
+ *   stats: n_pro / n_anc = R / C, width = columns propagated, d2h_bytes = 8 R C, alg_bytes = the plan's byte model
+ *   plus one read of the output block when the target side is summed per group. */
+int genlib_gc_groups(int32_t n, const int32_t *father, const int32_t *mother,
+                     int32_t n_pro, const int32_t *proband, const int32_t *pro_group, int32_t n_pro_groups,
+                     int32_t n_anc, const int32_t *ancestor, const int32_t *anc_group, int32_t n_anc_groups,
+                     double *out, int col_major, int32_t n_dev, const int32_t *devices, genlib_gc_stats *stats);
+/* genlib_gc_groups' schedule alone (host only), read with genlib_gc_plan_info / _layer / _layer_arrays.  A grouped
+ * column side has one column per group (row_seed = the member's group); a grouped target side keeps one output-block
+ * row per member, numbered in list order, and the sums per group follow the layers. */
+int genlib_gc_groups_plan_create(int32_t n, const int32_t *father, const int32_t *mother,
+                                 int32_t n_pro, const int32_t *proband, const int32_t *pro_group, int32_t n_pro_groups,
+                                 int32_t n_anc, const int32_t *ancestor, const int32_t *anc_group, int32_t n_anc_groups,
+                                 genlib_gc_plan **out);
+
 /* ---- gen.occ / gen.rec: descent-path counts and proband coverage (SURVEY.md 2: src/describe.jl:133-234) --------
  * The same plan and devices as genlib_gc (GENLIB_GC_DIRECTION applies), with the 1/2 dropped:
  *   O[a, p] = number of descent paths a -> ... -> p (the empty path when a == p)
