@@ -13,6 +13,7 @@ Usage mirrors the reference (`import GenLib as gen`):
     o = gen.phiOver(ped, 1 / 64)           # proband pairs at or above 1/64, selected on the device
     g = gen.phiMeanGroups(ped, {1: "a", 2: "a", 29: "b"})  # mean kinship within / between groups, and per proband
     c = gen.gcGroups(ped, {1: "a", 2: "a", 29: "b"})       # gen.gc summed over proband groups, no matrix formed
+    y = gen.phiProduct(ped, x)             # the proband kinship matrix times x (P, or P x k), no matrix fetched
 """
 import os as _os
 
@@ -20,7 +21,7 @@ from .pedigree import Individual, Pedigree, founder, genealogy, pro  # noqa: F40
 from .engine import (Engine, GcPlan, GenMatrix, GroupKinship, KinshipMatrix, PinnedMatrix, Plan, f, f_arrays,  # noqa: F401
                      findDistance, findMRCA, gc, gc_arrays, gc_groups_arrays, gcGroups, GroupContribution, meioses_arrays, mrca_arrays, occ, occ_arrays, phi, phi_arrays,
                      phi_distributed, phi_groups_arrays, phi_over_arrays, phi_pairs, phi_pairs_arrays, phiMean,
-                     phiMeanGroups, phiOver, PhiOver, rec, rec_arrays, run_distributed,
+                     phiMeanGroups, phiOver, phi_product_arrays, phiProduct, PhiOver, rec, rec_arrays, run_distributed,
                      sparse_phi)
 from . import synth  # noqa: F401
 from ._lib import GenlibError, GenlibOverflowError, LIB_PATH, PlanBoundsExceeded, lib  # noqa: F401

@@ -145,6 +145,8 @@ SYMBOLS = {
     "genlib_kinship_pairs_free": (C.c_int, [C.POINTER(KinshipPairs)]),
     "genlib_phi_groups": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, _P, C.c_int32, C.c_int, C.c_int32, _P, _P, _P,
                                     C.POINTER(Stats)]),
+    "genlib_phi_product": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, C.c_int, C.c_int32, _P, _P, _P,
+                                     C.POINTER(Stats)]),
     "genlib_plan_create_pairs": (C.c_int, [C.c_int32, _P, _P, C.c_int64, _P, _P, C.c_int32, C.c_int, C.POINTER(_P)]),
     "genlib_plan_pair_reads": (C.c_int64, [_P, C.c_int32, _P, _P, _P, _P, _P]),
     "genlib_plan_create_async": (C.c_int, [C.c_int32, _P, _P, _P, C.c_int32, _P, C.c_int32, C.c_int, C.POINTER(_P)]),
@@ -161,6 +163,7 @@ SYMBOLS = {
     "genlib_engine_ipc_attach": (C.c_int, [_P, _P, C.c_size_t]),
     "genlib_engine_phi_mean": (C.c_int, [_P, C.POINTER(C.c_double)]),
     "genlib_engine_row_sums": (C.c_int, [_P, _P]),
+    "genlib_engine_phi_product": (C.c_int, [_P, C.c_int32, _P, _P, _P]),
     "genlib_engine_set_layer_limit": (C.c_int, [_P, C.c_int32]),
     "genlib_engine_read_block": (C.c_int, [_P, C.c_int32, _P, _P]),
     "genlib_gc": (C.c_int, [C.c_int32, _P, _P, C.c_int32, _P, C.c_int32, _P, _P, C.c_int, C.c_int, C.c_int32, _P,

@@ -1,5 +1,5 @@
 // engine.cu -- the phi engine and the library-wide part of the C ABI of libgenlib_cuda.so (include/genlib_cuda.h):
-// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_phi_over / genlib_phi_groups / genlib_f / genlib_phi_pairs, errors and caches.  gen.gc, gen.occ and gen.rec are
+// plans, engines, the one-shot genlib_phi / genlib_phi_multi / genlib_phi_over / genlib_phi_groups / genlib_phi_product / genlib_f / genlib_phi_pairs, errors and caches.  gen.gc, gen.occ and gen.rec are
 // in gc_engine.cu; the host helpers both share are in runtime.hpp.
 //
 // The ABI stands where the reference's Julia method stands:
@@ -743,6 +743,85 @@ int phi_groups_rows(genlib_engine &E, const GroupColumns &C, double *dst) {
     return rc;
 }
 
+// ---- gen.phiProduct (genlib_phi_product, genlib_engine_phi_product) ---------------------------------------------
+// This device's rows of Y = M X (own_pro order) to host rows dst[0, nown) of k doubles each, and M[i, i] to diag[0,
+// nown) when diag is not null, in blocks of rows that fit one staging buffer (each block's Y rows, then its diagonal).
+// X (P x k, list order) is on the device for the call only, outside the arena.
+template <typename T>
+int phi_product_rows(genlib_engine &E, const double *X, int32_t k, double *dst, double *diag) {
+    const Plan &P = E.plan->p;
+    const int32_t np = P.n_unique, nown = (int32_t)E.own_pro.size();
+    if (nown == 0 || (k == 0 && !diag)) return GENLIB_OK;
+    const size_t row_bytes = ((size_t)k + (diag ? 1 : 0)) * sizeof(double);
+    if (row_bytes > kFetchStageBytes) return fail(GENLIB_EINVAL, "phiProduct: one proband's row of the product does not fit the staging buffer");
+    const int64_t rows_per = (int64_t)std::min<size_t>((size_t)nown, kFetchStageBytes / row_bytes);
+    const size_t x_bytes = (size_t)np * (size_t)k * sizeof(double);
+    double *d_x = nullptr;                                       // X (P k), then d_index (nown)
+    FreeOnExit<double> free_x{d_x};
+    if (cudaMalloc(&d_x, x_bytes + (size_t)nown * sizeof(int32_t)) != cudaSuccess) {
+        cudaGetLastError();
+        size_t free_b = 0, total_b = 0;
+        cudaMemGetInfo(&free_b, &total_b);
+        return fail(GENLIB_ENOMEM, "phiProduct: X needs " + std::to_string(x_bytes) + " bytes on the device next to the engine's arena, " +
+                                   std::to_string(free_b) + " bytes are free");
+    }
+    int32_t *d_index = reinterpret_cast<int32_t *>(reinterpret_cast<unsigned char *>(d_x) + x_bytes);
+    if (k > 0) CU(cudaMemcpyAsync(d_x, X, x_bytes, cudaMemcpyHostToDevice, E.stream));
+    CU(cudaMemcpyAsync(d_index, E.own_pro.data(), (size_t)nown * sizeof(int32_t), cudaMemcpyHostToDevice, E.stream));
+    const int rc = staged_d2h(E.stream, E.copy_stream, reinterpret_cast<double *>(E.fetch_stage[0]),
+                              reinterpret_cast<double *>(E.fetch_stage[1]), nown, rows_per, "phiProduct fetch",
+        [&](double *stage, int64_t r0, int64_t nr) {
+            const T *A = static_cast<const T *>(E.A);
+            double *d = diag ? stage + (size_t)nr * k : nullptr;
+            // One column: one row per CTA, as rowsum_kernel reads the block.  Several: 4 rows per CTA share each X load.
+            if (k <= 1)
+                phi_product_kernel<T, 1, 1><<<(unsigned)nr, kThreads, 0, E.stream>>>(A, P.capacity, E.own_pro_row.p, d_index, E.pro_slot.p,
+                                                                                   np, d_x, k, (int32_t)r0, (int32_t)nr, stage, d);
+            else
+                phi_product_kernel<T, 8, 4><<<(unsigned)((nr + 3) / 4) * (unsigned)((k + 7) / 8), kThreads, 0, E.stream>>>(
+                    A, P.capacity, E.own_pro_row.p, d_index, E.pro_slot.p, np, d_x, k, (int32_t)r0, (int32_t)nr, stage, d);
+        },
+        [&](const double *stage, int64_t r0, int64_t nr) {
+            cudaError_t ce = cudaSuccess;
+            if (k > 0) ce = cudaMemcpyAsync(dst + (size_t)r0 * k, stage, (size_t)nr * k * sizeof(double), cudaMemcpyDeviceToHost, E.copy_stream);
+            if (ce == cudaSuccess && diag)
+                ce = cudaMemcpyAsync(diag + r0, stage + (size_t)nr * k, (size_t)nr * sizeof(double), cudaMemcpyDeviceToHost, E.copy_stream);
+            return ce;
+        });
+    if (rc == GENLIB_OK) {
+        E.stats.h2d_bytes += (int64_t)x_bytes;
+        E.stats.d2h_bytes += (int64_t)nown * (int64_t)row_bytes;
+    }
+    return rc;
+}
+
+// Several devices of one process copy their own proband rows to a list-ordered output, device after device in own_pro
+// order (one device: row i lands at row i); afterwards the host moves the rows to list order in place.
+struct ListOrderRows {
+    std::vector<int64_t> base;      // device g's rows land at [base[g], base[g + 1])
+    std::vector<int32_t> at;        // at[p]: the list position of the row landed at p
+    void prepare(const Plan &P, int n_dev) {
+        const int32_t np = P.n_unique;        // (no duplicates: the plan's proband u is list position u)
+        base.assign((size_t)n_dev + 1, 0);
+        for (int32_t u = 0; u < np; u++) base[(size_t)P.pro_owner[(size_t)u] + 1]++;
+        for (int g = 0; g < n_dev; g++) base[(size_t)g + 1] += base[(size_t)g];
+        at.resize((size_t)np);
+        std::vector<int64_t> fill(base.begin(), base.end() - 1);
+        for (int32_t u = 0; u < np; u++) at[(size_t)fill[(size_t)P.pro_owner[(size_t)u]]++] = u;   // own_pro: ascending
+    }
+    // every output (rows of `width` doubles; a null one is skipped) moved by the same permutation; runs once
+    void to_list_order(std::initializer_list<std::pair<double *, size_t>> outs) {
+        for (int32_t p = 0; p < (int32_t)at.size(); p++)
+            while (at[(size_t)p] != p) {
+                const int32_t q = at[(size_t)p];
+                for (const auto &o : outs)
+                    if (o.first && o.second)
+                        std::swap_ranges(o.first + (size_t)p * o.second, o.first + (size_t)(p + 1) * o.second, o.first + (size_t)q * o.second);
+                std::swap(at[(size_t)p], at[(size_t)q]);
+            }
+    }
+};
+
 // Compulsory traffic of every layer on this rank (genlib_layer_info), from the plan.
 void account_layers(genlib_engine &E) {
     if (E.info_ready) return;
@@ -1378,6 +1457,16 @@ int genlib_engine_row_sums(genlib_engine *eng, double *out) {
     return GENLIB_OK;
 }
 
+int genlib_engine_phi_product(genlib_engine *eng, int32_t k, const double *X, double *out, double *diag) {
+    if (!eng || k < 0) return fail(GENLIB_EINVAL, "genlib_engine_phi_product: null engine or k < 0");
+    if (!eng->ran) return fail(GENLIB_EINVAL, "genlib_engine_phi_product before genlib_engine_run");
+    if (k > 0 && (!X || (!out && !eng->own_pro.empty()))) return fail(GENLIB_EINVAL, "genlib_engine_phi_product: null argument");
+    DeviceGuard guard;
+    if (int rc = guard.enter(eng->device)) return rc;
+    return eng->numerics == GENLIB_NUMERICS_FP64 ? phi_product_rows<double>(*eng, X, k, out, diag)
+                                                 : phi_product_rows<float>(*eng, X, k, out, diag);
+}
+
 int genlib_engine_phi_mean(genlib_engine *eng, double *out) {
     if (!eng || !out) return fail(GENLIB_EINVAL, "null argument");
     if (eng->world != 1) return fail(GENLIB_EINVAL, "genlib_engine_phi_mean: one rank only; sharded engines combine genlib_engine_row_sums in proband order");
@@ -1760,8 +1849,7 @@ int genlib_phi_groups(int32_t n, const int32_t *father, const int32_t *mother, i
         return GENLIB_OK;
     }
     GroupColumns cols;
-    std::vector<int64_t> base((size_t)n_dev + 1, 0);             // where each device's rows land in proband_mean
-    std::vector<int32_t> at;                                     // at[p]: the list position of the row landed at p
+    ListOrderRows rows;                                          // where each device's rows land in proband_mean
     double t0 = 0;
     OneshotFetch fetch;
     fetch.prepare = [&](const Plan &P) {
@@ -1776,26 +1864,17 @@ int genlib_phi_groups(int32_t n, const int32_t *father, const int32_t *mother, i
             cols.gcol[(size_t)k] = P.pro_slot[(size_t)u];
             cols.gat[(size_t)u] = k;
         }
-        for (int32_t u = 0; u < n_pro; u++) base[(size_t)P.pro_owner[(size_t)u] + 1]++;
-        for (int32_t g = 0; g < n_dev; g++) base[(size_t)g + 1] += base[(size_t)g];
-        at.resize((size_t)n_pro);
-        std::vector<int64_t> fill(base.begin(), base.end() - 1);
-        for (int32_t u = 0; u < n_pro; u++) at[(size_t)fill[(size_t)P.pro_owner[(size_t)u]]++] = u;   // own_pro: ascending
+        rows.prepare(P, n_dev);
     };
     fetch.device = [&](genlib_engine &E, int g) {
         DeviceGuard guard;
         if (int r = guard.enter(E.device)) return r;
-        double *dst = proband_mean + (size_t)base[(size_t)g] * G;
+        double *dst = proband_mean + (size_t)rows.base[(size_t)g] * G;
         return numerics == GENLIB_NUMERICS_FP64 ? phi_groups_rows<double>(E, cols, dst) : phi_groups_rows<float>(E, cols, dst);
     };
     fetch.combine = [&]() {
         const size_t Gs = (size_t)G;
-        for (int32_t p = 0; p < n_pro; p++)                      // rows to list order (one device: in place already)
-            while (at[(size_t)p] != p) {
-                const int32_t q = at[(size_t)p];
-                std::swap_ranges(proband_mean + (size_t)p * Gs, proband_mean + (size_t)(p + 1) * Gs, proband_mean + (size_t)q * Gs);
-                std::swap(at[(size_t)p], at[(size_t)q]);
-            }
+        rows.to_list_order({{proband_mean, Gs}});                // (one device: in place already)
         std::fill(group_mean, group_mean + Gs * Gs, 0.0);         // T, in list order
         for (int32_t i = 0; i < n_pro; i++) {
             double *t = group_mean + (size_t)group[i] * Gs;
@@ -1822,6 +1901,55 @@ int genlib_phi_groups(int32_t n, const int32_t *father, const int32_t *mother, i
         return (int)GENLIB_OK;
     };
     return oneshot("genlib_phi_groups", GENLIB_SCHEDULE_PHI, n, father, mother, n_pro, proband, true, numerics, n_dev,
+                   devices, stats, fetch);
+}
+
+// genlib_phi_product: the genlib_phi run, then every device multiplies its own proband rows by X (phi_product_rows)
+// into out and diag, device after device in own_pro order; the host moves the rows to list order in place.
+int genlib_phi_product(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                       int32_t k, const double *X, int numerics, int32_t n_dev, const int32_t *devices, double *out,
+                       double *diag, genlib_stats *stats) {
+    if (n < 0 || n_pro < 0 || k < 0 || (n > 0 && (!father || !mother)) || (n_pro > 0 && (!proband || (k > 0 && (!X || !out)))))
+        return fail(GENLIB_EINVAL, "genlib_phi_product: null pointer or negative size");
+    if (numerics != GENLIB_NUMERICS_REFERENCE && numerics != GENLIB_NUMERICS_FP64) return fail(GENLIB_EINVAL, "unknown numerics mode");
+    if (n_dev < 1 || n_dev > kMaxWorld || !devices) return fail(GENLIB_EINVAL, "genlib_phi_product: 1 .. 16 devices");
+    std::vector<char> seen((size_t)n, 0);
+    for (int32_t p = 0; p < n_pro; p++) {
+        const int32_t x = proband[p];
+        if (x < 0 || x >= n) {
+            std::string err;
+            if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);   // (a broken pedigree is reported first)
+            return fail(GENLIB_EKEY, "KeyError: index " + std::to_string(x) + " not in pedigree");
+        }
+        if (seen[(size_t)x]) return fail(GENLIB_EINVAL, "genlib_phi_product: duplicate proband rank " + std::to_string(x));
+        seen[(size_t)x] = 1;
+    }
+    if (n_pro == 0 || (k == 0 && !diag)) {                       // nothing to compute: no plan, no device
+        std::string err;
+        if (int rc = check_pedigree(n, father, mother, err)) return fail(rc, err);
+        if (stats) { std::memset(stats, 0, sizeof *stats); stats->n_unique = n_pro; }
+        return GENLIB_OK;
+    }
+    ListOrderRows rows;
+    double t0 = 0;
+    OneshotFetch fetch;
+    fetch.prepare = [&](const Plan &P) { t0 = now_ms(); rows.prepare(P, n_dev); };
+    fetch.device = [&](genlib_engine &E, int g) {
+        DeviceGuard guard;
+        if (int r = guard.enter(E.device)) return r;
+        const int64_t b = rows.base[(size_t)g];
+        double *dst = k > 0 ? out + (size_t)b * k : nullptr, *d = diag ? diag + b : nullptr;
+        return numerics == GENLIB_NUMERICS_FP64 ? phi_product_rows<double>(E, X, k, dst, d) : phi_product_rows<float>(E, X, k, dst, d);
+    };
+    fetch.combine = [&]() {
+        rows.to_list_order({{k > 0 ? out : nullptr, (size_t)k}, {diag, 1}});   // (one device: in place already)
+        return (int)GENLIB_OK;
+    };
+    fetch.finish = [&](genlib_engine &E, int) {                  // (one device: stats come from its engine)
+        E.stats.ms_fetch = now_ms() - t0;
+        return (int)GENLIB_OK;
+    };
+    return oneshot("genlib_phi_product", GENLIB_SCHEDULE_PHI, n, father, mother, n_pro, proband, true, numerics, n_dev,
                    devices, stats, fetch);
 }
 

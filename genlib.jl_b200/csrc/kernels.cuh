@@ -1,6 +1,6 @@
 // kernels.cuh -- device-side vocabulary shared by the sm_100a kernels of the kinship sweep, and the
 // small kernels around the layer kernel (layer_kernel.cuh): proband gather, gen.phiOver's selection, gen.phiMeanGroups'
-// and phiMean's reductions, the inter-GPU barrier, sparse_phi's misfiled pairs, gen.f's parents' kinships and gen.phi_pairs' reads.
+// and phiMean's reductions, gen.phiProduct's products, the inter-GPU barrier, sparse_phi's misfiled pairs, gen.f's parents' kinships and gen.phi_pairs' reads.
 //
 // Arithmetic is binary64 in the reference's grouping; storage type T is float
 // (GENLIB_NUMERICS_REFERENCE: one RN32 per step, like src/compute.jl:296) or double.
@@ -364,6 +364,71 @@ rowsum_kernel(const T *__restrict__ A, int64_t ld, const int32_t *__restrict__ o
         for (int w = 1; w < kThreads / 32; w++) s += part[w];
         out[2 * r] = s;
         out[2 * r + 1] = (double)row[slots[own_index[r]]];
+    }
+}
+
+// =====================================================================================
+// gen.phiProduct: Y[i][c] = sum over all probands j of M[i, j] X[j][c], for this rank's own proband rows
+// row0 + rb * R + q (rows[] local rows, index[] their list positions; columns gathered through slots[] in list order,
+// as rowsum_kernel reads them, so no peer reads).  X is P x k row-major (binary64), Y is nrows x k row-major, diag[r] =
+// M[i, i] (when not null, written by the first column block).  One CTA per R rows and CB columns: each M entry loaded
+// from memory serves its CB columns from registers, and each X row segment its R rows.
+// The order of every sum depends only on P, and is rowsum_kernel's: thread t accumulates the columns j = t, t + 256,
+// ... ascending with one FMA each (acc = fma(M[i, j], X[j][c], acc), rounded once), then a shuffle tree inside each
+// warp and the warps' totals in warp order.  So a column of a k-column call is the same bits as a one-column call, X
+// = 1 gives rowsum_kernel's sums, and neither CB, R, the row block nor the rank changes a result.
+// =====================================================================================
+template <typename T, int CB, int R>
+__global__ void __launch_bounds__(kThreads)
+phi_product_kernel(const T *__restrict__ A, int64_t ld, const int32_t *__restrict__ rows, const int32_t *__restrict__ index,
+                   const int32_t *__restrict__ slots, int32_t P, const double *__restrict__ X, int32_t k, int32_t row0,
+                   int32_t nrows, double *__restrict__ Y, double *__restrict__ diag) {
+    __shared__ double part[kThreads / 32][R * CB];
+    const int ncb = k > 0 ? (k + CB - 1) / CB : 1;
+    const int cb = blockIdx.x % ncb, r0 = (int)(blockIdx.x / ncb) * R, c0 = cb * CB;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const T *row[R];
+#pragma unroll
+    for (int q = 0; q < R; q++) row[q] = A + (int64_t)rows[row0 + min(r0 + q, nrows - 1)] * ld;   // (past the block: a copy, not written)
+    if (k > 0) {
+        double acc[R][CB];
+#pragma unroll
+        for (int q = 0; q < R; q++)
+#pragma unroll
+            for (int c = 0; c < CB; c++) acc[q][c] = 0.0;
+        for (int j = threadIdx.x; j < P; j += kThreads) {
+            const int s = slots[j];
+            const double *xj = X + (size_t)j * k + c0;
+            double x[CB];
+#pragma unroll
+            for (int c = 0; c < CB; c++) x[c] = c0 + c < k ? __ldg(xj + c) : 0.0;
+#pragma unroll
+            for (int q = 0; q < R; q++) {
+                const double m = (double)row[q][s];
+#pragma unroll
+                for (int c = 0; c < CB; c++) acc[q][c] = __fma_rn(m, x[c], acc[q][c]);
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < R; q++)
+#pragma unroll
+            for (int c = 0; c < CB; c++) {
+                double v = acc[q][c];
+                for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+                if (lane == 0) part[w][q * CB + c] = v;
+            }
+        __syncthreads();
+        for (int e = threadIdx.x; e < R * CB; e += kThreads) {
+            const int q = e / CB, c = e % CB;
+            if (r0 + q >= nrows || c0 + c >= k) continue;
+            double v = part[0][e];
+            for (int u = 1; u < kThreads / 32; u++) v += part[u][e];
+            Y[(size_t)(r0 + q) * k + c0 + c] = v;
+        }
+    }
+    if (diag && cb == 0 && threadIdx.x < R && r0 + (int)threadIdx.x < nrows) {
+        const int r = row0 + r0 + (int)threadIdx.x;
+        diag[r - row0] = (double)A[(int64_t)rows[r] * ld + slots[index[r]]];
     }
 }
 

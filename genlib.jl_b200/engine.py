@@ -248,6 +248,23 @@ class Engine:
             check(lib().genlib_engine_row_sums(self._h, ptr(out)))
         return out
 
+    def phi_product(self, X, return_diagonal: bool = False):
+        """Y = M X for this rank's proband rows (genlib_engine_phi_product), M the proband block of the run: X has
+        plan.n_unique rows in the plan's proband order, the result one row per own proband (own_probands() order; one
+        rank: list order).  A 1-D X gives a 1-D result.  The bits are gen.phiProduct's; the layers are not run again,
+        so an iterative method can call this as often as it needs.  return_diagonal=True also returns M[i, i]."""
+        X = np.asarray(X, np.float64)
+        one = X.ndim == 1
+        X2 = np.ascontiguousarray(X[:, None] if one else X)
+        if X2.ndim != 2 or X2.shape[0] != self.plan.n_unique:
+            raise ValueError(f"phi_product: X needs {self.plan.n_unique} rows, one per proband; it has shape {X.shape}")
+        n = lib().genlib_engine_own_probands(self._h, None)
+        Y = np.empty((n, X2.shape[1]), np.float64)
+        d = np.empty(n, np.float64) if return_diagonal else None
+        check(lib().genlib_engine_phi_product(self._h, X2.shape[1], ptr(X2), ptr(Y), ptr(d)))
+        Y = Y[:, 0] if one else Y
+        return (Y, d) if return_diagonal else Y
+
     def read_block(self, slots) -> np.ndarray:
         slots = np.ascontiguousarray(slots, np.int32)
         out = np.zeros((len(slots), len(slots)), np.float64)
@@ -606,6 +623,54 @@ def phi_groups_arrays(father, mother, proband_ranks, group_index, n_groups, *, n
     check(lib().genlib_phi_groups(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), ptr(gi), n_groups,
                                   _lib.NUMERICS[numerics], len(dv), ptr(dv), ptr(pm), ptr(gm), C.byref(st)))
     return pm, gm, st.as_dict()
+
+
+def phiProduct(pedigree: Pedigree, X, probandIDs=None, *, numerics="reference", device: int = -1, devices=None,
+               return_diagonal: bool = False, return_stats: bool = False):
+    """The proband kinship matrix times a block of vectors, Y = M X, formed on the device (genlib_phi_product).
+
+    M is the matrix gen.phi(pedigree, probandIDs, numerics=numerics) returns, widened exactly to float64; probandIDs
+    defaults to pro(pedigree) and must not repeat an ID.  X has one row per proband in probandIDs order (P x k, or a
+    vector of P for a 1-D result); Y[i, c] = sum over all j of M[i, j] X[j, c], the diagonal included.  With
+    return_diagonal=True the result is (Y, diag), diag[i] = M[i, i], so that the sum over relatives j != i is
+    Y - diag[:, None] * X.  gen.phi's plan and layers run on the device and every device multiplies the proband rows
+    it holds: only P x k doubles leave the device, never the matrix.  Each entry is summed in a fixed order that
+    depends only on P, so a column of X gives the same bits alone or in a block, on any number of devices and through
+    Engine.phi_product; where every product and partial sum is a float64 number (integer X on geneaJi or genea140) Y
+    is exact.  ValueError on a repeated ID or a row count that is not P, KeyError on an unknown ID, both before any
+    device work."""
+    IDs = pro(pedigree) if probandIDs is None else np.asarray(probandIDs, np.int64).reshape(-1)
+    if len(np.unique(IDs)) != len(IDs):
+        raise ValueError("phiProduct: duplicate proband IDs")
+    X = np.asarray(X, np.float64)
+    if X.ndim not in (1, 2) or X.shape[0] != len(IDs):
+        raise ValueError(f"phiProduct: X needs {len(IDs)} rows, one per proband; it has shape {X.shape}")
+    ranks = pedigree.rank_of(IDs)                       # KeyError, like pedigree[ID]
+    Y, d, stats = phi_product_arrays(pedigree.father, pedigree.mother, ranks, X[:, None] if X.ndim == 1 else X,
+                                     numerics=numerics, device=device, devices=devices, diagonal=return_diagonal)
+    Y = Y[:, 0] if X.ndim == 1 else Y
+    res = (Y, d) if return_diagonal else Y
+    return (res, stats) if return_stats else res
+
+
+def phi_product_arrays(father, mother, proband_ranks, X, *, numerics="reference", device: int = -1, devices=None,
+                       diagonal: bool = False):
+    """One-shot C-ABI call `genlib_phi_product` on flat arrays (what the Julia shim ccalls): distinct proband ranks in
+    list order and X (P x k, its rows in that order).  Returns (Y (P x k), diag (P) or None, stats)."""
+    father = np.ascontiguousarray(father, np.int32)
+    mother = np.ascontiguousarray(mother, np.int32)
+    pr = np.ascontiguousarray(proband_ranks, np.int32).reshape(-1)
+    X = np.ascontiguousarray(X, np.float64)
+    if X.ndim != 2 or X.shape[0] != len(pr):
+        raise ValueError(f"phi_product_arrays: X of shape {X.shape} for {len(pr)} probands")
+    k = X.shape[1]
+    Y = np.empty((len(pr), k), np.float64)
+    d = np.empty(len(pr), np.float64) if diagonal else None
+    dv = np.ascontiguousarray([device] if devices is None else devices, np.int32)
+    st = Stats()
+    check(lib().genlib_phi_product(len(father), ptr(father), ptr(mother), len(pr), ptr(pr), k, ptr(X),
+                                   _lib.NUMERICS[numerics], len(dv), ptr(dv), ptr(Y), ptr(d), C.byref(st)))
+    return Y, d, st.as_dict()
 
 
 class GcPlan:

@@ -292,6 +292,38 @@ function phiMeanGroups(pedigree::GenLib.Pedigree, groups::AbstractDict{Int}; num
 end
 
 """
+    phiProduct(pedigree, X, probandIDs = pro(pedigree); numerics = :reference, device = -1, devices = Int[],
+               diagonal = false) -> Y, or (Y, diag) with diagonal = true
+
+`phi(pedigree, probandIDs; numerics)` widened exactly to `Float64`, times `X`, without the matrix leaving the device
+(`genlib_phi_product`): `Y[i, c] = Σⱼ ϕ[i, j] X[j, c]` over all `j`, the diagonal included; `diag[i] = ϕ[i, i]`, so
+the kinship-weighted sum over relatives is `Y .- diag .* X`.  `X` is a `Vector` (a `Vector` comes back) or a
+`Matrix` with one row per proband, in `probandIDs` order; no ID may repeat.  Every entry is summed in an order that
+depends only on the number of probands: a column gives the same bits alone or in a block, on any number of devices.
+ArgumentError on a repeated ID or a row count that is not the number of probands, KeyError on an unknown ID.
+"""
+function phiProduct(pedigree::GenLib.Pedigree, X::AbstractVecOrMat{<:Real}, probandIDs::Vector{Int} = GenLib.pro(pedigree);
+                    numerics::Symbol = :reference, device::Integer = -1, devices::Vector{<:Integer} = Int[],
+                    diagonal::Bool = false)
+    allunique(probandIDs) || throw(ArgumentError("phiProduct: duplicate proband IDs"))
+    P, k = length(probandIDs), size(X, 2)
+    size(X, 1) == P || throw(ArgumentError("phiProduct: X has $(size(X, 1)) rows for $P probands"))
+    father, mother = flatten(pedigree)
+    probands = Int32[pedigree[ID].rank - 1 for ID in probandIDs]        # KeyError on unknown ID
+    Xt = Matrix{Float64}(permutedims(X isa AbstractVector ? reshape(X, P, 1) : X))   # column-major k x P = C's row-major P x k
+    Yt = Matrix{Float64}(undef, k, P)
+    d = diagonal ? Vector{Float64}(undef, P) : Float64[]
+    devs = isempty(devices) ? Int32[device] : Int32.(devices)
+    GC.@preserve Xt Yt d check(ccall((:genlib_phi_product, libgenlib[]), Cint,
+        (Int32, Ptr{Int32}, Ptr{Int32}, Int32, Ptr{Int32}, Int32, Ptr{Float64}, Cint, Int32, Ptr{Int32},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Cvoid}),
+        length(father), father, mother, P, probands, k, Xt, numerics === :fp64 ? 1 : 0, length(devs), devs,
+        Yt, diagonal ? pointer(d) : Ptr{Float64}(C_NULL), C_NULL))
+    Y = X isa AbstractVector ? vec(Yt) : permutedims(Yt)
+    diagonal ? (Y, d) : Y
+end
+
+"""
     sparse_phi(pedigree, probandIDs = pro(pedigree)) -> GenLib.KinshipMatrix
 
 `gen.sparse_phi` (src/compute.jl:321-447) on the GPU: the same engine, planned for sparse_phi's own

@@ -367,6 +367,32 @@ int genlib_phi_groups(int32_t n, const int32_t *father, const int32_t *mother, i
                       const int32_t *group, int32_t n_groups, int numerics, int32_t n_dev, const int32_t *devices,
                       double *proband_mean, double *group_mean, genlib_stats *stats);
 
+/* ---- gen.phiProduct: the proband kinship matrix times a block of vectors, Y = M X ---------------------------------
+ * proband[0 .. n_pro) are distinct ranks in list order; X is n_pro x k binary64, row-major (X[j k + c]), its rows in
+ * list order.  M is the matrix genlib_phi returns for the same list and numerics (Float32 or Float64 storage), each
+ * entry widened exactly to binary64:
+ *   out[i k + c] = sum over ALL j of M[i, j] X[j][c]       (the diagonal included: a true matrix product)
+ *   diag[i]      = M[i, i]      (when diag is not null: the sum over j != i is then out[i k + c] - diag[i] X[i][c])
+ * both n_pro rows in list order.  Every out[i k + c] is accumulated in binary64 with one FMA per term, in an order that
+ * depends only on n_pro: column j goes to partial j mod 256, each partial ascending in j, the 256 partials combined
+ * by a fixed tree (genlib_engine_row_sums' order).  So a column of a k-column call is the same bits as a one-column
+ * call on that column, and the result does not depend on the number of devices, on which device holds a row or on
+ * genlib_engine_phi_product against this call.  Where every product and every partial sum is a binary64 number
+ * (kinships that are multiples of 2^-32 and at most 1 times integers with n_pro max|x| <= 2^21), out is the exact
+ * sum.  Non-finite entries of X are not checked; they propagate as in IEEE arithmetic.  The genlib_phi plan runs
+ * unchanged (streamed, several devices as genlib_phi_multi); then every device multiplies the proband rows it holds
+ * (no peer reads) and copies back k (+ 1) doubles per row: no matrix leaves the device.  X takes 8 n_pro k bytes of
+ * device memory for the call, next to the engine's arena.  The caller owns X, out and diag.
+ *   GENLIB_EINVAL: a null pointer or negative size (k < 0 included), unknown numerics, not 1 .. 16 devices, a rank
+ *   listed twice.  A rank out of range gives GENLIB_EKEY (a broken pedigree is reported first).  GENLIB_ENOMEM when
+ *   the device has no room for X (the message names the bytes).  n_pro == 0, or k == 0 with diag == NULL, writes
+ *   nothing and touches no device.  devices[0] < 0 = the current device (one device).
+ *   stats as genlib_phi's, but ms_fetch = the products, the copies back and the host's part, d2h_bytes = 8 n_pro k
+ *   (+ 8 n_pro with diag), h2d_bytes includes X once per device. */
+int genlib_phi_product(int32_t n, const int32_t *father, const int32_t *mother, int32_t n_pro, const int32_t *proband,
+                       int32_t k, const double *X, int numerics, int32_t n_dev, const int32_t *devices, double *out,
+                       double *diag, genlib_stats *stats);
+
 /* ---- handle API: keep the schedule on the device, run, fetch ---------------
  * (what the benchmark and a multi-call Julia session use) */
 int genlib_engine_create(const genlib_plan *plan, int numerics, int device, genlib_engine **out);
@@ -401,6 +427,12 @@ int genlib_engine_phi_mean(genlib_engine *eng, double *out);
  * columns, out[2 r + 1] = its diagonal entry.  Adding the rows of all ranks in proband order gives
  * the same bits whatever the number of ranks. */
 int genlib_engine_row_sums(genlib_engine *eng, double *out);
+/* gen.phiProduct on an engine that has run: Y = M X for the rows of the probands this rank holds, out[r k + c] and
+ * diag[r] (nullable) for its r-th own proband (genlib_engine_own_probands order; one rank: list order).  X is
+ * n_unique x k, row-major, its rows in the plan's proband order.  The bits are genlib_phi_product's, whatever the
+ * rank.  Not collective, no peer reads; call it any number of times without running the layers again.  Errors as
+ * genlib_phi_product's where they apply, and GENLIB_EINVAL before genlib_engine_run. */
+int genlib_engine_phi_product(genlib_engine *eng, int32_t k, const double *X, double *out, double *diag);
 /* Debug/test: stop genlib_engine_run after `n_layers` layers (< 0: no limit). */
 int genlib_engine_set_layer_limit(genlib_engine *eng, int32_t n_layers);
 /* Debug/test: copy the frontier entry block [slots x slots] (as double). */
